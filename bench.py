@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric on BASELINE.json's configs, on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline (`metric`/`value`): genomes sketched per second, config[1] of BASELINE.json —
 1,000 synthetic 5 Mbp genomes, k=21 scaled=1500 D=4096 per GPU (weak scaling: every rank
@@ -18,6 +18,10 @@ the ranks and exchanged through the library's NVLink windows (csrc/peer.cu).
 
 `--impl reference` times the reference's CPU path restated in C (oracle/hg_oracle.c — the
 Rust crate cannot be built here: no cargo/rustc) on the host cores.
+
+`--steps K` is the number of timed steps of every leg.  `--dump-outputs DIR` writes what the sketch
+call returned in the last timed step as DIR/<name>.npy (see dump_outputs); the inputs are generated
+from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -34,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: leave no __pycache__ in it
 
 K, SCALED, SEED, HV_D = 21, 1500, 123, 4096
 GENOME_LEN = 5_000_000
@@ -66,6 +71,26 @@ def load_peaks():
         return dict(hbm_gbs=float(d["hbm_gbs"]), bf16_tflops=float(d["bf16_tflops"]),
                     bf16_tflops_sustained=float(d.get("bf16_tflops_sustained", d["bf16_tflops"])), source="measured")
     return dict(hbm_gbs=6650.0, bf16_tflops=1590.0, bf16_tflops_sustained=1400.0, source="fallback")
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, outputs: dict):
+    """--dump-outputs: one DIR/<name>.npy per array the sketch call returned (one row per genome), converted
+    exactly to float32 (8- and 16-bit integers) or float64 (32-bit integers), and DIR/genome.npy, the batch index of
+    every row.  A batch whose rows would exceed DUMP_LIMIT_BYTES in all is cut to a sample of rows drawn with a fixed
+    seed, the same in every run."""
+    wide = {k: np.float64 if v.dtype.itemsize >= 4 else np.float32 for k, v in outputs.items()}
+    n = len(next(iter(outputs.values())))
+    row_bytes = 8 + sum(np.dtype(wide[k]).itemsize * v[0].size for k, v in outputs.items())
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "genome.npy"), rows.astype(np.float64))
+    for k, v in outputs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[rows].astype(wide[k]))
 
 
 class ClockSampler:
@@ -209,9 +234,11 @@ def run_reference(args, rank):
     times = []
     for step in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        O.sketch_batch(seq, off, k=K, scaled=SCALED, seed=SEED, hv_d=HV_D, want_hv=False)
+        r = O.sketch_batch(seq, off, k=K, scaled=SCALED, seed=SEED, hv_d=HV_D, want_hv=False)
         if step >= args.warmup:
             times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for k, v in r.items() if v is not None})
     total = sum(times)
     value = n * len(times) / total
     line = {
@@ -258,7 +285,10 @@ def main():
     ap.add_argument("--no-dist", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-fasta", action="store_true", help="skip the raw-FASTA end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the sketch outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -345,6 +375,10 @@ def main():
     launches = ctx.launches - l0
     dev_ms = max_over_ranks(e0.elapsed_time(e1))
     ctx.sketch_status()
+    if args.dump_outputs and rank == 0:  # rank 0's genomes (every rank sketches its own)
+        dump_outputs(args.dump_outputs, {"hv": d_hv.cpu().numpy(), "packed": d_packed.cpu().numpy(),
+                                         "quant_bits": d_bits.cpu().numpy(), "norm2": d_norm.cpu().numpy(),
+                                         "n_hashes": d_nh.cpu().numpy()})
     value = world * n * args.steps / (dev_ms * 1e-3)
     kmer_ms = statistics.mean(s[1] for s in stage)
     enc_ms = statistics.mean(s[2] for s in stage)
@@ -382,7 +416,7 @@ def main():
     h2d_only_gbs = 3 * n * GENOME_LEN / (h0.elapsed_time(h1) * 1e-3) / 1e9
     del scratch_dev
 
-    e2e_steps = max(3, args.steps // 2)
+    e2e_steps = args.steps
     for _ in range(2):
         e2e_step()
     barrier()
@@ -704,7 +738,7 @@ def bench_dist_config(cfg, args, ctx, ext, hg, multigpu, synth, dev, rank, world
     with torch.cuda.stream(ext):
         step(0)  # auto: single-plane tensor kernel if the rows are narrow, else two-limb; records why
     path, path_reason = ctx.dist_last_path, ctx.dist_last_reason
-    steps = max(5, args.steps)
+    steps = args.steps
     tot_ms, kern_ms, hits, stages = 0.0, [], None, []
 
     def one_step(timed):
@@ -795,7 +829,7 @@ def bench_dist_config(cfg, args, ctx, ext, hg, multigpu, synth, dev, rank, world
     import ctypes as C
     lib = hg.ffi.load()
     if world == 1 and cfg["key"] == "dist":
-        out.update(dist_e2e_single(ctx, hg, lib, ref_hv, ref_norm, bits, packed, n_ref, D, cap, path, n_pairs, hits))
+        out.update(dist_e2e_single(ctx, hg, lib, ref_hv, ref_norm, bits, packed, n_ref, D, cap, path, n_pairs, hits, args.steps))
     if cfg["key"] in ("dist", "dist_cfg4") and world > 1:
         # `hyper-gen dist` with all GPUs behind one process (hg_group_dist_packed): rank 0 drives the N GPUs from packed
         # sketch rows in pinned host memory while the other ranks wait on the host
@@ -826,7 +860,7 @@ def bench_dist_config(cfg, args, ctx, ext, hg, multigpu, synth, dev, rank, world
 
             gcall(); gcall()
             t0 = time.perf_counter()
-            reps = 5
+            reps = args.steps
             for _ in range(reps):
                 gcall()
             dtg = (time.perf_counter() - t0) / reps
@@ -848,7 +882,7 @@ def bench_dist_config(cfg, args, ctx, ext, hg, multigpu, synth, dev, rank, world
     return out
 
 
-def dist_e2e_single(ctx, hg, lib, hv, norm, bits, packed_d, nq, D, cap, path, n_pairs, hits_ref):
+def dist_e2e_single(ctx, hg, lib, hv, norm, bits, packed_d, nq, D, cap, path, n_pairs, hits_ref, reps):
     """config 3 through the single-GPU host-pointer entries (hg_dist, hg_dist_sorted, hg_dist_packed)"""
     import ctypes as C
     import torch
@@ -869,7 +903,6 @@ def dist_e2e_single(ctx, hg, lib, hv, norm, bits, packed_d, nq, D, cap, path, n_
 
     e2e()
     t0 = time.perf_counter()
-    reps = 5
     for _ in range(reps):
         e2e()
     dt = (time.perf_counter() - t0) / reps

@@ -87,16 +87,25 @@ def test_u_and_iupac_bytes_break_kmers_like_the_reference_gpu_path(ctx, hg, orac
         assert np.isin(ref, got).all()
 
 
-def test_kmer_hash_matches_reference_kernel_compiled_for_host(ctx, hg, oracle):
-    """The reference's own cuda_kmer_t1ha2 (compiled as host code in oracle/_ref) agrees too."""
-    if oracle.ref() is None:
-        pytest.skip("oracle/_ref not built")
+def test_kmer_hash_matches_reference_kernel_compiled_for_host(ctx, hg):
+    """The reference's own cuda_kmer_t1ha2 (compiled as host code) agrees too: its hash sets of one genome with an N run
+    and a lower-case stretch, at three (k, scaled) and both strand modes, are stored in golden/kmer_ref_sets.json."""
+    import hashlib
+    import json
+    import os
     from hypergen_b200 import synth
-    g = synth.genome(0xB200 + 5, 400_000).numpy()
-    g[1000:1040] = ord("N")
-    p = hg.make_params()
-    hashes, hoff = ctx.kmer_hash(g, np.array([0, g.size], np.uint64), p)
-    assert np.array_equal(hashes, oracle.ref_kmer_hash_set(g))
+    with open(os.path.join(os.path.dirname(__file__), "golden", "kmer_ref_sets.json")) as f:
+        sets = json.load(f)["sets"]
+    g = synth.genome(0xB200 + 77, 60_000).numpy().copy()
+    g[5000:5030] = ord("N")
+    g[20000:26000] |= 0x20
+    off = np.array([0, g.size], np.uint64)
+    assert len(sets) == 6
+    for name, c in sets.items():
+        hashes, _ = ctx.kmer_hash(g, off, hg.make_params(k=c["k"], scaled=c["scaled"], canonical=c["canonical"]))
+        assert hashes.size == c["n"], name
+        assert [int(x) for x in hashes[:4]] == c["head"], name
+        assert hashlib.sha256(hashes.tobytes()).hexdigest() == c["sha256"], name
 
 
 @pytest.mark.parametrize("hv_d,scaled", [(256, 200), (1024, 1500), (4096, 1500), (8192, 500), (4096, 60)])

@@ -27,8 +27,6 @@ def test_sort_matches_reference_order(ctx, hg, oracle, n, R, Q, levels, multi, m
     """multi=False: one cooperative kernel up to ~600 k records (4 or 16 rounds per warp), the multi-kernel
     path beyond; multi=True: the multi-kernel path at every size"""
     if multi:
-        if n > 300_000:
-            pytest.skip("already the multi-kernel path (or covered at 300 k)")
         monkeypatch.setenv("HG_SORT_MULTI", "1")
     rng = np.random.default_rng(n + levels)
     # full R x Q enumeration; a few distinct ANI levels so that ties dominate
