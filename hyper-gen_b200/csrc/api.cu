@@ -55,8 +55,8 @@ extern "C" int hg_init(int device, hg_ctx **out) {
   cudaDeviceProp prop;
   HG_CUDA(cudaGetDeviceProperties(&prop, device));
   c->sm_count = prop.multiProcessorCount;
-  {  // highest priority: work other streams of the library run NEXT TO this one (a multi-GPU member's operand pushes,
-     // peer.cu) must not get in front of the kernels launched here
+  {  // highest priority: work on other streams running next to this one (the H2D copy stream of the host entries, or the
+     // caller's own) must not get in front of the kernels launched here
     int lo = 0, hi = 0;
     HG_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
     HG_CUDA(cudaStreamCreateWithPriority(&c->stream, cudaStreamNonBlocking, hi));

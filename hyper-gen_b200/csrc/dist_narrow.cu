@@ -41,21 +41,14 @@ using namespace hgtc;
 constexpr int N1_BN = 256;                              // tile columns (the pair's N)
 constexpr int N1_A_BYTES = 128 * TC_BK;                 // 128 of my ref rows
 constexpr int N1_B_BYTES = 128 * TC_BK;                 // my half of the 256 query rows
-// NACC = accumulators (256 TMEM columns each) per tile.  NACC = 1 (default): 256 x 256 pair tiles, the accumulator
-// double buffered (epilogue fully hidden), 32 KB per stage.  NACC = 2: 512 x 256 pair tiles - two A tiles per CTA
-// share one B stage, 25 % fewer operand bytes per MAC - at the price of a single-buffered accumulator pair, i.e. an
-// exposed epilogue; 48 KB per stage.  Measured slower (see the launcher), kept selectable.
-template <int NACC> struct N1Cfg {
-  static constexpr int STAGES = NACC == 1 ? 6 : 4;
-  static constexpr int STAGE_BYTES = NACC * N1_A_BYTES + N1_B_BYTES;
-  static constexpr int TILE_ROWS = 256 * NACC;
-};
+constexpr int N1_STAGES = 6;
+constexpr int N1_STAGE_BYTES = N1_A_BYTES + N1_B_BYTES;  // 32 KB
 constexpr int N1_EPI_WARPS = 8;                         // two per TMEM lane quarter, half the columns each
 constexpr int N1_THREADS = 64 + 32 * N1_EPI_WARPS;      // producer, MMA issuer, epilogue warps (+ 32 per pusher warp of a multi-GPU member)
 constexpr int N1_PUSH_WARPS = 2;
 constexpr int N1_LIST_CAP = 256;                        // candidates per warp list (8 B each)
 constexpr int N1_COL_WORDS = 3 * N1_BN;                 // per tile: bound, centre, 2 sum(b) of every column
-constexpr int N1_SMEM_BYTES = 6 * (N1_A_BYTES + N1_B_BYTES) /* == 4 * (2 A + B) */ + 1024 /*align slack*/ + 256 /*barriers*/ +
+constexpr int N1_SMEM_BYTES = N1_STAGES * N1_STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/ +
                               2 * N1_COL_WORDS * 4 /*column constants, double buffered*/ + N1_EPI_WARPS * N1_LIST_CAP * 8 +
                               N1_EPI_WARPS * N1_LIST_CAP * 4 /*ANI of the evaluated candidates*/;
 constexpr uint32_t N1_TMEM_COLS = 512;                  // two accumulator buffers of 256 columns
@@ -247,28 +240,27 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
   }
 }
 
-// ---- tile walk: non-empty (256 NACC) x 256 tiles, row-block major ------------------------------------
+// ---- tile walk: non-empty 256 x 256 tiles, row-block major ------------------------------------------
 struct N1Tiles {
-  uint32_t gx, gy, R, C, tile_rows;
+  uint32_t gx, gy, R, C;
   int64_t delta;  // i0 - j0
   int sym;
   const uint2 *list;  // multi-GPU member: its tiles in the order the host chose (hg_tile_feed); NULL: the arithmetic walk below
   uint32_t n_list, cur, need;
   __device__ uint32_t cmin(uint32_t r) const {  // symmetric: tiles whose largest j is not above their smallest i are empty
     if (!sym) return 0;
-    const int64_t v = delta + (int64_t)tile_rows * (int64_t)r + 1;
+    const int64_t v = delta + 256ll * (int64_t)r + 1;
     if (v <= 0) return 0;
     const uint64_t c = (uint64_t)v / (uint32_t)N1_BN;
     return c > gx ? gx : (uint32_t)c;
   }
-  __device__ void init(const hg::DistEpilogue &ep, uint32_t rows_per_tile, const hg_tile_feed &f) {
+  __device__ void init(const hg::DistEpilogue &ep, const hg_tile_feed &f) {
     list = f.list;
     n_list = f.n_list;
     cur = 0;
     need = 0;
-    tile_rows = rows_per_tile;
     gx = (ep.n_qry + N1_BN - 1) / N1_BN;
-    gy = (ep.n_ref + tile_rows - 1) / tile_rows;
+    gy = (ep.n_ref + 255) / 256;
     delta = (int64_t)ep.i0 - (int64_t)ep.j0;
     sym = ep.symmetric;
     R = 0;
@@ -447,14 +439,11 @@ __device__ __forceinline__ uint32_t n1_drain(const hg::DistEpilogue &ep, const N
   return n_list;
 }
 
-template <int NACC, int PUSHW>
+template <int PUSHW>
 __global__ void __launch_bounds__(N1_THREADS + 32 * PUSHW, 1)
 dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry, uint32_t ref_row_base,
                uint32_t qry_row_base, hg::DistEpilogue ep, NarrowArgs na, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan) {
-  using Cfg = N1Cfg<NACC>;
-  constexpr int STAGES = Cfg::STAGES, STAGE_BYTES = Cfg::STAGE_BYTES;
-  constexpr uint32_t TILE_ROWS = Cfg::TILE_ROWS;
-  constexpr uint32_t NBUF = NACC == 1 ? 2 : 1;  // accumulator sets in TMEM
+  constexpr int STAGES = N1_STAGES, STAGE_BYTES = N1_STAGE_BYTES;
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
   if (feed.seq_ptr) feed.seq = *feed.seq_ptr;
@@ -510,7 +499,7 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
   for (uint32_t t = 0; t < na.r_nsets; ++t) { declined |= na.r_stats[4 * t + 3]; r_tmax = max(r_tmax, na.r_stats[4 * t + 1]); }
 
   N1Tiles tiles;
-  tiles.init(ep, TILE_ROWS, feed);
+  tiles.init(ep, feed);
   bool valid = !declined && tiles.advance(pair);
 
   if (warp == 0) {
@@ -519,7 +508,7 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
     uint32_t s = 0, ph = 0;
     unsigned long long waited = 0;  // (timeline) ns this producer spent waiting for other members' rows
     for (; valid; valid = tiles.advance(n_pairs)) {
-      const uint32_t row0 = tiles.R * TILE_ROWS + rank * 128u, colh = tiles.C * N1_BN + rank * 128u;
+      const uint32_t row0 = tiles.R * 256u + rank * 128u, colh = tiles.C * N1_BN + rank * 128u;
       if (tiles.need) {  // the rows this tile reads have arrived from their owners
         const unsigned long long w0 = feed.dbg ? hg::feed_ns() : 0ull;
         hg::feed_wait(feed, tiles.need, have);
@@ -531,10 +520,8 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
         const uint32_t fb = mapa_u32(full_bar(s), 0);
         const uint32_t st = base + s * STAGE_BYTES;
         const int k0 = (int)(kb * TC_BK);
-#pragma unroll
-        for (int a = 0; a < NACC; ++a)  // 128 of my ref rows per accumulator (accumulator a: tile rows 256 a .. 256 a + 255)
-          tma_load_2d_pair(st + a * N1_A_BYTES, &tm_ref, fb, k0, (int)(ref_row_base + row0 + 256u * a), on);
-        tma_load_2d_pair(st + NACC * N1_A_BYTES, &tm_qry, fb, k0, (int)(qry_row_base + colh), on);  // my half of the query rows
+        tma_load_2d_pair(st, &tm_ref, fb, k0, (int)(ref_row_base + row0), on);                     // my 128 ref rows
+        tma_load_2d_pair(st + N1_A_BYTES, &tm_qry, fb, k0, (int)(qry_row_base + colh), on);      // my half of the query rows
         if (++s == STAGES) { s = 0; ph ^= 1u; }
       }
     }
@@ -546,22 +533,19 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
       const uint32_t d0 = umma_desc_lo(base);
       uint32_t s = 0, ph = 0, tile_n = 0;
       for (; valid; valid = tiles.advance(n_pairs), ++tile_n) {
-        const uint32_t b = tile_n % NBUF, use = tile_n / NBUF;
+        const uint32_t b = tile_n & 1u, use = tile_n >> 1;  // accumulator buffer, and how often it was used before
         // both epilogues have drained this buffer's previous tile (passes at once for its first use)
         mbar_wait_cluster(tmem_empty_bar(b), (use & 1u) ^ 1u);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t tacc = tmem_base + (NACC == 1 ? b * N1_BN : 0u);
+        const uint32_t tacc = tmem_base + b * N1_BN;
         for (uint32_t kb = 0; kb < num_kb; ++kb) {
           mbar_wait(full_bar(s), ph);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t a0 = d0 + s * (uint32_t)(STAGE_BYTES >> 4);
 #pragma unroll
-          for (int ks = 0; ks < TC_BK / 32; ++ks) {  // one MMA covers K = 32 int8
-#pragma unroll
-            for (int a = 0; a < NACC; ++a)
-              umma_i8_pair(tacc + a * N1_BN, a0 + (uint32_t)((a * N1_A_BYTES + 32 * ks) >> 4),
-                           a0 + (uint32_t)((NACC * N1_A_BYTES + 32 * ks) >> 4), N1_IDESC, (kb | (uint32_t)ks) != 0u, on);
-          }
+          for (int ks = 0; ks < TC_BK / 32; ++ks)  // one MMA covers K = 32 int8
+            umma_i8_pair(tacc, a0 + (uint32_t)((32 * ks) >> 4), a0 + (uint32_t)((N1_A_BYTES + 32 * ks) >> 4), N1_IDESC,
+                         (kb | (uint32_t)ks) != 0u, on);
           umma_commit_pair(empty_bar(s), on);  // the stage is free in both CTAs once these MMAs have read it
           if (++s == STAGES) { s = 0; ph ^= 1u; }
         }
@@ -569,7 +553,7 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
       }
     }
   } else {
-    // ===== epilogue (both CTAs, each its own 128 rows of every accumulator) =====
+    // ===== epilogue (both CTAs, each its own 128 rows of the accumulator) =====
     const int ew = warp - 2;
     const uint32_t q = warp & 3;  // TMEM lane quarter this warp may read
     const int half = (ew >> 2);   // which 128 columns this warp drains
@@ -579,8 +563,8 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
     uint32_t tile_n = 0, have_e = 0, have_l = 0;
     volatile uint32_t *s_early = reinterpret_cast<volatile uint32_t *>(aligned + STAGES * STAGE_BYTES + 240);
     for (; valid; valid = tiles.advance(n_pairs), ++tile_n) {
-      const uint32_t b = tile_n % NBUF, use = tile_n / NBUF;
-      const uint32_t row0 = tiles.R * TILE_ROWS + rank * 128u, col0 = tiles.C * N1_BN;
+      const uint32_t b = tile_n & 1u, use = tile_n >> 1;
+      const uint32_t row0 = tiles.R * 256u + rank * 128u, col0 = tiles.C * N1_BN;
       // The per-row / per-column constants are read BEFORE the accumulator is waited for, to hide their latency - in a
       // multi-GPU launch possibly before the rows they belong to have arrived.  One epilogue warp looks at the arrival
       // flags (no spinning here: the producer does the waiting) and all eight take the same route: constants now, or
@@ -595,8 +579,8 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
         early = *s_early != 0u;
       }
       int32_t *s_col = s_col_all + (tile_n & 1u) * N1_COL_WORDS;  // double buffered: one barrier per tile is enough
-      int32_t tr[NACC], sr[NACC], xr[NACC];
-      bool live[NACC];
+      int32_t tr, sr, xr;
+      bool live;
       auto constants = [&]() {
         {
           const uint32_t t = threadIdx.x - 64, lj = col0 + t;  // one column per epilogue thread
@@ -615,20 +599,17 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
           s_col[2 * N1_BN + t] = tt;
         }
         asm volatile("bar.sync 1, %0;" ::"r"(32 * N1_EPI_WARPS) : "memory");  // epilogue warps only
-        // row constants of my row in every accumulator
-#pragma unroll
-        for (int a = 0; a < NACC; ++a) {
-          const uint32_t li = row0 + 256u * a + q * 32 + lane;
-          tr[a] = ROW_ALWAYS; sr[a] = 0; xr[a] = 0;
-          live[a] = li < ep.n_ref;
-          if (live[a]) {
-            if (ep.cfrac > 0.0f) {
-              const int32_t nr = ep.ref_norm[li];
-              if (nr > 0) tr[a] = n1_loosen(__float2int_rd(ep.cfrac * __int2float_rz(nr)) - 1, na.r.e[li], q_absmax, ROW_ALWAYS);
-            }
-            sr[a] = na.r.s[li];
-            xr[a] = (int32_t)((uint32_t)na.r.a2[li] + na.hv_d * (uint32_t)sr[a]);  // sum x~ = 2 sum a + D s
+        // row constants of my row
+        const uint32_t li = row0 + q * 32 + lane;
+        tr = ROW_ALWAYS; sr = 0; xr = 0;
+        live = li < ep.n_ref;
+        if (live) {
+          if (ep.cfrac > 0.0f) {
+            const int32_t nr = ep.ref_norm[li];
+            if (nr > 0) tr = n1_loosen(__float2int_rd(ep.cfrac * __int2float_rz(nr)) - 1, na.r.e[li], q_absmax, ROW_ALWAYS);
           }
+          sr = na.r.s[li];
+          xr = (int32_t)((uint32_t)na.r.a2[li] + na.hv_d * (uint32_t)sr);  // sum x~ = 2 sum a + D s
         }
       };
       if (early) constants();
@@ -639,16 +620,11 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
         constants();
       }
       uint32_t n_list = 0;
-#pragma unroll
-      for (int a = 0; a < NACC; ++a) {
-        const uint32_t rowa = row0 + 256u * a;
-        // my 128 x 256 part of this accumulator may be empty (below the diagonal, or past the last ref row)
-        const bool mine_empty = rowa >= ep.n_ref || (ep.symmetric && (uint64_t)ep.j0 + col0 + N1_BN - 1 <= (uint64_t)ep.i0 + rowa);
-        if (!mine_empty)
-          n_list = n1_drain(ep, na, tmem_base + ((q * 32u) << 16) + (NACC == 1 ? b * N1_BN : a * N1_BN), half * (N1_BN / 2),
-                            (half + 1) * (N1_BN / 2), s_col, tr[a], sr[a], xr[a], live[a], 256u * a + q * 32 + lane, row0, col0,
-                            list, anis, n_list);
-      }
+      // my 128 x 256 part of the tile may be empty (below the diagonal, or past the last ref row)
+      const bool mine_empty = row0 >= ep.n_ref || (ep.symmetric && (uint64_t)ep.j0 + col0 + N1_BN - 1 <= (uint64_t)ep.i0 + row0);
+      if (!mine_empty)
+        n_list = n1_drain(ep, na, tmem_base + ((q * 32u) << 16) + b * N1_BN, half * (N1_BN / 2), (half + 1) * (N1_BN / 2), s_col, tr,
+                          sr, xr, live, q * 32 + lane, row0, col0, list, anis, 0u);
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(mapa_u32(tmem_empty_bar(b), 0));  // this warp's TMEM reads of buffer b are done
@@ -724,11 +700,8 @@ uint32_t hg_narrow_set_cap(uint32_t n_rows) { return (uint32_t)std::min<uint64_t
 
 static int narrow_attrs(hg_ctx *ctx) {
   if (!ctx->n1_attr_set) {
-    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<1, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<N1_PUSH_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
     ctx->n1_attr_set = 1;
   }
   return HG_OK;
@@ -855,34 +828,22 @@ int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32
   cfg.numAttrs = 1;
   cfg.blockDim = dim3(N1_THREADS, 1, 1);
   cfg.stream = ctx->stream;
-  // one CTA pair per TPC, each walking its tiles with stride n_pairs.  256-row tiles by default: the 512-row
-  // variant (two accumulators, 25 % fewer operand bytes per MAC, exposed epilogue) measured 13 % slower on
-  // config 3 (0.239 vs 0.212 ms) and 5 % slower on config 4; HG_NARROW_NACC=2 selects it.
-  int nacc = 1;
-  if (const char *e = getenv("HG_NARROW_NACC")) nacc = atoi(e) == 2 ? 2 : 1;
-  const uint32_t tile_rows = 256u * nacc;
-  const uint64_t tiles_all = (uint64_t)((n_qry + N1_BN - 1) / N1_BN) * ((n_ref + tile_rows - 1) / tile_rows);
+  // one CTA pair per TPC, each walking its 256 x 256 tiles with stride n_pairs
+  const uint64_t tiles_all = (uint64_t)((n_qry + N1_BN - 1) / N1_BN) * ((n_ref + 255) / 256);
   hg_tile_feed fd = {};
   if (feed) fd = *feed;
-  if (fd.list && nacc != 1) { hg_set_error("a tile list is built for 256-row tiles (HG_NARROW_NACC=2 is a single-GPU experiment)"); return HG_E_UNSUPPORTED; }
   // this launch's share of the tiles (an upper bound when symmetric)
   const uint64_t tiles = fd.list ? fd.n_list : (tiles_all + walk_mul - 1) / walk_mul;
   if (tiles == 0) return HG_OK;
-  const uint32_t n_pairs = (uint32_t)std::min<uint64_t>(tiles, (uint64_t)std::max(ctx->sm_count / 2 - fd.reserve_tpcs, 1));
+  const uint32_t n_pairs = (uint32_t)std::min<uint64_t>(tiles, (uint64_t)std::max(ctx->sm_count / 2, 1));
   cfg.gridDim = dim3(2 * n_pairs, 1, 1);
   cfg.dynamicSmemBytes = N1_SMEM_BYTES;
   static const hg_push_plan no_push = {};
   if (push) {  // a member of several GPUs: the launch carries pusher warps that send my operand rows while the tiles are computed
-    if (nacc != 1) { hg_set_error("pusher warps come with the 256-row tile kernel"); return HG_E_UNSUPPORTED; }
-    const int pw = hg_push_warps(N1_PUSH_WARPS);
-    cfg.blockDim = dim3(N1_THREADS + 32 * pw, 1, 1);
-    if (pw == 2) HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<1, 2>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push));
-    else if (pw == 4) HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<1, 4>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push));
-    else HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<1, 6>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push));
-  } else if (nacc == 2) {
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<2, 0>, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push));
+    cfg.blockDim = dim3(N1_THREADS + 32 * N1_PUSH_WARPS, 1, 1);
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<N1_PUSH_WARPS>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push));
   } else {
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<1, 0>, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push));
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<0>, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push));
   }
   ctx->launches++;
   HG_CUDA(cudaGetLastError());

@@ -12,7 +12,7 @@
 // is accumulated as three s32 accumulators (the two cross products share one), each < 2^31
 // for D <= 32768.  The recombination wraps in i32 exactly like the reference's i32 sum.
 //
-// Default kernel (dist_tc2_kernel): persistent CTA PAIRS (cluster 2 x 1, tcgen05 cta_group::2), one pair
+// Kernel (dist_tc2_kernel): persistent CTA PAIRS (cluster 2 x 1, tcgen05 cta_group::2), one pair
 // per TPC, each walking 256 x 128 output tiles.  Per k-block a CTA TMA-loads its own 128 ref rows and
 // only HALF of the query tile (64 rows) - 48 KB instead of 64 KB for the same MMA work - because the
 // pair's MMA reads the query half of both CTAs; the kernel is bound by operand bytes arriving per SM
@@ -21,11 +21,11 @@
 // tile while the epilogue drains, one thread of the leader CTA's warp 1 issues the tcgen05.mma stream
 // (M = 256) and multicasts the stage releases to both CTAs, warps 2-9 of each CTA drain their three
 // TMEM accumulators with tcgen05.ld, apply a division-free bound and run the shared exact epilogue
-// (dist_common.cuh) only where a pair can reach the threshold.
-// Fallback (HG_DIST_KERNEL=1): dist_tc_kernel, one stand-alone CTA per 128 x 128 tile.
+// (dist_common.cuh) only where a pair can reach the threshold.  The K loop always runs whole trips of the
+// stage ring: when hv_d is not a multiple of 512 the tensor maps' zero fill supplies the missing columns.
 #include <cuda.h>
 
-#include <cstdlib>
+#include <algorithm>
 
 #include "dist_common.cuh"
 #include "tc_ptx.cuh"
@@ -34,22 +34,13 @@ namespace {
 
 using namespace hgtc;
 
-constexpr int TC_BM = 128, TC_BN = 128;
-constexpr int TC_STAGES = 3;
-constexpr int TC_TILE_BYTES = 128 * TC_BK;            // one operand tile
-constexpr int TC_STAGE_BYTES = 4 * TC_TILE_BYTES;     // A_hi, A_lo, B_hi, B_lo
+constexpr int TC_BN = 128;
 constexpr int TC_EPI_WARPS = 8;                      // two per TMEM lane quarter, half the columns each
 constexpr int TC_THREADS = 64 + 32 * TC_EPI_WARPS;  // producer, MMA issuer, epilogue warps (+ 32 per pusher warp of a multi-GPU member)
 constexpr int TC_PUSH_WARPS = 2;
-constexpr int TC_SMEM_BYTES = TC_STAGES * TC_STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/ + 512 /*col bounds*/ +
-                              8 * 256 * 8 /*candidate lists: TC_EPI_WARPS x TC_LIST_CAP x 8 B*/ + 8 * 256 * 4 /*their ANIs*/;
 constexpr uint32_t TC_TMEM_COLS = 512;
 
-// instruction descriptor, kind::i8: D = s32, A = B = signed 8-bit, both K-major, M = 128, N = 128
-constexpr uint32_t TC_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((TC_BN >> 3) << 17) | ((TC_BM >> 4) << 24);
-
-
-// ---- epilogue pieces shared by both kernels ---------------------------------------------------
+// ---- epilogue pieces --------------------------------------------------------------------------
 // Cheap per-element test first: ani >= ani_th implies dot >= cfrac * (norm_r + norm_q)
 // (dist_common.cuh), split into a per-row and a per-column integer so that an element costs
 // two shift-adds, one add and one compare.  Only lanes that pass run the exact f32 ANI sequence
@@ -69,8 +60,8 @@ __device__ __forceinline__ int32_t tc_row_bound(const hg::DistEpilogue &ep, uint
 
 // Candidates are not evaluated while the accumulators are being drained: each epilogue warp parks
 // them (row, column, exact dot) in its own shared-memory list and runs the exact f32 ANI + append
-// (dist_common.cuh) over the list afterwards, 32 candidates per round.  In the persistent kernel
-// that second phase starts after TMEM has been handed back, so it overlaps the next tile's MMAs;
+// (dist_common.cuh) over the list afterwards, 32 candidates per round.  That second phase starts
+// after TMEM has been handed back, so it overlaps the next tile's MMAs;
 // it also balances the lanes (hits cluster on a few rows of the diagonal tiles).
 constexpr int TC_LIST_CAP = 256;  // candidates per warp list (8 B each); a full list is evaluated in place
 
@@ -187,126 +178,14 @@ __device__ __forceinline__ uint32_t tc_drain(const hg::DistEpilogue &ep, uint32_
   return n_list;
 }
 
-// ---- fallback kernel: one stand-alone CTA per 128 x 128 tile ----------------------------------
-__global__ void __launch_bounds__(TC_THREADS, 1)
-dist_tc_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
-               uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t hv_d,
-               hg::DistEpilogue ep) {
-  const uint32_t row0 = blockIdx.y * TC_BM, col0 = blockIdx.x * TC_BN;
-  // symmetric: a tile whose largest global j is not above its smallest global i is empty
-  if (ep.symmetric && (uint64_t)ep.j0 + col0 + TC_BN - 1 <= (uint64_t)ep.i0 + row0) return;
-
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;  // 128B swizzle wants 1024 B alignment
-  uint8_t *aligned = smem_raw + (base - smem_u32(smem_raw));
-  const uint32_t bar_base = base + TC_STAGES * TC_STAGE_BYTES;
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (TC_STAGES + s); };
-  const uint32_t accum_bar = bar_base + 8u * (2 * TC_STAGES);
-  volatile uint32_t *tmem_slot = reinterpret_cast<volatile uint32_t *>(aligned + TC_STAGES * TC_STAGE_BYTES + 8 * (2 * TC_STAGES + 1));
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < TC_STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    mbar_init(accum_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void *)tmem_slot)),
-                 "r"(TC_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t num_kb = hv_d / TC_BK;
-
-  if (warp == 0) {
-    // ===== TMA producer (whole warp in step, one elected lane issues) =====
-    {
-      const uint32_t on = elect_one();
-      for (uint32_t kb = 0; kb < num_kb; ++kb) {
-        const int s = kb % TC_STAGES;
-        const uint32_t ph = (kb / TC_STAGES) & 1u;
-        mbar_wait(empty_bar(s), ph ^ 1u);
-        mbar_expect_tx(full_bar(s), TC_STAGE_BYTES, on);
-        const uint32_t st = base + s * TC_STAGE_BYTES;
-        const int k0 = (int)(kb * TC_BK);
-        tma_load_2d(st + 0 * TC_TILE_BYTES, &tm_ref, full_bar(s), k0, (int)(ref_row_base + row0), on);  // ref hi limbs
-        tma_load_2d(st + 1 * TC_TILE_BYTES, &tm_ref, full_bar(s), k0, (int)(ref_plane_rows + ref_row_base + row0), on);  // ref lo
-        tma_load_2d(st + 2 * TC_TILE_BYTES, &tm_qry, full_bar(s), k0, (int)(qry_row_base + col0), on);                    // qry hi limbs
-        tma_load_2d(st + 3 * TC_TILE_BYTES, &tm_qry, full_bar(s), k0, (int)(qry_plane_rows + qry_row_base + col0), on);  // qry lo limbs
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer (one elected thread drives the tensor core; the warp stays converged) =====
-    {
-      const uint32_t on = elect_one();
-      const uint32_t d0 = umma_desc_lo(base);
-      // the stage ring is walked with a compile-time stage index so that every descriptor is d0 + constant
-      for (uint32_t kb0 = 0; kb0 < num_kb; kb0 += TC_STAGES) {
-        const uint32_t ph = (kb0 / TC_STAGES) & 1u;
-#pragma unroll
-        for (int s = 0; s < TC_STAGES; ++s) {
-          if (kb0 + s < num_kb) {
-            mbar_wait(full_bar(s), ph);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int ks = 0; ks < TC_BK / 32; ++ks) {  // one MMA covers K = 32 int8
-              const uint32_t off = (uint32_t)(s * TC_STAGE_BYTES + 32 * ks) >> 4;
-              const uint32_t a_hi = d0 + off, a_lo = a_hi + (TC_TILE_BYTES >> 4);
-              const uint32_t b_hi = a_hi + (2 * TC_TILE_BYTES >> 4), b_lo = a_hi + (3 * TC_TILE_BYTES >> 4);
-              const uint32_t acc = (kb0 | (uint32_t)s | (uint32_t)ks) != 0u;
-              umma_i8(tmem_base + 0 * TC_BN, a_hi, b_hi, TC_IDESC, acc, on);  // Hr.Hq
-              umma_i8(tmem_base + 1 * TC_BN, a_hi, b_lo, TC_IDESC, acc, on);  // Hr.Lq
-              umma_i8(tmem_base + 1 * TC_BN, a_lo, b_hi, TC_IDESC, 1u, on);   //   + Lr.Hq
-              umma_i8(tmem_base + 2 * TC_BN, a_lo, b_lo, TC_IDESC, acc, on);  // Lr.Lq
-            }
-            umma_commit(empty_bar(s), on);  // the stage is free once these MMAs have read it
-          }
-        }
-      }
-      umma_commit(accum_bar, on);       // all accumulators final
-    }
-  } else {
-    // ===== epilogue: TMEM -> registers -> exact i32 dot -> bound test -> (rare) ANI + append =====
-    const int ew = warp - 2;                 // 0..7
-    const uint32_t q = warp & 3;             // TMEM lane quarter this warp may read
-    const int half = (ew >> 2);              // which 64 columns this warp drains
-    int32_t *s_tq = reinterpret_cast<int32_t *>(aligned + TC_STAGES * TC_STAGE_BYTES + 256);
-    {  // per-column bounds, one column per epilogue thread of the first four warps
-      const int t = threadIdx.x - 64;
-      if (t < TC_BN) s_tq[t] = tc_col_bound(ep, col0 + t);
-    }
-    asm volatile("bar.sync 1, %0;" ::"r"(32 * TC_EPI_WARPS) : "memory");  // epilogue warps only
-    const uint32_t li = row0 + q * 32 + lane;
-    const int32_t tr = tc_row_bound(ep, li);
-    mbar_wait(accum_bar, 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    uint2 *list = reinterpret_cast<uint2 *>(aligned + TC_STAGES * TC_STAGE_BYTES + 256 + 512) + ew * TC_LIST_CAP;
-    float *anis = reinterpret_cast<float *>(aligned + TC_STAGES * TC_STAGE_BYTES + 256 + 512 + TC_EPI_WARPS * TC_LIST_CAP * 8) + ew * TC_LIST_CAP;
-    const uint32_t n_list = tc_drain(ep, tmem_base + ((q * 32u) << 16), half * (TC_BN / 2), (half + 1) * (TC_BN / 2), s_tq, tr,
-                                     li < ep.n_ref, q * 32 + lane, row0, col0, list, anis, 0u);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    tc_process(ep, list, anis, n_list, row0, col0);
-  }
-  __syncthreads();
-  if (warp == 2) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
-  }
-}
-
-// ---- default kernel: persistent CTA pairs, cta_group::2, 256 x 128 tiles ----------------------
+// ---- the kernel: persistent CTA pairs, cta_group::2, 256 x 128 tiles ---------------------------
 constexpr int T2_STAGES = 4;
 constexpr int T2_A_BYTES = 128 * TC_BK;               // my 128 ref rows, one limb plane
 constexpr int T2_B_BYTES = 64 * TC_BK;                // my half of the 128 query rows, one limb plane
 constexpr int T2_STAGE_BYTES = 2 * T2_A_BYTES + 2 * T2_B_BYTES;  // 48 KB
 constexpr int T2_SMEM_BYTES = T2_STAGES * T2_STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/ + 1024 /*col bounds x 2*/ +
                               8 * 256 * 8 /*candidate lists*/ + 8 * 256 * 4 /*their ANIs*/;
-// instruction descriptor as TC_IDESC with M = 256 (the pair's rows)
+// instruction descriptor, kind::i8: D = s32, A = B = signed 8-bit, both K-major, M = 256 (the pair's rows), N = 128
 constexpr uint32_t T2_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((TC_BN >> 3) << 17) | ((256u >> 4) << 24);
 
 
@@ -362,7 +241,7 @@ struct PairTiles {
 template <int PUSHW>
 __global__ void __launch_bounds__(TC_THREADS + 32 * PUSHW, 1)
 dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
-                uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t hv_d,
+                uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len,
                 hg::DistEpilogue ep, uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan) {
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
@@ -401,7 +280,7 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
   cluster_sync_all();  // the peer's barriers are initialised before anyone signals them
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t num_kb = hv_d / TC_BK;
+  const uint32_t num_kb = k_len / TC_BK;
 
   if (PUSHW > 0 && warp >= TC_THREADS / 32) {
     // ===== pusher warps (a member of several GPUs): my limb-plane rows to the windows of the members that compute with them, unit by unit =====
@@ -457,7 +336,7 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
           mbar_wait_cluster(tmem_empty_bar, (tile_n - 1) & 1u);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         }
-        // num_kb is a multiple of T2_STAGES (host-checked), so every tile starts at stage 0 and the ring is
+        // num_kb is a multiple of T2_STAGES (k_len is), so every tile starts at stage 0 and the ring is
         // walked with a compile-time stage index: every descriptor is d0 + constant
         for (uint32_t kb0 = 0; kb0 < num_kb; kb0 += T2_STAGES, ++it) {
           const uint32_t ph = it & 1u;
@@ -571,6 +450,15 @@ __global__ void split_limbs_kernel(const int16_t *__restrict__ hv, uint64_t n_el
 
 void hg_tc_tile_shape(uint32_t *rows, uint32_t *cols) { *rows = 256; *cols = TC_BN; }
 
+static int tc_attrs(hg_ctx *ctx) {
+  if (!ctx->tc_attr_set) {
+    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<TC_PUSH_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
+    ctx->tc_attr_set = 1;
+  }
+  return HG_OK;
+}
+
 // ---- one matrix as two s8 limb planes [2][n_rows][hv_d]; its rows may be split piecewise, as they arrive ----
 int hg_tc_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b) {
   if (hv_d % TC_BK != 0 || hv_d > 32768) {
@@ -592,15 +480,7 @@ int hg_tc_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d
   m->planes = (int8_t *)p;
   m->n_rows = n_rows;
   m->hv_d = hv_d;
-  if (!ctx->tc_attr_set) {
-    HG_CUDA(cudaFuncSetAttribute(dist_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    ctx->tc_attr_set = 1;
-  }
-  return HG_OK;
+  return tc_attrs(ctx);
 }
 
 // limb split of rows [row0, row0 + rows) (asynchronous)
@@ -629,15 +509,7 @@ int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_
   m->planes = planes;
   m->n_rows = n_rows;
   m->hv_d = hv_d;
-  if (!ctx->tc_attr_set) {
-    HG_CUDA(cudaFuncSetAttribute(dist_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
-    ctx->tc_attr_set = 1;
-  }
-  return HG_OK;
+  return tc_attrs(ctx);
 }
 
 int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
@@ -650,73 +522,54 @@ int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref
   if (walk_mul == 0 || walk_add >= walk_mul) { hg_set_error("hg_tc_launch: tile walk %u / %u", walk_add, walk_mul); return HG_E_INVALID; }
   int rc;
   const uint32_t hv_d = R->hv_d;
-  const uint32_t gx = (n_qry + TC_BN - 1) / TC_BN, gy_total = (n_ref + TC_BM - 1) / TC_BM;
-  // HG_DIST_KERNEL=1 selects the stand-alone-CTA fallback; default is the persistent CTA-pair kernel
-  int pair_kernel = 1;
-  if (const char *e = getenv("HG_DIST_KERNEL")) pair_kernel = atoi(e) == 1 ? 0 : 1;
-  if (hv_d % (TC_BK * T2_STAGES) != 0) pair_kernel = 0;  // the pair kernel walks whole trips of its 4-stage ring
-  if (!pair_kernel && (walk_mul != 1 || fd.list || push)) { hg_set_error("a shared tile walk needs the pair kernel (hv_d %% 512 == 0)"); return HG_E_UNSUPPORTED; }
+  // the K loop runs whole trips of the 4-stage ring; the tensor maps end at hv_d and fill the boxes past it with zeros,
+  // which add nothing to the dot products
+  const uint32_t k_len = (hv_d + TC_BK * T2_STAGES - 1) / (TC_BK * T2_STAGES) * (TC_BK * T2_STAGES);
   CUtensorMap tm_ref, tm_qry;
-  if ((rc = make_plane_map(&tm_qry, Q->planes, 2ull * Q->n_rows, hv_d, pair_kernel ? 64 : 128))) return rc;
+  if ((rc = make_plane_map(&tm_qry, Q->planes, 2ull * Q->n_rows, hv_d, 64))) return rc;
   if ((rc = make_plane_map(&tm_ref, R->planes, 2ull * R->n_rows, hv_d, 128))) return rc;
-  auto make_ep = [&](uint32_t y0) {
-    hg::DistEpilogue ep;
-    ep.ref_norm = d_ref_norm + (size_t)y0 * TC_BM;
-    ep.qry_norm = d_qry_norm;
-    ep.n_ref = n_ref - y0 * TC_BM;
-    ep.n_qry = n_qry;
-    ep.i0 = i0 + y0 * TC_BM;
-    ep.j0 = j0;
-    ep.ksize_f = (float)ksize;
-    ep.ani_th = ani_th;
-    ep.jmin = hg::dist_jmin(ani_th, ksize);
-    ep.cfrac = ep.jmin > 0.0f ? (float)((double)ep.jmin / (1.0 + (double)ep.jmin)) : 0.0f;
-    ep.symmetric = symmetric;
-    ep.hits = d_hits;
-    ep.cap = cap;
-    ep.n_hits = d_n_hits;
-    return ep;
-  };
+  hg::DistEpilogue ep;
+  ep.ref_norm = d_ref_norm;
+  ep.qry_norm = d_qry_norm;
+  ep.n_ref = n_ref;
+  ep.n_qry = n_qry;
+  ep.i0 = i0;
+  ep.j0 = j0;
+  ep.ksize_f = (float)ksize;
+  ep.ani_th = ani_th;
+  ep.jmin = hg::dist_jmin(ani_th, ksize);
+  ep.cfrac = ep.jmin > 0.0f ? (float)((double)ep.jmin / (1.0 + (double)ep.jmin)) : 0.0f;
+  ep.symmetric = symmetric;
+  ep.hits = d_hits;
+  ep.cap = cap;
+  ep.n_hits = d_n_hits;
+  // one CTA pair per TPC, each walking the 256 x 128 tiles with stride n_pairs
+  const uint32_t gx = (n_qry + TC_BN - 1) / TC_BN;
+  const uint64_t tiles = fd.list ? fd.n_list : ((uint64_t)gx * ((n_ref + 255) / 256) + walk_mul - 1) / walk_mul;
+  if (tiles == 0) return HG_OK;
+  const uint32_t n_pairs = (uint32_t)std::min<uint64_t>(tiles, (uint64_t)std::max(ctx->sm_count / 2, 1));
   cudaLaunchConfig_t cfg = {};
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   cfg.blockDim = dim3(TC_THREADS, 1, 1);
+  cfg.gridDim = dim3(2 * n_pairs, 1, 1);
+  cfg.dynamicSmemBytes = T2_SMEM_BYTES;
   cfg.stream = ctx->stream;
-  if (pair_kernel) {
-    // one CTA pair per TPC, each walking the 256 x 128 tiles with stride n_pairs
-    const uint64_t tiles = fd.list ? fd.n_list : ((uint64_t)gx * ((n_ref + 255) / 256) + walk_mul - 1) / walk_mul;
-    if (tiles == 0) return HG_OK;
-    const uint32_t n_pairs = (uint32_t)std::min<uint64_t>(tiles, (uint64_t)std::max(ctx->sm_count / 2 - fd.reserve_tpcs, 1));
-    cfg.gridDim = dim3(2 * n_pairs, 1, 1);
-    cfg.dynamicSmemBytes = T2_SMEM_BYTES;
-    attr[0].val.clusterDim.x = 2;
-    static const hg_push_plan no_push = {};
-    if (push) {  // a member of several GPUs: pusher warps send my limb-plane rows while the tiles are computed
-      const int pw = hg_push_warps(TC_PUSH_WARPS);
-      cfg.blockDim = dim3(TC_THREADS + 32 * pw, 1, 1);
-      if (pw == 2) HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<2>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, hv_d, make_ep(0), walk_mul, walk_add, fd, *push));
-      else if (pw == 4) HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<4>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, hv_d, make_ep(0), walk_mul, walk_add, fd, *push));
-      else HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<6>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, hv_d, make_ep(0), walk_mul, walk_add, fd, *push));
-    } else {
-      HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, hv_d, make_ep(0), walk_mul, walk_add,
-                                 fd, no_push));
-    }
-    ctx->launches++;
+  static const hg_push_plan no_push = {};
+  if (push) {  // a member of several GPUs: pusher warps send my limb-plane rows while the tiles are computed
+    cfg.blockDim = dim3(TC_THREADS + 32 * TC_PUSH_WARPS, 1, 1);
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<TC_PUSH_WARPS>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul,
+                               walk_add, fd, *push));
   } else {
-    const uint32_t y_step = 65534;  // <= the gridDim.y limit
-    for (uint32_t y0 = 0; y0 < gy_total; y0 += y_step) {
-      const uint32_t gy = gy_total - y0 < y_step ? gy_total - y0 : y_step;
-      cfg.gridDim = dim3(gx, gy, 1);
-      cfg.dynamicSmemBytes = TC_SMEM_BYTES;
-      attr[0].val.clusterDim.x = 1;
-      HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc_kernel, tm_ref, tm_qry, R->n_rows, r0 + y0 * TC_BM, Q->n_rows, q0, hv_d, make_ep(y0)));
-      ctx->launches++;
-    }
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul, walk_add, fd,
+                               no_push));
   }
+  ctx->launches++;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
 }

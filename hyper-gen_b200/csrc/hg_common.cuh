@@ -242,10 +242,6 @@ int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_
 // or this member's start flag - when all pusher warps of the grid are through with it.  All-vs-all on three or more
 // GPUs sends a member's rows only to the floor(N/2) members that compute tiles with them, nearest ring neighbour first
 // (csrc/peer.cu); otherwise every chunk goes to everybody.  One kernel computes tiles and moves operands.
-// TPCs a multi-GPU dist launch leaves free when this member's pushes run as kernels of their own NEXT TO it (on a
-// second, lower-priority stream): the dist kernel is resident and waiting for the other members' chunks while they run, so
-// the pushes must never need one of its SMs.
-#define HG_PEER_RESERVED_TPCS 8
 #define HG_PUSH_CHUNKS 4
 #define HG_PUSH_SETS (HG_PUSH_CHUNKS + 1)
 #define HG_PUSH_START_SET HG_PUSH_CHUNKS
@@ -269,12 +265,6 @@ struct hg_push_plan {
   uint32_t dyn_base;
   unsigned long long *dbg;  // timeline stamps (HG_PEER_TIMELINE=1, hg_peer_timeline), else NULL
 };
-// pusher warps per CTA of a multi-GPU dist launch: 2, 4 or 6 (HG_PEER_PUSH_WARPS overrides the kernels' default)
-inline int hg_push_warps(int dflt) {
-  int w = dflt;
-  if (const char *e = getenv("HG_PEER_PUSH_WARPS")) w = atoi(e);
-  return w <= 2 ? 2 : (w <= 4 ? 4 : 6);
-}
 struct hg_tile_feed {
   const uint2 *list;        // x = tile row | tile column << 16, y = mask of the arrival flags the tile needs; NULL: arithmetic walk
   uint32_t n_list;
@@ -286,7 +276,6 @@ struct hg_tile_feed {
                             // outlier entries are here; the root has reset its gather counter)
   uint32_t *status;         // set to 1 if a wait times out (the host turns it into an error)
   unsigned long long timeout_ns;
-  int reserve_tpcs;         // TPCs the launch leaves free (for the push kernel running next to it)
   unsigned long long *dbg;  // timeline stamps (HG_PEER_TIMELINE=1, hg_peer_timeline), else NULL
 };
 

@@ -228,10 +228,6 @@ struct hg_peer {
                              // last call, written by the call's last node
   // The launch sequence of a sharded dist with asserted path (same pointers, same shapes, call after call) is captured
   // once and replayed as a CUDA graph: one launch instead of ~10, no gaps between the nodes.
-  // chunk pushes as kernels of their own run on this (default-priority) stream, next to the dist kernel on the context's
-  // (highest-priority) stream, on the TPCs the dist launch leaves free
-  cudaStream_t push_stream = nullptr;
-  cudaEvent_t ev_operands = nullptr, ev_pushed = nullptr;
   cudaGraphExec_t graph = nullptr;
   std::vector<uint8_t> graph_key, last_key;
   unsigned graph_nodes = 0;
@@ -282,12 +278,6 @@ static int peer_alloc(hg_ctx *ctx, int rank, int world, uint64_t window_bytes, h
   p->timeout_ns = 10ull * 1000000000ull;
   if (const char *e = getenv("HG_PEER_TIMEOUT_MS")) p->timeout_ns = (unsigned long long)std::max(1, atoi(e)) * 1000000ull;
   if (const char *e = getenv("HG_PEER_TIMELINE")) p->timeline = atoi(e) != 0;
-  if (cudaStreamCreateWithFlags(&p->push_stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&p->ev_operands, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&p->ev_pushed, cudaEventDisableTiming) != cudaSuccess) {
-    delete p;
-    return hg_cuda_fail(cudaGetLastError(), "push stream", __FILE__, __LINE__);
-  }
   void *w = nullptr;
   cudaError_t e = cudaMalloc(&w, window_bytes);
   if (e != cudaSuccess) { delete p; return hg_cuda_fail(e, "cudaMalloc(window)", __FILE__, __LINE__); }
@@ -377,9 +367,6 @@ extern "C" void hg_peer_destroy(hg_peer *p) {
   for (int i = 0; i < 6; ++i) if (p->ev[i]) cudaEventDestroy(p->ev[i]);
   if (p->graph) cudaGraphExecDestroy(p->graph);
   if (p->h_hdr) cudaFreeHost(p->h_hdr);
-  if (p->push_stream) { cudaStreamSynchronize(p->push_stream); cudaStreamDestroy(p->push_stream); }
-  if (p->ev_operands) cudaEventDestroy(p->ev_operands);
-  if (p->ev_pushed) cudaEventDestroy(p->ev_pushed);
   delete p;
 }
 
@@ -403,13 +390,13 @@ extern "C" int hg_peer_barrier(hg_peer *p) {
 // Stand-alone push of one unit (a member that has rows to contribute but no tile to compute - otherwise the dist
 // kernel's pusher warps do this, see hg_push_plan): the ranges to the members in `dest`, then the flag at byte offset
 // `flag_off` of those windows
-static int peer_push(hg_peer *p, const PushArgs &a, uint32_t dest, uint64_t flag_off, int unit, cudaStream_t stream, unsigned max_blocks) {
+static int peer_push(hg_peer *p, const PushArgs &a, uint32_t dest, uint64_t flag_off, int unit) {
   if (p->world == 1) return HG_OK;
   uint64_t bytes = 0;
   for (int k = 0; k < a.n; ++k) bytes += a.r[k].bytes;
-  const unsigned blocks = (unsigned)std::min<uint64_t>(std::max<uint64_t>(bytes / (16 * 256 * 4), 1), (uint64_t)max_blocks);
+  const unsigned blocks = (unsigned)std::min<uint64_t>(std::max<uint64_t>(bytes / (16 * 256 * 4), 1), (uint64_t)p->ctx->sm_count * 4u);
   uint32_t *done = reinterpret_cast<uint32_t *>(p->win[p->rank] + OFF_DONE) + unit;
-  peer_push_kernel<<<blocks, 256, 0, stream>>>(peer_ptrs(p), p->rank, p->world, a, dest, flag_off, done);
+  peer_push_kernel<<<blocks, 256, 0, p->ctx->stream>>>(peer_ptrs(p), p->rank, p->world, a, dest, flag_off, done);
   p->ctx->launches++;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
@@ -447,7 +434,7 @@ XPlan make_xplan(int world, int symmetric, int path, uint32_t hv_d, const uint32
     if (rows == 0) nonempty = false;
     if (m > 0 && qb[m] % 256 != 0) aligned = false;  // a tile (256 rows x 128 or 256 columns) lies inside one block on either side
   }
-  x.ring = symmetric && world >= 2 && aligned && nonempty && !getenv("HG_PEER_NO_RING");
+  x.ring = symmetric && world >= 2 && aligned && nonempty;
   return x;
 }
 // chunk c of member m's block: rows [chunk_lo(c), chunk_lo(c + 1))
@@ -545,7 +532,7 @@ static void plan_tiles(const TileKey &k, int world, int rank, std::vector<uint2>
   // all-vs-all: tiles that read only my own rows first, then in the order the other members' chunks arrive (row-major
   // within each group).  ref x query stays row-major: the queries are few and arrive early, while a column-wise sweep
   // would stream my whole ref plane from HBM once per query tile column.
-  if (k.sym && !getenv("HG_PEER_NOSORT")) std::stable_sort(v.begin(), v.end(), [](const T &a, const T &b) { return a.key < b.key; });
+  if (k.sym) std::stable_sort(v.begin(), v.end(), [](const T &a, const T &b) { return a.key < b.key; });
   out.resize(v.size());
   for (size_t i = 0; i < v.size(); ++i) out[i] = v[i].e;
 }
@@ -629,7 +616,7 @@ static int shard_reserve(hg_peer *p, const ShardCall &a, int use_path) {
     if ((rc = hg_scratch(c, HG_S_REF_LIMBS, 2 * (uint64_t)a.n_ref_local * a.hv_d + 1024, &x))) return rc;
     if ((rc = hg_scratch(c, HG_S_NARROW_META, hg_narrow_arrays_bytes(a.n_ref_local) + (uint64_t)hg_narrow_set_cap(a.n_ref_local) * 4 + 256, &x))) return rc;
   }
-  if (p->world > 1 || getenv("HG_PEER_FORCE_LIST")) {
+  if (p->world > 1) {
     build_tiles(p, a, use_path);
     const size_t bytes = p->tiles.size() * sizeof(uint2) + 256;
     if ((rc = hg_scratch(c, HG_S_TILES, bytes, &x))) return rc;
@@ -670,7 +657,7 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
   c->launches++;
   HG_CUDA(cudaGetLastError());
   hg_tile_feed feed = {};
-  const bool use_list = world > 1 || getenv("HG_PEER_FORCE_LIST");  // (the env: list walk on a single GPU, for measurements)
+  const bool use_list = world > 1;
   if (use_list) {
     if (!p->tiles_on_device) {
       HG_CUDA(cudaMemcpyAsync(c->d_scratch[HG_S_TILES], c->h_pinned[2], p->tiles.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
@@ -761,36 +748,21 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
     if (plan.n_units > 0) plan.unit_stamp[0] = 8;
     if (plan.n_units > 1) { plan.unit_stamp[1] = 9; plan.unit_stamp[plan.n_units - 1] = 11; }
   }
-  // Who pushes?  mode 1 (default): pusher warps inside the dist kernel - one kernel computes tiles and moves operands, no
-  // SM is given up.  mode 0 (HG_PEER_PUSH=concurrent): a kernel of its own per unit on the push stream, next to the dist
-  // kernel, which then leaves HG_PEER_RESERVED_TPCS TPCs free for it.  mode 2 (HG_PEER_PUSH=ahead, or a member without a
-  // tile to compute): the push kernels on the main stream, ahead of the dist kernel.
+  // Who pushes?  A member with tiles to compute: the pusher warps inside its dist kernel - one kernel computes tiles and
+  // moves operands, no SM is given up.  A member without a tile to compute: stand-alone push kernels on its stream, ahead
+  // of the dist launch (which then has nothing to do).
   const bool have_tiles = world > 1 && !p->tiles.empty() && (a.symmetric || a.n_ref_local > 0);
-  int mode = have_tiles ? 1 : 2;
-  if (const char *e = getenv("HG_PEER_PUSH")) {
-    if (have_tiles && !strcmp(e, "concurrent")) mode = 0;
-    if (!strcmp(e, "ahead")) mode = 2;
-  }
-  if (world > 1 && mode != 1) {
-    cudaStream_t ps = mode == 0 ? p->push_stream : c->stream;
-    if (mode == 0) {
-      HG_CUDA(cudaEventRecord(p->ev_operands, c->stream));
-      HG_CUDA(cudaStreamWaitEvent(ps, p->ev_operands, 0));
-      feed.reserve_tpcs = HG_PEER_RESERVED_TPCS;
-    }
-    const unsigned max_blocks = mode == 0 ? 2u * HG_PEER_RESERVED_TPCS * 8u : (unsigned)c->sm_count * 4u;
+  if (world > 1 && !have_tiles) {
     for (int u = 0; u < plan.n_units; ++u) {
       const int set = plan.unit_set[u];
       PushArgs pa;
       pa.n = plan.n[set];
       for (int k = 0; k < pa.n; ++k) { pa.r[k].off = plan.off[set][k]; pa.r[k].bytes = plan.bytes[set][k]; }
       const uint64_t flag_off = set == HG_PUSH_START_SET ? OFF_START + 4 * (uint64_t)rank : OFF_READY + 4 * (uint64_t)(rank * N_CHUNKS + set);
-      if ((rc = peer_push(p, pa, plan.unit_dest[u], flag_off, u, ps, max_blocks))) return rc;
+      if ((rc = peer_push(p, pa, plan.unit_dest[u], flag_off, u))) return rc;
     }
-    if (mode == 0) HG_CUDA(cudaEventRecord(p->ev_pushed, ps));
   }
-  const bool fused = mode == 1, concurrent = world > 1 && mode == 0;
-  const hg_push_plan *pp = fused ? &plan : nullptr;
+  const hg_push_plan *pp = have_tiles ? &plan : nullptr;
   PEER_PROF(p, 2);
   const hg_tile_feed *fp = use_list ? &feed : nullptr;
   if (use_path == 3) {
@@ -809,7 +781,6 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
   if (rc) return rc;
   HG_PROF(c, 5);
   PEER_PROF(p, 3);
-  if (concurrent) HG_CUDA(cudaStreamWaitEvent(c->stream, p->ev_pushed, 0));  // my window is not reused before my pushes have read it
   {  // my hits to the root: its gather list (NVLink), or the host buffer every member has mapped (my own PCIe link)
     hg_hit *dst = a.mapped_hits ? a.mapped_hits : (hg_hit *)(p->win[a.root] + lay.gather);
     unsigned long long *total = (unsigned long long *)(p->win[a.root] + OFF_TOTAL);
@@ -914,7 +885,7 @@ extern "C" int hg_dist_sharded_dev(hg_peer *p, const int16_t *d_ref_hv, const in
     // The first call runs directly, the second is captured, the following ones are one cudaGraphLaunch each.
     std::vector<uint8_t> key(sizeof(ShardCall) + 4 * sizeof(void *));
     memcpy(key.data(), &a, sizeof(ShardCall));
-    const void *extra[4] = {c->d_scratch[HG_S_REF_LIMBS], c->d_scratch[HG_S_NARROW_META], c->d_scratch[HG_S_TILES], (const void *)(uintptr_t)(path | hg_push_warps(0) << 8)};
+    const void *extra[4] = {c->d_scratch[HG_S_REF_LIMBS], c->d_scratch[HG_S_NARROW_META], c->d_scratch[HG_S_TILES], (const void *)(uintptr_t)path};
     memcpy(key.data() + sizeof(ShardCall), extra, sizeof(extra));
     const bool can_graph = !c->prof && !getenv("HG_PEER_NO_GRAPH");
     if (can_graph && p->graph && key == p->graph_key) {
@@ -927,7 +898,7 @@ extern "C" int hg_dist_sharded_dev(hg_peer *p, const int16_t *d_ref_hv, const in
     if (p->graph) { cudaGraphExecDestroy(p->graph); p->graph = nullptr; p->graph_key.clear(); }
     if ((rc = shard_reserve(p, a, path))) return rc;
     memcpy(key.data() + sizeof(ShardCall), extra, 0);  // (scratch pointers may have changed in shard_reserve: refresh below)
-    const void *extra2[4] = {c->d_scratch[HG_S_REF_LIMBS], c->d_scratch[HG_S_NARROW_META], c->d_scratch[HG_S_TILES], (const void *)(uintptr_t)(path | hg_push_warps(0) << 8)};
+    const void *extra2[4] = {c->d_scratch[HG_S_REF_LIMBS], c->d_scratch[HG_S_NARROW_META], c->d_scratch[HG_S_TILES], (const void *)(uintptr_t)path};
     memcpy(key.data() + sizeof(ShardCall), extra2, sizeof(extra2));
     if (can_graph && key == p->last_key && p->tiles_on_device) {
       HG_CUDA(cudaSetDevice(c->device));

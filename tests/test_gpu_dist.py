@@ -150,12 +150,12 @@ def _norms(oracle, hv):
     return np.array([oracle.hv_l2_norm_sq(v) for v in hv], np.int32)
 
 
-@pytest.mark.parametrize("nacc", [1, 2])
+@pytest.mark.parametrize("chunks", [1, 2])
 @pytest.mark.parametrize("symmetric", [False, True])
-def test_narrow_many_tiles_exact(ctx, hg, oracle, symmetric, nacc, monkeypatch):
-    """several tiles per CTA pair (stage ring across tiles, ragged edges): 256 x 256 tiles with the TMEM
-    accumulator double buffered (nacc 1) and 512 x 256 tiles with two accumulators (nacc 2)"""
-    monkeypatch.setenv("HG_NARROW_NACC", str(nacc))
+def test_narrow_many_tiles_exact(ctx, hg, oracle, symmetric, chunks, monkeypatch):
+    """several 256 x 256 tiles per CTA pair (stage ring across tiles, TMEM accumulator double buffered, ragged edges).
+    chunks = 2: the host entry streams the ref rows in two chunks, i.e. two launches into one hit list, the second
+    with a tile walk that starts at a row offset (symmetric: j0 > i0, so the walk skips the tiles below the diagonal)"""
     rng = np.random.default_rng(31)
     D = 512
     hv = _narrow_rows(rng, 700, D)
@@ -166,21 +166,28 @@ def test_narrow_many_tiles_exact(ctx, hg, oracle, symmetric, nacc, monkeypatch):
         r, rn, q, qn = hv, norm, hv, norm
     else:
         r, rn, q, qn = hv[:300], norm[:300], hv[100:], norm[100:]
+    if chunks == 2:  # chunk size: half of the ref rows, rounded up to a multiple of 256 as the library does
+        half = (r.shape[0] + 1) // 2
+        monkeypatch.setenv("HG_DIST_CHUNK_ROWS", str((half + 255) // 256 * 256))
     ani, dot = oracle.dist_all(r, rn, q, qn, symmetric=symmetric)
     hits = ctx.dist(r, rn, q, qn, ani_th=0.0, symmetric=symmetric, path=3, cap=ani.size + 16)
     assert ctx.dist_last_path == 3
+    assert "%d row chunk" % chunks in ctx.dist_last_reason, ctx.dist_last_reason
     idx = _as_pairs(hits, r.shape[0], q.shape[0], symmetric)
     assert np.array_equal(np.sort(idx), np.arange(ani.size))
     assert np.array_equal(hits["dot"], dot[idx])
     assert np.array_equal(hits["ani"].view(np.uint32), ani[idx].view(np.uint32))
 
 
-@pytest.mark.parametrize("nacc", [1, 2])
+@pytest.mark.parametrize("chunks", [1, 2])
 @pytest.mark.parametrize("ani_th", [0.0, 85.0])
-def test_narrow_outlier_corrections(ctx, hg, oracle, ani_th, nacc, monkeypatch):
+def test_narrow_outlier_corrections(ctx, hg, oracle, ani_th, chunks, monkeypatch):
     """rows with a few elements outside the s8 plane (range and parity outliers, both sides): the kernel
-    loosens their bound and corrects each candidate exactly"""
-    monkeypatch.setenv("HG_NARROW_NACC", str(nacc))
+    loosens their bound and corrects each candidate exactly.  chunks = 2: the host entry streams the symmetric run's
+    300 rows in two chunks of 256 rows, so the outlier entries of the second chunk's pre-pass follow those of the
+    first and a launch reads both (the ref x query run has 130 ref rows: one chunk either way)"""
+    if chunks == 2:
+        monkeypatch.setenv("HG_DIST_CHUNK_ROWS", "256")
     hv, norm = _sketches(oracle, 300, length=120_000, hv_d=1024, scaled=300)
     hv = hv.copy()
     rng = np.random.default_rng(7)
@@ -202,6 +209,7 @@ def test_narrow_outlier_corrections(ctx, hg, oracle, ani_th, nacc, monkeypatch):
         ani, dot = oracle.dist_all(r_, rn, q_, qn, symmetric=symmetric)
         hits = ctx.dist(r_, rn, q_, qn, ani_th=ani_th, symmetric=symmetric, path=0, cap=ani.size + 16)
         assert ctx.dist_last_path == 3 and "narrow" in ctx.dist_last_reason, ctx.dist_last_reason
+        assert "%d row chunk" % (chunks if symmetric else 1) in ctx.dist_last_reason, ctx.dist_last_reason
         idx = _as_pairs(hits, r_.shape[0], q_.shape[0], symmetric)
         want = np.nonzero(ani >= np.float32(ani_th))[0]
         assert np.array_equal(np.sort(idx), want)
@@ -230,12 +238,12 @@ def test_auto_path_narrow_for_sketches_and_two_limb_for_wide_rows(ctx, hg, oracl
     assert ei.value.code == hg.ffi.HG_E_UNSUPPORTED
 
 
-@pytest.mark.parametrize("nacc", [1, 2])
-def test_narrow_row_shard_offsets(ctx, hg, oracle, nacc, monkeypatch):
+@pytest.mark.parametrize("shards", [1, 2])
+def test_narrow_row_shard_offsets(ctx, hg, oracle, shards):
     """hg_dist_dev on a row shard of the query matrix (i0 > 0, symmetric filter on global indices) - the
-    multi-GPU dist step - through the single-plane path"""
+    multi-GPU dist step - through the single-plane path.  shards = 2: the same rows as two calls at row offsets
+    273 and 423, as two members of a GPU group would compute them"""
     import torch
-    monkeypatch.setenv("HG_NARROW_NACC", str(nacc))
     rng = np.random.default_rng(11)
     D, n = 2048, 600
     hv = _narrow_rows(rng, n, D)
@@ -249,11 +257,15 @@ def test_narrow_row_shard_offsets(ctx, hg, oracle, nacc, monkeypatch):
     d_hits = torch.empty(cap * 16, dtype=torch.uint8, device="cuda")
     d_cnt = torch.zeros(1, dtype=torch.int64, device="cuda")
     torch.cuda.synchronize()
-    ctx.dist_dev(d_hv.data_ptr() + i0 * D * 2, d_n.data_ptr() + i0 * 4, rows, i0, d_hv.data_ptr(), d_n.data_ptr(), n, 0, D, 21,
-                 0.0, True, 3, d_hits.data_ptr(), cap, d_cnt.data_ptr())
-    ctx.sync()
-    cnt = int(d_cnt.item())
-    hits = np.frombuffer(d_hits.cpu().numpy().tobytes(), dtype=hg.ffi.HIT_DTYPE)[:cnt]
+    parts = []
+    bounds = [i0 + rows * s // shards for s in range(shards + 1)]
+    for a, b in zip(bounds[:-1], bounds[1:]):  # every call resets the hit counter: read its hits before the next one
+        ctx.dist_dev(d_hv.data_ptr() + a * D * 2, d_n.data_ptr() + a * 4, b - a, a, d_hv.data_ptr(), d_n.data_ptr(), n, 0, D, 21,
+                     0.0, True, 3, d_hits.data_ptr(), cap, d_cnt.data_ptr())
+        ctx.sync()
+        cnt = int(d_cnt.item())
+        parts.append(np.frombuffer(d_hits.cpu().numpy().tobytes(), dtype=hg.ffi.HIT_DTYPE)[:cnt])
+    hits = np.concatenate(parts)
     idx = _as_pairs(hits, n, n, True)
     ii, jj = np.meshgrid(np.arange(i0, i0 + rows), np.arange(n), indexing="ij")
     keep = jj > ii
@@ -273,6 +285,29 @@ def test_narrow_short_and_mid_k(ctx, hg, oracle, hv_d):
     ani, dot = oracle.dist_all(hv, norm, hv, norm, symmetric=True)
     hits = ctx.dist(hv, norm, hv, norm, ani_th=0.0, symmetric=True, path=3, cap=ani.size + 16)
     idx = _as_pairs(hits, 330, 330, True)
+    assert np.array_equal(np.sort(idx), np.arange(ani.size))
+    assert np.array_equal(hits["dot"], dot[idx])
+    assert np.array_equal(hits["ani"].view(np.uint32), ani[idx].view(np.uint32))
+
+
+@pytest.mark.parametrize("hv_d", [256, 768, 1280])
+@pytest.mark.parametrize("symmetric", [False, True])
+def test_two_limb_k_not_a_multiple_of_512(ctx, hg, oracle, hv_d, symmetric):
+    """two-limb kernel at hv_d % 512 != 0: its K loop runs whole trips of the 4-stage ring (512 columns) and the
+    tensor maps fill the columns past hv_d with zeros; several 256 x 128 tiles with ragged edges, both limbs in use"""
+    rng = np.random.default_rng(hv_d + symmetric)
+    hv = _narrow_rows(rng, 420, hv_d, spread=1000)  # |hv| <= 2001: the high limb is not zero
+    hv[9] = hv[333]
+    hv[200] = hv[201]
+    norm = _norms(oracle, hv)
+    if symmetric:
+        r, rn, q, qn = hv, norm, hv, norm
+    else:
+        r, rn, q, qn = hv[:300], norm[:300], hv[90:], norm[90:]
+    ani, dot = oracle.dist_all(r, rn, q, qn, symmetric=symmetric)
+    hits = ctx.dist(r, rn, q, qn, ani_th=0.0, symmetric=symmetric, path=2, cap=ani.size + 16)
+    assert ctx.dist_last_path == 2, ctx.dist_last_reason
+    idx = _as_pairs(hits, r.shape[0], q.shape[0], symmetric)
     assert np.array_equal(np.sort(idx), np.arange(ani.size))
     assert np.array_equal(hits["dot"], dot[idx])
     assert np.array_equal(hits["ani"].view(np.uint32), ani[idx].view(np.uint32))

@@ -45,22 +45,23 @@ def _dev(t):
     return torch.from_numpy(np.ascontiguousarray(t)).cuda()
 
 
-@pytest.mark.parametrize("path", [0, 2, 3])
+@pytest.mark.parametrize("path,hv_d", [(0, 1024), (2, 1024), (3, 1024), (2, 768)], ids=["0", "2", "3", "2-768"])
 @pytest.mark.parametrize("symmetric", [True, False])
-def test_world1_sharded_equals_oracle(ctx, hg, oracle, path, symmetric):
-    """One member: the window path (operands prepared inside the window, tile walk 0/1) must equal the plain path."""
-    hv, norm, _, _ = _sketch_sets(ctx, 700, 1024, 800, 1500)
+def test_world1_sharded_equals_oracle(ctx, hg, oracle, path, hv_d, symmetric):
+    """One member: the window path (operands prepared inside the window, tile walk 0/1) must equal the plain path.
+    hv_d = 768: the two-limb kernel's K loop runs past hv_d into the tensor maps' zero fill."""
+    hv, norm, _, _ = _sketch_sets(ctx, 700, hv_d, 800, 1500)
     cap = 700 * 700
-    peer = hg.Peer(ctx, 0, 1, hg.ffi.peer_window_need(700, 1024, cap))
+    peer = hg.Peer(ctx, 0, 1, hg.ffi.peer_window_need(700, hv_d, cap))
     try:
         d_hv, d_n = _dev(hv), _dev(norm)
         if symmetric:
-            peer.dist_sharded_dev(None, None, 0, 0, d_hv.data_ptr(), d_n.data_ptr(), [0, 700], 1024, 21, 80.0, True, path, 0, cap)
+            peer.dist_sharded_dev(None, None, 0, 0, d_hv.data_ptr(), d_n.data_ptr(), [0, 700], hv_d, 21, 80.0, True, path, 0, cap)
             hits, _ = peer.dist_sharded_hits(cap)
             _check_hits(oracle, hits, hv, norm, hv, norm, True, 80.0)
         else:
             peer.dist_sharded_dev(d_hv[:300].data_ptr(), d_n[:300].data_ptr(), 300, 1000, d_hv.data_ptr(), d_n.data_ptr(), [0, 700],
-                                  1024, 21, 0.0, False, path, 0, cap)
+                                  hv_d, 21, 0.0, False, path, 0, cap)
             hits, _ = peer.dist_sharded_hits(cap)
             _check_hits(oracle, hits, hv[:300], norm[:300], hv, norm, False, 0.0, i0=1000)
         assert ctx.dist_last_path == (path or 3)
