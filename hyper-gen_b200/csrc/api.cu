@@ -198,6 +198,18 @@ int hg_pinned(hg_ctx *c, int slot, size_t bytes, void **out) {
   return HG_OK;
 }
 
+// the copy stream of the host-pointer entries (H2D next to the compute stream) and its events, created on first use
+static int ensure_copy_stream(hg_ctx *c) {
+  if (c->copy_stream) return HG_OK;
+  HG_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; i++) {
+    HG_CUDA(cudaEventCreateWithFlags(&c->ev_copied[i], cudaEventDisableTiming));
+    HG_CUDA(cudaEventCreateWithFlags(&c->ev_done[i], cudaEventDisableTiming));
+  }
+  for (int i = 0; i < 10; i++) HG_CUDA(cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming));
+  return HG_OK;
+}
+
 // ---------------------------------------------------------------------------------------
 // sketch
 // ---------------------------------------------------------------------------------------
@@ -444,13 +456,7 @@ extern "C" int hg_sketch_batch(hg_ctx *c, const uint8_t *seq, const uint64_t *se
   uint8_t *d_bits = (uint8_t *)d_small + (size_t)n * 8;
   int32_t *d_norm = (int32_t *)d_small;
   uint32_t *d_nh = (uint32_t *)d_small + n;
-  if (!c->copy_stream) {
-    HG_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; i++) {
-      HG_CUDA(cudaEventCreateWithFlags(&c->ev_copied[i], cudaEventDisableTiming));
-      HG_CUDA(cudaEventCreateWithFlags(&c->ev_done[i], cudaEventDisableTiming));
-    }
-  }
+  if ((rc = ensure_copy_stream(c))) return rc;
   c->ev_used = 0;
   HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
   HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * n, c->stream));
@@ -699,13 +705,7 @@ extern "C" int hg_sketch_fasta_batch(hg_ctx *c, const uint8_t *raw, const uint64
   uint64_t *dm_off = (uint64_t *)d_meta, *dm_blk = dm_off + (max_m + 1), *dm_out = dm_blk + (max_m + 1);
   uint8_t *dm_sums = (uint8_t *)(dm_out + max_blk);
   uint8_t *dm_carry = dm_sums + max_blk * 16;
-  if (!c->copy_stream) {
-    HG_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; i++) {
-      HG_CUDA(cudaEventCreateWithFlags(&c->ev_copied[i], cudaEventDisableTiming));
-      HG_CUDA(cudaEventCreateWithFlags(&c->ev_done[i], cudaEventDisableTiming));
-    }
-  }
+  if ((rc = ensure_copy_stream(c))) return rc;
   c->ev_used = 0;
   HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
   HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * n, c->stream));
@@ -792,109 +792,269 @@ extern "C" int hg_unpack(hg_ctx *c, const uint8_t *packed, uint64_t row_stride, 
 // ---------------------------------------------------------------------------------------
 // dist
 // ---------------------------------------------------------------------------------------
-static const int32_t HG_TC_MAX_ABS = 8127;  // |x| <= 8127 splits into two s8 limbs (x = 128 h + l)
+void hg_dist_record(hg_ctx *c, int path, const char *fmt, ...) {
+  c->dist_path = path;
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(c->dist_reason, sizeof(c->dist_reason), fmt, ap);
+  va_end(ap);
+}
 
-// allow_narrow = false: the single-plane path has already been tried (and declined) on these matrices, absmax is
-// max |hv| from its pre-pass
-static int dist_dev_impl(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t i0,
-                         const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry, uint32_t j0,
-                         uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric, int path, hg_hit *d_hits,
-                         uint64_t cap, unsigned long long *d_n_hits, bool allow_narrow, int32_t absmax, bool defer_forced = false) {
-  if (!c || !d_n_hits) { hg_set_error("hg_dist_dev: NULL argument"); return HG_E_INVALID; }
-  c->pending_stats[0] = c->pending_stats[1] = nullptr;
-  if ((n_ref && (!d_ref || !d_ref_norm)) || (n_qry && (!d_qry || !d_qry_norm)) || (cap && !d_hits)) {
-    hg_set_error("hg_dist_dev: NULL argument"); return HG_E_INVALID;
+// one dist call: ref rows [i0, i0 + n_ref) against query rows [j0, j0 + n_qry), both matrices in HBM (or arriving there)
+struct DistOp {
+  const int16_t *ref;
+  const int32_t *ref_norm;
+  uint32_t n_ref, i0;
+  const int16_t *qry;
+  const int32_t *qry_norm;
+  uint32_t n_qry, j0;
+  uint32_t hv_d, ksize;
+  float ani_th;
+  int symmetric;
+  hg_hit *hits;
+  uint64_t cap;
+  unsigned long long *n_hits;
+};
+
+// The kernel a dist call tries first, chosen before anything runs.
+struct DistChoice {
+  int kernel;     // HG_PATH_SIMT, HG_PATH_TWO_LIMB or HG_PATH_NARROW
+  bool fallback;  // the single plane may decline the rows: then two-limb if max |hv| fits the limb split, else SIMT
+  char why[96];   // why this kernel (the reason of a run that had no facts to report)
+};
+
+// What a run found out on the way (the reason reports it).
+struct DistFacts {
+  int32_t absmax = -1;    // max |hv| once a pre-pass or a scan has produced it
+  uint64_t outliers = 0;  // outlier elements the single-plane run corrects per candidate
+  uint32_t chunks = 0;    // row chunks streamed from the host (0: the rows were in HBM)
+};
+
+// path: as requested (0 auto).  shape_ok: hg_tensor_shape_ok.  bits: what the caller knows about the rows - 0 for i16
+// rows, the largest hv_quant_bits for packed rows.  b-bit two's-complement values are below 2^(b-1): above 10 bits no
+// row fits the single s8 plane (x = 2a + s spans 510), and up to 13 bits every element fits the int8 limb split.
+static int dist_choose(int path, uint32_t n_ref, uint32_t n_qry, bool shape_ok, uint32_t bits, DistChoice *ch) {
+  ch->kernel = path;
+  ch->fallback = false;
+  snprintf(ch->why, sizeof(ch->why), "forced by caller");
+  if (path != HG_PATH_AUTO) return path == HG_PATH_SIMT || shape_ok ? HG_OK : HG_E_UNSUPPORTED;  // (error set by the predicate)
+  if ((uint64_t)n_ref * n_qry < 128ull * 128ull) {
+    ch->kernel = HG_PATH_SIMT;
+    snprintf(ch->why, sizeof(ch->why), "%u x %u pairs do not fill one 128x128 tensor tile", n_ref, n_qry);
+  } else if (!shape_ok) {
+    ch->kernel = HG_PATH_SIMT;
+    snprintf(ch->why, sizeof(ch->why), "the tensor kernels declined this shape (hv_d <= 32768, 16-byte aligned matrices)");
+  } else if (bits > 10 && bits <= 13) {
+    ch->kernel = HG_PATH_TWO_LIMB;
+    snprintf(ch->why, sizeof(ch->why), "hv_quant_bits <= %u fits two s8 limbs; tcgen05 kind::i8", bits);
+  } else {
+    ch->kernel = HG_PATH_NARROW;  // its pre-pass (one read of both matrices) tells whether the rows fit one s8 plane
+    ch->fallback = true;
   }
-  if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("hg_dist_dev: hv_d %u must be a multiple of 256", hv_d); return HG_E_INVALID; }
-  if (path < 0 || path > 3) { hg_set_error("hg_dist_dev: path %d", path); return HG_E_INVALID; }
-  HG_CUDA(cudaSetDevice(c->device));
-  HG_CUDA(cudaMemsetAsync(d_n_hits, 0, sizeof(unsigned long long), c->stream));
-  if (n_ref == 0 || n_qry == 0) return HG_OK;
-  c->ev_used &= ~(3 << 4);
+  return HG_OK;
+}
+
+// dist_path and dist_reason of a finished run; `ran` is the kernel whose hits the call returns
+static void dist_note(hg_ctx *c, const DistChoice &ch, int ran, const DistFacts &f, bool deferred) {
+  static const char *const name[4] = {"", "SIMT", "tensor", "tensor-narrow"};
+  char chunks[64] = "";
+  if (f.chunks) snprintf(chunks, sizeof(chunks), "; %u row chunk(s) overlapping their H2D", f.chunks);
+  if (ran != ch.kernel && ran == HG_PATH_TWO_LIMB)
+    hg_dist_record(c, ran, "tensor: max |hv| = %d fits two s8 limbs, tcgen05 kind::i8 (one s8 plane declined: rows are not narrow)",
+                   f.absmax);
+  else if (ran != ch.kernel)
+    hg_dist_record(c, ran, "SIMT: max |hv| = %d exceeds the 13-bit budget (%d) of the int8 limb split (one s8 plane declined)",
+                   f.absmax, HG_LIMB_MAX_ABS);
+  else if (ran == HG_PATH_NARROW && !deferred)
+    hg_dist_record(c, ran,
+                   "tensor-narrow%s: rows fit one s8 plane as x = 2a + s (max |hv| = %d, %llu outlier elements corrected per "
+                   "candidate); tcgen05 kind::i8, one MMA per K step%s",
+                   ch.fallback ? "" : " (forced)", f.absmax, (unsigned long long)f.outliers, chunks);
+  else
+    hg_dist_record(c, ran, "%s: %s%s%s", name[ran], ch.why, deferred ? " (verdict deferred to hg_dist_status)" : "", chunks);
+}
+
+// ---- host matrices streamed in row chunks: H2D of chunk c + 1 under unpack / pre-pass / dist kernel of chunk c ----
+struct HostRows {
+  const uint8_t *base;  // first row on the host
+  uint64_t stride;      // bytes between host rows
+  uint64_t width;       // bytes of a row that travel (int16 rows: 2 hv_d; packed rows: max hv_quant_bits * hv_d / 8)
+  const uint8_t *bits;  // packed rows: hv_quant_bits per row (host); int16 rows: NULL
+  const int32_t *norm;  // host
+  uint32_t n;
+  uint8_t *d_stage;     // packed rows: where they land (width apart); int16 rows: the matrix itself
+  uint8_t *d_bits;      // packed rows
+  int16_t *d_hv;
+  int32_t *d_norm;
+};
+
+static uint32_t dist_chunk_rows(uint32_t n) {
+  uint32_t rows = 0;
+  if (const char *e = getenv("HG_DIST_CHUNK_ROWS")) rows = (uint32_t)std::max(0, atoi(e));
+  if (rows == 0) {
+    const uint32_t want = std::min<uint32_t>(8, std::max<uint32_t>(1, n / 1280));  // measured on config 3: 6-8 chunks beat 2-4
+    rows = (n + want - 1) / want;
+  }
+  rows = std::max<uint32_t>(256, (rows + 255) & ~255u);
+  if ((uint64_t)rows * 8 < n) rows = (uint32_t)((((uint64_t)n + 7) / 8 + 255) & ~255ull);  // at most 8 chunks
+  return rows;
+}
+
+// The tensor dist (two-limb or single-plane kernel): the query matrix is prepared (limb split or pre-pass), then the
+// ref rows chunk by chunk, each chunk launched against the query rows.  Rows already in HBM are one chunk and no
+// copies.  With hr / hq the rows arrive from the host: all copies are queued first on the copy stream, so that chunk
+// k + 1 crosses PCIe under the kernels of chunk k.  The ref block may lie inside the query matrix (all-vs-all on one
+// matrix, or a row shard of it as hg_dist_dev gets it): then it shares the query's preparation.  When it IS the query
+// matrix, chunk k is compared against the rows up to its own end (j in the chunk, i < j): the later rows are still
+// on their way.  Single plane: HG_E_UNSUPPORTED, with max |hv| in f, if the rows turn out not to be narrow - unless
+// `defer`: then nothing waits and hg_dist_status reads the verdict.
+static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, HostRows *hq, bool defer, DistFacts *f) {
   int rc;
-
-  // ---- choose: 3 = single-plane tensor kernel, 2 = two-limb tensor kernel, 1 = SIMT ----
-  int use = path;  // absmax: max |hv| once some scan has produced it (-1: not yet)
-  if (path == 0 && (uint64_t)n_ref * n_qry < 128ull * 128ull) {
-    use = 1;
-    snprintf(c->dist_reason, sizeof(c->dist_reason), "SIMT: %u x %u pairs do not fill one 128x128 tensor tile", n_ref, n_qry);
-  } else if (!allow_narrow && (path == 0 || path == 3)) {
-    if (path == 3) { hg_set_error("rows are not narrow (single-plane path declined)"); return HG_E_UNSUPPORTED; }
-    snprintf(c->dist_reason, sizeof(c->dist_reason), "rows are not narrow");
-    hg_set_error("rows are not narrow");
-    use = 0;
-  } else if (path == 0 || path == 3) {
-    // the narrow path's own pre-pass (one read of both matrices) tells whether the rows fit one s8 plane
-    uint64_t outliers = 0;
-    rc = hg_launch_dist_narrow(c, d_ref, d_ref_norm, n_ref, i0, d_qry, d_qry_norm, n_qry, j0, hv_d, ksize, ani_th, symmetric,
-                               d_hits, cap, d_n_hits, &absmax, &outliers, path == 3 && defer_forced);
-    if (rc == HG_OK) {
-      c->dist_path = 3;
-      if (path == 3)
-        snprintf(c->dist_reason, sizeof(c->dist_reason), "tensor-narrow: forced by caller%s", defer_forced ? " (verdict deferred to hg_dist_status)" : "");
-      else
-        snprintf(c->dist_reason, sizeof(c->dist_reason),
-                 "tensor-narrow: rows fit one s8 plane as x = 2a + s (max |hv| = %d, %llu outlier elements corrected per candidate); "
-                 "tcgen05 kind::i8, one MMA per K step", absmax, (unsigned long long)outliers);
+  const uint32_t hv_d = op.hv_d;
+  const bool in_q = op.ref >= op.qry && op.ref + (uint64_t)op.n_ref * hv_d <= op.qry + (uint64_t)op.n_qry * hv_d &&
+                    (op.ref - op.qry) % hv_d == 0;
+  const uint32_t r_off = in_q ? (uint32_t)((op.ref - op.qry) / hv_d) : 0u;
+  const bool one = in_q && r_off == 0 && op.n_ref == op.n_qry;
+  if (hr && (rc = ensure_copy_stream(c))) return rc;
+  hg_narrow_mat Qm, Rm;
+  hg_tc_mat Qt, Rt;
+  if (narrow) {
+    const size_t mq = hg_narrow_meta_bytes(op.n_qry), mr = in_q ? 0 : hg_narrow_meta_bytes(op.n_ref);
+    void *meta;
+    if ((rc = hg_scratch(c, HG_S_NARROW_META, mq + mr, &meta))) return rc;
+    if ((rc = hg_narrow_setup(c, op.qry, op.n_qry, hv_d, HG_S_QRY_LIMBS, meta, &Qm))) return rc;
+    if (!in_q && (rc = hg_narrow_setup(c, op.ref, op.n_ref, hv_d, HG_S_REF_LIMBS, (uint8_t *)meta + mq, &Rm))) return rc;
+  } else {
+    if ((rc = hg_tc_setup(c, op.qry, op.n_qry, hv_d, HG_S_QRY_LIMBS, &Qt))) return rc;
+    if (!in_q && (rc = hg_tc_setup(c, op.ref, op.n_ref, hv_d, HG_S_REF_LIMBS, &Rt))) return rc;
+  }
+  const hg_narrow_mat *Rn = in_q ? &Qm : &Rm;
+  const hg_tc_mat *Rl = in_q ? &Qt : &Rt;
+  std::vector<std::pair<uint32_t, uint32_t>> chunks;
+  const uint32_t step = hr ? dist_chunk_rows(op.n_ref) : op.n_ref;
+  for (uint32_t a = 0; a < op.n_ref; a += step) chunks.push_back({a, std::min(step, op.n_ref - a)});
+  if (hr) {
+    auto small = [&](HostRows &S) -> int {
+      HG_CUDA(cudaMemcpyAsync(S.d_norm, S.norm, (size_t)S.n * 4, cudaMemcpyHostToDevice, c->stream));
+      if (S.bits) HG_CUDA(cudaMemcpyAsync(S.d_bits, S.bits, S.n, cudaMemcpyHostToDevice, c->stream));
       return HG_OK;
-    }
-    if (rc != HG_E_UNSUPPORTED || path == 3) return rc;
-    use = 0;  // declined: two-limb tensor kernel if every |hv| fits 13 bits, else SIMT
-  }
-  if (use == 0) {
-    char why[96];
-    snprintf(why, sizeof(why), "%s", hg_last_error());
-    if (absmax < 0) {  // the narrow path declined before its scan: one read of both matrices and one 4-byte D2H each
-      void *d_max;
-      if ((rc = hg_scratch(c, HG_S_MISC, 256, &d_max))) return rc;
-      int32_t m1 = 0, m2 = 0;
-      if ((rc = hg_launch_absmax(c, d_ref, (uint64_t)n_ref * hv_d, (int32_t *)d_max))) return rc;
-      HG_CUDA(cudaMemcpyAsync(&m1, d_max, 4, cudaMemcpyDeviceToHost, c->stream));
-      HG_CUDA(cudaStreamSynchronize(c->stream));
-      if (d_qry != d_ref) {
-        if ((rc = hg_launch_absmax(c, d_qry, (uint64_t)n_qry * hv_d, (int32_t *)d_max))) return rc;
-        HG_CUDA(cudaMemcpyAsync(&m2, d_max, 4, cudaMemcpyDeviceToHost, c->stream));
-        HG_CUDA(cudaStreamSynchronize(c->stream));
-      }
-      absmax = m1 > m2 ? m1 : m2;
-    }
-    if (absmax > HG_TC_MAX_ABS) {
-      use = 1;
-      snprintf(c->dist_reason, sizeof(c->dist_reason),
-               "SIMT: max |hv| = %d exceeds the 13-bit budget (%d) of the int8 limb split", absmax, HG_TC_MAX_ABS);
-    } else {
-      use = 2;
-      snprintf(c->dist_reason, sizeof(c->dist_reason),
-               "tensor: max |hv| = %d fits two s8 limbs, tcgen05 kind::i8 (one s8 plane declined: %.80s)", absmax, why);
-    }
-  } else if (path != 0) {
-    snprintf(c->dist_reason, sizeof(c->dist_reason), "%s: forced by caller", use == 1 ? "SIMT" : "tensor");
-  }
-  c->dist_path = use;
-  int rc2 = HG_OK;
-  if (use == 2) {
-    rc2 = hg_launch_dist_tc(c, d_ref, d_ref_norm, n_ref, i0, d_qry, d_qry_norm, n_qry, j0, hv_d, ksize, ani_th,
-                            symmetric, d_hits, cap, d_n_hits);
-    if (rc2 == HG_E_UNSUPPORTED && (path == 0 || c->tc_is_hint)) {  // shape outside the tensor kernel's tiling: exact SIMT path
-      use = c->dist_path = 1;
-      snprintf(c->dist_reason, sizeof(c->dist_reason), "SIMT: tensor kernel declined this shape (%s)", hg_last_error());
-    }
-  }
-  if (use != 2) {
+    };
+    auto stage = [&](HostRows &S, uint32_t a, uint32_t rows, cudaEvent_t ev) -> int {
+      HG_CUDA(cudaMemcpy2DAsync(S.d_stage + (size_t)a * S.width, S.width, S.base + (size_t)a * S.stride, S.stride, S.width, rows,
+                                cudaMemcpyHostToDevice, c->copy_stream));
+      HG_CUDA(cudaEventRecord(ev, c->copy_stream));
+      return HG_OK;
+    };
+    if ((rc = small(*hr))) return rc;
+    if (!in_q && (rc = small(*hq))) return rc;
+    // the copy stream starts once the compute stream has got here (the buffers may still be in use by an earlier call)
+    HG_CUDA(cudaEventRecord(c->ev_chunk[0], c->stream));
+    HG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_chunk[0], 0));
+    if (!in_q && (rc = stage(*hq, 0, op.n_qry, c->ev_chunk[1]))) return rc;
+    for (size_t k = 0; k < chunks.size(); k++)
+      if ((rc = stage(*hr, chunks[k].first, chunks[k].second, c->ev_chunk[2 + k]))) return rc;
+  } else {
     HG_PROF(c, 4);
-    rc2 = hg_launch_dist_simt(c, d_ref, d_ref_norm, n_ref, i0, d_qry, d_qry_norm, n_qry, j0, hv_d, ksize, ani_th,
-                              symmetric, d_hits, cap, d_n_hits);
-    HG_PROF(c, 5);
   }
-  return rc2;
+  // rows [a, a + rows) of one matrix: once they have arrived (and packed rows are unpacked), split or pre-passed
+  auto prep = [&](HostRows *S, const hg_narrow_mat *M, const hg_tc_mat *T, uint32_t a, uint32_t rows, cudaEvent_t ev) -> int {
+    if (S) {
+      HG_CUDA(cudaStreamWaitEvent(c->stream, ev, 0));
+      int r2 = S->bits ? hg_launch_unpack(c, S->d_stage + (size_t)a * S->width, S->width, S->d_bits + a, rows, hv_d, S->d_hv + (size_t)a * hv_d)
+                       : HG_OK;
+      if (r2) return r2;
+    }
+    return narrow ? hg_narrow_prep_rows(c, M, a, rows) : hg_tc_split_rows(c, T, a, rows);
+  };
+  auto launch = [&](uint32_t r0, uint32_t nr, uint32_t i0, const int32_t *rn, uint32_t q0, uint32_t nq, uint32_t j0, const int32_t *qn) {
+    return narrow ? hg_narrow_launch(c, Rn, r0, nr, i0, rn, &Qm, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits)
+                  : hg_tc_launch(c, Rl, r0, nr, i0, rn, &Qt, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits);
+  };
+  if (!one && (rc = prep(hq, &Qm, &Qt, 0, op.n_qry, c->ev_chunk[1]))) return rc;
+  for (size_t k = 0; k < chunks.size(); k++) {
+    const uint32_t a = chunks[k].first, rows = chunks[k].second;
+    if ((!in_q || one) && (rc = prep(hr, Rn, Rl, a, rows, c->ev_chunk[2 + k]))) return rc;
+    rc = one ? launch(0, a + rows, op.i0, op.ref_norm, a, rows, op.j0 + a, op.qry_norm + a)
+             : launch(r_off + a, rows, op.i0 + a, op.ref_norm + a, 0, op.n_qry, op.j0, op.qry_norm);
+    if (rc) return rc;
+  }
+  if (!hr) HG_PROF(c, 5);
+  f->chunks = hr ? (uint32_t)chunks.size() : 0;
+  if (!narrow) return HG_OK;
+  if (defer) {  // the kernel itself honours the pre-pass's verdict (it does nothing when the rows are not narrow)
+    c->pending_stats[0] = Qm.stats_all;
+    c->pending_nsets[0] = Qm.n_sets;
+    c->pending_stats[1] = in_q ? nullptr : Rm.stats_all;
+    c->pending_nsets[1] = in_q ? 0 : Rm.n_sets;
+    return HG_OK;
+  }
+  return hg_narrow_verdict(c, &Qm, in_q ? nullptr : &Rm, &f->absmax, &f->outliers);
+}
+
+// max |hv| over both matrices when no pre-pass has produced it: one read of each and one 4-byte D2H each
+static int dist_absmax(hg_ctx *c, const DistOp &op, int32_t *absmax) {
+  void *d_max;
+  int rc;
+  if ((rc = hg_scratch(c, HG_S_MISC, 256, &d_max))) return rc;
+  int32_t m[2] = {0, 0};
+  for (int k = 0; k < (op.qry == op.ref ? 1 : 2); ++k) {
+    if ((rc = hg_launch_absmax(c, k ? op.qry : op.ref, (uint64_t)(k ? op.n_qry : op.n_ref) * op.hv_d, (int32_t *)d_max))) return rc;
+    HG_CUDA(cudaMemcpyAsync(&m[k], d_max, 4, cudaMemcpyDeviceToHost, c->stream));
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+  }
+  *absmax = std::max(m[0], m[1]);
+  return HG_OK;
+}
+
+// Runs the chosen kernel (streaming the rows from the host when hr / hq are given).  When the single plane declines
+// and the choice allows it, the kernel max |hv| calls for runs on the same rows, complete in HBM by then.
+static int dist_run(hg_ctx *c, const DistOp &op, const DistChoice &ch, HostRows *hr, HostRows *hq, bool defer) {
+  DistFacts f;
+  int ran = ch.kernel, rc;
+  if (ran != HG_PATH_SIMT) {
+    rc = dist_tensor(c, op, ran == HG_PATH_NARROW, hr, hq, defer, &f);
+    if (rc == HG_E_UNSUPPORTED && ran == HG_PATH_NARROW && ch.fallback) {
+      if (f.absmax < 0 && (rc = dist_absmax(c, op, &f.absmax))) return rc;  // declined before its pre-pass
+      ran = f.absmax > HG_LIMB_MAX_ABS ? HG_PATH_SIMT : HG_PATH_TWO_LIMB;
+      HG_CUDA(cudaMemsetAsync(op.n_hits, 0, sizeof(unsigned long long), c->stream));  // what the declined chunks appended
+      rc = ran == HG_PATH_TWO_LIMB ? dist_tensor(c, op, false, nullptr, nullptr, false, &f) : HG_OK;
+    } else if (rc == HG_E_UNSUPPORTED && ran == HG_PATH_NARROW && f.absmax >= 0) {
+      hg_set_error("rows are not narrow (max |hv| = %d): more outlier entries than the single-plane path's budget", f.absmax);
+    }
+    if (rc) return rc;
+  }
+  if (ran == HG_PATH_SIMT) {
+    HG_PROF(c, 4);
+    rc = hg_launch_dist_simt(c, op.ref, op.ref_norm, op.n_ref, op.i0, op.qry, op.qry_norm, op.n_qry, op.j0, op.hv_d, op.ksize, op.ani_th,
+                             op.symmetric, op.hits, op.cap, op.n_hits);
+    HG_PROF(c, 5);
+    if (rc) return rc;
+  }
+  dist_note(c, ch, ran, f, defer);
+  return HG_OK;
 }
 
 extern "C" int hg_dist_dev(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t i0,
                            const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry, uint32_t j0,
                            uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric, int path, hg_hit *d_hits,
                            uint64_t cap, unsigned long long *d_n_hits) {
-  return dist_dev_impl(c, d_ref, d_ref_norm, n_ref, i0, d_qry, d_qry_norm, n_qry, j0, hv_d, ksize, ani_th, symmetric, path, d_hits,
-                       cap, d_n_hits, true, -1, true);
+  if (!c || !d_n_hits) { hg_set_error("hg_dist_dev: NULL argument"); return HG_E_INVALID; }
+  c->pending_stats[0] = c->pending_stats[1] = nullptr;
+  if ((n_ref && (!d_ref || !d_ref_norm)) || (n_qry && (!d_qry || !d_qry_norm)) || (cap && !d_hits)) {
+    hg_set_error("hg_dist_dev: NULL argument"); return HG_E_INVALID;
+  }
+  if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("hg_dist_dev: hv_d %u must be a multiple of 256", hv_d); return HG_E_INVALID; }
+  if (path < HG_PATH_AUTO || path > HG_PATH_NARROW) { hg_set_error("hg_dist_dev: path %d", path); return HG_E_INVALID; }
+  HG_CUDA(cudaSetDevice(c->device));
+  HG_CUDA(cudaMemsetAsync(d_n_hits, 0, sizeof(unsigned long long), c->stream));
+  if (n_ref == 0 || n_qry == 0) return HG_OK;
+  c->ev_used &= ~(3 << 4);
+  int rc;
+  DistChoice ch;
+  if ((rc = dist_choose(path, n_ref, n_qry, hg_tensor_shape_ok(hv_d, d_ref, d_qry) == HG_OK, 0, &ch))) return rc;
+  const DistOp op = {d_ref, d_ref_norm, n_ref, i0, d_qry, d_qry_norm, n_qry, j0, hv_d, ksize, ani_th, symmetric, d_hits, cap, d_n_hits};
+  // a caller that forces the single plane on device rows does not wait for its verdict here
+  return dist_run(c, op, ch, nullptr, nullptr, path == HG_PATH_NARROW);
 }
 
 // After hg_dist_dev(path = 3): the pre-pass verdict that call did not wait for.
@@ -943,196 +1103,40 @@ static int dist_tail(hg_ctx *c, void *d_hits, void *d_cnt, hg_hit *hits, uint64_
   return HG_OK;
 }
 
-static int dist_out_buffers(hg_ctx *c, uint64_t cap, void **d_hits, void **d_cnt) {
-  int rc;
-  if ((rc = hg_scratch(c, HG_S_PACKED, cap * sizeof(hg_hit) + 256, d_hits))) return rc;
-  return hg_scratch(c, HG_S_COUNTS, 256, d_cnt);
-}
-
-// matrices already on the device: dist kernel (auto / forced path) + tail
-static int dist_finish(hg_ctx *c, const int16_t *d_ref, const int32_t *d_rn, uint32_t n_ref, const int16_t *d_qry,
-                       const int32_t *d_qn, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric, int path,
-                       hg_hit *hits, uint64_t cap, uint64_t *n_hits, bool sorted, uint32_t *ani_milli, bool allow_narrow = true,
-                       int32_t absmax = -1) {
-  int rc;
-  void *d_hits, *d_cnt;
-  if ((rc = dist_out_buffers(c, cap, &d_hits, &d_cnt))) return rc;
-  rc = dist_dev_impl(c, d_ref, d_rn, n_ref, 0, d_qry, d_qn, n_qry, 0, hv_d, ksize, ani_th, symmetric, path, (hg_hit *)d_hits, cap,
-                     (unsigned long long *)d_cnt, allow_narrow, absmax);
-  if (rc) return rc;
-  return dist_tail(c, d_hits, d_cnt, hits, cap, n_hits, sorted, ani_milli);
-}
-
-// ---- host matrices streamed in row chunks: H2D of chunk c + 1 under unpack / pre-pass / dist kernel of chunk c ----
-struct HostRows {
-  const uint8_t *base;  // first row on the host
-  uint64_t stride;      // bytes between host rows
-  uint64_t width;       // bytes of a row that travel (int16 rows: 2 hv_d; packed rows: max hv_quant_bits * hv_d / 8)
-  const uint8_t *bits;  // packed rows: hv_quant_bits per row (host); int16 rows: NULL
-  const int32_t *norm;  // host
-  uint32_t n;
-  uint8_t *d_stage;     // packed rows: where they land (width apart); int16 rows: the matrix itself
-  uint8_t *d_bits;      // packed rows
-  int16_t *d_hv;
-  int32_t *d_norm;
-};
-
-static bool dist_stream_eligible(int path, bool same, int symmetric, uint32_t n_ref, uint32_t n_qry, uint32_t hv_d,
-                                 const void *d_a, const void *d_b) {
-  if (path != 0 && path != 3) return false;
-  if ((uint64_t)n_ref * n_qry < 128ull * 128ull && path == 0) return false;  // SIMT territory
-  if (same && !symmetric) return false;  // full n x n of one matrix: both (i, j) and (j, i) - not worth a special walk
-  return hg_narrow_shape_ok(hv_d, d_a, d_b) == HG_OK;
-}
-
-// Dist with the rows arriving in chunks.  same: ONE matrix, symmetric all-vs-all - chunk c is compared against
-// every row up to its own end (j in the chunk, i < j).  Otherwise the queries go first, whole, and every ref chunk
-// is compared against all of them.
-//   narrow = true: single-plane kernel; returns HG_E_UNSUPPORTED (with max |hv|) if the rows turn out not to be
-//     narrow: by then both matrices are complete in HBM and the caller runs another kernel on them.
-//   narrow = false: two-limb kernel (the caller knows every |hv| fits 13 bits: packed rows of <= 13 bits), the
-//     rows of a chunk split into the matrix-wide limb planes when they arrive.
-static int dist_stream(hg_ctx *c, HostRows &R, HostRows &Q, bool same, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric,
-                       bool narrow, hg_hit *d_hits, uint64_t cap, unsigned long long *d_cnt, int32_t *absmax, uint64_t *outliers,
-                       uint32_t *n_chunks_out) {
-  int rc;
-  if (!c->copy_stream) {
-    HG_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; i++) {
-      HG_CUDA(cudaEventCreateWithFlags(&c->ev_copied[i], cudaEventDisableTiming));
-      HG_CUDA(cudaEventCreateWithFlags(&c->ev_done[i], cudaEventDisableTiming));
-    }
-  }
-  if (!c->ev_chunk[0])
-    for (int i = 0; i < 10; i++) HG_CUDA(cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming));
-  hg_narrow_mat Qm, Rm;
-  hg_tc_mat Qt, Rt;
-  if (narrow) {
-    const size_t mq = hg_narrow_meta_bytes(Q.n), mr = same ? 0 : hg_narrow_meta_bytes(R.n);
-    void *p_meta;
-    if ((rc = hg_scratch(c, HG_S_NARROW_META, mq + mr, &p_meta))) return rc;
-    if ((rc = hg_narrow_setup(c, Q.d_hv, Q.n, hv_d, HG_S_QRY_LIMBS, p_meta, &Qm))) return rc;
-    if (!same && (rc = hg_narrow_setup(c, R.d_hv, R.n, hv_d, HG_S_REF_LIMBS, (uint8_t *)p_meta + mq, &Rm))) return rc;
-  } else {
-    if ((rc = hg_tc_setup(c, Q.d_hv, Q.n, hv_d, HG_S_QRY_LIMBS, &Qt))) return rc;
-    if (!same && (rc = hg_tc_setup(c, R.d_hv, R.n, hv_d, HG_S_REF_LIMBS, &Rt))) return rc;
-  }
-  HG_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), c->stream));
-  auto small = [&](HostRows &S) -> int {
-    HG_CUDA(cudaMemcpyAsync(S.d_norm, S.norm, (size_t)S.n * 4, cudaMemcpyHostToDevice, c->stream));
-    if (S.bits) HG_CUDA(cudaMemcpyAsync(S.d_bits, S.bits, S.n, cudaMemcpyHostToDevice, c->stream));
-    return HG_OK;
-  };
-  if ((rc = small(R))) return rc;
-  if (!same && (rc = small(Q))) return rc;
-  // the copy stream starts once the compute stream has got here (the buffers may still be in use by an earlier call)
-  HG_CUDA(cudaEventRecord(c->ev_chunk[0], c->stream));
-  HG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_chunk[0], 0));
-  auto stage = [&](HostRows &S, uint32_t a, uint32_t rows, cudaEvent_t ev) -> int {  // copy stream
-    HG_CUDA(cudaMemcpy2DAsync(S.d_stage + (size_t)a * S.width, S.width, S.base + (size_t)a * S.stride, S.stride, S.width, rows,
-                              cudaMemcpyHostToDevice, c->copy_stream));
-    HG_CUDA(cudaEventRecord(ev, c->copy_stream));
-    return HG_OK;
-  };
-  auto ready = [&](HostRows &S, const hg_narrow_mat *M, const hg_tc_mat *T, uint32_t a, uint32_t rows, cudaEvent_t ev) -> int {  // compute stream
-    HG_CUDA(cudaStreamWaitEvent(c->stream, ev, 0));
-    if (S.bits) {
-      int r2 = hg_launch_unpack(c, S.d_stage + (size_t)a * S.width, S.width, S.d_bits + a, rows, hv_d, S.d_hv + (size_t)a * hv_d);
-      if (r2) return r2;
-    }
-    return M ? hg_narrow_prep_rows(c, M, a, rows) : hg_tc_split_rows(c, T, a, rows);
-  };
-  uint32_t chunk_rows = 0;
-  if (const char *e = getenv("HG_DIST_CHUNK_ROWS")) chunk_rows = (uint32_t)std::max(0, atoi(e));
-  if (chunk_rows == 0) {
-    const uint32_t want = std::min<uint32_t>(8, std::max<uint32_t>(1, R.n / 1280));  // measured on config 3: 6-8 chunks beat 2-4
-    chunk_rows = (R.n + want - 1) / want;
-  }
-  chunk_rows = std::max<uint32_t>(256, (chunk_rows + 255) & ~255u);
-  if ((uint64_t)chunk_rows * 8 < R.n) chunk_rows = (uint32_t)((((uint64_t)R.n + 7) / 8 + 255) & ~255ull);  // at most 8 chunks
-  // all copies are queued first so that PCIe never waits for the host
-  std::vector<std::pair<uint32_t, uint32_t>> chunks;
-  for (uint32_t a = 0; a < R.n; a += chunk_rows) chunks.push_back({a, std::min(chunk_rows, R.n - a)});
-  if (!same && (rc = stage(Q, 0, Q.n, c->ev_chunk[1]))) return rc;
-  for (size_t k = 0; k < chunks.size(); k++)
-    if ((rc = stage(R, chunks[k].first, chunks[k].second, c->ev_chunk[2 + k]))) return rc;
-  if (!same && (rc = ready(Q, narrow ? &Qm : nullptr, &Qt, 0, Q.n, c->ev_chunk[1]))) return rc;
-  for (size_t k = 0; k < chunks.size(); k++) {
-    const uint32_t a = chunks[k].first, rows = chunks[k].second;
-    if ((rc = ready(R, narrow ? (same ? &Qm : &Rm) : nullptr, same ? &Qt : &Rt, a, rows, c->ev_chunk[2 + k]))) return rc;
-    if (narrow) {
-      if (same)  // pairs (i, j): j in this chunk, i < j
-        rc = hg_narrow_launch(c, &Qm, 0, a + rows, 0, R.d_norm, &Qm, a, rows, a, R.d_norm + a, ksize, ani_th, 1, d_hits, cap, d_cnt);
-      else
-        rc = hg_narrow_launch(c, &Rm, a, rows, a, R.d_norm + a, &Qm, 0, Q.n, 0, Q.d_norm, ksize, ani_th, symmetric, d_hits, cap, d_cnt);
-    } else if (same) {
-      rc = hg_tc_launch(c, &Qt, 0, a + rows, 0, R.d_norm, &Qt, a, rows, a, R.d_norm + a, ksize, ani_th, 1, d_hits, cap, d_cnt);
-    } else {
-      rc = hg_tc_launch(c, &Rt, a, rows, a, R.d_norm + a, &Qt, 0, Q.n, 0, Q.d_norm, ksize, ani_th, symmetric, d_hits, cap, d_cnt);
-    }
-    if (rc) return rc;
-  }
-  if (n_chunks_out) *n_chunks_out = (uint32_t)chunks.size();
-  if (!narrow) return HG_OK;
-  return hg_narrow_verdict(c, &Qm, same ? nullptr : &Rm, absmax, outliers);
-}
-
-// common driver of the host entries: streamed single-plane path if eligible, else (or if it declines) whole
-// copies + the kernel the rows call for
+// Common driver of the host entries: the kernel chosen for these rows, streamed from the host when it can be, else
+// after whole copies on the compute stream; then the tail.  bits: as dist_choose.
 static int dist_from_host(hg_ctx *c, HostRows &R, HostRows &Q, bool same, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric,
-                          int path, int stream_mode /*0 no, 1 single-plane, 2 two-limb*/, hg_hit *hits, uint64_t cap,
-                          uint64_t *n_hits, bool sorted, uint32_t *ani_milli) {
+                          int path, uint32_t bits, hg_hit *hits, uint64_t cap, uint64_t *n_hits, bool sorted, uint32_t *ani_milli) {
   int rc;
-  bool allow_narrow = true;
-  int32_t absmax = -1;
-  const bool shape_ok = !(same && !symmetric) && hg_narrow_shape_ok(hv_d, R.d_hv, Q.d_hv) == HG_OK;
+  DistChoice ch;
+  if ((rc = dist_choose(path, R.n, Q.n, hg_tensor_shape_ok(hv_d, R.d_hv, Q.d_hv) == HG_OK, bits, &ch))) return rc;
+  void *d_hits, *d_cnt;
+  if ((rc = hg_scratch(c, HG_S_PACKED, cap * sizeof(hg_hit) + 256, &d_hits))) return rc;
+  if ((rc = hg_scratch(c, HG_S_COUNTS, 256, &d_cnt))) return rc;
   bool stream_on = true;
   if (const char *e = getenv("HG_DIST_STREAM")) stream_on = atoi(e) != 0;
-  if (stream_on && stream_mode == 1 && dist_stream_eligible(path, same, symmetric, R.n, Q.n, hv_d, R.d_hv, Q.d_hv)) {
-    void *d_hits, *d_cnt;
-    if ((rc = dist_out_buffers(c, cap, &d_hits, &d_cnt))) return rc;
-    uint64_t outliers = 0;
-    uint32_t n_chunks = 0;
-    rc = dist_stream(c, R, Q, same, hv_d, ksize, ani_th, symmetric, true, (hg_hit *)d_hits, cap, (unsigned long long *)d_cnt, &absmax,
-                     &outliers, &n_chunks);
-    if (rc == HG_OK) {
-      c->dist_path = 3;
-      c->ev_used &= ~(3 << 4);
-      snprintf(c->dist_reason, sizeof(c->dist_reason),
-               "tensor-narrow%s: rows fit one s8 plane as x = 2a + s (max |hv| = %d, %llu outlier elements corrected per candidate); "
-               "tcgen05 kind::i8, one MMA per K step; %u row chunk(s) overlapping their H2D",
-               path == 3 ? " (forced)" : "", absmax, (unsigned long long)outliers, n_chunks);
-      return dist_tail(c, d_hits, d_cnt, hits, cap, n_hits, sorted, ani_milli);
+  // Streamed: the single plane on rows that may be narrow, and the two-limb kernel that packed rows of 11..13 bits
+  // chose.  The full n x n of one matrix (both (i, j) and (j, i)) is not worth a special walk.
+  const bool stream = stream_on && !(same && !symmetric) &&
+                      (ch.kernel == HG_PATH_NARROW ? bits <= 10
+                                                   : ch.kernel == HG_PATH_TWO_LIMB && path == HG_PATH_AUTO && hv_d % 512 == 0);
+  c->pending_stats[0] = c->pending_stats[1] = nullptr;
+  c->ev_used &= ~(3 << 4);
+  HG_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), c->stream));
+  auto whole = [&](HostRows &S) -> int {
+    HG_CUDA(cudaMemcpy2DAsync(S.d_stage, S.width, S.base, S.stride, S.width, S.n, cudaMemcpyHostToDevice, c->stream));
+    HG_CUDA(cudaMemcpyAsync(S.d_norm, S.norm, (size_t)S.n * 4, cudaMemcpyHostToDevice, c->stream));
+    if (S.bits) {
+      HG_CUDA(cudaMemcpyAsync(S.d_bits, S.bits, S.n, cudaMemcpyHostToDevice, c->stream));
+      return hg_launch_unpack(c, S.d_stage, S.width, S.d_bits, S.n, hv_d, S.d_hv);
     }
-    if (rc != HG_E_UNSUPPORTED || path == 3) return rc;
-    allow_narrow = false;  // both matrices are complete in HBM now: another kernel on the same data
-  } else if (stream_on && stream_mode == 2 && shape_ok && hv_d % 512 == 0 && (uint64_t)R.n * Q.n >= 128ull * 128ull) {
-    void *d_hits, *d_cnt;
-    if ((rc = dist_out_buffers(c, cap, &d_hits, &d_cnt))) return rc;
-    uint32_t n_chunks = 0;
-    rc = dist_stream(c, R, Q, same, hv_d, ksize, ani_th, symmetric, false, (hg_hit *)d_hits, cap, (unsigned long long *)d_cnt, nullptr,
-                     nullptr, &n_chunks);
-    if (rc) return rc;
-    c->dist_path = 2;
-    c->ev_used &= ~(3 << 4);
-    snprintf(c->dist_reason, sizeof(c->dist_reason),
-             "tensor: hv_quant_bits fit two s8 limbs; tcgen05 kind::i8; %u row chunk(s) overlapping their H2D", n_chunks);
-    return dist_tail(c, d_hits, d_cnt, hits, cap, n_hits, sorted, ani_milli);
-  } else {
-    auto whole = [&](HostRows &S) -> int {
-      HG_CUDA(cudaMemcpy2DAsync(S.d_stage, S.width, S.base, S.stride, S.width, S.n, cudaMemcpyHostToDevice, c->stream));
-      HG_CUDA(cudaMemcpyAsync(S.d_norm, S.norm, (size_t)S.n * 4, cudaMemcpyHostToDevice, c->stream));
-      if (S.bits) {
-        HG_CUDA(cudaMemcpyAsync(S.d_bits, S.bits, S.n, cudaMemcpyHostToDevice, c->stream));
-        return hg_launch_unpack(c, S.d_stage, S.width, S.d_bits, S.n, hv_d, S.d_hv);
-      }
-      return HG_OK;
-    };
-    if ((rc = whole(R))) return rc;
-    if (!same && (rc = whole(Q))) return rc;
-  }
-  return dist_finish(c, R.d_hv, R.d_norm, R.n, Q.d_hv, Q.d_norm, Q.n, hv_d, ksize, ani_th, symmetric, path, hits, cap, n_hits, sorted,
-                     ani_milli, allow_narrow, absmax);
+    return HG_OK;
+  };
+  if (!stream && ((rc = whole(R)) || (!same && (rc = whole(Q))))) return rc;
+  const DistOp op = {R.d_hv, R.d_norm, R.n, 0, Q.d_hv, Q.d_norm, Q.n, 0, hv_d, ksize, ani_th, symmetric, (hg_hit *)d_hits, cap,
+                     (unsigned long long *)d_cnt};
+  if ((rc = dist_run(c, op, ch, stream ? &R : nullptr, stream ? &Q : nullptr, false))) return rc;
+  return dist_tail(c, d_hits, d_cnt, hits, cap, n_hits, sorted, ani_milli);
 }
 
 static int dist_host(hg_ctx *c, const int16_t *ref, const int32_t *ref_norm, uint32_t n_ref, const int16_t *qry,
@@ -1157,7 +1161,7 @@ static int dist_host(hg_ctx *c, const int16_t *ref, const int32_t *ref_norm, uin
   int32_t *d_rn = (int32_t *)d_norm, *d_qn = same ? d_rn : d_rn + n_ref;
   HostRows R = {(const uint8_t *)ref, (uint64_t)hv_d * 2, (uint64_t)hv_d * 2, nullptr, ref_norm, n_ref, (uint8_t *)d_ref, nullptr, d_ref, d_rn};
   HostRows Q = {(const uint8_t *)qry, (uint64_t)hv_d * 2, (uint64_t)hv_d * 2, nullptr, qry_norm, n_qry, (uint8_t *)d_qry, nullptr, d_qry, d_qn};
-  return dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, path, 1, hits, cap, n_hits, sorted, ani_milli);
+  return dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, path, 0, hits, cap, n_hits, sorted, ani_milli);
 }
 
 // `dist` straight from what the sketch file holds (FileSketch.hv bit-packed + hv_quant_bits + hv_norm_2,
@@ -1204,20 +1208,8 @@ extern "C" int hg_dist_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t ref
   uint8_t *d_rp = (uint8_t *)d_pk, *d_qp = d_rp + rp;
   HostRows R = {ref_packed, ref_stride, rw, ref_bits, ref_norm, n_ref, d_rp, d_rbits, d_ref, d_rn};
   HostRows Q = {qry_packed, qry_stride, qw, qry_bits, qry_norm, n_qry, d_qp, d_qbits, d_qry, d_qn};
-  // b-bit two's-complement values are below 2^(b-1): with b > 10 no row can fit the single s8 plane
-  // (x = 2a + s spans 510), and with b <= 13 every element fits the int8 limb split, so that case needs no scan
-  const uint32_t bmax = std::max(rmax, qmax);
-  const bool wide = bmax > 10;
-  if (path == 0 && wide && bmax <= 13 && (uint64_t)n_ref * n_qry >= 128ull * 128ull) {
-    c->tc_is_hint = 1;  // the caller asked for auto: if the tensor kernel declines the shape (hv_d > 32768 ...) SIMT takes over
-    rc = dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, 2, 2, hits, cap, n_hits, sorted != 0, ani_milli);
-    c->tc_is_hint = 0;
-    if (c->dist_path == 2 && !strstr(c->dist_reason, "chunk"))
-      snprintf(c->dist_reason, sizeof(c->dist_reason), "tensor: hv_quant_bits <= %u fits two s8 limbs; tcgen05 kind::i8", bmax);
-    return rc;
-  }
-  return dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, path, wide ? 0 : 1, hits, cap, n_hits, sorted != 0,
-                        ani_milli);
+  return dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, path, std::max(rmax, qmax), hits, cap, n_hits,
+                        sorted != 0, ani_milli);
 }
 
 extern "C" int hg_dist(hg_ctx *c, const int16_t *ref, const int32_t *ref_norm, uint32_t n_ref, const int16_t *qry,

@@ -680,18 +680,6 @@ uint32_t narrow_budget() {  // outlier entries per row on average (HG_NARROW_BUD
 void hg_narrow_tile_shape(uint32_t *rows, uint32_t *cols) { *rows = 256; *cols = N1_BN; }
 
 // ---- one matrix in single-plane form; its rows may be prepared piecewise, as they arrive ------
-int hg_narrow_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b) {
-  if (hv_d % TC_BK != 0 || hv_d > 32768) {
-    hg_set_error("narrow tensor path needs hv_d %% 128 == 0 and hv_d <= 32768, got %u", hv_d);
-    return HG_E_UNSUPPORTED;
-  }
-  if (((uintptr_t)d_a | (uintptr_t)d_b) & 15) {
-    hg_set_error("narrow tensor path needs 16-byte aligned HV matrices");
-    return HG_E_UNSUPPORTED;
-  }
-  return HG_OK;
-}
-
 size_t hg_narrow_meta_bytes(uint32_t n_rows) {
   return ((((size_t)n_rows * 5 + ((size_t)n_rows * narrow_budget() + 1024) + 4) * 4 + 256) + 255) & ~(size_t)255;
 }
@@ -851,8 +839,8 @@ int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32
 }
 
 // Reads the pre-pass statistics (synchronises the stream): HG_OK if every row prepared so far fits the single
-// plane within the budget, else HG_E_UNSUPPORTED (then the kernels launched so far have done nothing useful and
-// the caller must discard their hits).  B may be NULL or equal to A.
+// plane within the budget, else HG_E_UNSUPPORTED, a result that sets no error (then the kernels launched so far
+// have done nothing useful and the caller must discard their hits).  B may be NULL or equal to A.
 int hg_narrow_verdict(hg_ctx *ctx, const hg_narrow_mat *A, const hg_narrow_mat *B, int32_t *absmax_out, uint64_t *outliers_out) {
   uint32_t sa[4 * 8] = {0}, sb[4 * 8] = {0};
   if (A->n_sets > 8 || (B && B->n_sets > 8)) { hg_set_error("hg_narrow_verdict: more than 8 statistic sets"); return HG_E_INVALID; }
@@ -869,52 +857,5 @@ int hg_narrow_verdict(hg_ctx *ctx, const hg_narrow_mat *A, const hg_narrow_mat *
   used += two && B->n_sets == 1 ? sb[2] - B->entry_base : 0;
   if (absmax_out) *absmax_out = (int32_t)amax;
   if (outliers_out) *outliers_out = used;
-  if (declined) {
-    hg_set_error("rows are not narrow: more than %u outlier entries per row on average (x = 2a + s, a in s8)", narrow_budget());
-    return HG_E_UNSUPPORTED;
-  }
-  return HG_OK;
-}
-
-// One-shot form: both matrices already in HBM.  Returns HG_OK when the narrow kernel ran; HG_E_UNSUPPORTED when it
-// declines (shape, or the rows need more outlier entries than the budget) — *absmax_out then holds max |hv| if the
-// scan ran, else -1.
-int hg_launch_dist_narrow(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t i0,
-                          const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry, uint32_t j0, uint32_t hv_d,
-                          uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                          unsigned long long *d_n_hits, int32_t *absmax_out, uint64_t *outliers_out, int defer_verdict) {
-  ctx->pending_stats[0] = ctx->pending_stats[1] = nullptr;
-  if (absmax_out) *absmax_out = -1;
-  if (outliers_out) *outliers_out = 0;
-  if (n_ref == 0 || n_qry == 0) return HG_OK;
-  int rc;
-  if ((rc = hg_narrow_shape_ok(hv_d, d_ref, d_qry))) return rc;
-  const uint64_t ref_elems = (uint64_t)n_ref * hv_d, qry_elems = (uint64_t)n_qry * hv_d;
-  // the query block may alias the ref block (all-vs-all) or contain it (row shard of the same matrix)
-  const bool qry_covers_ref = d_ref >= d_qry && d_ref + ref_elems <= d_qry + qry_elems && ((d_ref - d_qry) % hv_d) == 0;
-  const size_t mq = hg_narrow_meta_bytes(n_qry), mr = qry_covers_ref ? 0 : hg_narrow_meta_bytes(n_ref);
-  void *p_meta;
-  if ((rc = hg_scratch(ctx, HG_S_NARROW_META, mq + mr, &p_meta))) return rc;
-  hg_narrow_mat Q, R;
-  if ((rc = hg_narrow_setup(ctx, d_qry, n_qry, hv_d, HG_S_QRY_LIMBS, p_meta, &Q))) return rc;
-  if (!qry_covers_ref && (rc = hg_narrow_setup(ctx, d_ref, n_ref, hv_d, HG_S_REF_LIMBS, (uint8_t *)p_meta + mq, &R))) return rc;
-  HG_PROF(ctx, 4);
-  if ((rc = hg_narrow_prep_rows(ctx, &Q, 0, n_qry))) return rc;
-  if (!qry_covers_ref && (rc = hg_narrow_prep_rows(ctx, &R, 0, n_ref))) return rc;
-  const uint32_t ref_row_off = qry_covers_ref ? (uint32_t)((d_ref - d_qry) / hv_d) : 0u;
-  if ((rc = hg_narrow_launch(ctx, qry_covers_ref ? &Q : &R, ref_row_off, n_ref, i0, d_ref_norm, &Q, 0, n_qry, j0, d_qry_norm, ksize,
-                             ani_th, symmetric, d_hits, cap, d_n_hits)))
-    return rc;
-  HG_PROF(ctx, 5);
-  // The kernel itself honours the pre-pass's verdict (it does nothing when the rows are not narrow), so the
-  // host learns it only now, with no bubble between pre-pass and kernel - or, when the caller has asserted the
-  // path (defer_verdict), not at all here: hg_dist_status reads it whenever the caller synchronises anyway.
-  if (defer_verdict) {
-    ctx->pending_stats[0] = Q.stats_all;
-    ctx->pending_nsets[0] = Q.n_sets;
-    ctx->pending_stats[1] = qry_covers_ref ? nullptr : R.stats_all;
-    ctx->pending_nsets[1] = qry_covers_ref ? 0 : R.n_sets;
-    return HG_OK;
-  }
-  return hg_narrow_verdict(ctx, &Q, qry_covers_ref ? nullptr : &R, absmax_out, outliers_out);
+  return declined ? HG_E_UNSUPPORTED : HG_OK;
 }

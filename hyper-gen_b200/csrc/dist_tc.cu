@@ -459,18 +459,19 @@ static int tc_attrs(hg_ctx *ctx) {
   return HG_OK;
 }
 
-// ---- one matrix as two s8 limb planes [2][n_rows][hv_d]; its rows may be split piecewise, as they arrive ----
-int hg_tc_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b) {
+int hg_tensor_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b) {
   if (hv_d % TC_BK != 0 || hv_d > 32768) {
-    hg_set_error("tensor path needs hv_d %% 128 == 0 and hv_d <= 32768 (s32 accumulator bound), got %u", hv_d);
+    hg_set_error("tensor paths need hv_d %% 128 == 0 and hv_d <= 32768 (s32 accumulator bound), got %u", hv_d);
     return HG_E_UNSUPPORTED;
   }
   if (((uintptr_t)d_a | (uintptr_t)d_b) & 15) {
-    hg_set_error("tensor path needs 16-byte aligned HV matrices");
+    hg_set_error("tensor paths need 16-byte aligned HV matrices");
     return HG_E_UNSUPPORTED;
   }
   return HG_OK;
 }
+
+// ---- one matrix as two s8 limb planes [2][n_rows][hv_d]; its rows may be split piecewise, as they arrive ----
 
 int hg_tc_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int plane_slot, hg_tc_mat *m) {
   void *p;
@@ -572,29 +573,4 @@ int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref
   ctx->launches++;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
-}
-
-// one-shot form: both matrices already in HBM
-int hg_launch_dist_tc(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t i0,
-                      const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry, uint32_t j0, uint32_t hv_d,
-                      uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                      unsigned long long *d_n_hits) {
-  if (n_ref == 0 || n_qry == 0) return HG_OK;
-  int rc;
-  if ((rc = hg_tc_shape_ok(hv_d, d_ref, d_qry))) return rc;
-  const uint64_t ref_elems = (uint64_t)n_ref * hv_d, qry_elems = (uint64_t)n_qry * hv_d;
-  // the query block may alias the ref block (all-vs-all) or contain it (row shard of the same matrix)
-  const bool qry_covers_ref = d_ref >= d_qry && d_ref + ref_elems <= d_qry + qry_elems && ((d_ref - d_qry) % hv_d) == 0;
-  hg_tc_mat Q, R;
-  if ((rc = hg_tc_setup(ctx, d_qry, n_qry, hv_d, HG_S_QRY_LIMBS, &Q))) return rc;
-  if (!qry_covers_ref && (rc = hg_tc_setup(ctx, d_ref, n_ref, hv_d, HG_S_REF_LIMBS, &R))) return rc;
-  // ---- GPU work starts here (stage timer 4..5 brackets exactly this) ----
-  HG_PROF(ctx, 4);
-  if ((rc = hg_tc_split_rows(ctx, &Q, 0, n_qry))) return rc;
-  if (!qry_covers_ref && (rc = hg_tc_split_rows(ctx, &R, 0, n_ref))) return rc;
-  const uint32_t ref_row_off = qry_covers_ref ? (uint32_t)((d_ref - d_qry) / hv_d) : 0u;
-  rc = hg_tc_launch(ctx, qry_covers_ref ? &Q : &R, ref_row_off, n_ref, i0, d_ref_norm, &Q, 0, n_qry, j0, d_qry_norm, ksize, ani_th,
-                    symmetric, d_hits, cap, d_n_hits);
-  HG_PROF(ctx, 5);
-  return rc;
 }

@@ -140,7 +140,7 @@ struct hg_ctx {
   // pinned host scratch
   void *h_pinned[4];
   size_t h_pinned_bytes[4];
-  // last dist decision
+  // last dist decision (hg_dist_record)
   int dist_path;
   char dist_reason[288];
   // status words of the last sketch batch (device + host copy)
@@ -152,12 +152,11 @@ struct hg_ctx {
   int ev_used;           // which stage boundaries were recorded in the last call
   // H2D pipeline of the host-pointer sketch entry
   int tc_attr_set;
-  int tc_is_hint;   // the two-limb path was chosen by the library (packed rows of 11..13 bits), not forced by the caller: SIMT fallback allowed
   int n1_attr_set;
   const uint64_t *d_actual_len;  // optional per-genome true lengths for the next k-mer launch (raw-FASTA path)
-  cudaStream_t copy_stream;
+  cudaStream_t copy_stream;      // created on first use, with the events below
   cudaEvent_t ev_copied[2], ev_done[2];
-  cudaEvent_t ev_chunk[10];  // dist streaming: fork + one per row chunk (created with the copy stream)
+  cudaEvent_t ev_chunk[10];  // dist streaming: fork + query matrix + one per row chunk
   // hg_dist_dev with the single-plane path forced: the pre-pass verdict is not waited for (hg_dist_status reads it)
   const uint32_t *pending_stats[2];
   uint32_t pending_nsets[2];
@@ -203,6 +202,12 @@ enum hg_scratch_slot {
 // scratch slot `slot` grown to at least `bytes` (contents not preserved)
 int hg_scratch(hg_ctx *ctx, int slot, size_t bytes, void **out);
 int hg_pinned(hg_ctx *ctx, int slot, size_t bytes, void **out);
+
+// The dist kernels, numbered as the `path` argument of the dist entries (include/hypergen_b200.h).
+enum hg_dist_path { HG_PATH_AUTO = 0, HG_PATH_SIMT = 1, HG_PATH_TWO_LIMB = 2, HG_PATH_NARROW = 3 };
+constexpr int32_t HG_LIMB_MAX_ABS = 8127;  // the largest |x| that splits into two s8 limbs x = 128 h + l (13 bits)
+// sets what hg_dist_last_path / hg_dist_last_reason report
+void hg_dist_record(hg_ctx *ctx, int path, const char *fmt, ...);
 
 // ---- kernel launchers (all asynchronous on ctx->stream) ----
 
@@ -279,13 +284,16 @@ struct hg_tile_feed {
   unsigned long long *dbg;  // timeline stamps (HG_PEER_TIMELINE=1, hg_peer_timeline), else NULL
 };
 
+// HG_OK when both tensor kernels (two-limb and single-plane) tile this shape: hv_d % 128 == 0, hv_d <= 32768 (s32
+// accumulator bound) and 16-byte aligned matrices; else HG_E_UNSUPPORTED with the reason in hg_last_error()
+int hg_tensor_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b);
+
 // two s8 limb planes of one matrix (dist_tc.cu), split piecewise or at once
 struct hg_tc_mat {
   const int16_t *hv;
   int8_t *planes;  // [2][n_rows][hv_d]
   uint32_t n_rows, hv_d;
 };
-int hg_tc_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b);
 int hg_tc_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int plane_slot, hg_tc_mat *m);
 int hg_tc_split_rows(hg_ctx *ctx, const hg_tc_mat *m, uint32_t row0, uint32_t rows);
 int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
@@ -297,10 +305,6 @@ int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref
                     float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, uint32_t walk_mul,
                     uint32_t walk_add, const hg_tile_feed *feed = nullptr, const hg_push_plan *push = nullptr);
 void hg_tc_tile_shape(uint32_t *rows, uint32_t *cols);
-int hg_launch_dist_tc(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref,
-                      uint32_t i0, const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry,
-                      uint32_t j0, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric,
-                      hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits);
 // single s8 plane (x = 2a + s) + sparse outlier corrections (dist_narrow.cu): one matrix in that form, prepared
 // piecewise (rows as they arrive over PCIe) or at once
 struct hg_narrow_mat {
@@ -317,7 +321,6 @@ struct hg_narrow_mat {
   uint32_t cap;         // ... and the limit (exclusive)
   uint32_t n_rows, hv_d;
 };
-int hg_narrow_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b);
 size_t hg_narrow_meta_bytes(uint32_t n_rows);
 int hg_narrow_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int plane_slot, void *meta,
                     hg_narrow_mat *m);
@@ -340,12 +343,6 @@ int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32
                         const hg_push_plan *push = nullptr);
 void hg_narrow_tile_shape(uint32_t *rows, uint32_t *cols);
 int hg_narrow_verdict(hg_ctx *ctx, const hg_narrow_mat *A, const hg_narrow_mat *B, int32_t *absmax_out, uint64_t *outliers_out);
-// one-shot form of the above; HG_E_UNSUPPORTED when the rows are not narrow
-int hg_launch_dist_narrow(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref,
-                          uint32_t i0, const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry,
-                          uint32_t j0, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric,
-                          hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, int32_t *absmax_out,
-                          uint64_t *outliers_out, int defer_verdict);
 int hg_launch_int_peak(hg_ctx *ctx, int which, uint32_t iters, uint32_t *d_sink, uint32_t blocks);
 // max |hv| over a device matrix (decides the dist path); result in *d_out (int32)
 int hg_launch_sort_hits(hg_ctx *ctx, hg_hit *d_hits, uint64_t n, uint32_t *d_milli);

@@ -52,7 +52,6 @@ constexpr int N_CHUNKS = HG_PUSH_CHUNKS;
 constexpr uint64_t CHUNK_TARGET_BYTES = 2u << 20;  // a member's block is cut into chunks of at least about this much
 static_assert(OFF_DONE + 4 * HG_PUSH_UNITS <= OFF_DBG, "header layout");
 constexpr size_t OFF_HITS = 4096;    // hg_hit[cap]
-constexpr int32_t TC_MAX_ABS = 8127; // |x| <= 8127 splits into two s8 limbs
 
 struct PeerPtrs { uint8_t *p[HG_MAX_PEERS]; };
 
@@ -429,7 +428,7 @@ XPlan make_xplan(int world, int symmetric, int path, uint32_t hv_d, const uint32
   bool aligned = true, nonempty = true;
   for (int m = 0; m <= world; ++m) x.qb[m] = qb[m];
   for (int m = 0; m < world; ++m) {
-    const uint64_t rows = qb[m + 1] - qb[m], bytes = rows * hv_d * (path == 3 ? 1 : 2);
+    const uint64_t rows = qb[m + 1] - qb[m], bytes = rows * hv_d * (path == HG_PATH_NARROW ? 1 : 2);
     x.n_chunks[m] = (int)std::min<uint64_t>(std::max<uint64_t>((bytes + CHUNK_TARGET_BYTES - 1) / CHUNK_TARGET_BYTES, 1), N_CHUNKS);
     if (rows == 0) nonempty = false;
     if (m > 0 && qb[m] % 256 != 0) aligned = false;  // a tile (256 rows x 128 or 256 columns) lies inside one block on either side
@@ -544,7 +543,7 @@ static TileKey tile_key(int world, int symmetric, int use_path, uint32_t hv_d, u
   k.hv_d = hv_d;
   k.n_ref = symmetric ? qb[world] : n_ref;
   k.n_qry = qb[world];
-  if (use_path == 3) hg_narrow_tile_shape(&k.tr, &k.tc); else hg_tc_tile_shape(&k.tr, &k.tc);
+  if (use_path == HG_PATH_NARROW) hg_narrow_tile_shape(&k.tr, &k.tc); else hg_tc_tile_shape(&k.tr, &k.tc);
   for (int m = 0; m <= world; ++m) k.qb[m] = qb[m];
   return k;
 }
@@ -563,7 +562,7 @@ static void build_tiles(hg_peer *p, const ShardCall &a, int use_path) {
 // pairs; *n_tiles the count (HG_E_CAPACITY if it exceeds cap).
 extern "C" int hg_peer_plan_tiles(int world, int rank, int symmetric, int path, uint32_t hv_d, uint32_t n_ref_local,
                                   const uint32_t *qry_bounds, uint32_t *tiles_out, uint64_t cap, uint64_t *n_tiles) {
-  if (!qry_bounds || !n_tiles || world < 1 || world > HG_MAX_PEERS || rank < 0 || rank >= world || (path != 2 && path != 3) || hv_d == 0) {
+  if (!qry_bounds || !n_tiles || world < 1 || world > HG_MAX_PEERS || rank < 0 || rank >= world || (path != HG_PATH_TWO_LIMB && path != HG_PATH_NARROW) || hv_d == 0) {
     hg_set_error("hg_peer_plan_tiles: bad argument"); return HG_E_INVALID;
   }
   std::vector<uint2> v;
@@ -591,7 +590,7 @@ static void plan_units(const XPlan &x, int rank, bool have_rows, std::vector<std
 extern "C" int hg_peer_plan_push(int world, int rank, int symmetric, int path, uint32_t hv_d, const uint32_t *qry_bounds,
                                  uint32_t chunk_rows_out[HG_PUSH_CHUNKS + 1], uint32_t *units_out, uint64_t cap, uint64_t *n_units,
                                  int *ring) {
-  if (!qry_bounds || !n_units || !chunk_rows_out || world < 1 || world > HG_MAX_PEERS || rank < 0 || rank >= world || (path != 2 && path != 3) || hv_d == 0) {
+  if (!qry_bounds || !n_units || !chunk_rows_out || world < 1 || world > HG_MAX_PEERS || rank < 0 || rank >= world || (path != HG_PATH_TWO_LIMB && path != HG_PATH_NARROW) || hv_d == 0) {
     hg_set_error("hg_peer_plan_push: bad argument"); return HG_E_INVALID;
   }
   const XPlan x = make_xplan(world, symmetric, path, hv_d, qry_bounds);
@@ -639,7 +638,7 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
   const int rank = p->rank, world = p->world;
   const uint32_t n_total = a.qb[world], r0 = a.qb[rank], nl = a.qb[rank + 1] - a.qb[rank];
   uint8_t *W = p->win[rank];
-  const ShardLayout lay = make_layout(world, n_total, a.hv_d, a.cap, use_path == 3 ? 1 : 2, a.mapped_hits != nullptr);
+  const ShardLayout lay = make_layout(world, n_total, a.hv_d, a.cap, use_path == HG_PATH_NARROW ? 1 : 2, a.mapped_hits != nullptr);
   int32_t *normW = (int32_t *)(W + lay.norm);
   // every member appends to ITS OWN list (local atomics and stores); peer_flush_kernel moves the list to the root afterwards
   hg_hit *hits = (hg_hit *)(W + OFF_HITS);
@@ -653,7 +652,7 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
   p->ev_n = 0;
   PEER_PROF(p, 0);
   // sequence number + 1, my hit counter and statistics reset, the root's gather counter reset
-  peer_tick_kernel<<<1, 32, 0, c->stream>>>(W, rank, rank == a.root, use_path == 3 ? (uint32_t)rank * lay.set_cap : 0u, p->timeline);
+  peer_tick_kernel<<<1, 32, 0, c->stream>>>(W, rank, rank == a.root, use_path == HG_PATH_NARROW ? (uint32_t)rank * lay.set_cap : 0u, p->timeline);
   c->launches++;
   HG_CUDA(cudaGetLastError());
   hg_tile_feed feed = {};
@@ -678,7 +677,7 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
   if (nl) HG_CUDA(cudaMemcpyAsync(normW + r0, a.d_qry_norm, (size_t)nl * 4, cudaMemcpyDeviceToDevice, c->stream));
   hg_narrow_mat Qn, Rn;
   hg_tc_mat Qt, Rt;
-  if (use_path == 3) {
+  if (use_path == HG_PATH_NARROW) {
     if ((rc = hg_narrow_attach(c, matrix_base(a.d_qry_hv, r0, a.hv_d), n_total, a.hv_d, (int8_t *)(W + lay.plane), W + lay.arrays,
                                (uint32_t *)(W + lay.entries), (uint32_t *)(W + OFF_STATS_Q), (uint32_t)world, (uint32_t)rank,
                                (uint32_t)rank * lay.set_cap, lay.set_cap, &Qn, /*init_stats=*/false)))
@@ -693,7 +692,7 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
       if ((rc = hg_narrow_prep_rows(c, &Rn, 0, nr))) return rc;
     }
   } else {
-    if ((rc = hg_tc_shape_ok(a.hv_d, a.d_qry_hv, a.d_ref_hv))) return rc;
+    if ((rc = hg_tensor_shape_ok(a.hv_d, a.d_qry_hv, a.d_ref_hv))) return rc;
     if ((rc = hg_tc_attach(c, matrix_base(a.d_qry_hv, r0, a.hv_d), n_total, a.hv_d, (int8_t *)(W + lay.plane), &Qt))) return rc;
     if ((rc = hg_tc_split_rows(c, &Qt, r0, nl))) return rc;
     if (!a.symmetric && a.n_ref_local) {
@@ -723,10 +722,10 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
     const uint64_t lo = chunk_lo(xp, rank, ch), n = chunk_lo(xp, rank, ch + 1) - lo;
     add(ch, lay.norm + lo * 4, n * 4);
     add(ch, lay.plane + lo * a.hv_d, n * a.hv_d);
-    if (use_path == 3) for (int k = 0; k < 5; ++k) add(ch, lay.arrays + ((uint64_t)k * n_total + lo) * 4, n * 4);
+    if (use_path == HG_PATH_NARROW) for (int k = 0; k < 5; ++k) add(ch, lay.arrays + ((uint64_t)k * n_total + lo) * 4, n * 4);
     else add(ch, lay.plane + ((uint64_t)n_total + lo) * a.hv_d, n * a.hv_d);
   }
-  if (use_path == 3 && world > 1) {  // the statistics and the outlier entries of ALL my rows (the pre-pass above is complete)
+  if (use_path == HG_PATH_NARROW && world > 1) {  // the statistics and the outlier entries of ALL my rows (the pre-pass above is complete)
     if (nl) {  // (range 0 of the start set: the pushers cut it down to the entries the pre-pass actually wrote)
       add(HG_PUSH_START_SET, lay.entries + (uint64_t)rank * lay.set_cap * 4, (uint64_t)lay.set_cap * 4);
       plan.dyn_count = (const uint32_t *)(W + OFF_STATS_Q) + 4 * rank + 2;
@@ -765,7 +764,7 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
   const hg_push_plan *pp = have_tiles ? &plan : nullptr;
   PEER_PROF(p, 2);
   const hg_tile_feed *fp = use_list ? &feed : nullptr;
-  if (use_path == 3) {
+  if (use_path == HG_PATH_NARROW) {
     if (a.symmetric)
       rc = hg_narrow_launch_ex(c, &Qn, 0, n_total, 0, normW, &Qn, 0, n_total, 0, normW, a.ksize, a.ani_th, 1, hits, a.cap, counter, 1, 0, fp, pp);
     else
@@ -853,13 +852,12 @@ static int shard_verdict(hg_peer *p, const ShardCall &a, int32_t *absmax) {
 
 static void shard_reason(hg_peer *p, int path, int32_t absmax, bool forced) {
   hg_ctx *c = p->ctx;
-  c->dist_path = path;
-  if (path == 3)
-    snprintf(c->dist_reason, sizeof(c->dist_reason), "tensor-narrow%s: member %d of %d GPUs, operand planes pushed over NVLink windows in chunks, %s, tiles ordered by arrival%s",
+  if (path == HG_PATH_NARROW)
+    hg_dist_record(c, path, "tensor-narrow%s: member %d of %d GPUs, operand planes pushed over NVLink windows in chunks, %s, tiles ordered by arrival%s",
              forced ? " (forced)" : "", p->rank, p->world, p->last_ring ? "block pairs owned along the ring (rows go to N/2 members)" : "tiles dealt round-robin (rows go to every member)",
              forced ? "" : "; rows fit one s8 plane as x = 2a + s");
   else
-    snprintf(c->dist_reason, sizeof(c->dist_reason), "tensor%s: member %d of %d GPUs, two s8 limb planes pushed over NVLink windows in chunks, %s, tiles ordered by arrival (max |hv| = %d)",
+    hg_dist_record(c, path, "tensor%s: member %d of %d GPUs, two s8 limb planes pushed over NVLink windows in chunks, %s, tiles ordered by arrival (max |hv| = %d)",
              forced ? " (forced)" : "", p->rank, p->world, p->last_ring ? "block pairs owned along the ring (rows go to N/2 members)" : "tiles dealt round-robin (rows go to every member)", absmax);
 }
 
@@ -876,10 +874,10 @@ extern "C" int hg_dist_sharded_dev(hg_peer *p, const int16_t *d_ref_hv, const in
   a.hv_d = hv_d; a.ksize = ksize; a.ani_th = ani_th; a.symmetric = symmetric; a.root = root; a.cap = cap; a.mapped_hits = mapped_hits;
   int rc;
   if ((rc = shard_check(p, a))) return rc;
-  if (path != 0 && path != 2 && path != 3) { hg_set_error("hg_dist_sharded_dev: path %d (0 auto, 2 two-limb, 3 single plane)", path); return HG_E_INVALID; }
+  if (path != HG_PATH_AUTO && path != HG_PATH_TWO_LIMB && path != HG_PATH_NARROW) { hg_set_error("hg_dist_sharded_dev: path %d (0 auto, 2 two-limb, 3 single plane)", path); return HG_E_INVALID; }
   if (a.qb[p->world] == 0) return HG_OK;
-  if (path == 2 || path == 3) {
-    if (path == 3 && (rc = hg_narrow_shape_ok(hv_d, d_qry_hv, d_ref_hv))) return rc;
+  if (path == HG_PATH_TWO_LIMB || path == HG_PATH_NARROW) {
+    if (path == HG_PATH_NARROW && (rc = hg_tensor_shape_ok(hv_d, d_qry_hv, d_ref_hv))) return rc;
     hg_ctx *c = p->ctx;
     // The same call again (same pointers, shapes and scratch buffers): replay its launch sequence as a CUDA graph.
     // The first call runs directly, the second is captured, the following ones are one cudaGraphLaunch each.
@@ -925,21 +923,21 @@ extern "C" int hg_dist_sharded_dev(hg_peer *p, const int16_t *d_ref_hv, const in
   int32_t absmax = -1;
   if (p->graph) { cudaGraphExecDestroy(p->graph); p->graph = nullptr; p->graph_key.clear(); }
   p->last_key.clear();
-  rc = hg_narrow_shape_ok(hv_d, d_qry_hv, d_ref_hv);
+  rc = hg_tensor_shape_ok(hv_d, d_qry_hv, d_ref_hv);
   if (rc == HG_OK) {
-    if ((rc = shard_reserve(p, a, 3))) return rc;
-    if ((rc = shard_enqueue(p, a, 3))) return rc;
+    if ((rc = shard_reserve(p, a, HG_PATH_NARROW))) return rc;
+    if ((rc = shard_enqueue(p, a, HG_PATH_NARROW))) return rc;
     rc = shard_verdict(p, a, &absmax);
-    if (rc == HG_OK) { shard_reason(p, 3, absmax, false); return HG_OK; }
+    if (rc == HG_OK) { shard_reason(p, HG_PATH_NARROW, absmax, false); return HG_OK; }
     if (rc != HG_E_UNSUPPORTED) return rc;
   }
-  if (absmax > TC_MAX_ABS) {
+  if (absmax > HG_LIMB_MAX_ABS) {
     hg_set_error("hg_dist_sharded_dev: max |hv| = %d exceeds the 13-bit budget of the int8 limb split; the sharded path has no SIMT kernel", absmax);
     return HG_E_UNSUPPORTED;
   }
-  if ((rc = shard_reserve(p, a, 2))) return rc;
-  if ((rc = shard_enqueue(p, a, 2))) return rc;
-  shard_reason(p, 2, absmax, false);
+  if ((rc = shard_reserve(p, a, HG_PATH_TWO_LIMB))) return rc;
+  if ((rc = shard_enqueue(p, a, HG_PATH_TWO_LIMB))) return rc;
+  shard_reason(p, HG_PATH_TWO_LIMB, absmax, false);
   return HG_OK;
 }
 
@@ -1165,7 +1163,7 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
     if ((rc = shard_check(g->peer[k], a))) return rc;
   }
   // b-bit values are below 2^(b-1): above 10 bits no row fits the single plane, and up to 13 bits every element fits two limbs
-  int used = bmax > 10 ? 2 : 3;
+  int used = bmax > 10 ? HG_PATH_TWO_LIMB : HG_PATH_NARROW;
   for (int k = 0; k < N; ++k)
     if ((rc = shard_reserve(g->peer[k], make_call(M[k]), used))) return rc;
   // phase 2: H2D + unpack + sharded dist enqueued on every GPU; nothing here waits for another GPU
@@ -1198,7 +1196,7 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
   }
   int32_t absmax = -1;
   if ((rc = enqueue_all(used))) return rc;
-  if (used == 3) {
+  if (used == HG_PATH_NARROW) {
     int verdict = HG_OK;
     for (int k = 0; k < N; ++k) {
       cudaSetDevice(g->ctx[k]->device);
@@ -1207,10 +1205,10 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
       if (v) verdict = v;
     }
     if (verdict == HG_E_UNSUPPORTED) {  // not narrow (the same answer on every GPU): the two-limb kernel on the rows already in HBM
-      used = 2;
+      used = HG_PATH_TWO_LIMB;
       for (int k = 0; k < N; ++k)
-        if ((rc = shard_reserve(g->peer[k], make_call(M[k]), 2))) return rc;
-      if ((rc = enqueue_all(2))) return rc;
+        if ((rc = shard_reserve(g->peer[k], make_call(M[k]), HG_PATH_TWO_LIMB))) return rc;
+      if ((rc = enqueue_all(HG_PATH_TWO_LIMB))) return rc;
     }
   }
   for (int k = 0; k < N; ++k) shard_reason(g->peer[k], used, absmax, false);
