@@ -17,7 +17,8 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(ROOT, "build", "obj")
 LIB = os.path.join(HERE, "libhypergen_b200.so")
 
-SOURCES = ["api.cu", "kmer_hash.cu", "encode.cu", "dist_simt.cu", "dist_tc.cu", "dist_narrow.cu", "probe.cu", "fasta.cu", "sort.cu", "peer.cu"]
+SOURCES = ["api.cu", "kmer_hash.cu", "encode.cu", "dist_simt.cu", "dist_tc.cu", "dist_narrow.cu", "probe.cu", "fasta.cu", "sort.cu", "peer.cu",
+           "search.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC,-fvisibility=hidden", "-diag-suppress", "177",

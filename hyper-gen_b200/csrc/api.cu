@@ -2,6 +2,7 @@
 // entry points (H2D / D2H inside), device-pointer entry points (inputs resident in HBM).
 // Replaces the cudarc plumbing of reference src/sketch_cuda.rs:52-60,119-166.
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -74,6 +75,7 @@ extern "C" void hg_destroy(hg_ctx *c) {
   cudaSetDevice(c->device);
   if (c->stream) cudaStreamSynchronize(c->stream);
   for (int i = 0; i < 10; i++) if (c->ev_chunk[i]) cudaEventDestroy(c->ev_chunk[i]);
+  for (int i = 0; i < 5; i++) if (c->ev_search[i]) cudaEventDestroy(c->ev_search[i]);
   for (int i = 0; i < HG_S_COUNT; i++) if (c->d_scratch[i]) cudaFree(c->d_scratch[i]);
   for (int i = 0; i < 4; i++) if (c->h_pinned[i]) cudaFreeHost(c->h_pinned[i]);
   if (c->d_status) cudaFree(c->d_status);
@@ -814,6 +816,8 @@ struct DistOp {
   hg_hit *hits;
   uint64_t cap;
   unsigned long long *n_hits;
+  const hg_floor *floors = nullptr;  // a search's main pass: per-query thresholds in place of ani_th (hg_floors)
+  const float *cfrac_row = nullptr;
 };
 
 // The kernel a dist call tries first, chosen before anything runs.
@@ -967,8 +971,10 @@ static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, H
     return narrow ? hg_narrow_prep_rows(c, M, a, rows) : hg_tc_split_rows(c, T, a, rows);
   };
   auto launch = [&](uint32_t r0, uint32_t nr, uint32_t i0, const int32_t *rn, uint32_t q0, uint32_t nq, uint32_t j0, const int32_t *qn) {
-    return narrow ? hg_narrow_launch(c, Rn, r0, nr, i0, rn, &Qm, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits)
-                  : hg_tc_launch(c, Rl, r0, nr, i0, rn, &Qt, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits);
+    const hg_floors fl = {op.floors ? op.floors + q0 : nullptr, op.cfrac_row};  // indexed like qn = qry_norm + q0
+    const hg_floors *flp = op.floors ? &fl : nullptr;
+    return narrow ? hg_narrow_launch(c, Rn, r0, nr, i0, rn, &Qm, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits, flp)
+                  : hg_tc_launch(c, Rl, r0, nr, i0, rn, &Qt, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits, flp);
   };
   if (!one && (rc = prep(hq, &Qm, &Qt, 0, op.n_qry, c->ev_chunk[1]))) return rc;
   for (size_t k = 0; k < chunks.size(); k++) {
@@ -1025,8 +1031,9 @@ static int dist_run(hg_ctx *c, const DistOp &op, const DistChoice &ch, HostRows 
   }
   if (ran == HG_PATH_SIMT) {
     HG_PROF(c, 4);
+    const hg_floors fl = {op.floors, op.cfrac_row};
     rc = hg_launch_dist_simt(c, op.ref, op.ref_norm, op.n_ref, op.i0, op.qry, op.qry_norm, op.n_qry, op.j0, op.hv_d, op.ksize, op.ani_th,
-                             op.symmetric, op.hits, op.cap, op.n_hits);
+                             op.symmetric, op.hits, op.cap, op.n_hits, op.floors ? &fl : nullptr);
     HG_PROF(c, 5);
     if (rc) return rc;
   }
@@ -1230,4 +1237,212 @@ extern "C" int hg_sort_hits_dev(hg_ctx *c, hg_hit *d_hits, uint64_t n, uint32_t 
   if (!c || (n && !d_hits)) { hg_set_error("hg_sort_hits_dev: NULL argument"); return HG_E_INVALID; }
   HG_CUDA(cudaSetDevice(c->device));
   return hg_launch_sort_hits(c, d_hits, n, d_ani_milli);
+}
+
+// ---------------------------------------------------------------------------------------
+// search: the top_k best refs of every query (DESIGN.md §4, "Top-k search")
+// ---------------------------------------------------------------------------------------
+
+// rows of the floor pass's sample: about sqrt(top_k * n_ref) in [1024, 16384], a multiple of 256 and at least top_k;
+// all of them (one pass) when that is not fewer than n_ref
+static uint32_t search_sample_rows(uint32_t top_k, uint32_t n_ref) {
+  const double want = std::min(16384.0, std::max(1024.0, std::sqrt((double)top_k * (double)n_ref)));
+  const uint32_t s = std::max(((uint32_t)want + 255u) & ~255u, (top_k + 255u) & ~255u);
+  return s < n_ref ? s : n_ref;
+}
+
+static void search_mark(hg_ctx *c, int k) {
+  if (!c->prof) return;
+  cudaEventRecord(c->ev_search[k], c->stream);
+  c->search_ev_used |= 1 << k;
+}
+
+// One dist pass of a search: every pair that passes op's threshold(s), into the candidate scratch.  When they do not
+// fit, the scratch grows to their count and the pass reruns: no candidate is dropped.
+static int search_pass(hg_ctx *c, DistOp op, int path, uint32_t bits, uint64_t want, hg_hit **cand, uint64_t *n_cand) {
+  int rc;
+  DistChoice ch;
+  if ((rc = dist_choose(path, op.n_ref, op.n_qry, hg_tensor_shape_ok(op.hv_d, op.ref, op.qry) == HG_OK, bits, &ch))) return rc;
+  void *d_cnt, *d_hits;
+  if ((rc = hg_scratch(c, HG_S_COUNTS, 256, &d_cnt))) return rc;
+  for (;;) {
+    if ((rc = hg_scratch(c, HG_S_PACKED, want * sizeof(hg_hit), &d_hits))) return rc;
+    op.hits = (hg_hit *)d_hits;
+    op.cap = c->d_scratch_bytes[HG_S_PACKED] / sizeof(hg_hit);
+    op.n_hits = (unsigned long long *)d_cnt;
+    HG_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), c->stream));
+    if ((rc = dist_run(c, op, ch, nullptr, nullptr, false))) return rc;
+    unsigned long long cnt = 0;
+    HG_CUDA(cudaMemcpyAsync(&cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, c->stream));
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+    if (cnt <= op.cap) {
+      *cand = op.hits;
+      *n_cand = cnt;
+      return HG_OK;
+    }
+    want = cnt;
+    c->search_stats[3]++;
+  }
+}
+
+// Exact by construction.  Floor pass: the dist kernel on s sample rows S x Q at ani_min, and per query the top_k-th
+// key (ANI desc, i asc) of the sample.  S is a subset of the refs, so every member of the true top_k of query j has a
+// key at least that large: the main pass over R x Q keeps exactly those pairs (hg_floors) - a superset of the answer -
+// and the select kernel takes the top_k of each query from them.  With s = n_ref the first pass is the answer.
+static int search_run(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, const int16_t *d_qry,
+                      const int32_t *d_qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
+                      int path, uint32_t bits, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli) {
+  int rc;
+  memset(c->search_stats, 0, sizeof(c->search_stats));
+  c->search_ev_used = 0;
+  c->pending_stats[0] = c->pending_stats[1] = nullptr;
+  c->ev_used &= ~(3 << 4);
+  if (n_qry == 0) return HG_OK;
+  if (n_ref == 0) {
+    HG_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n_qry * top_k * sizeof(hg_hit), c->stream));
+    HG_CUDA(cudaMemsetAsync(d_n_found, 0, (size_t)n_qry * 4, c->stream));
+    if (d_milli) HG_CUDA(cudaMemsetAsync(d_milli, 0, (size_t)n_qry * top_k * 4, c->stream));
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+    return HG_OK;
+  }
+  if (c->prof && !c->ev_search[0])
+    for (int k = 0; k < 5; k++) HG_CUDA(cudaEventCreate(&c->ev_search[k]));
+  const uint32_t s = search_sample_rows(top_k, n_ref);
+  c->search_stats[0] = s;
+  const uint64_t want = 4096 + 4ull * n_qry * top_k;  // initial candidate room; grows as the passes need
+  DistOp op = {d_ref, d_ref_norm, n_ref, 0, d_qry, d_qry_norm, n_qry, 0, hv_d, ksize, ani_min, 0, nullptr, 0, nullptr};
+  hg_hit *cand;
+  uint64_t n_cand;
+  search_mark(c, 0);
+  if (s < n_ref) {
+    void *d_sample, *d_fl;
+    const size_t sb = ((size_t)s * hv_d * 2 + 255) & ~(size_t)255;
+    if ((rc = hg_scratch(c, HG_S_SEQ, sb + (size_t)s * 4, &d_sample))) return rc;
+    if ((rc = hg_scratch(c, HG_S_DESC, (size_t)n_qry * (sizeof(hg_floor) + 8) + 256, &d_fl))) return rc;
+    hg_floor *floors = (hg_floor *)d_fl;
+    unsigned long long *fkey = (unsigned long long *)(floors + n_qry);
+    float *cfrac_row = (float *)(fkey + n_qry);
+    int16_t *S = (int16_t *)d_sample;
+    int32_t *Sn = (int32_t *)((uint8_t *)d_sample + sb);
+    if ((rc = hg_launch_search_gather(c, d_ref, d_ref_norm, n_ref, hv_d, s, S, Sn))) return rc;
+    DistOp fo = op;
+    fo.ref = S;
+    fo.ref_norm = Sn;
+    fo.n_ref = s;
+    if ((rc = search_pass(c, fo, path, bits, want, &cand, &n_cand))) return rc;
+    c->search_stats[1] = n_cand;
+    search_mark(c, 1);
+    if ((rc = hg_launch_search_select(c, cand, n_cand, n_qry, top_k, nullptr, nullptr, nullptr, fkey))) return rc;
+    if ((rc = hg_launch_search_floors(c, fkey, n_qry, ani_min, ksize, n_ref, s, floors, cfrac_row))) return rc;
+    search_mark(c, 2);
+    op.floors = floors;
+    op.cfrac_row = cfrac_row;
+  }
+  if ((rc = search_pass(c, op, path, bits, want, &cand, &n_cand))) return rc;
+  c->search_stats[2] = n_cand;
+  search_mark(c, 3);
+  if ((rc = hg_launch_search_select(c, cand, n_cand, n_qry, top_k, d_out, d_n_found, d_milli, nullptr))) return rc;
+  search_mark(c, 4);
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  return HG_OK;
+}
+
+static int search_check(const char *who, uint32_t hv_d, uint32_t top_k, int path) {
+  if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("%s: hv_d %u must be a multiple of 256", who, hv_d); return HG_E_INVALID; }
+  if (top_k < 1 || top_k > 1024) { hg_set_error("%s: top_k %u outside 1..1024", who, top_k); return HG_E_INVALID; }
+  if (path < HG_PATH_AUTO || path > HG_PATH_NARROW) { hg_set_error("%s: path %d", who, path); return HG_E_INVALID; }
+  return HG_OK;
+}
+
+extern "C" int hg_search_dev(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm2, uint32_t n_ref, const int16_t *d_qry,
+                             const int32_t *d_qry_norm2, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
+                             int path, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_ani_milli) {
+  if (!c || (n_ref && (!d_ref || !d_ref_norm2)) || (n_qry && (!d_qry || !d_qry_norm2 || !d_out || !d_n_found))) {
+    hg_set_error("hg_search_dev: NULL argument"); return HG_E_INVALID;
+  }
+  int rc;
+  if ((rc = search_check("hg_search_dev", hv_d, top_k, path))) return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  return search_run(c, d_ref, d_ref_norm2, n_ref, d_qry, d_qry_norm2, n_qry, hv_d, ksize, top_k, ani_min, path, 0, d_out, d_n_found,
+                    d_ani_milli);
+}
+
+// The rows as the sketch files hold them: whole copies of the packed bytes, decompress_file_sketch on the device (as
+// hg_dist_packed), then the search; the results come back to the host.
+extern "C" int hg_search_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits, const int32_t *ref_norm,
+                                uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
+                                const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
+                                int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli) {
+  if (!c || (n_ref && (!ref_packed || !ref_bits || !ref_norm)) || (n_qry && (!qry_packed || !qry_bits || !qry_norm || !out || !n_found))) {
+    hg_set_error("hg_search_packed: NULL argument"); return HG_E_INVALID;
+  }
+  int rc;
+  if ((rc = search_check("hg_search_packed", hv_d, top_k, path))) return rc;
+  if (ref_stride % 4 != 0 || qry_stride % 4 != 0) { hg_set_error("hg_search_packed: row stride %% 4"); return HG_E_INVALID; }
+  memset(c->search_stats, 0, sizeof(c->search_stats));
+  if (n_qry == 0) return HG_OK;
+  if (n_ref == 0) {
+    memset(out, 0, (size_t)n_qry * top_k * sizeof(hg_hit));
+    memset(n_found, 0, (size_t)n_qry * 4);
+    if (ani_milli) memset(ani_milli, 0, (size_t)n_qry * top_k * 4);
+    return HG_OK;
+  }
+  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
+  uint32_t rmax = 0, qmax = 0;
+  for (uint32_t g = 0; g < n_ref; g++) {
+    if (ref_bits[g] < 1 || ref_bits[g] > 16) { hg_set_error("hg_search_packed: ref sketch %u has hv_quant_bits %u", g, (unsigned)ref_bits[g]); return HG_E_INVALID; }
+    rmax = std::max<uint32_t>(rmax, ref_bits[g]);
+  }
+  for (uint32_t g = 0; g < n_qry && !same; g++) {
+    if (qry_bits[g] < 1 || qry_bits[g] > 16) { hg_set_error("hg_search_packed: query sketch %u has hv_quant_bits %u", g, (unsigned)qry_bits[g]); return HG_E_INVALID; }
+    qmax = std::max<uint32_t>(qmax, qry_bits[g]);
+  }
+  const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;
+  if (rw > ref_stride || (!same && qw > qry_stride)) { hg_set_error("hg_search_packed: row stride below hv_quant_bits * hv_d / 8"); return HG_E_INVALID; }
+  HG_CUDA(cudaSetDevice(c->device));
+  const size_t rb = (size_t)n_ref * hv_d * 2, qb = same ? 0 : (size_t)n_qry * hv_d * 2;
+  const size_t rb_al = (rb + 255) & ~(size_t)255;
+  const size_t rp = ((size_t)n_ref * rw + 255) & ~(size_t)255, qp = same ? 0 : (size_t)n_qry * qw;
+  const size_t n_out = (size_t)n_qry * top_k;
+  void *d_mat, *d_small, *d_pk, *d_res;
+  if ((rc = hg_scratch(c, HG_S_HV, rb + qb + 512, &d_mat))) return rc;
+  if ((rc = hg_scratch(c, HG_S_SMALL, ((size_t)n_ref + n_qry) * 5 + 512, &d_small))) return rc;
+  if ((rc = hg_scratch(c, HG_S_TABLES, rp + qp + 256, &d_pk))) return rc;
+  if ((rc = hg_scratch(c, HG_S_TILES, n_out * (sizeof(hg_hit) + 4) + (size_t)n_qry * 4 + 256, &d_res))) return rc;
+  int16_t *d_ref = (int16_t *)d_mat, *d_qry = same ? d_ref : (int16_t *)((uint8_t *)d_mat + rb_al);
+  int32_t *d_rn = (int32_t *)d_small, *d_qn = same ? d_rn : d_rn + n_ref;
+  uint8_t *d_rbits = (uint8_t *)d_small + ((size_t)n_ref + n_qry) * 4, *d_qbits = same ? d_rbits : d_rbits + n_ref;
+  uint8_t *d_rp = (uint8_t *)d_pk, *d_qp = d_rp + rp;
+  hg_hit *d_out = (hg_hit *)d_res;
+  uint32_t *d_milli = (uint32_t *)(d_out + n_out), *d_nf = d_milli + n_out;
+  auto whole = [&](const uint8_t *packed, uint64_t stride, size_t width, const uint8_t *bits, const int32_t *norm, uint32_t n,
+                   uint8_t *d_stage, uint8_t *d_bits, int32_t *d_norm, int16_t *d_hv) -> int {
+    HG_CUDA(cudaMemcpy2DAsync(d_stage, width, packed, stride, width, n, cudaMemcpyHostToDevice, c->stream));
+    HG_CUDA(cudaMemcpyAsync(d_norm, norm, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
+    HG_CUDA(cudaMemcpyAsync(d_bits, bits, n, cudaMemcpyHostToDevice, c->stream));
+    return hg_launch_unpack(c, d_stage, width, d_bits, n, hv_d, d_hv);
+  };
+  if ((rc = whole(ref_packed, ref_stride, rw, ref_bits, ref_norm, n_ref, d_rp, d_rbits, d_rn, d_ref))) return rc;
+  if (!same && (rc = whole(qry_packed, qry_stride, qw, qry_bits, qry_norm, n_qry, d_qp, d_qbits, d_qn, d_qry))) return rc;
+  if ((rc = search_run(c, d_ref, d_rn, n_ref, d_qry, d_qn, n_qry, hv_d, ksize, top_k, ani_min, path, std::max(rmax, qmax), d_out, d_nf,
+                       d_milli)))
+    return rc;
+  HG_CUDA(cudaMemcpyAsync(out, d_out, n_out * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaMemcpyAsync(n_found, d_nf, (size_t)n_qry * 4, cudaMemcpyDeviceToHost, c->stream));
+  if (ani_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, n_out * 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  return HG_OK;
+}
+
+extern "C" int hg_search_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
+  if (!c || !counts || !ms) { hg_set_error("hg_search_stats: NULL argument"); return HG_E_INVALID; }
+  memcpy(counts, c->search_stats, sizeof(c->search_stats));
+  // floor pass (gather + dist), its select, main pass, its select; the main pass of a one-pass search starts at mark 0
+  const int from[4] = {0, 1, (c->search_ev_used >> 2 & 1) ? 2 : 0, 3};
+  for (int k = 0; k < 4; k++) {
+    ms[k] = -1.0f;
+    if ((c->search_ev_used >> from[k] & 1) && (c->search_ev_used >> (k + 1) & 1))
+      HG_CUDA(cudaEventElapsedTime(&ms[k], c->ev_search[from[k]], c->ev_search[k + 1]));
+  }
+  return HG_OK;
 }

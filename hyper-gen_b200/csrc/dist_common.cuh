@@ -25,7 +25,11 @@ struct DistEpilogue {
 
 // Called by every lane of a warp (converged) with its own candidate; `live` marks lanes
 // whose (li, lj) is inside the matrices.  Survivors are appended with one atomic per warp.
-__device__ __forceinline__ void dist_emit(const DistEpilogue &e, bool live, uint32_t li, uint32_t lj, int32_t dot) {
+// QF: the threshold, its ref-index tie bound and the pre-filter of query column lj come from fl (a search pass,
+// hg_floor) instead of e.ani_th / e.jmin.
+template <bool QF = false>
+__device__ __forceinline__ void dist_emit(const DistEpilogue &e, bool live, uint32_t li, uint32_t lj, int32_t dot,
+                                          const hg_floors &fl = {}) {
   bool keep = false;
   float ani = 0.0f;
   uint32_t gi = 0, gj = 0;
@@ -34,14 +38,18 @@ __device__ __forceinline__ void dist_emit(const DistEpilogue &e, bool live, uint
     gj = e.j0 + lj;
     if (!e.symmetric || gj > gi) {  // dist.rs:253-265: only j > i when ref == query
       const int32_t nr = e.ref_norm[li], nq = e.qry_norm[lj];
+      float th = e.ani_th, jmin = e.jmin;
+      uint32_t imax = 0;
+      if constexpr (QF) { const hg_floor f = fl.q[lj]; th = f.ani; jmin = f.jmin; imax = f.imax; }
       bool cand = true;
-      if (e.jmin > 0.0f) {  // cheap monotone bound first; the exact f32 sequence decides
+      if (jmin > 0.0f) {  // cheap monotone bound first; the exact f32 sequence decides
         const int32_t den = (int32_t)((uint32_t)nr + (uint32_t)nq - (uint32_t)dot);
-        cand = den <= 0 || __int2float_rn(dot) >= e.jmin * __int2float_rn(den);
+        cand = den <= 0 || __int2float_rn(dot) >= jmin * __int2float_rn(den);
       }
       if (cand) {
         ani = ani_from_dot(dot, nr, nq, e.ksize_f);
-        keep = ani >= e.ani_th;
+        if constexpr (QF) keep = ani > th || (ani == th && gi <= imax);
+        else keep = ani >= th;
       }
     }
   }
@@ -64,18 +72,24 @@ __device__ __forceinline__ void dist_emit(const DistEpilogue &e, bool live, uint
 // The same decision without the append: used by the tensor kernels' candidate lists, which evaluate a whole list first
 // and then reserve room for all its survivors with ONE atomic (the counter may live on another GPU: a round trip over
 // NVLink per 32 candidates is what made remote members slow).
-__device__ __forceinline__ bool dist_eval(const DistEpilogue &e, bool live, uint32_t li, uint32_t lj, int32_t dot, float *ani_out) {
+template <bool QF = false>
+__device__ __forceinline__ bool dist_eval(const DistEpilogue &e, bool live, uint32_t li, uint32_t lj, int32_t dot, float *ani_out,
+                                          const hg_floors &fl = {}) {
   if (!live) return false;
   const uint32_t gi = e.i0 + li, gj = e.j0 + lj;
   if (e.symmetric && gj <= gi) return false;
   const int32_t nr = e.ref_norm[li], nq = e.qry_norm[lj];
-  if (e.jmin > 0.0f) {
+  float th = e.ani_th, jmin = e.jmin;
+  uint32_t imax = 0;
+  if constexpr (QF) { const hg_floor f = fl.q[lj]; th = f.ani; jmin = f.jmin; imax = f.imax; }
+  if (jmin > 0.0f) {
     const int32_t den = (int32_t)((uint32_t)nr + (uint32_t)nq - (uint32_t)dot);
-    if (!(den <= 0 || __int2float_rn(dot) >= e.jmin * __int2float_rn(den))) return false;
+    if (!(den <= 0 || __int2float_rn(dot) >= jmin * __int2float_rn(den))) return false;
   }
   const float ani = ani_from_dot(dot, nr, nq, e.ksize_f);
   *ani_out = ani;
-  return ani >= e.ani_th;
+  if constexpr (QF) return ani > th || (ani == th && gi <= imax);
+  return ani >= th;
 }
 
 // ---- arrival flags of a multi-GPU launch (hg_tile_feed) ----
@@ -198,9 +212,10 @@ __device__ __forceinline__ void push_my_units(const hg_push_plan *__restrict__ p
   }
 }
 
-// Host: the Jaccard value below which ANI (dist.rs:154) cannot reach ani_th, lowered by a safety
+// The Jaccard value below which ANI (dist.rs:154) cannot reach ani_th, lowered by a safety
 // margin (0.01 ANI points and 0.1 % relative) that dwarfs every f32 rounding in the exact path.
-inline float dist_jmin(float ani_th, uint32_t ksize) {
+// Host for a scalar threshold; device for the per-query floors of a search pass.
+__host__ __device__ inline float dist_jmin(float ani_th, uint32_t ksize) {
   const double a = (double)ani_th / 100.0 - 1e-4;
   if (!(a > 0.0)) return 0.0f;            // everything (ani >= 0 always) must be evaluated exactly
   if (a >= 1.0) return 1e30f;             // ani is clamped to 100: nothing can pass, J bound irrelevant

@@ -323,8 +323,9 @@ __device__ __noinline__ int32_t n1_correction(const NarrowArgs &na, uint32_t li,
 // Evaluate a warp's parked candidates and append the survivors: pass 1 runs the exact correction + f32 ANI sequence and
 // leaves (keep flag, dot, ANI) in shared memory, ONE atomic reserves room for all survivors (the counter may sit on another
 // GPU), pass 2 writes the records.
-__device__ __forceinline__ void n1_process(const hg::DistEpilogue &ep, const NarrowArgs &na, uint2 *list, float *anis, uint32_t n,
-                                           uint32_t row0, uint32_t col0) {
+template <bool QF>
+__device__ __forceinline__ void n1_process(const hg::DistEpilogue &ep, const hg_floors &fl, const NarrowArgs &na, uint2 *list, float *anis,
+                                           uint32_t n, uint32_t row0, uint32_t col0) {
   if (n == 0) return;
   const uint32_t lane = threadIdx.x & 31;
   uint32_t mine = 0;
@@ -338,7 +339,7 @@ __device__ __forceinline__ void n1_process(const hg::DistEpilogue &ep, const Nar
       if (er | eq) dot = (int32_t)((uint32_t)dot + (uint32_t)n1_correction(na, li, lj, er, eq));
     }
     float ani = 0.0f;
-    const bool keep = hg::dist_eval(ep, live, li, lj, dot, &ani);
+    const bool keep = hg::dist_eval<QF>(ep, live, li, lj, dot, &ani, fl);
     list[e] = make_uint2(c.x | (keep ? 0x80000000u : 0u), (uint32_t)dot);
     anis[e] = ani;
     mine += keep;
@@ -379,7 +380,8 @@ __device__ __forceinline__ void n1_process(const hg::DistEpilogue &ep, const Nar
 // One epilogue warp drains columns [c_begin, c_end) of its 32 TMEM lanes: row `rowl` of the CTA's
 // 128 rows per lane.  x~ . y~ = 4 acc + s_q * X_r + s_r * T_q with X_r = sum x~ of my row and, per
 // column, the centre s_q and T_q = 2 sum(b).  Candidates (rowl, column, x~ . y~) go to `list`.
-__device__ __forceinline__ uint32_t n1_drain(const hg::DistEpilogue &ep, const NarrowArgs &na, uint32_t taddr, int c_begin,
+template <bool QF>
+__device__ __forceinline__ uint32_t n1_drain(const hg::DistEpilogue &ep, const hg_floors &fl, const NarrowArgs &na, uint32_t taddr, int c_begin,
                                              int c_end, const int32_t *s_col, int32_t tr, int32_t sr, int32_t xr, bool row_live,
                                              uint32_t rowl, uint32_t row0, uint32_t col0, uint2 *list, float *anis, uint32_t n_list) {
   const uint32_t lane = threadIdx.x & 31;
@@ -425,7 +427,7 @@ __device__ __forceinline__ uint32_t n1_drain(const hg::DistEpilogue &ep, const N
       const uint32_t total = __shfl_sync(0xffffffffu, inc, 31);
       if (total == 0) continue;
       if (n_list + total > N1_LIST_CAP) {  // evaluate what is parked (slow path: the accumulator stays held)
-        n1_process(ep, na, list, anis, n_list, row0, col0);
+        n1_process<QF>(ep, fl, na, list, anis, n_list, row0, col0);
         n_list = 0;
       }
       uint32_t pos = n_list + inc - cnt;
@@ -439,10 +441,12 @@ __device__ __forceinline__ uint32_t n1_drain(const hg::DistEpilogue &ep, const N
   return n_list;
 }
 
-template <int PUSHW>
+// QF: per-query thresholds (a search pass, PUSHW = 0 only); `fl` is not read otherwise
+template <int PUSHW, bool QF = false>
 __global__ void __launch_bounds__(N1_THREADS + 32 * PUSHW, 1)
 dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry, uint32_t ref_row_base,
-               uint32_t qry_row_base, hg::DistEpilogue ep, NarrowArgs na, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan) {
+               uint32_t qry_row_base, hg::DistEpilogue ep, NarrowArgs na, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan,
+               hg_floors fl) {
   constexpr int STAGES = N1_STAGES, STAGE_BYTES = N1_STAGE_BYTES;
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
@@ -587,9 +591,11 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
           int32_t tq = COL_NEVER, sq = 0, tt = 0;
           if (lj < ep.n_qry) {
             tq = COL_ALWAYS;
-            if (ep.cfrac > 0.0f) {
+            float cq = ep.cfrac;
+            if constexpr (QF) cq = fl.q[lj].cfrac;
+            if (cq > 0.0f) {
               const int32_t nq = ep.qry_norm[lj];
-              if (nq > 0) tq = n1_loosen(__float2int_rd(ep.cfrac * __int2float_rz(nq)) - 1, na.q.e[lj], r_tmax, COL_ALWAYS);
+              if (nq > 0) tq = n1_loosen(__float2int_rd(cq * __int2float_rz(nq)) - 1, na.q.e[lj], r_tmax, COL_ALWAYS);
             }
             sq = na.q.s[lj];
             tt = na.q.a2[lj];
@@ -604,9 +610,11 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
         tr = ROW_ALWAYS; sr = 0; xr = 0;
         live = li < ep.n_ref;
         if (live) {
-          if (ep.cfrac > 0.0f) {
+          float cr = ep.cfrac;
+          if constexpr (QF) cr = *fl.cfrac_row;
+          if (cr > 0.0f) {
             const int32_t nr = ep.ref_norm[li];
-            if (nr > 0) tr = n1_loosen(__float2int_rd(ep.cfrac * __int2float_rz(nr)) - 1, na.r.e[li], q_absmax, ROW_ALWAYS);
+            if (nr > 0) tr = n1_loosen(__float2int_rd(cr * __int2float_rz(nr)) - 1, na.r.e[li], q_absmax, ROW_ALWAYS);
           }
           sr = na.r.s[li];
           xr = (int32_t)((uint32_t)na.r.a2[li] + na.hv_d * (uint32_t)sr);  // sum x~ = 2 sum a + D s
@@ -623,12 +631,12 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
       // my 128 x 256 part of the tile may be empty (below the diagonal, or past the last ref row)
       const bool mine_empty = row0 >= ep.n_ref || (ep.symmetric && (uint64_t)ep.j0 + col0 + N1_BN - 1 <= (uint64_t)ep.i0 + row0);
       if (!mine_empty)
-        n_list = n1_drain(ep, na, tmem_base + ((q * 32u) << 16) + b * N1_BN, half * (N1_BN / 2), (half + 1) * (N1_BN / 2), s_col, tr,
+        n_list = n1_drain<QF>(ep, fl, na, tmem_base + ((q * 32u) << 16) + b * N1_BN, half * (N1_BN / 2), (half + 1) * (N1_BN / 2), s_col, tr,
                           sr, xr, live, q * 32 + lane, row0, col0, list, anis, 0u);
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(mapa_u32(tmem_empty_bar(b), 0));  // this warp's TMEM reads of buffer b are done
-      n1_process(ep, na, list, anis, n_list, row0, col0);                  // exact ANI + append, under the next tiles' MMAs
+      n1_process<QF>(ep, fl, na, list, anis, n_list, row0, col0);          // exact ANI + append, under the next tiles' MMAs
     }
   }
   }  // compute roles
@@ -690,6 +698,7 @@ static int narrow_attrs(hg_ctx *ctx) {
   if (!ctx->n1_attr_set) {
     HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
     HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<N1_PUSH_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
     ctx->n1_attr_set = 1;
   }
   return HG_OK;
@@ -757,17 +766,18 @@ int hg_narrow_prep_rows(hg_ctx *ctx, const hg_narrow_mat *m, uint32_t row0, uint
 int hg_narrow_launch(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                      const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                      uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                     unsigned long long *d_n_hits) {
+                     unsigned long long *d_n_hits, const hg_floors *floors) {
   return hg_narrow_launch_ex(ctx, R, r0, n_ref, i0, d_ref_norm, Q, q0, n_qry, j0, d_qry_norm, ksize, ani_th, symmetric, d_hits, cap,
-                             d_n_hits, 1, 0);
+                             d_n_hits, 1, 0, nullptr, nullptr, floors);
 }
 
 int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                         const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                         uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
                         unsigned long long *d_n_hits, uint32_t walk_mul, uint32_t walk_add, const hg_tile_feed *feed,
-                        const hg_push_plan *push) {
+                        const hg_push_plan *push, const hg_floors *floors) {
   if (n_ref == 0 || n_qry == 0) return HG_OK;
+  if (floors && push) { hg_set_error("hg_narrow_launch: per-query thresholds on a multi-GPU member"); return HG_E_UNSUPPORTED; }
   if (walk_mul == 0 || walk_add >= walk_mul) { hg_set_error("hg_narrow_launch: tile walk %u / %u", walk_add, walk_mul); return HG_E_INVALID; }
   int rc;
   const uint32_t hv_d = R->hv_d;
@@ -829,9 +839,11 @@ int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32
   static const hg_push_plan no_push = {};
   if (push) {  // a member of several GPUs: the launch carries pusher warps that send my operand rows while the tiles are computed
     cfg.blockDim = dim3(N1_THREADS + 32 * N1_PUSH_WARPS, 1, 1);
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<N1_PUSH_WARPS>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push));
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<N1_PUSH_WARPS>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push, hg_floors{}));
+  } else if (floors) {
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<0, true>, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push, *floors));
   } else {
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<0>, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push));
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<0>, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push, hg_floors{}));
   }
   ctx->launches++;
   HG_CUDA(cudaGetLastError());

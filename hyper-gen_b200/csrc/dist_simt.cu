@@ -30,9 +30,11 @@ __device__ __forceinline__ void mac8(int32_t &acc, const uint4 &a, const uint4 &
   }
 }
 
+// QF: per-query thresholds (a search pass); `fl` is not read otherwise
+template <bool QF>
 __global__ void __launch_bounds__(DS_THREADS)
 dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qry, uint32_t hv_d,
-                 hg::DistEpilogue ep) {
+                 hg::DistEpilogue ep, hg_floors fl) {
   __shared__ __align__(16) unsigned char s_a[DS_TILE * DS_ROW_BYTES];
   __shared__ __align__(16) unsigned char s_b[DS_TILE * DS_ROW_BYTES];
 
@@ -83,7 +85,7 @@ dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qr
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const uint32_t li = row0 + ty + 16 * i, lj = col0 + tx + 16 * j;
-      hg::dist_emit(ep, li < ep.n_ref && lj < ep.n_qry, li, lj, acc[i][j]);
+      hg::dist_emit<QF>(ep, li < ep.n_ref && lj < ep.n_qry, li, lj, acc[i][j], fl);
     }
 }
 
@@ -92,7 +94,7 @@ dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qr
 int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t i0,
                         const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry, uint32_t j0,
                         uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                        unsigned long long *d_n_hits) {
+                        unsigned long long *d_n_hits, const hg_floors *floors) {
   if (n_ref == 0 || n_qry == 0) return HG_OK;
   if (hv_d % DS_KS != 0) {
     hg_set_error("hv_d %u must be a multiple of %d", hv_d, DS_KS);
@@ -113,8 +115,12 @@ int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_
     e2.ref_norm = d_ref_norm + (size_t)y0 * DS_TILE;
     e2.n_ref = n_ref - y0 * DS_TILE;
     e2.i0 = i0 + y0 * DS_TILE;
-    dist_simt_kernel<<<dim3(gx, gy), DS_THREADS, 0, ctx->stream>>>(d_ref + (size_t)y0 * DS_TILE * hv_d, d_qry,
-                                                                   hv_d, e2);
+    if (floors)
+      dist_simt_kernel<true><<<dim3(gx, gy), DS_THREADS, 0, ctx->stream>>>(d_ref + (size_t)y0 * DS_TILE * hv_d, d_qry, hv_d, e2,
+                                                                           *floors);
+    else
+      dist_simt_kernel<false><<<dim3(gx, gy), DS_THREADS, 0, ctx->stream>>>(d_ref + (size_t)y0 * DS_TILE * hv_d, d_qry, hv_d, e2,
+                                                                            hg_floors{});
     ctx->launches++;
   }
   HG_CUDA(cudaGetLastError());

@@ -46,16 +46,23 @@ constexpr uint32_t TC_TMEM_COLS = 512;
 // two shift-adds, one add and one compare.  Only lanes that pass run the exact f32 ANI sequence
 // and the compacted append.
 
-// per-column bound of query column lj (INT32_MIN = always take the exact path)
-__device__ __forceinline__ int32_t tc_col_bound(const hg::DistEpilogue &ep, uint32_t lj) {
-  if (!(ep.cfrac > 0.0f) || lj >= ep.n_qry) return INT32_MIN;
+// per-column bound of query column lj (INT32_MIN = always take the exact path).  QF (a search pass): the column's own
+// cfrac, and the launch's smallest positive one for the rows (hg_floors).
+template <bool QF>
+__device__ __forceinline__ int32_t tc_col_bound(const hg::DistEpilogue &ep, const hg_floors &fl, uint32_t lj) {
+  float cfrac = ep.cfrac;
+  if constexpr (QF) cfrac = lj < ep.n_qry ? fl.q[lj].cfrac : 0.0f;
+  if (!(cfrac > 0.0f) || lj >= ep.n_qry) return INT32_MIN;
   const int32_t nq = ep.qry_norm[lj];
-  return nq > 0 ? __float2int_rd(ep.cfrac * __int2float_rz(nq)) - 1 : INT32_MIN;
+  return nq > 0 ? __float2int_rd(cfrac * __int2float_rz(nq)) - 1 : INT32_MIN;
 }
-__device__ __forceinline__ int32_t tc_row_bound(const hg::DistEpilogue &ep, uint32_t li) {
-  if (!(ep.cfrac > 0.0f) || li >= ep.n_ref) return INT32_MIN / 2;
+template <bool QF>
+__device__ __forceinline__ int32_t tc_row_bound(const hg::DistEpilogue &ep, const hg_floors &fl, uint32_t li) {
+  float cfrac = ep.cfrac;
+  if constexpr (QF) cfrac = *fl.cfrac_row;
+  if (!(cfrac > 0.0f) || li >= ep.n_ref) return INT32_MIN / 2;
   const int32_t nr = ep.ref_norm[li];
-  return nr > 0 ? __float2int_rd(ep.cfrac * __int2float_rz(nr)) - 1 : INT32_MIN / 2;
+  return nr > 0 ? __float2int_rd(cfrac * __int2float_rz(nr)) - 1 : INT32_MIN / 2;
 }
 
 // Candidates are not evaluated while the accumulators are being drained: each epilogue warp parks
@@ -67,7 +74,9 @@ constexpr int TC_LIST_CAP = 256;  // candidates per warp list (8 B each); a full
 
 // pass 1: exact f32 ANI of every parked candidate; ONE atomic reserves room for the survivors (the counter may sit on
 // another GPU); pass 2 writes the records
-__device__ __forceinline__ void tc_process(const hg::DistEpilogue &ep, uint2 *list, float *anis, uint32_t n, uint32_t row0, uint32_t col0) {
+template <bool QF>
+__device__ __forceinline__ void tc_process(const hg::DistEpilogue &ep, const hg_floors &fl, uint2 *list, float *anis, uint32_t n,
+                                           uint32_t row0, uint32_t col0) {
   if (n == 0) return;
   const uint32_t lane = threadIdx.x & 31;
   uint32_t mine = 0;
@@ -75,7 +84,7 @@ __device__ __forceinline__ void tc_process(const hg::DistEpilogue &ep, uint2 *li
     const uint2 c = list[e];
     const uint32_t li = row0 + (c.x >> 8), lj = col0 + (c.x & 255u);
     float ani = 0.0f;
-    const bool keep = hg::dist_eval(ep, li < ep.n_ref && lj < ep.n_qry, li, lj, (int32_t)c.y, &ani);
+    const bool keep = hg::dist_eval<QF>(ep, li < ep.n_ref && lj < ep.n_qry, li, lj, (int32_t)c.y, &ani, fl);
     if (keep) list[e].x = c.x | 0x80000000u;
     anis[e] = ani;
     mine += keep;
@@ -116,7 +125,8 @@ __device__ __forceinline__ void tc_process(const hg::DistEpilogue &ep, uint2 *li
 // One epilogue warp drains columns [c_begin, c_end) of its 32 TMEM lanes (three accumulators at
 // column offsets 0, BN, 2 BN from taddr): row `rowl` of the tile per lane, query columns col0 + c.
 // Appends the candidates to list[0..n_list); returns the new n_list.
-__device__ __forceinline__ uint32_t tc_drain(const hg::DistEpilogue &ep, uint32_t taddr, int c_begin, int c_end,
+template <bool QF>
+__device__ __forceinline__ uint32_t tc_drain(const hg::DistEpilogue &ep, const hg_floors &fl, uint32_t taddr, int c_begin, int c_end,
                                              const int32_t *s_tq, int32_t tr, bool row_live, uint32_t rowl, uint32_t row0,
                                              uint32_t col0, uint2 *list, float *anis, uint32_t n_list) {
   const uint32_t lane = threadIdx.x & 31;
@@ -164,7 +174,7 @@ __device__ __forceinline__ uint32_t tc_drain(const hg::DistEpilogue &ep, uint32_
       const uint32_t total = __shfl_sync(0xffffffffu, inc, 31);
       if (total == 0) continue;
       if (n_list + total > TC_LIST_CAP) {  // evaluate what is parked (slow path: TMEM stays held)
-        tc_process(ep, list, anis, n_list, row0, col0);
+        tc_process<QF>(ep, fl, list, anis, n_list, row0, col0);
         n_list = 0;
       }
       uint32_t pos = n_list + inc - cnt;
@@ -238,11 +248,13 @@ struct PairTiles {
   }
 };
 
-template <int PUSHW>
+// QF: per-query thresholds (a search pass, PUSHW = 0 only); `fl` is not read otherwise
+template <int PUSHW, bool QF = false>
 __global__ void __launch_bounds__(TC_THREADS + 32 * PUSHW, 1)
 dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
                 uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len,
-                hg::DistEpilogue ep, uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan) {
+                hg::DistEpilogue ep, uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan,
+                hg_floors fl) {
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
   if (feed.seq_ptr) feed.seq = *feed.seq_ptr;
@@ -391,9 +403,9 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
       int32_t tr = 0;
       auto bounds = [&]() {
         const int t = threadIdx.x - 64;
-        if (t < TC_BN) s_tq[t] = tc_col_bound(ep, col0 + t);
+        if (t < TC_BN) s_tq[t] = tc_col_bound<QF>(ep, fl, col0 + t);
         asm volatile("bar.sync 1, %0;" ::"r"(32 * TC_EPI_WARPS) : "memory");
-        tr = tc_row_bound(ep, li);
+        tr = tc_row_bound<QF>(ep, fl, li);
       };
       if (early) bounds();
       // my 128 x 128 part of the tile may be empty (below the diagonal, or past the last ref row)
@@ -406,12 +418,12 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
       }
       uint32_t n_list = 0;
       if (!mine_empty)
-        n_list = tc_drain(ep, tmem_base + ((q * 32u) << 16), half * (TC_BN / 2), (half + 1) * (TC_BN / 2), s_tq, tr,
+        n_list = tc_drain<QF>(ep, fl, tmem_base + ((q * 32u) << 16), half * (TC_BN / 2), (half + 1) * (TC_BN / 2), s_tq, tr,
                           li < ep.n_ref, q * 32 + lane, row0, col0, list, anis, 0u);
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(te);  // this warp's TMEM reads are done: the next tile's MMAs may start
-      tc_process(ep, list, anis, n_list, row0, col0);  // exact ANI + append, under the next tile's mainloop
+      tc_process<QF>(ep, fl, list, anis, n_list, row0, col0);  // exact ANI + append, under the next tile's mainloop
     }
   }
   }  // compute roles
@@ -454,6 +466,7 @@ static int tc_attrs(hg_ctx *ctx) {
   if (!ctx->tc_attr_set) {
     HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
     HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<TC_PUSH_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
     ctx->tc_attr_set = 1;
   }
   return HG_OK;
@@ -500,9 +513,9 @@ int hg_tc_split_rows(hg_ctx *ctx, const hg_tc_mat *m, uint32_t row0, uint32_t ro
 // rows [r0, r0 + n_ref) of R against rows [q0, q0 + n_qry) of Q (both split); norms point at the windows' first rows
 int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                  const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
-                 float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits) {
+                 float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, const hg_floors *floors) {
   return hg_tc_launch_ex(ctx, R, r0, n_ref, i0, d_ref_norm, Q, q0, n_qry, j0, d_qry_norm, ksize, ani_th, symmetric, d_hits, cap,
-                         d_n_hits, 1, 0);
+                         d_n_hits, 1, 0, nullptr, nullptr, floors);
 }
 
 int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int8_t *planes, hg_tc_mat *m) {
@@ -516,8 +529,9 @@ int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_
 int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                     const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
                     float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, uint32_t walk_mul,
-                    uint32_t walk_add, const hg_tile_feed *feed, const hg_push_plan *push) {
+                    uint32_t walk_add, const hg_tile_feed *feed, const hg_push_plan *push, const hg_floors *floors) {
   if (n_ref == 0 || n_qry == 0) return HG_OK;
+  if (floors && push) { hg_set_error("hg_tc_launch: per-query thresholds on a multi-GPU member"); return HG_E_UNSUPPORTED; }
   hg_tile_feed fd = {};
   if (feed) fd = *feed;
   if (walk_mul == 0 || walk_add >= walk_mul) { hg_set_error("hg_tc_launch: tile walk %u / %u", walk_add, walk_mul); return HG_E_INVALID; }
@@ -565,10 +579,13 @@ int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref
   if (push) {  // a member of several GPUs: pusher warps send my limb-plane rows while the tiles are computed
     cfg.blockDim = dim3(TC_THREADS + 32 * TC_PUSH_WARPS, 1, 1);
     HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<TC_PUSH_WARPS>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul,
-                               walk_add, fd, *push));
+                               walk_add, fd, *push, hg_floors{}));
+  } else if (floors) {
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0, true>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul,
+                               walk_add, fd, no_push, *floors));
   } else {
     HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul, walk_add, fd,
-                               no_push));
+                               no_push, hg_floors{}));
   }
   ctx->launches++;
   HG_CUDA(cudaGetLastError());

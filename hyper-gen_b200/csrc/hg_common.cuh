@@ -160,6 +160,11 @@ struct hg_ctx {
   // hg_dist_dev with the single-plane path forced: the pre-pass verdict is not waited for (hg_dist_status reads it)
   const uint32_t *pending_stats[2];
   uint32_t pending_nsets[2];
+  // the last search (hg_search_stats): sample rows, candidates of the floor and the main pass, reruns; with profiling
+  // on, events at its step boundaries (created on first use)
+  uint64_t search_stats[4];
+  cudaEvent_t ev_search[5];
+  int search_ev_used;
 };
 
 // stage boundaries: 0 start, 1 after staging/memsets, 2 after k-mer hash, 3 after encode,
@@ -183,20 +188,20 @@ int hg_cuda_fail(cudaError_t e, const char *what, const char *file, int line);
 // Grow-only device scratch slots.  A slot has one tenant per entry point; entry points of one
 // context never run concurrently (one stream), so slots may be shared between them.
 enum hg_scratch_slot {
-  HG_S_SEQ = 0,        // staged sequence bytes (two halves when the H2D pipeline is active)
-  HG_S_DESC = 1,       // hg_genome_desc[] (+ sentinels)
+  HG_S_SEQ = 0,        // staged sequence bytes (two halves when the H2D pipeline is active); search: the sample rows
+  HG_S_DESC = 1,       // hg_genome_desc[] (+ sentinels); search: the per-query floors
   HG_S_TABLES = 2,     // per-genome hash tables / explicit hash sets
   HG_S_COUNTS = 3,     // distinct-hash counters; dist: the hit counter of the host entry
   HG_S_HV = 4,         // int16 HVs (sketch output staging; dist: both matrices of the host entry)
-  HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry
+  HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass
   HG_S_SMALL = 6,      // norms / bits / counts per sketch
   HG_S_MISC = 7,       // CTA -> genome map, |hv| max, probe sink
   HG_S_REF_LIMBS = 8,  // s8 limb planes of the ref matrix (dist_tc)
   HG_S_QRY_LIMBS = 9,  // s8 limb planes of the query matrix (dist_tc)
-  HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort
-  HG_S_SORT_CNT = 11,  // digit counters of the hit sort
+  HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort; search: the per-query segments
+  HG_S_SORT_CNT = 11,  // digit counters of the hit sort; search: per-query counts and offsets
   HG_S_NARROW_META = 12,  // per-row constants + outlier lists of the single-plane dist path (dist_narrow)
-  HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu)
+  HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entry
   HG_S_COUNT = 14
 };
 // scratch slot `slot` grown to at least `bytes` (contents not preserved)
@@ -208,6 +213,18 @@ enum hg_dist_path { HG_PATH_AUTO = 0, HG_PATH_SIMT = 1, HG_PATH_TWO_LIMB = 2, HG
 constexpr int32_t HG_LIMB_MAX_ABS = 8127;  // the largest |x| that splits into two s8 limbs x = 128 h + l (13 bits)
 // sets what hg_dist_last_path / hg_dist_last_reason report
 void hg_dist_record(hg_ctx *ctx, int path, const char *fmt, ...);
+
+// Per-query thresholds of a search pass (hg_search_*), in place of the scalar ani_th: query column j of a launch keeps
+// the pairs (i, j) whose key (ANI desc, ref index i asc) is at least (q[j].ani, q[j].imax) - ani > q[j].ani, or
+// ani == q[j].ani and i <= q[j].imax - and q[j].jmin / q[j].cfrac are dist_jmin's pre-filter constants for q[j].ani.
+// *cfrac_row is the smallest POSITIVE cfrac of the launch: the row term of the tensor kernels' candidate bound, valid
+// for every column because cfrac_row * n_r + cfrac_j * n_q <= cfrac_j * (n_r + n_q).  A column whose cfrac is 0 (its
+// floor is <= 0) is always a candidate and does not lower the row term of the others.
+struct __align__(16) hg_floor { float ani, jmin, cfrac; uint32_t imax; };
+struct hg_floors {
+  const hg_floor *q;       // indexed like the launch's query norms
+  const float *cfrac_row;  // device scalar (0: no positive cfrac)
+};
 
 // ---- kernel launchers (all asynchronous on ctx->stream) ----
 
@@ -235,7 +252,7 @@ int hg_launch_unpack(hg_ctx *ctx, const uint8_t *d_packed, uint64_t row_stride,
 int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref,
                         uint32_t i0, const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry,
                         uint32_t j0, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric,
-                        hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits);
+                        hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, const hg_floors *floors = nullptr);
 // A dist launch that is one member of several GPUs (csrc/peer.cu) walks a host-built list of ITS tiles instead of the
 // arithmetic enumeration, ordered by when the rows they read arrive, and its TMA producer waits for the arrival flags
 // of those rows: the operand exchange over NVLink overlaps the tile computation.
@@ -298,12 +315,14 @@ int hg_tc_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d
 int hg_tc_split_rows(hg_ctx *ctx, const hg_tc_mat *m, uint32_t row0, uint32_t rows);
 int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                  const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
-                 float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits);
+                 float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits,
+                 const hg_floors *floors = nullptr);
 int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int8_t *planes, hg_tc_mat *m);
 int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                     const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
                     float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, uint32_t walk_mul,
-                    uint32_t walk_add, const hg_tile_feed *feed = nullptr, const hg_push_plan *push = nullptr);
+                    uint32_t walk_add, const hg_tile_feed *feed = nullptr, const hg_push_plan *push = nullptr,
+                    const hg_floors *floors = nullptr);
 void hg_tc_tile_shape(uint32_t *rows, uint32_t *cols);
 // single s8 plane (x = 2a + s) + sparse outlier corrections (dist_narrow.cu): one matrix in that form, prepared
 // piecewise (rows as they arrive over PCIe) or at once
@@ -334,16 +353,26 @@ int hg_narrow_prep_rows(hg_ctx *ctx, const hg_narrow_mat *m, uint32_t row0, uint
 int hg_narrow_launch(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                      const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                      uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                     unsigned long long *d_n_hits);
+                     unsigned long long *d_n_hits, const hg_floors *floors = nullptr);
 // as hg_narrow_launch for one member of `walk_mul` GPUs sharing the tile enumeration (takes tiles walk_add, walk_add + walk_mul, ...)
 int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                         const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                         uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
                         unsigned long long *d_n_hits, uint32_t walk_mul, uint32_t walk_add, const hg_tile_feed *feed = nullptr,
-                        const hg_push_plan *push = nullptr);
+                        const hg_push_plan *push = nullptr, const hg_floors *floors = nullptr);
 void hg_narrow_tile_shape(uint32_t *rows, uint32_t *cols);
 int hg_narrow_verdict(hg_ctx *ctx, const hg_narrow_mat *A, const hg_narrow_mat *B, int32_t *absmax_out, uint64_t *outliers_out);
 int hg_launch_int_peak(hg_ctx *ctx, int which, uint32_t iters, uint32_t *d_sink, uint32_t blocks);
 // max |hv| over a device matrix (decides the dist path); result in *d_out (int32)
 int hg_launch_sort_hits(hg_ctx *ctx, hg_hit *d_hits, uint64_t n, uint32_t *d_milli);
+// top-k search (search.cu): s sample rows of the ref matrix (row t = ref row t * n_ref / s) into d_out / d_out_norm
+int hg_launch_search_gather(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t hv_d, uint32_t s,
+                            int16_t *d_out, int32_t *d_out_norm);
+// candidates (query indices < n_qry) -> per query the top_k best by (ANI desc, i asc): out / n_found / milli as
+// hg_search_dev writes them, and the top_k-th key per query (0: fewer candidates) in d_floor_key; each may be NULL
+int hg_launch_search_select(hg_ctx *ctx, const hg_hit *d_cand, uint64_t n_cand, uint32_t n_qry, uint32_t top_k, hg_hit *d_out,
+                            uint32_t *d_n_found, uint32_t *d_milli, unsigned long long *d_floor_key);
+// the floor pass's top_k-th keys (over s sample rows of n_ref) -> the main pass's per-query thresholds (hg_floors)
+int hg_launch_search_floors(hg_ctx *ctx, const unsigned long long *d_floor_key, uint32_t n_qry, float ani_min, uint32_t ksize,
+                            uint32_t n_ref, uint32_t s, hg_floor *d_floors, float *d_cfrac_row);
 int hg_launch_absmax(hg_ctx *ctx, const int16_t *d_hv, uint64_t n_elems, int32_t *d_out);

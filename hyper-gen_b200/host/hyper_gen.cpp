@@ -13,6 +13,9 @@
 // CLI (same flags as src/utils.rs:44-126):
 //   hyper-gen sketch -p <dir> -o <out> [-k 21] [-s 1500] [-S 123] [-d 4096] [-C true] [-t 16]
 //   hyper-gen dist   -r <ref sketch> -q <query sketch> -o <out> [-a 85.0]
+//   hyper-gen search -r <ref sketch> -q <query sketch> -o <out> [-n 10] [-a 0.0]
+//       the -n best refs of every query with ANI >= -a (ties by ascending ref index), one line per result,
+//       queries in file order.  Runs on one GPU; sharding it over the GPUs of an hg_group is not done yet.
 // The GPU path is the only path (`-D gpu` is implied): there is no CPU fallback.
 #include <algorithm>
 #include <chrono>
@@ -55,6 +58,12 @@ struct FileSketch {  // src/types.rs:224-235
 struct SketchDist {  // src/types.rs:237-245
   std::string path_ref_sketch, path_query_sketch, out_file;
   float ani_threshold = 85.0f;
+};
+
+struct SketchSearch {
+  std::string path_ref_sketch, path_query_sketch, out_file;
+  uint32_t top_k = 10;
+  float ani_min = 0.0f;
 };
 
 }  // namespace types
@@ -351,24 +360,69 @@ void dist(const types::SketchDist &sd) {
 
 }  // namespace dist
 
+namespace search {
+
+void search(const types::SketchSearch &ss) {
+  auto ref = utils::load_sketch(ss.path_ref_sketch);
+  auto qry = utils::load_sketch(ss.path_query_sketch);
+  if (ref.empty() || qry.empty()) die("empty sketch file");
+  if (ref[0].ksize != qry[0].ksize) die("Ref and query sketches use different kmer sizes!");
+  if (ref[0].hv_d != qry[0].hv_d) die("Ref and query sketches use different HV dimensions!");
+  const size_t D = ref[0].hv_d, R = ref.size(), Q = qry.size(), K = ss.top_k;
+  const dist::Stacked rs = dist::stack(ref, D), qs = dist::stack(qry, D);
+  hg_ctx *ctx = nullptr;
+  check(hg_init(0, &ctx), "hg_init");
+  std::vector<hg_hit> hits(Q * K);
+  std::vector<uint32_t> n_found(Q), milli(Q * K);
+  check(hg_search_packed(ctx, rs.packed.data(), 2 * D, rs.bits.data(), rs.norm.data(), (uint32_t)R, qs.packed.data(), 2 * D,
+                         qs.bits.data(), qs.norm.data(), (uint32_t)Q, (uint32_t)D, ref[0].ksize, ss.top_k, ss.ani_min, 0, hits.data(),
+                         n_found.data(), milli.data()),
+        "hg_search_packed");
+  hg_destroy(ctx);
+  std::string out;
+  char buf[64];
+  size_t lines = 0;
+  for (size_t j = 0; j < Q; j++)
+    for (size_t r = 0; r < n_found[j]; r++, lines++) {
+      const size_t t = j * K + r;
+      out += ref[hits[t].i].file_str; out += '\t'; out += qry[j].file_str;
+      snprintf(buf, sizeof(buf), "\t%u.%03u\n", milli[t] / 1000u, milli[t] % 1000u);
+      out += buf;
+    }
+  std::ofstream f(ss.out_file, std::ios::binary);
+  if (!f) die("Dump search file failed!");
+  f.write(out.data(), (std::streamsize)out.size());
+  fprintf(stdout, "Output %zu results (top %u per query, ANI >= %.1f) for %zu queries to file %s\n", lines, ss.top_k,
+          (double)ss.ani_min, Q, ss.out_file.c_str());
+}
+
+}  // namespace search
+
 int main(int argc, char **argv) {
-  if (argc < 2) die("usage: hyper-gen <sketch|dist> ...");
+  if (argc < 2) die("usage: hyper-gen <sketch|dist|search> ...");
   const std::string mode = argv[1];
   types::SketchParams sp;
   types::SketchDist sd;
+  types::SketchSearch ss;
+  bool ani_given = false;
   for (int i = 2; i + 1 < argc; i += 2) {
     const std::string k = argv[i], v = argv[i + 1];
     if (k == "-p" || k == "--path") sp.path = v;
-    else if (k == "-o" || k == "--out") { sp.out_file = v; sd.out_file = v; }
-    else if (k == "-r" || k == "--path_r") sd.path_ref_sketch = v;
-    else if (k == "-q" || k == "--path_q") sd.path_query_sketch = v;
+    else if (k == "-o" || k == "--out") { sp.out_file = v; sd.out_file = v; ss.out_file = v; }
+    else if (k == "-r" || k == "--path_r") { sd.path_ref_sketch = v; ss.path_ref_sketch = v; }
+    else if (k == "-q" || k == "--path_q") { sd.path_query_sketch = v; ss.path_query_sketch = v; }
+    else if (k == "-n" || k == "--top_k") {
+      const long n = atol(v.c_str());
+      if (n < 1 || n > 1024) die("-n must be in 1..1024");
+      ss.top_k = (uint32_t)n;
+    }
     else if (k == "-t" || k == "--thread") sp.threads = atoi(v.c_str());
     else if (k == "-C" || k == "--canonical") sp.canonical = (v == "true" || v == "1");
     else if (k == "-k" || k == "--ksize") sp.ksize = (uint8_t)atoi(v.c_str());
     else if (k == "-S" || k == "--seed") sp.seed = strtoull(v.c_str(), nullptr, 10);
     else if (k == "-s" || k == "--scaled") sp.scaled = strtoull(v.c_str(), nullptr, 10);
     else if (k == "-d" || k == "--hv_d") sp.hv_d = strtoull(v.c_str(), nullptr, 10);
-    else if (k == "-a" || k == "--ani_th") sd.ani_threshold = (float)atof(v.c_str());
+    else if (k == "-a" || k == "--ani_th") { sd.ani_threshold = (float)atof(v.c_str()); ani_given = true; }
     else if (k == "-D" || k == "--device" || k == "-m" || k == "--sketch_method" || k == "-Q" || k == "--quant_scale") {}
     else die("unknown flag " + k);
   }
@@ -378,6 +432,10 @@ int main(int argc, char **argv) {
   } else if (mode == "dist") {
     if (sd.path_ref_sketch.empty() || sd.path_query_sketch.empty() || sd.out_file.empty()) die("dist needs -r -q -o");
     dist::dist(sd);
+  } else if (mode == "search") {
+    if (ss.path_ref_sketch.empty() || ss.path_query_sketch.empty() || ss.out_file.empty()) die("search needs -r -q -o");
+    if (ani_given) ss.ani_min = sd.ani_threshold;
+    search::search(ss);
   } else {
     die("unknown subcommand " + mode);
   }

@@ -342,6 +342,39 @@ HG_API int hg_peer_timeline(hg_peer *p, unsigned long long out_ns[32]);
 /* the root's hit list and counter as this member addresses them (device pointers) */
 HG_API int hg_peer_hit_buffers(hg_peer *p, int root, hg_hit **d_hits, unsigned long long **d_count);
 
+/* ---- top-k search: the best-matching refs of every query ------------------------------------------
+ * Every (i, j) of ref rows R x query rows Q, as hg_dist with symmetric = 0 (the same pointers for ref and
+ * query are a plain R x R search, self hits included).  For query j the result is the refs with the top_k
+ * largest ANIs among those with ani >= ani_min, ordered by ANI descending and, for equal ANIs, by ascending
+ * ref index i; the tie rule also decides membership at the top_k-th place, so the set is exact.  Every
+ * record's dot and ANI are bit-identical to hg_dist's.
+ *   out        n_qry * top_k records: query j's are out[j * top_k .. j * top_k + n_found[j]), with i = ref
+ *              index and j = query index; the unused slots are zeroed
+ *   n_found[j] = min(top_k, number of refs with ani >= ani_min)
+ *   ani_milli  may be NULL: each record's ANI in thousandths, rounded as hg_sort_hits_dev rounds it (0 in
+ *              the unused slots)
+ *   top_k      1..1024, else HG_E_INVALID.  n_ref == 0 or n_qry == 0: HG_OK with every n_found 0.
+ *   path       as hg_dist (0 auto, 1 SIMT, 2 two-limb, 3 single plane) with the same choice and fallbacks;
+ *              hg_dist_last_path / hg_dist_last_reason report the main pass.
+ * Both entries return with the result complete.  The candidate lists between the passes are library scratch
+ * that grows as a pass needs it (DESIGN.md §4, "Top-k search"); no candidate is dropped. */
+HG_API int hg_search_dev(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm2, uint32_t n_ref,
+                         const int16_t *d_qry, const int32_t *d_qry_norm2, uint32_t n_qry, uint32_t hv_d,
+                         uint32_t ksize, uint32_t top_k, float ani_min, int path,
+                         hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_ani_milli /* may be NULL */);
+/* The same from the rows as the sketch files hold them (as hg_dist_packed: packed bytes + hv_quant_bits +
+ * norms, unpacked on the device); results in host memory. */
+HG_API int hg_search_packed(hg_ctx *ctx, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_quant_bits,
+                            const int32_t *ref_norm2, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                            const uint8_t *qry_quant_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d,
+                            uint32_t ksize, uint32_t top_k, float ani_min, int path,
+                            hg_hit *out, uint32_t *n_found, uint32_t *ani_milli /* may be NULL */);
+/* Measurement hook of the last search: counts = {sample rows s (= n_ref: one pass), floor-pass candidates,
+ * main-pass candidates, reruns after a candidate list outgrew its scratch}; ms = device time of the floor
+ * pass (gather + dist), its select, the main pass, its select (-1 where not run or profiling is off, see
+ * hg_set_profiling). */
+HG_API int hg_search_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
+
 /* Which path the last hg_dist / hg_dist_dev took (1 SIMT, 2 two-limb tensor, 3 single-plane tensor) and why. */
 HG_API int hg_dist_last_path(hg_ctx *ctx);
 HG_API const char *hg_dist_last_reason(hg_ctx *ctx);
