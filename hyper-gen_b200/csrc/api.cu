@@ -1367,39 +1367,46 @@ extern "C" int hg_search_dev(hg_ctx *c, const int16_t *d_ref, const int32_t *d_r
                     d_ani_milli);
 }
 
-// The rows as the sketch files hold them: whole copies of the packed bytes, decompress_file_sketch on the device (as
-// hg_dist_packed), then the search; the results come back to the host.
-extern "C" int hg_search_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits, const int32_t *ref_norm,
-                                uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
-                                const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
-                                int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli) {
-  if (!c || (n_ref && (!ref_packed || !ref_bits || !ref_norm)) || (n_qry && (!qry_packed || !qry_bits || !qry_norm || !out || !n_found))) {
-    hg_set_error("hg_search_packed: NULL argument"); return HG_E_INVALID;
+int hg_search_packed_check(const char *who, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                           const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
+                           const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t top_k, int path, const hg_hit *out,
+                           const uint32_t *n_found) {
+  if ((n_ref && (!ref_packed || !ref_bits || !ref_norm)) || (n_qry && (!qry_packed || !qry_bits || !qry_norm || !out || !n_found))) {
+    hg_set_error("%s: NULL argument", who); return HG_E_INVALID;
   }
   int rc;
-  if ((rc = search_check("hg_search_packed", hv_d, top_k, path))) return rc;
-  if (ref_stride % 4 != 0 || qry_stride % 4 != 0) { hg_set_error("hg_search_packed: row stride %% 4"); return HG_E_INVALID; }
-  memset(c->search_stats, 0, sizeof(c->search_stats));
-  if (n_qry == 0) return HG_OK;
-  if (n_ref == 0) {
-    memset(out, 0, (size_t)n_qry * top_k * sizeof(hg_hit));
-    memset(n_found, 0, (size_t)n_qry * 4);
-    if (ani_milli) memset(ani_milli, 0, (size_t)n_qry * top_k * 4);
-    return HG_OK;
-  }
-  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
+  if ((rc = search_check(who, hv_d, top_k, path))) return rc;
+  if (ref_stride % 4 != 0 || qry_stride % 4 != 0) { hg_set_error("%s: row stride %% 4", who); return HG_E_INVALID; }
+  return HG_OK;
+}
+
+int hg_search_packed_bits(const char *who, const uint8_t *ref_bits, uint32_t n_ref, uint64_t ref_stride, const uint8_t *qry_bits,
+                          uint32_t n_qry, uint64_t qry_stride, bool same, uint32_t hv_d, uint32_t *rmax_out, uint32_t *qmax_out) {
   uint32_t rmax = 0, qmax = 0;
   for (uint32_t g = 0; g < n_ref; g++) {
-    if (ref_bits[g] < 1 || ref_bits[g] > 16) { hg_set_error("hg_search_packed: ref sketch %u has hv_quant_bits %u", g, (unsigned)ref_bits[g]); return HG_E_INVALID; }
+    if (ref_bits[g] < 1 || ref_bits[g] > 16) { hg_set_error("%s: ref sketch %u has hv_quant_bits %u", who, g, (unsigned)ref_bits[g]); return HG_E_INVALID; }
     rmax = std::max<uint32_t>(rmax, ref_bits[g]);
   }
   for (uint32_t g = 0; g < n_qry && !same; g++) {
-    if (qry_bits[g] < 1 || qry_bits[g] > 16) { hg_set_error("hg_search_packed: query sketch %u has hv_quant_bits %u", g, (unsigned)qry_bits[g]); return HG_E_INVALID; }
+    if (qry_bits[g] < 1 || qry_bits[g] > 16) { hg_set_error("%s: query sketch %u has hv_quant_bits %u", who, g, (unsigned)qry_bits[g]); return HG_E_INVALID; }
     qmax = std::max<uint32_t>(qmax, qry_bits[g]);
   }
   const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;
-  if (rw > ref_stride || (!same && qw > qry_stride)) { hg_set_error("hg_search_packed: row stride below hv_quant_bits * hv_d / 8"); return HG_E_INVALID; }
-  HG_CUDA(cudaSetDevice(c->device));
+  if (rw > ref_stride || (!same && qw > qry_stride)) { hg_set_error("%s: row stride below hv_quant_bits * hv_d / 8", who); return HG_E_INVALID; }
+  *rmax_out = rmax;
+  *qmax_out = qmax;
+  return HG_OK;
+}
+
+// The rows as the sketch files hold them: whole copies of the packed bytes (rmax * hv_d / 8 bytes of every ref row,
+// qmax * hv_d / 8 of every query row), decompress_file_sketch on the device (as hg_dist_packed), then the search.  The
+// result stays in the context's HG_S_TILES scratch: *d_out / *d_n_found / *d_milli.
+int hg_search_packed_run(hg_ctx *c, bool same, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                         const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
+                         const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min, int path,
+                         uint32_t rmax, uint32_t qmax, hg_hit **d_out_p, uint32_t **d_nf_p, uint32_t **d_milli_p) {
+  int rc;
+  const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;
   const size_t rb = (size_t)n_ref * hv_d * 2, qb = same ? 0 : (size_t)n_qry * hv_d * 2;
   const size_t rb_al = (rb + 255) & ~(size_t)255;
   const size_t rp = ((size_t)n_ref * rw + 255) & ~(size_t)255, qp = same ? 0 : (size_t)n_qry * qw;
@@ -1427,11 +1434,73 @@ extern "C" int hg_search_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t r
   if ((rc = search_run(c, d_ref, d_rn, n_ref, d_qry, d_qn, n_qry, hv_d, ksize, top_k, ani_min, path, std::max(rmax, qmax), d_out, d_nf,
                        d_milli)))
     return rc;
+  *d_out_p = d_out;
+  *d_nf_p = d_nf;
+  *d_milli_p = d_milli;
+  return HG_OK;
+}
+
+extern "C" int hg_search_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits, const int32_t *ref_norm,
+                                uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
+                                const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
+                                int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli) {
+  if (!c) { hg_set_error("hg_search_packed: NULL argument"); return HG_E_INVALID; }
+  int rc;
+  if ((rc = hg_search_packed_check("hg_search_packed", ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits,
+                                   qry_norm, n_qry, hv_d, top_k, path, out, n_found)))
+    return rc;
+  memset(c->search_stats, 0, sizeof(c->search_stats));
+  if (n_qry == 0) return HG_OK;
+  if (n_ref == 0) {
+    memset(out, 0, (size_t)n_qry * top_k * sizeof(hg_hit));
+    memset(n_found, 0, (size_t)n_qry * 4);
+    if (ani_milli) memset(ani_milli, 0, (size_t)n_qry * top_k * 4);
+    return HG_OK;
+  }
+  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
+  uint32_t rmax, qmax;
+  if ((rc = hg_search_packed_bits("hg_search_packed", ref_bits, n_ref, ref_stride, qry_bits, n_qry, qry_stride, same, hv_d, &rmax, &qmax)))
+    return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  hg_hit *d_out;
+  uint32_t *d_nf, *d_milli;
+  if ((rc = hg_search_packed_run(c, same, ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits, qry_norm,
+                                 n_qry, hv_d, ksize, top_k, ani_min, path, rmax, qmax, &d_out, &d_nf, &d_milli)))
+    return rc;
+  const size_t n_out = (size_t)n_qry * top_k;
   HG_CUDA(cudaMemcpyAsync(out, d_out, n_out * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
   HG_CUDA(cudaMemcpyAsync(n_found, d_nf, (size_t)n_qry * 4, cudaMemcpyDeviceToHost, c->stream));
   if (ani_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, n_out * 4, cudaMemcpyDeviceToHost, c->stream));
   HG_CUDA(cudaStreamSynchronize(c->stream));
   return HG_OK;
+}
+
+int hg_search_merge(hg_ctx *c, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0, uint32_t n_qry,
+                    uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli) {
+  if (n_qry == 0) return HG_OK;
+  int rc;
+  void *d_status;
+  if ((rc = hg_scratch(c, HG_S_MISC, 256, &d_status))) return rc;
+  HG_CUDA(cudaMemsetAsync(d_status, 0, 4, c->stream));
+  if ((rc = hg_launch_search_merge(c, n_lists, d_in, d_in_found, i0, n_qry, top_k, d_out, d_n_found, d_milli, (uint32_t *)d_status)))
+    return rc;
+  uint32_t status = 0;
+  HG_CUDA(cudaMemcpyAsync(&status, d_status, 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  if (status & 1) { hg_set_error("hg_search_merge_dev: a ref index i + i0 does not fit 32 bits"); return HG_E_INVALID; }
+  if (status & 2) { hg_set_error("hg_search_merge_dev: an input n_found exceeds top_k %u", top_k); return HG_E_INVALID; }
+  return HG_OK;
+}
+
+extern "C" int hg_search_merge_dev(hg_ctx *c, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0,
+                                   uint32_t n_qry, uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_ani_milli) {
+  if (!c || !i0 || (n_qry && (!d_in || !d_in_found || !d_out || !d_n_found))) { hg_set_error("hg_search_merge_dev: NULL argument"); return HG_E_INVALID; }
+  if (n_lists < 1 || n_lists > HG_SEARCH_MERGE_MAX_LISTS) {
+    hg_set_error("hg_search_merge_dev: n_lists %u outside 1..%d", n_lists, HG_SEARCH_MERGE_MAX_LISTS); return HG_E_INVALID;
+  }
+  if (top_k < 1 || top_k > 1024) { hg_set_error("hg_search_merge_dev: top_k %u outside 1..1024", top_k); return HG_E_INVALID; }
+  HG_CUDA(cudaSetDevice(c->device));
+  return hg_search_merge(c, n_lists, d_in, d_in_found, i0, n_qry, top_k, d_out, d_n_found, d_ani_milli);
 }
 
 extern "C" int hg_search_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {

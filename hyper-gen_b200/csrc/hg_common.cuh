@@ -193,15 +193,16 @@ enum hg_scratch_slot {
   HG_S_TABLES = 2,     // per-genome hash tables / explicit hash sets
   HG_S_COUNTS = 3,     // distinct-hash counters; dist: the hit counter of the host entry
   HG_S_HV = 4,         // int16 HVs (sketch output staging; dist: both matrices of the host entry)
-  HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass
+  HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass;
+                       // group search: the members' results gathered on GPU 0
   HG_S_SMALL = 6,      // norms / bits / counts per sketch
-  HG_S_MISC = 7,       // CTA -> genome map, |hv| max, probe sink
+  HG_S_MISC = 7,       // CTA -> genome map, |hv| max, probe sink, status word of a search merge
   HG_S_REF_LIMBS = 8,  // s8 limb planes of the ref matrix (dist_tc)
   HG_S_QRY_LIMBS = 9,  // s8 limb planes of the query matrix (dist_tc)
-  HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort; search: the per-query segments
+  HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort; search: the per-query segments; group search: the merged result
   HG_S_SORT_CNT = 11,  // digit counters of the hit sort; search: per-query counts and offsets
   HG_S_NARROW_META = 12,  // per-row constants + outlier lists of the single-plane dist path (dist_narrow)
-  HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entry
+  HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entries
   HG_S_COUNT = 14
 };
 // scratch slot `slot` grown to at least `bytes` (contents not preserved)
@@ -375,4 +376,24 @@ int hg_launch_search_select(hg_ctx *ctx, const hg_hit *d_cand, uint64_t n_cand, 
 // the floor pass's top_k-th keys (over s sample rows of n_ref) -> the main pass's per-query thresholds (hg_floors)
 int hg_launch_search_floors(hg_ctx *ctx, const unsigned long long *d_floor_key, uint32_t n_qry, float ani_min, uint32_t ksize,
                             uint32_t n_ref, uint32_t s, hg_floor *d_floors, float *d_cfrac_row);
+// n_lists (1..HG_SEARCH_MERGE_MAX_LISTS) per-block results -> one, as hg_search_merge_dev describes; *d_status |= 1 if some
+// i + i0[m] does not fit 32 bits, |= 2 if some input n_found exceeds top_k (the caller zeroes it before)
+int hg_launch_search_merge(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0,
+                           uint32_t n_qry, uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli, uint32_t *d_status);
+// The pieces of hg_search_packed (api.cu) that hg_group_search_packed (peer.cu) shares: the argument checks (`who` names
+// the entry in the error), every row's hv_quant_bits checked -> the largest of the refs and of the queries (0 when
+// `same`), and one search of packed host rows whose result stays on the device (HG_S_TILES of the context).
+int hg_search_packed_check(const char *who, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                           const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
+                           const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t top_k, int path, const hg_hit *out,
+                           const uint32_t *n_found);
+int hg_search_packed_bits(const char *who, const uint8_t *ref_bits, uint32_t n_ref, uint64_t ref_stride, const uint8_t *qry_bits,
+                          uint32_t n_qry, uint64_t qry_stride, bool same, uint32_t hv_d, uint32_t *rmax, uint32_t *qmax);
+int hg_search_packed_run(hg_ctx *ctx, bool same, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                         const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
+                         const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min, int path,
+                         uint32_t rmax, uint32_t qmax, hg_hit **d_out, uint32_t **d_n_found, uint32_t **d_milli);
+// hg_search_merge_dev after its argument checks (the context's device is current); returns with the result complete
+int hg_search_merge(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0, uint32_t n_qry,
+                    uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli);
 int hg_launch_absmax(hg_ctx *ctx, const int16_t *d_hv, uint64_t n_elems, int32_t *d_out);

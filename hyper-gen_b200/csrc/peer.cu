@@ -1220,3 +1220,85 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
   }
   return HG_OK;
 }
+
+// hg_search_packed over all GPUs of the group (DESIGN.md §4.8).  The refs are cut into contiguous blocks of about equal
+// size, one per member that gets at least 1024 of them; each member copies its ref block and all query rows over its own
+// PCIe link and searches them.  One host thread per GPU drives its members: members that share a device ordinal run one
+// after another (the dist kernels were never checked running next to another context's on the same GPU).  The blocks'
+// results are copied to GPU 0 and merged there; the only exchange is n_qry * top_k records per member, so no windows.
+extern "C" int hg_group_search_packed(hg_group *g, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                                      const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                                      const uint8_t *qry_bits, const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize,
+                                      uint32_t top_k, float ani_min, int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli) {
+  if (!g) { hg_set_error("hg_group_search_packed: NULL argument"); return HG_E_INVALID; }
+  for (int k = 0; k < g->n; ++k) {  // a member without a block reports no passes
+    memset(g->ctx[k]->search_stats, 0, sizeof(g->ctx[k]->search_stats));
+    g->ctx[k]->search_ev_used = 0;
+  }
+  const int parts = (int)std::min<uint32_t>((uint32_t)g->n, std::max<uint32_t>(1u, n_ref / 1024u));
+  if (parts == 1)
+    return hg_search_packed(g->ctx[0], ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits, qry_norm, n_qry,
+                            hv_d, ksize, top_k, ani_min, path, out, n_found, ani_milli);
+  int rc;
+  if ((rc = hg_search_packed_check("hg_group_search_packed", ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride,
+                                   qry_bits, qry_norm, n_qry, hv_d, top_k, path, out, n_found)))
+    return rc;
+  if (n_qry == 0) return HG_OK;
+  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
+  uint32_t rmax, qmax;
+  if ((rc = hg_search_packed_bits("hg_group_search_packed", ref_bits, n_ref, ref_stride, qry_bits, n_qry, qry_stride, same, hv_d, &rmax,
+                                  &qmax)))
+    return rc;
+  if (same) qmax = rmax;  // every member holds a ref block and all queries: two matrices
+  std::vector<uint32_t> b(parts + 1);
+  for (int k = 0; k <= parts; ++k) b[k] = (uint32_t)((uint64_t)n_ref * k / parts);
+  std::vector<hg_hit *> d_out(parts);
+  std::vector<uint32_t *> d_nf(parts), d_milli(parts);
+  std::vector<int> rcs(parts, HG_OK);
+  std::vector<std::string> msgs(parts);
+  auto member = [&](int m) -> int {
+    hg_ctx *c = g->ctx[m];
+    HG_CUDA(cudaSetDevice(c->device));
+    return hg_search_packed_run(c, false, ref_packed + (size_t)b[m] * ref_stride, ref_stride, ref_bits + b[m], ref_norm + b[m],
+                                b[m + 1] - b[m], qry_packed, qry_stride, qry_bits, qry_norm, n_qry, hv_d, ksize, top_k, ani_min, path,
+                                rmax, qmax, &d_out[m], &d_nf[m], &d_milli[m]);
+  };
+  std::vector<std::thread> th;
+  for (int k = 0; k < parts; ++k) {
+    bool first_on_device = true;
+    for (int l = 0; l < k; ++l) first_on_device &= g->ctx[l]->device != g->ctx[k]->device;
+    if (!first_on_device) continue;
+    th.emplace_back([&, k]() {
+      for (int m = k; m < parts; ++m) {
+        if (g->ctx[m]->device != g->ctx[k]->device) continue;
+        if ((rcs[m] = member(m))) msgs[m] = hg_last_error();
+      }
+    });
+  }
+  for (auto &t : th) t.join();
+  for (int k = 0; k < parts; ++k)
+    if (rcs[k]) { hg_set_error("GPU %d (refs %u..%u): %s", g->ctx[k]->device, b[k], b[k + 1], msgs[k].c_str()); return rcs[k]; }
+  // gather: the members' results next to each other on GPU 0, in a slot apart from member 0's own result (HG_S_TILES)
+  hg_ctx *c0 = g->ctx[0];
+  HG_CUDA(cudaSetDevice(c0->device));
+  const size_t n_out = (size_t)n_qry * top_k;
+  void *d_gather, *d_res;
+  if ((rc = hg_scratch(c0, HG_S_PACKED, (size_t)parts * (n_out * sizeof(hg_hit) + (size_t)n_qry * 4) + 256, &d_gather))) return rc;
+  if ((rc = hg_scratch(c0, HG_S_SORT_TMP, n_out * (sizeof(hg_hit) + 4) + (size_t)n_qry * 4 + 256, &d_res))) return rc;
+  hg_hit *g_hits = (hg_hit *)d_gather;
+  uint32_t *g_found = (uint32_t *)(g_hits + (size_t)parts * n_out);
+  for (int k = 0; k < parts; ++k) {
+    const int dev = g->ctx[k]->device;
+    HG_CUDA(cudaMemcpyPeerAsync(g_hits + (size_t)k * n_out, c0->device, d_out[k], dev, n_out * sizeof(hg_hit), c0->stream));
+    HG_CUDA(cudaMemcpyPeerAsync(g_found + (size_t)k * n_qry, c0->device, d_nf[k], dev, (size_t)n_qry * 4, c0->stream));
+  }
+  hg_hit *r_out = (hg_hit *)d_res;
+  uint32_t *r_milli = (uint32_t *)(r_out + n_out), *r_nf = r_milli + n_out;
+  if ((rc = hg_search_merge(c0, (uint32_t)parts, g_hits, g_found, b.data(), n_qry, top_k, r_out, r_nf, ani_milli ? r_milli : nullptr)))
+    return rc;
+  HG_CUDA(cudaMemcpyAsync(out, r_out, n_out * sizeof(hg_hit), cudaMemcpyDeviceToHost, c0->stream));
+  HG_CUDA(cudaMemcpyAsync(n_found, r_nf, (size_t)n_qry * 4, cudaMemcpyDeviceToHost, c0->stream));
+  if (ani_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, r_milli, n_out * 4, cudaMemcpyDeviceToHost, c0->stream));
+  HG_CUDA(cudaStreamSynchronize(c0->stream));
+  return HG_OK;
+}

@@ -7,7 +7,8 @@
 //            floor is 0) first finds its top_k-th largest key by a radix select over the 64-bit key (8 passes of 8
 //            bits), keeps the top_k keys at or above it and sorts those.  The pair enumeration emits every (i, j)
 //            at most once, so the keys of a segment are distinct and the selected set is exact;
-//   floors   the top_k-th key of every query after the floor pass -> the per-query threshold (hg_floor) of the main pass.
+//   floors   the top_k-th key of every query after the floor pass -> the per-query threshold (hg_floor) of the main pass;
+//   merge    the results of searches over contiguous ref blocks -> the result over all of them (hg_search_merge_dev).
 //
 // The key of a candidate is (ANI bits << 32) | ~i: ANI is a non-negative f32, so its bits order like the value, and the
 // complemented index puts the smaller i first among equal ANIs.  No real key is 0 (that would need i = 2^32 - 1).
@@ -214,7 +215,87 @@ __global__ void __launch_bounds__(1024) floor_prep_kernel(const unsigned long lo
   }
 }
 
+// Merge of n_lists per-block results (each as hg_search_dev writes it, block m's ref indices offset by i0[m]) into one,
+// by rank: live element p of list m for query j has the output rank p + #(keys >= its key in the lists before m) +
+// #(keys > its key in the lists after m), each count a binary search in a list that is already in key order.  Keys are
+// distinct within a list, so the ranks are a permutation of 0 .. sum(n_found) - 1 - the asymmetric >= / > keeps them
+// one even when the same key is in two lists.  The thread of list 0 at position p also zeroes output slot p if it is
+// unused.  status: bit 0 = some i + i0 does not fit 32 bits, bit 1 = some n_found above top_k (counted as top_k).
+struct MergeOffsets { uint32_t i0[HG_SEARCH_MERGE_MAX_LISTS]; };
+
+__device__ __forceinline__ unsigned long long merge_key(const uint4 &h, uint32_t i0) {
+  return ((unsigned long long)h.w << 32) | (unsigned long long)(~(h.x + i0));
+}
+
+__device__ __forceinline__ uint32_t merge_found(const uint32_t *in_found, uint32_t m, uint32_t n_qry, uint32_t j, uint32_t top_k,
+                                                uint32_t *status) {
+  const uint32_t nf = in_found[(uint64_t)m * n_qry + j];
+  if (nf > top_k) { atomicOr(status, 2u); return top_k; }
+  return nf;
+}
+
+__global__ void search_merge_kernel(const uint4 *__restrict__ in, const uint32_t *__restrict__ in_found, MergeOffsets off,
+                                    uint32_t n_lists, uint32_t n_qry, uint32_t top_k, hg_hit *__restrict__ out,
+                                    uint32_t *__restrict__ n_found, uint32_t *__restrict__ milli, uint32_t *__restrict__ status) {
+  const uint64_t total = (uint64_t)n_lists * n_qry * top_k;
+  for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (uint64_t)gridDim.x * blockDim.x) {
+    const uint32_t p = (uint32_t)(t % top_k);
+    const uint64_t r = t / top_k;
+    const uint32_t j = (uint32_t)(r % n_qry), m = (uint32_t)(r / n_qry);
+    const uint64_t o = (uint64_t)j * top_k;
+    if (m == 0) {
+      uint64_t sum = 0;
+      for (uint32_t l = 0; l < n_lists; ++l) sum += merge_found(in_found, l, n_qry, j, top_k, status);
+      const uint32_t nf = sum < top_k ? (uint32_t)sum : top_k;
+      if (p == 0) n_found[j] = nf;
+      if (p >= nf) {
+        out[o + p] = hg_hit{0u, 0u, 0, 0.0f};
+        if (milli) milli[o + p] = 0;
+      }
+    }
+    if (p >= merge_found(in_found, m, n_qry, j, top_k, status)) continue;
+    const uint4 h = in[((uint64_t)m * n_qry + j) * top_k + p];
+    if ((uint64_t)h.x + off.i0[m] > 0xFFFFFFFFull) { atomicOr(status, 1u); continue; }
+    const unsigned long long key = merge_key(h, off.i0[m]);
+    uint32_t rank = p;
+    for (uint32_t l = 0; l < n_lists && rank < top_k; ++l) {
+      if (l == m) continue;
+      const uint4 *L = in + ((uint64_t)l * n_qry + j) * top_k;
+      uint32_t lo = 0, hi = merge_found(in_found, l, n_qry, j, top_k, status);  // first position that does not count
+      while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        const unsigned long long k = merge_key(L[mid], off.i0[l]);
+        if (l < m ? k >= key : k > key) lo = mid + 1;
+        else hi = mid;
+      }
+      rank += lo;
+    }
+    if (rank >= top_k) continue;
+    hg_hit hit;
+    hit.i = h.x + off.i0[m];
+    hit.j = h.y;
+    hit.dot = (int32_t)h.z;
+    hit.ani = __uint_as_float(h.w);
+    out[o + rank] = hit;
+    if (milli) milli[o + rank] = (uint32_t)__double2ll_rn((double)hit.ani * 1000.0);  // as seg_select_kernel
+  }
+}
+
 }  // namespace
+
+int hg_launch_search_merge(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0,
+                           uint32_t n_qry, uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli, uint32_t *d_status) {
+  if (n_qry == 0) return HG_OK;
+  MergeOffsets off = {};
+  for (uint32_t m = 0; m < n_lists; ++m) off.i0[m] = i0[m];
+  const uint64_t total = (uint64_t)n_lists * n_qry * top_k;
+  const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((total + 255) / 256, (uint64_t)ctx->sm_count * 16));
+  search_merge_kernel<<<grid, 256, 0, ctx->stream>>>((const uint4 *)d_in, d_in_found, off, n_lists, n_qry, top_k, d_out, d_n_found,
+                                                     d_milli, d_status);
+  ctx->launches++;
+  HG_CUDA(cudaGetLastError());
+  return HG_OK;
+}
 
 int hg_launch_search_gather(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t hv_d, uint32_t s,
                             int16_t *d_out, int32_t *d_out_norm) {

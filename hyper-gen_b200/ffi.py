@@ -21,8 +21,9 @@ EXPORTS = [
     "hg_fasta_merge", "hg_sketch_fasta_batch",
     "hg_kmer_hash", "hg_sketch_batch", "hg_sketch_batch_dev", "hg_sketch_status", "hg_unpack", "hg_unpack_dev",
     "hg_dist", "hg_dist_dev", "hg_dist_status", "hg_dist_last_path", "hg_dist_last_reason", "hg_sort_hits_dev", "hg_dist_sorted", "hg_dist_packed",
-    "hg_search_dev", "hg_search_packed", "hg_search_stats",
+    "hg_search_dev", "hg_search_packed", "hg_search_stats", "hg_search_merge_dev",
     "hg_group_create", "hg_group_destroy", "hg_group_size", "hg_group_ctx", "hg_group_sketch_fasta_batch", "hg_group_dist_packed",
+    "hg_group_search_packed",
     "hg_peer_window_need", "hg_peer_create", "hg_peer_connect", "hg_peer_create_local", "hg_peer_destroy", "hg_peer_rank",
     "hg_peer_world", "hg_peer_barrier", "hg_peer_stage_ms", "hg_peer_timeline", "hg_peer_plan_tiles", "hg_peer_plan_push", "hg_dist_sharded_dev", "hg_dist_sharded_hits", "hg_peer_hit_buffers",
 ]
@@ -106,6 +107,7 @@ def load() -> C.CDLL:
     L.hg_search_packed.restype = i32
     L.hg_search_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, u32, C.c_float, i32, vp, vp, vp]
     L.hg_search_stats.restype = i32; L.hg_search_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
+    L.hg_search_merge_dev.restype = i32; L.hg_search_merge_dev.argtypes = [vp, u32, vp, vp, vp, u32, u32, vp, vp, vp]
     L.hg_group_create.restype = i32; L.hg_group_create.argtypes = [i32, vp, C.POINTER(vp)]
     L.hg_group_destroy.restype = None; L.hg_group_destroy.argtypes = [vp]
     L.hg_group_size.restype = i32; L.hg_group_size.argtypes = [vp]
@@ -114,6 +116,8 @@ def load() -> C.CDLL:
     L.hg_group_dist_packed.restype = i32
     L.hg_group_dist_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, i32, vp, vp, u64,
                                        C.POINTER(u64)]
+    L.hg_group_search_packed.restype = i32
+    L.hg_group_search_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, u32, C.c_float, i32, vp, vp, vp]
     L.hg_peer_window_need.restype = u64; L.hg_peer_window_need.argtypes = [u32, u32, u64]
     L.hg_peer_create.restype = i32; L.hg_peer_create.argtypes = [vp, i32, i32, u64, vp, C.POINTER(vp)]
     L.hg_peer_connect.restype = i32; L.hg_peer_connect.argtypes = [vp, vp]
@@ -152,6 +156,30 @@ def _ptr(a) -> int:
 
 def make_params(k=21, scaled=1500, seed=123, canonical=True, hv_d=4096) -> SketchParams:
     return SketchParams(scaled=scaled, seed=seed, hv_d=hv_d, ksize=k, canonical=int(bool(canonical)))
+
+
+def _search_packed(fn, h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize, top_k, ani_min, path):
+    """hg_search_packed / hg_group_search_packed (fn) on the context / group h"""
+    rp = np.ascontiguousarray(ref_packed, np.uint8)
+    rb = np.ascontiguousarray(ref_bits, np.uint8)
+    rn = np.ascontiguousarray(ref_norm2, np.int32)
+    same = qry_packed is ref_packed
+    qp = rp if same else np.ascontiguousarray(qry_packed, np.uint8)
+    qb = rb if same else np.ascontiguousarray(qry_bits, np.uint8)
+    qn = rn if same else np.ascontiguousarray(qry_norm2, np.int32)
+    R, Q = rp.shape[0], qp.shape[0]
+    hits = np.zeros((Q, top_k), HIT_DTYPE)
+    n_found = np.zeros(Q, np.uint32)
+    milli = np.zeros((Q, top_k), np.uint32)
+    _check(fn(h, _ptr(rp), rp.strides[0] if R else 0, _ptr(rb), _ptr(rn), R, _ptr(qp), qp.strides[0] if Q else 0, _ptr(qb), _ptr(qn),
+              Q, hv_d, ksize, top_k, ani_min, path, _ptr(hits), _ptr(n_found), _ptr(milli)))
+    return hits, n_found, milli
+
+
+def _search_stats(ctx_handle):
+    counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
+    _check(load().hg_search_stats(ctx_handle, counts, ms))
+    return [int(x) for x in counts], [float(x) for x in ms]
 
 
 class Context:
@@ -398,28 +426,21 @@ class Context:
                       ani_min=0.0, path=0):
         """hg_search_packed: packed sketch rows (n x stride uint8) + quant bits + norms ->
         (hits[n_qry, top_k], n_found[n_qry], ani_milli[n_qry, top_k]); query j's results are hits[j, :n_found[j]]."""
-        rp = np.ascontiguousarray(ref_packed, np.uint8)
-        rb = np.ascontiguousarray(ref_bits, np.uint8)
-        rn = np.ascontiguousarray(ref_norm2, np.int32)
-        same = qry_packed is ref_packed
-        qp = rp if same else np.ascontiguousarray(qry_packed, np.uint8)
-        qb = rb if same else np.ascontiguousarray(qry_bits, np.uint8)
-        qn = rn if same else np.ascontiguousarray(qry_norm2, np.int32)
-        R, Q = rp.shape[0], qp.shape[0]
-        hits = np.zeros((Q, top_k), HIT_DTYPE)
-        n_found = np.zeros(Q, np.uint32)
-        milli = np.zeros((Q, top_k), np.uint32)
-        _check(load().hg_search_packed(self._h, _ptr(rp), rp.strides[0] if R else 0, _ptr(rb), _ptr(rn), R, _ptr(qp),
-                                       qp.strides[0] if Q else 0, _ptr(qb), _ptr(qn), Q, hv_d, ksize, top_k, ani_min, path,
-                                       _ptr(hits), _ptr(n_found), _ptr(milli)))
-        return hits, n_found, milli
+        return _search_packed(load().hg_search_packed, self._h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2,
+                              hv_d, ksize, top_k, ani_min, path)
 
     def search_stats(self):
         """hg_search_stats of the last search -> ([s, floor-pass candidates, main-pass candidates, reruns],
         [ms of floor pass, its select, main pass, its select] (-1: not run or profiling off))"""
-        counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
-        _check(load().hg_search_stats(self._h, counts, ms))
-        return [int(x) for x in counts], [float(x) for x in ms]
+        return _search_stats(self._h)
+
+    def search_merge_dev(self, n_lists, d_in, d_in_found, i0, n_qry, top_k, d_out, d_n_found, d_ani_milli=None):
+        """hg_search_merge_dev: n_lists per-block results (device pointers as ints; list m's refs start at global index
+        i0[m]) -> the result over all blocks; returns when it is complete."""
+        off = np.ascontiguousarray(i0, np.uint32)
+        assert off.size == n_lists
+        _check(load().hg_search_merge_dev(self._h, n_lists, d_in, d_in_found, _ptr(off), n_qry, top_k, d_out, d_n_found,
+                                          d_ani_milli))
 
     def sort_hits_dev(self, d_hits, n, d_ani_milli=None):
         """hg_sort_hits_dev: device records to the reference's output order, in place."""
@@ -601,3 +622,13 @@ class Group:
                 continue
             _check(rc)
             return hits[: n_hits.value].copy(), (milli[: n_hits.value].copy() if sorted_output else None)
+
+    def search_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize=21, top_k=10,
+                      ani_min=0.0, path=0):
+        """hg_group_search_packed: Context.search_packed with the refs split into one block per GPU; same results."""
+        return _search_packed(load().hg_group_search_packed, self._h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits,
+                              qry_norm2, hv_d, ksize, top_k, ani_min, path)
+
+    def search_stats(self, i: int = 0):
+        """Context.search_stats of member i's part of the last group search"""
+        return _search_stats(load().hg_group_ctx(self._h, i))

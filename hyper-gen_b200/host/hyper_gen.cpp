@@ -15,7 +15,7 @@
 //   hyper-gen dist   -r <ref sketch> -q <query sketch> -o <out> [-a 85.0]
 //   hyper-gen search -r <ref sketch> -q <query sketch> -o <out> [-n 10] [-a 0.0]
 //       the -n best refs of every query with ANI >= -a (ties by ascending ref index), one line per result,
-//       queries in file order.  Runs on one GPU; sharding it over the GPUs of an hg_group is not done yet.
+//       queries in file order.  The refs are split over every visible GPU (hg_group_search_packed); HG_GPUS=n limits it.
 // The GPU path is the only path (`-D gpu` is implied): there is no CPU fallback.
 #include <algorithm>
 #include <chrono>
@@ -370,15 +370,14 @@ void search(const types::SketchSearch &ss) {
   if (ref[0].hv_d != qry[0].hv_d) die("Ref and query sketches use different HV dimensions!");
   const size_t D = ref[0].hv_d, R = ref.size(), Q = qry.size(), K = ss.top_k;
   const dist::Stacked rs = dist::stack(ref, D), qs = dist::stack(qry, D);
-  hg_ctx *ctx = nullptr;
-  check(hg_init(0, &ctx), "hg_init");
+  hg_group *group = open_group();
   std::vector<hg_hit> hits(Q * K);
   std::vector<uint32_t> n_found(Q), milli(Q * K);
-  check(hg_search_packed(ctx, rs.packed.data(), 2 * D, rs.bits.data(), rs.norm.data(), (uint32_t)R, qs.packed.data(), 2 * D,
-                         qs.bits.data(), qs.norm.data(), (uint32_t)Q, (uint32_t)D, ref[0].ksize, ss.top_k, ss.ani_min, 0, hits.data(),
-                         n_found.data(), milli.data()),
-        "hg_search_packed");
-  hg_destroy(ctx);
+  check(hg_group_search_packed(group, rs.packed.data(), 2 * D, rs.bits.data(), rs.norm.data(), (uint32_t)R, qs.packed.data(), 2 * D,
+                               qs.bits.data(), qs.norm.data(), (uint32_t)Q, (uint32_t)D, ref[0].ksize, ss.top_k, ss.ani_min, 0,
+                               hits.data(), n_found.data(), milli.data()),
+        "hg_group_search_packed");
+  hg_group_destroy(group);
   std::string out;
   char buf[64];
   size_t lines = 0;

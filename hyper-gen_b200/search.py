@@ -1,12 +1,13 @@
 """Host mirror of the `search` subcommand: load two sketch files, and for every query sketch write its top-k
-best-matching refs (hg_search_packed: unpack, floor pass, main pass and selection all on the GPU)."""
+best-matching refs (hg_search_packed: unpack, floor pass, main pass and selection all on the GPU; with a Group,
+hg_group_search_packed: one block of refs per GPU, the blocks' results merged on GPU 0)."""
 from __future__ import annotations
 
 from dataclasses import dataclass
 
 from . import fileio
 from .dist import _stack_packed
-from .ffi import Context
+from .ffi import Context, Group
 
 
 @dataclass
@@ -28,10 +29,11 @@ def format_search_lines(ref_names, qry_names, hits, n_found, milli) -> str:
     return "".join(out)
 
 
-def search(ss: SketchSearch, ctx: Context | None = None, path: int = 0) -> str:
-    """Returns the text written to ss.out_file."""
-    own = ctx is None
-    ctx = ctx or Context(0)
+def search(ss: SketchSearch, ctx: Context | None = None, path: int = 0, group: Group | None = None) -> str:
+    """Returns the text written to ss.out_file.  With `group` the search runs on its GPUs (Group.search_packed)."""
+    own = ctx is None and group is None
+    if own:
+        ctx = Context(0)
     try:
         ref = fileio.load_sketch(ss.path_ref_sketch)
         qry = fileio.load_sketch(ss.path_query_sketch)
@@ -42,8 +44,8 @@ def search(ss: SketchSearch, ctx: Context | None = None, path: int = 0) -> str:
         hv_d, ksize = ref[0].hv_d, ref[0].ksize
         rp, rb, rn = _stack_packed(ref)
         qp, qb, qn = _stack_packed(qry)
-        hits, n_found, milli = ctx.search_packed(rp, rb, rn, qp, qb, qn, hv_d, ksize=ksize, top_k=ss.top_k,
-                                                 ani_min=ss.ani_min, path=path)
+        hits, n_found, milli = (group or ctx).search_packed(rp, rb, rn, qp, qb, qn, hv_d, ksize=ksize, top_k=ss.top_k,
+                                                            ani_min=ss.ani_min, path=path)
         text = format_search_lines([s.file_str for s in ref], [s.file_str for s in qry], hits, n_found, milli)
         if ss.out_file:
             with open(ss.out_file, "w") as f:

@@ -273,6 +273,17 @@ HG_API int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint64_t
                                 const uint8_t *qry_quant_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d,
                                 uint32_t ksize, float ani_th, int symmetric, int sorted, hg_hit *hits, uint32_t *ani_milli,
                                 uint64_t cap, uint64_t *n_hits);
+/* hg_search_packed with the refs split into contiguous blocks of about equal size, one per GPU (as many GPUs as give
+ * every block at least 1024 refs): each GPU receives its ref block and all query rows over its own PCIe link and
+ * searches them; the per-block results are copied to GPU 0 and merged there (hg_search_merge_dev).  Same arguments,
+ * results identical to hg_search_packed.  One GPU in use (g has one member, or fewer than 2048 refs): hg_search_packed
+ * on member 0.  Members that share a device ordinal run one after another.  hg_search_stats on hg_group_ctx(g, m)
+ * reports member m's passes (all zero for a member without a block). */
+HG_API int hg_group_search_packed(hg_group *g, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_quant_bits,
+                                  const int32_t *ref_norm2, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                                  const uint8_t *qry_quant_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d,
+                                  uint32_t ksize, uint32_t top_k, float ani_min, int path,
+                                  hg_hit *out, uint32_t *n_found, uint32_t *ani_milli /* may be NULL */);
 
 /* hg_peer: one member of a group of GPUs, for hosts that run ONE PROCESS PER GPU.  Every member
  * allocates a window (hg_peer_create), the host exchanges the HG_IPC_HANDLE_BYTES-byte handles by its
@@ -374,6 +385,19 @@ HG_API int hg_search_packed(hg_ctx *ctx, const uint8_t *ref_packed, uint64_t ref
  * pass (gather + dist), its select, the main pass, its select (-1 where not run or profiling is off, see
  * hg_set_profiling). */
 HG_API int hg_search_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
+/* The search over refs cut into contiguous blocks, from the search of each block: list m (m < n_lists) is what
+ * hg_search_dev wrote for block m, which starts at global ref index i0[m] - records d_in[(m * n_qry + j) * top_k ..],
+ * counts d_in_found[m * n_qry + j].  The result is what one search over all blocks writes (d_out, d_n_found,
+ * d_ani_milli as hg_search_dev), with i = block index + i0[m].  Exact: the global top_k of a query is a subset of the
+ * union of the blocks' top_k, and within a contiguous block the ref order is the global order, so ties come out by
+ * ascending global index.  Device pointers; returns with the result complete.  A host that runs one process per GPU
+ * searches its own ref block, gathers the ranks' lists into one device buffer by its own means and calls this.
+ *   n_lists 1..HG_SEARCH_MERGE_MAX_LISTS, top_k 1..1024; an i + i0[m] beyond 32 bits or an input count above top_k:
+ *   HG_E_INVALID. */
+#define HG_SEARCH_MERGE_MAX_LISTS 64
+HG_API int hg_search_merge_dev(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found,
+                               const uint32_t *i0 /* host, n_lists entries */, uint32_t n_qry, uint32_t top_k, hg_hit *d_out,
+                               uint32_t *d_n_found, uint32_t *d_ani_milli /* may be NULL */);
 
 /* Which path the last hg_dist / hg_dist_dev took (1 SIMT, 2 two-limb tensor, 3 single-plane tensor) and why. */
 HG_API int hg_dist_last_path(hg_ctx *ctx);

@@ -32,6 +32,14 @@ extern "C" {
         ref_norm2: *const i32, n_ref: u32, qry_packed: *const u8, qry_stride: u64, qry_quant_bits: *const u8,
         qry_norm2: *const i32, n_qry: u32, hv_d: u32, ksize: u32, ani_th: f32, symmetric: c_int, sorted: c_int,
         hits: *mut hg_hit, ani_milli: *mut u32, cap: u64, n_hits: *mut u64) -> c_int;
+    // top-k search with one contiguous ref block per GPU; results identical to hg_search_packed
+    pub fn hg_group_search_packed(g: *mut hg_group, ref_packed: *const u8, ref_stride: u64, ref_quant_bits: *const u8,
+        ref_norm2: *const i32, n_ref: u32, qry_packed: *const u8, qry_stride: u64, qry_quant_bits: *const u8,
+        qry_norm2: *const i32, n_qry: u32, hv_d: u32, ksize: u32, top_k: u32, ani_min: f32, path: c_int,
+        out: *mut hg_hit, n_found: *mut u32, ani_milli: *mut u32) -> c_int;
+    // the per-block top-k lists (device memory, block m starting at global ref i0[m]) merged into one
+    pub fn hg_search_merge_dev(ctx: *mut hg_ctx, n_lists: u32, d_in: *const hg_hit, d_in_found: *const u32, i0: *const u32,
+        n_qry: u32, top_k: u32, d_out: *mut hg_hit, d_n_found: *mut u32, d_ani_milli: *mut u32) -> c_int;
 }
 
 /// status -> panic with the library's message, the reference's error style (`unwrap()`, Cargo.toml:67-70)

@@ -7,7 +7,14 @@ alternately with CUDA events on the library's stream.  One extra profiled search
 the candidates of each pass and the device time of each step.  64 sampled queries per case are checked against the
 oracle (every i, dot, ANI bit, n_found).  Prints one JSON line per case, with the GPU's name and power limit.
 
+With --gpus N the tool times the host entries instead, end to end from packed host rows as a sketch file holds them
+(the H2D copies, the unpack, the search and the copy of the result back): hg_search_packed on one GPU next to
+hg_group_search_packed on groups of 1..N GPUs (--same-gpu: groups of 1..N contexts on GPU 0, which measures what the
+block split, gather and merge add and nothing of the scaling).  Host clock around each call (the call returns with the
+result on the host), calls alternated; every group result is compared with the single-GPU result, slot for slot.
+
     python tools/search_bench.py [--shapes cfg4,10k] [--top-k 1,10,100] [--steps 5] [--warmup 2] [--out FILE]
+                                 [--gpus N [--same-gpu]]
 """
 from __future__ import annotations
 
@@ -17,6 +24,7 @@ import os
 import statistics
 import subprocess
 import sys
+import time
 
 import numpy as np
 
@@ -33,7 +41,8 @@ def gpu_info():
     return out[0] if out else "unknown"
 
 
-def encode_family(ctx, synth, n, D, n_per=3333, scaled=1500, seed=0xD157, first=0):
+def encode_family(ctx, synth, n, D, n_per=3333, scaled=1500, seed=0xD157, first=0, packed=None):
+    """-> device (hv, norm); with `packed` (a device uint8 tensor of n x 2D) also the packed rows there, and the bits"""
     import torch
     hv = torch.empty((n, D), dtype=torch.int16, device="cuda")
     norm = torch.empty(n, dtype=torch.int32, device="cuda")
@@ -43,9 +52,12 @@ def encode_family(ctx, synth, n, D, n_per=3333, scaled=1500, seed=0xD157, first=
         m = min(chunk, n - c0)
         hashes, off = synth.hash_sets_family_dev(m, n_per=n_per, scaled=scaled, seed=seed, device="cuda", first=first + c0)
         torch.cuda.current_stream().synchronize()  # the encoder runs on the library's stream
-        ctx.encode_sets_dev(hashes.data_ptr(), off, D, hv[c0:].data_ptr(), None, bits[c0:].data_ptr(), norm[c0:].data_ptr())
+        ctx.encode_sets_dev(hashes.data_ptr(), off, D, hv[c0:].data_ptr(), None if packed is None else packed[c0:].data_ptr(),
+                            bits[c0:].data_ptr(), norm[c0:].data_ptr())
         ctx.sync()
         del hashes
+    if packed is not None:
+        return hv, norm, bits
     return hv, norm
 
 
@@ -63,6 +75,64 @@ def shapes(names):
             yield "10000 refs x 10000 queries (non-symmetric), D 4096", hv[:10000], norm[:10000], hv[5000:].contiguous(), norm[5000:].contiguous()
         else:
             raise SystemExit("unknown shape " + name)
+
+
+def packed_shapes(names):
+    """the shapes above as host (packed, bits, norm) of refs and queries: rows of 2 D bytes, as the CLI stacks a sketch file"""
+    import torch
+    from hypergen_b200 import synth
+    D = 4096
+    for name in names:
+        n, label = {"cfg4": (100000, "config 4: 100000 refs x 1000 queries, D 4096"),
+                    "10k": (15000, "10000 refs x 10000 queries (non-symmetric), D 4096")}.get(name, (0, ""))
+        if not n:
+            raise SystemExit("unknown shape " + name)
+        d_packed = torch.empty((n, 2 * D), dtype=torch.uint8, device="cuda")
+        hv, norm, bits = encode_family(CTX, synth, n, D, packed=d_packed)
+        del hv
+        packed, norm, bits = d_packed.cpu().numpy(), norm.cpu().numpy(), bits.cpu().numpy()
+        del d_packed
+        torch.cuda.empty_cache()
+        if name == "cfg4":
+            r, q = slice(0, 100000), np.arange(5, 100000, 100)[:1000]
+        else:
+            r, q = slice(0, 10000), slice(5000, 15000)
+        yield label, (packed[r], bits[r], norm[r]), (np.ascontiguousarray(packed[q]), bits[q].copy(), norm[q].copy())
+
+
+def group_bench(args, hg):
+    """hg_search_packed next to hg_group_search_packed at 1..N GPUs (or N contexts on GPU 0), end to end from host rows"""
+    ctx = CTX
+    sizes = list(range(1, args.gpus + 1))
+    groups = {n: hg.Group(ordinals=[0] * n if args.same_gpu else list(range(n))) for n in sizes}
+    card = gpu_info()
+    lines = []
+    for label, (rp, rb, rn), (qp, qb, qn) in packed_shapes(args.shapes.split(",")):
+        for top_k in [int(x) for x in args.top_k.split(",")]:
+            calls = {"single": lambda: ctx.search_packed(rp, rb, rn, qp, qb, qn, 4096, ksize=K, top_k=top_k)}
+            for n in sizes:
+                calls["group%d" % n] = (lambda g: lambda: g.search_packed(rp, rb, rn, qp, qb, qn, 4096, ksize=K, top_k=top_k))(groups[n])
+            results = {}
+            for _ in range(args.warmup):
+                for name, fn in calls.items():
+                    results[name] = fn()
+            times = {name: [] for name in calls}
+            for _ in range(args.steps):
+                for name, fn in calls.items():
+                    t0 = time.perf_counter()
+                    fn()
+                    times[name].append((time.perf_counter() - t0) * 1e3)
+            identical = all(all(np.array_equal(a, b) for a, b in zip(results[name], results["single"])) for name in calls)
+            rec = dict(shape=label, top_k=top_k, ani_min=0.0, same_gpu=bool(args.same_gpu),
+                       ms={name: statistics.median(t) for name, t in times.items()},
+                       ms_all=times, identical_to_single=identical,
+                       members_used={n: sum(groups[n].search_stats(m)[0][0] > 0 for m in range(n)) for n in sizes},
+                       ref_bytes_h2d=int(rb.astype(np.int64).sum() * 4096 // 8), gpu=card)
+            print(json.dumps(rec), flush=True)
+            lines.append(rec)
+    for g in groups.values():
+        g.close()
+    return lines
 
 
 def oracle_check(ref, rn, qry, qn, hits, n_found, top_k, rng):
@@ -94,11 +164,19 @@ def main():
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--no-check", action="store_true")
     ap.add_argument("--out", default="")
+    ap.add_argument("--gpus", type=int, default=0)
+    ap.add_argument("--same-gpu", action="store_true")
     args = ap.parse_args()
     import torch
     import hypergen_b200 as hg
     CTX = hg.Context(0)
     ctx = CTX
+    if args.gpus:
+        if not args.same_gpu and torch.cuda.device_count() < args.gpus:
+            raise SystemExit("--gpus %d: %d GPUs visible" % (args.gpus, torch.cuda.device_count()))
+        write_lines(args.out, group_bench(args, hg))
+        ctx.close()
+        return
     stream = torch.cuda.ExternalStream(ctx.stream)
     card = gpu_info()
     rng = np.random.default_rng(1)
@@ -157,11 +235,15 @@ def main():
             lines.append(rec)
         del ref, rn, qry, qn
         torch.cuda.empty_cache()
-    if args.out:
-        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
-        with open(args.out, "w") as f:
-            f.write("".join(json.dumps(x) + "\n" for x in lines))
+    write_lines(args.out, lines)
     ctx.close()
+
+
+def write_lines(path, lines):
+    if path:
+        os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+        with open(path, "w") as f:
+            f.write("".join(json.dumps(x) + "\n" for x in lines))
 
 
 CTX = None
