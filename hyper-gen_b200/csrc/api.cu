@@ -879,19 +879,6 @@ static void dist_note(hg_ctx *c, const DistChoice &ch, int ran, const DistFacts 
 }
 
 // ---- host matrices streamed in row chunks: H2D of chunk c + 1 under unpack / pre-pass / dist kernel of chunk c ----
-struct HostRows {
-  const uint8_t *base;  // first row on the host
-  uint64_t stride;      // bytes between host rows
-  uint64_t width;       // bytes of a row that travel (int16 rows: 2 hv_d; packed rows: max hv_quant_bits * hv_d / 8)
-  const uint8_t *bits;  // packed rows: hv_quant_bits per row (host); int16 rows: NULL
-  const int32_t *norm;  // host
-  uint32_t n;
-  uint8_t *d_stage;     // packed rows: where they land (width apart); int16 rows: the matrix itself
-  uint8_t *d_bits;      // packed rows
-  int16_t *d_hv;
-  int32_t *d_norm;
-};
-
 static uint32_t dist_chunk_rows(uint32_t n) {
   uint32_t rows = 0;
   if (const char *e = getenv("HG_DIST_CHUNK_ROWS")) rows = (uint32_t)std::max(0, atoi(e));
@@ -1085,10 +1072,22 @@ extern "C" int hg_dist_status(hg_ctx *c) {
 extern "C" int hg_dist_last_path(hg_ctx *c) { return c ? c->dist_path : 0; }
 extern "C" const char *hg_dist_last_reason(hg_ctx *c) { return c ? c->dist_reason : ""; }
 
-// shared tail of the host-pointer dist entries: hit count back, output-stage sort if asked, hits back
+int hg_hits_to_host(hg_ctx *c, hg_hit *d_hits, uint64_t n, bool sorted, hg_hit *hits, uint32_t *ani_milli) {
+  int rc;
+  void *d_milli = nullptr;
+  if (sorted) {  // output stage on the device (src/utils.rs:262-269); unsorted: append order is unspecified
+    if (ani_milli && (rc = hg_scratch(c, HG_S_MISC, n * 4 + 256, &d_milli))) return rc;
+    if ((rc = hg_launch_sort_hits(c, d_hits, n, (uint32_t *)d_milli))) return rc;
+  }
+  HG_CUDA(cudaMemcpyAsync(hits, d_hits, n * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
+  if (d_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, n * 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  return HG_OK;
+}
+
+// shared tail of the host-pointer dist entries: hit count back, then the output stage
 static int dist_tail(hg_ctx *c, void *d_hits, void *d_cnt, hg_hit *hits, uint64_t cap, uint64_t *n_hits, bool sorted,
                      uint32_t *ani_milli) {
-  int rc;
   unsigned long long cnt = 0;
   HG_CUDA(cudaMemcpyAsync(&cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, c->stream));
   HG_CUDA(cudaStreamSynchronize(c->stream));
@@ -1097,17 +1096,16 @@ static int dist_tail(hg_ctx *c, void *d_hits, void *d_cnt, hg_hit *hits, uint64_
     hg_set_error("hg_dist: %llu pairs pass the threshold, capacity is %llu", cnt, (unsigned long long)cap);
     return HG_E_CAPACITY;
   }
-  if (cnt) {
-    void *d_milli = nullptr;
-    if (sorted) {  // output stage on the device (src/utils.rs:262-269)
-      if (ani_milli && (rc = hg_scratch(c, HG_S_MISC, cnt * 4 + 256, &d_milli))) return rc;
-      if ((rc = hg_launch_sort_hits(c, (hg_hit *)d_hits, cnt, (uint32_t *)d_milli))) return rc;
-    }
-    HG_CUDA(cudaMemcpyAsync(hits, d_hits, cnt * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
-    if (d_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, cnt * 4, cudaMemcpyDeviceToHost, c->stream));
-    HG_CUDA(cudaStreamSynchronize(c->stream));  // unsorted: append order is unspecified
-  }
-  return HG_OK;
+  return cnt ? hg_hits_to_host(c, (hg_hit *)d_hits, cnt, sorted, hits, ani_milli) : HG_OK;
+}
+
+int hg_rows_to_device(hg_ctx *c, const HostRows &S, uint32_t hv_d) {
+  if (S.n == 0) return HG_OK;
+  HG_CUDA(cudaMemcpy2DAsync(S.d_stage, S.width, S.base, S.stride, S.width, S.n, cudaMemcpyHostToDevice, c->stream));
+  HG_CUDA(cudaMemcpyAsync(S.d_norm, S.norm, (size_t)S.n * 4, cudaMemcpyHostToDevice, c->stream));
+  if (!S.bits) return HG_OK;
+  HG_CUDA(cudaMemcpyAsync(S.d_bits, S.bits, S.n, cudaMemcpyHostToDevice, c->stream));
+  return hg_launch_unpack(c, S.d_stage, S.width, S.d_bits, S.n, hv_d, S.d_hv);
 }
 
 // Common driver of the host entries: the kernel chosen for these rows, streamed from the host when it can be, else
@@ -1130,16 +1128,7 @@ static int dist_from_host(hg_ctx *c, HostRows &R, HostRows &Q, bool same, uint32
   c->pending_stats[0] = c->pending_stats[1] = nullptr;
   c->ev_used &= ~(3 << 4);
   HG_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), c->stream));
-  auto whole = [&](HostRows &S) -> int {
-    HG_CUDA(cudaMemcpy2DAsync(S.d_stage, S.width, S.base, S.stride, S.width, S.n, cudaMemcpyHostToDevice, c->stream));
-    HG_CUDA(cudaMemcpyAsync(S.d_norm, S.norm, (size_t)S.n * 4, cudaMemcpyHostToDevice, c->stream));
-    if (S.bits) {
-      HG_CUDA(cudaMemcpyAsync(S.d_bits, S.bits, S.n, cudaMemcpyHostToDevice, c->stream));
-      return hg_launch_unpack(c, S.d_stage, S.width, S.d_bits, S.n, hv_d, S.d_hv);
-    }
-    return HG_OK;
-  };
-  if (!stream && ((rc = whole(R)) || (!same && (rc = whole(Q))))) return rc;
+  if (!stream && ((rc = hg_rows_to_device(c, R, hv_d)) || (!same && (rc = hg_rows_to_device(c, Q, hv_d))))) return rc;
   const DistOp op = {R.d_hv, R.d_norm, R.n, 0, Q.d_hv, Q.d_norm, Q.n, 0, hv_d, ksize, ani_th, symmetric, (hg_hit *)d_hits, cap,
                      (unsigned long long *)d_cnt};
   if ((rc = dist_run(c, op, ch, stream ? &R : nullptr, stream ? &Q : nullptr, false))) return rc;
@@ -1171,6 +1160,65 @@ static int dist_host(hg_ctx *c, const int16_t *ref, const int32_t *ref_norm, uin
   return dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, path, 0, hits, cap, n_hits, sorted, ani_milli);
 }
 
+int hg_packed_args_check(const char *who, const hg_packed_rows &R, const hg_packed_rows &Q, uint32_t hv_d) {
+  for (const hg_packed_rows *S : {&R, &Q})
+    if (S->n && (!S->packed || !S->bits || !S->norm)) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
+  if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("%s: hv_d %u must be a multiple of 256", who, hv_d); return HG_E_INVALID; }
+  if (R.stride % 4 != 0 || Q.stride % 4 != 0) { hg_set_error("%s: row stride %% 4", who); return HG_E_INVALID; }
+  return HG_OK;
+}
+
+int hg_packed_rows_check(const char *who, hg_packed_rows *R, hg_packed_rows *Q, uint32_t hv_d, bool *same) {
+  *same = R->packed == Q->packed && R->bits == Q->bits && R->norm == Q->norm && R->n == Q->n;
+  for (int k = 0; k < (*same ? 1 : 2); ++k) {
+    hg_packed_rows &S = k ? *Q : *R;
+    S.max_bits = 0;
+    for (uint32_t g = 0; g < S.n; g++) {
+      if (S.bits[g] < 1 || S.bits[g] > 16) {
+        hg_set_error("%s: %s sketch %u has hv_quant_bits %u", who, k ? "query" : "ref", g, (unsigned)S.bits[g]);
+        return HG_E_INVALID;
+      }
+      S.max_bits = std::max<uint32_t>(S.max_bits, S.bits[g]);
+    }
+  }
+  if (*same) *Q = *R;
+  if (R->width(hv_d) > R->stride || Q->width(hv_d) > Q->stride) {
+    hg_set_error("%s: row stride below hv_quant_bits * hv_d / 8", who); return HG_E_INVALID;
+  }
+  return HG_OK;
+}
+
+int hg_packed_stage(hg_ctx *c, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, HostRows *hr,
+                    HostRows *hq) {
+  const uint64_t rw = R.width(hv_d), qw = Q.width(hv_d);
+  const uint32_t nq = same ? 0 : Q.n;  // rows of a second block
+  const size_t rb = (size_t)R.n * hv_d * 2, rb_al = (rb + 255) & ~(size_t)255, qb = (size_t)nq * hv_d * 2;
+  const size_t rp = ((size_t)R.n * rw + 255) & ~(size_t)255, qp = (size_t)nq * qw;
+  int rc;
+  void *d_mat, *d_small, *d_pk;
+  if ((rc = hg_scratch(c, HG_S_HV, rb + qb + 512, &d_mat))) return rc;
+  if ((rc = hg_scratch(c, HG_S_SMALL, ((size_t)R.n + nq) * 5 + 512, &d_small))) return rc;
+  if ((rc = hg_scratch(c, HG_S_TABLES, rp + qp + 256, &d_pk))) return rc;
+  int32_t *d_norm = (int32_t *)d_small;
+  uint8_t *d_bits = (uint8_t *)(d_norm + R.n + nq);
+  *hr = {R.packed, R.stride, rw, R.bits, R.norm, R.n, (uint8_t *)d_pk, d_bits, (int16_t *)d_mat, d_norm};
+  *hq = same ? *hr
+             : HostRows{Q.packed, Q.stride, qw, Q.bits, Q.norm, Q.n, (uint8_t *)d_pk + rp, d_bits + R.n,
+                        (int16_t *)((uint8_t *)d_mat + rb_al), d_norm + R.n};
+  return HG_OK;
+}
+
+int hg_dist_packed_run(hg_ctx *c, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, uint32_t ksize,
+                       float ani_th, int symmetric, int path, bool sorted, hg_hit *hits, uint32_t *ani_milli, uint64_t cap,
+                       uint64_t *n_hits) {
+  HG_CUDA(cudaSetDevice(c->device));
+  int rc;
+  HostRows hr, hq;
+  if ((rc = hg_packed_stage(c, R, Q, same, hv_d, &hr, &hq))) return rc;
+  return dist_from_host(c, hr, hq, same, hv_d, ksize, ani_th, symmetric, path, std::max(R.max_bits, Q.max_bits), hits, cap, n_hits,
+                        sorted, ani_milli);
+}
+
 // `dist` straight from what the sketch file holds (FileSketch.hv bit-packed + hv_quant_bits + hv_norm_2,
 // src/types.rs:224-235): only the packed bytes cross PCIe (b/16 of the i16 matrix), decompress_file_sketch
 // (src/hd.rs:171-232) runs on the device, then the dist kernel and, if asked, the output-stage sort.
@@ -1181,42 +1229,14 @@ extern "C" int hg_dist_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t ref
                               uint64_t *n_hits) {
   if (!c || !n_hits) { hg_set_error("hg_dist_packed: NULL argument"); return HG_E_INVALID; }
   *n_hits = 0;
-  if ((n_ref && (!ref_packed || !ref_bits || !ref_norm)) || (n_qry && (!qry_packed || !qry_bits || !qry_norm)) || (cap && !hits)) {
-    hg_set_error("hg_dist_packed: NULL argument"); return HG_E_INVALID;
-  }
-  if (hv_d == 0 || hv_d % 256 != 0 || ref_stride % 4 != 0 || qry_stride % 4 != 0) {
-    hg_set_error("hg_dist_packed: hv_d %% 256 or row stride %% 4"); return HG_E_INVALID;
-  }
-  if (n_ref == 0 || n_qry == 0) return HG_OK;
-  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
-  uint32_t rmax = 0, qmax = 0;
-  for (uint32_t g = 0; g < n_ref; g++) {
-    if (ref_bits[g] < 1 || ref_bits[g] > 16) { hg_set_error("hg_dist_packed: ref sketch %u has hv_quant_bits %u", g, (unsigned)ref_bits[g]); return HG_E_INVALID; }
-    rmax = std::max<uint32_t>(rmax, ref_bits[g]);
-  }
-  for (uint32_t g = 0; g < n_qry && !same; g++) {
-    if (qry_bits[g] < 1 || qry_bits[g] > 16) { hg_set_error("hg_dist_packed: query sketch %u has hv_quant_bits %u", g, (unsigned)qry_bits[g]); return HG_E_INVALID; }
-    qmax = std::max<uint32_t>(qmax, qry_bits[g]);
-  }
-  const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;  // bytes of a row that can be live
-  if (rw > ref_stride || (!same && qw > qry_stride)) { hg_set_error("hg_dist_packed: row stride below hv_quant_bits * hv_d / 8"); return HG_E_INVALID; }
-  HG_CUDA(cudaSetDevice(c->device));
+  hg_packed_rows R = {ref_packed, ref_stride, ref_bits, ref_norm, n_ref}, Q = {qry_packed, qry_stride, qry_bits, qry_norm, n_qry};
   int rc;
-  const size_t rb = (size_t)n_ref * hv_d * 2, qb = same ? 0 : (size_t)n_qry * hv_d * 2;
-  const size_t rb_al = (rb + 255) & ~(size_t)255;
-  const size_t rp = ((size_t)n_ref * rw + 255) & ~(size_t)255, qp = same ? 0 : (size_t)n_qry * qw;
-  void *d_mat, *d_small, *d_pk;
-  if ((rc = hg_scratch(c, HG_S_HV, rb + qb + 512, &d_mat))) return rc;
-  if ((rc = hg_scratch(c, HG_S_SMALL, ((size_t)n_ref + n_qry) * 5 + 512, &d_small))) return rc;
-  if ((rc = hg_scratch(c, HG_S_TABLES, rp + qp + 256, &d_pk))) return rc;
-  int16_t *d_ref = (int16_t *)d_mat, *d_qry = same ? d_ref : (int16_t *)((uint8_t *)d_mat + rb_al);
-  int32_t *d_rn = (int32_t *)d_small, *d_qn = same ? d_rn : d_rn + n_ref;
-  uint8_t *d_rbits = (uint8_t *)d_small + ((size_t)n_ref + n_qry) * 4, *d_qbits = same ? d_rbits : d_rbits + n_ref;
-  uint8_t *d_rp = (uint8_t *)d_pk, *d_qp = d_rp + rp;
-  HostRows R = {ref_packed, ref_stride, rw, ref_bits, ref_norm, n_ref, d_rp, d_rbits, d_ref, d_rn};
-  HostRows Q = {qry_packed, qry_stride, qw, qry_bits, qry_norm, n_qry, d_qp, d_qbits, d_qry, d_qn};
-  return dist_from_host(c, R, same ? R : Q, same, hv_d, ksize, ani_th, symmetric, path, std::max(rmax, qmax), hits, cap, n_hits,
-                        sorted != 0, ani_milli);
+  if (cap && !hits) { hg_set_error("hg_dist_packed: NULL argument"); return HG_E_INVALID; }
+  if ((rc = hg_packed_args_check("hg_dist_packed", R, Q, hv_d))) return rc;
+  if (n_ref == 0 || n_qry == 0) return HG_OK;
+  bool same;
+  if ((rc = hg_packed_rows_check("hg_dist_packed", &R, &Q, hv_d, &same))) return rc;
+  return hg_dist_packed_run(c, R, Q, same, hv_d, ksize, ani_th, symmetric, path, sorted != 0, hits, ani_milli, cap, n_hits);
 }
 
 extern "C" int hg_dist(hg_ctx *c, const int16_t *ref, const int32_t *ref_norm, uint32_t n_ref, const int16_t *qry,
@@ -1347,7 +1367,9 @@ static int search_run(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm
   return HG_OK;
 }
 
-static int search_check(const char *who, uint32_t hv_d, uint32_t top_k, int path) {
+int hg_search_check(const char *who, uint32_t n_qry, const hg_hit *out, const uint32_t *n_found, uint32_t hv_d, uint32_t top_k,
+                    int path) {
+  if (n_qry && (!out || !n_found)) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
   if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("%s: hv_d %u must be a multiple of 256", who, hv_d); return HG_E_INVALID; }
   if (top_k < 1 || top_k > 1024) { hg_set_error("%s: top_k %u outside 1..1024", who, top_k); return HG_E_INVALID; }
   if (path < HG_PATH_AUTO || path > HG_PATH_NARROW) { hg_set_error("%s: path %d", who, path); return HG_E_INVALID; }
@@ -1357,86 +1379,60 @@ static int search_check(const char *who, uint32_t hv_d, uint32_t top_k, int path
 extern "C" int hg_search_dev(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm2, uint32_t n_ref, const int16_t *d_qry,
                              const int32_t *d_qry_norm2, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
                              int path, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_ani_milli) {
-  if (!c || (n_ref && (!d_ref || !d_ref_norm2)) || (n_qry && (!d_qry || !d_qry_norm2 || !d_out || !d_n_found))) {
+  if (!c || (n_ref && (!d_ref || !d_ref_norm2)) || (n_qry && (!d_qry || !d_qry_norm2))) {
     hg_set_error("hg_search_dev: NULL argument"); return HG_E_INVALID;
   }
   int rc;
-  if ((rc = search_check("hg_search_dev", hv_d, top_k, path))) return rc;
+  if ((rc = hg_search_check("hg_search_dev", n_qry, d_out, d_n_found, hv_d, top_k, path))) return rc;
   HG_CUDA(cudaSetDevice(c->device));
   return search_run(c, d_ref, d_ref_norm2, n_ref, d_qry, d_qry_norm2, n_qry, hv_d, ksize, top_k, ani_min, path, 0, d_out, d_n_found,
                     d_ani_milli);
 }
 
-int hg_search_packed_check(const char *who, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
-                           const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
-                           const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t top_k, int path, const hg_hit *out,
-                           const uint32_t *n_found) {
-  if ((n_ref && (!ref_packed || !ref_bits || !ref_norm)) || (n_qry && (!qry_packed || !qry_bits || !qry_norm || !out || !n_found))) {
-    hg_set_error("%s: NULL argument", who); return HG_E_INVALID;
-  }
+// The rows as the sketch files hold them: whole copies of the packed bytes (the live width of every row),
+// decompress_file_sketch on the device (as hg_dist_packed), then the search.
+int hg_search_packed_run(hg_ctx *c, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, uint32_t ksize,
+                         uint32_t top_k, float ani_min, int path, hg_hit **d_out_p, uint32_t **d_nf_p, uint32_t **d_milli_p) {
   int rc;
-  if ((rc = search_check(who, hv_d, top_k, path))) return rc;
-  if (ref_stride % 4 != 0 || qry_stride % 4 != 0) { hg_set_error("%s: row stride %% 4", who); return HG_E_INVALID; }
-  return HG_OK;
-}
-
-int hg_search_packed_bits(const char *who, const uint8_t *ref_bits, uint32_t n_ref, uint64_t ref_stride, const uint8_t *qry_bits,
-                          uint32_t n_qry, uint64_t qry_stride, bool same, uint32_t hv_d, uint32_t *rmax_out, uint32_t *qmax_out) {
-  uint32_t rmax = 0, qmax = 0;
-  for (uint32_t g = 0; g < n_ref; g++) {
-    if (ref_bits[g] < 1 || ref_bits[g] > 16) { hg_set_error("%s: ref sketch %u has hv_quant_bits %u", who, g, (unsigned)ref_bits[g]); return HG_E_INVALID; }
-    rmax = std::max<uint32_t>(rmax, ref_bits[g]);
-  }
-  for (uint32_t g = 0; g < n_qry && !same; g++) {
-    if (qry_bits[g] < 1 || qry_bits[g] > 16) { hg_set_error("%s: query sketch %u has hv_quant_bits %u", who, g, (unsigned)qry_bits[g]); return HG_E_INVALID; }
-    qmax = std::max<uint32_t>(qmax, qry_bits[g]);
-  }
-  const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;
-  if (rw > ref_stride || (!same && qw > qry_stride)) { hg_set_error("%s: row stride below hv_quant_bits * hv_d / 8", who); return HG_E_INVALID; }
-  *rmax_out = rmax;
-  *qmax_out = qmax;
-  return HG_OK;
-}
-
-// The rows as the sketch files hold them: whole copies of the packed bytes (rmax * hv_d / 8 bytes of every ref row,
-// qmax * hv_d / 8 of every query row), decompress_file_sketch on the device (as hg_dist_packed), then the search.  The
-// result stays in the context's HG_S_TILES scratch: *d_out / *d_n_found / *d_milli.
-int hg_search_packed_run(hg_ctx *c, bool same, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
-                         const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
-                         const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min, int path,
-                         uint32_t rmax, uint32_t qmax, hg_hit **d_out_p, uint32_t **d_nf_p, uint32_t **d_milli_p) {
-  int rc;
-  const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;
-  const size_t rb = (size_t)n_ref * hv_d * 2, qb = same ? 0 : (size_t)n_qry * hv_d * 2;
-  const size_t rb_al = (rb + 255) & ~(size_t)255;
-  const size_t rp = ((size_t)n_ref * rw + 255) & ~(size_t)255, qp = same ? 0 : (size_t)n_qry * qw;
-  const size_t n_out = (size_t)n_qry * top_k;
-  void *d_mat, *d_small, *d_pk, *d_res;
-  if ((rc = hg_scratch(c, HG_S_HV, rb + qb + 512, &d_mat))) return rc;
-  if ((rc = hg_scratch(c, HG_S_SMALL, ((size_t)n_ref + n_qry) * 5 + 512, &d_small))) return rc;
-  if ((rc = hg_scratch(c, HG_S_TABLES, rp + qp + 256, &d_pk))) return rc;
-  if ((rc = hg_scratch(c, HG_S_TILES, n_out * (sizeof(hg_hit) + 4) + (size_t)n_qry * 4 + 256, &d_res))) return rc;
-  int16_t *d_ref = (int16_t *)d_mat, *d_qry = same ? d_ref : (int16_t *)((uint8_t *)d_mat + rb_al);
-  int32_t *d_rn = (int32_t *)d_small, *d_qn = same ? d_rn : d_rn + n_ref;
-  uint8_t *d_rbits = (uint8_t *)d_small + ((size_t)n_ref + n_qry) * 4, *d_qbits = same ? d_rbits : d_rbits + n_ref;
-  uint8_t *d_rp = (uint8_t *)d_pk, *d_qp = d_rp + rp;
+  HostRows hr, hq;
+  if ((rc = hg_packed_stage(c, R, Q, same, hv_d, &hr, &hq))) return rc;
+  const size_t n_out = (size_t)Q.n * top_k;
+  void *d_res;
+  if ((rc = hg_scratch(c, HG_S_TILES, n_out * (sizeof(hg_hit) + 4) + (size_t)Q.n * 4 + 256, &d_res))) return rc;
   hg_hit *d_out = (hg_hit *)d_res;
   uint32_t *d_milli = (uint32_t *)(d_out + n_out), *d_nf = d_milli + n_out;
-  auto whole = [&](const uint8_t *packed, uint64_t stride, size_t width, const uint8_t *bits, const int32_t *norm, uint32_t n,
-                   uint8_t *d_stage, uint8_t *d_bits, int32_t *d_norm, int16_t *d_hv) -> int {
-    HG_CUDA(cudaMemcpy2DAsync(d_stage, width, packed, stride, width, n, cudaMemcpyHostToDevice, c->stream));
-    HG_CUDA(cudaMemcpyAsync(d_norm, norm, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
-    HG_CUDA(cudaMemcpyAsync(d_bits, bits, n, cudaMemcpyHostToDevice, c->stream));
-    return hg_launch_unpack(c, d_stage, width, d_bits, n, hv_d, d_hv);
-  };
-  if ((rc = whole(ref_packed, ref_stride, rw, ref_bits, ref_norm, n_ref, d_rp, d_rbits, d_rn, d_ref))) return rc;
-  if (!same && (rc = whole(qry_packed, qry_stride, qw, qry_bits, qry_norm, n_qry, d_qp, d_qbits, d_qn, d_qry))) return rc;
-  if ((rc = search_run(c, d_ref, d_rn, n_ref, d_qry, d_qn, n_qry, hv_d, ksize, top_k, ani_min, path, std::max(rmax, qmax), d_out, d_nf,
-                       d_milli)))
+  if ((rc = hg_rows_to_device(c, hr, hv_d)) || (!same && (rc = hg_rows_to_device(c, hq, hv_d)))) return rc;
+  if ((rc = search_run(c, hr.d_hv, hr.d_norm, R.n, hq.d_hv, hq.d_norm, Q.n, hv_d, ksize, top_k, ani_min, path,
+                       std::max(R.max_bits, Q.max_bits), d_out, d_nf, d_milli)))
     return rc;
   *d_out_p = d_out;
   *d_nf_p = d_nf;
   *d_milli_p = d_milli;
+  return HG_OK;
+}
+
+int hg_search_packed_host(hg_ctx *c, const char *who, hg_packed_rows R, hg_packed_rows Q, uint32_t hv_d, uint32_t ksize,
+                          uint32_t top_k, float ani_min, int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli) {
+  memset(c->search_stats, 0, sizeof(c->search_stats));
+  const size_t n_out = (size_t)Q.n * top_k;
+  if (Q.n == 0) return HG_OK;
+  if (R.n == 0) {
+    memset(out, 0, n_out * sizeof(hg_hit));
+    memset(n_found, 0, (size_t)Q.n * 4);
+    if (ani_milli) memset(ani_milli, 0, n_out * 4);
+    return HG_OK;
+  }
+  int rc;
+  bool same;
+  if ((rc = hg_packed_rows_check(who, &R, &Q, hv_d, &same))) return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  hg_hit *d_out;
+  uint32_t *d_nf, *d_milli;
+  if ((rc = hg_search_packed_run(c, R, Q, same, hv_d, ksize, top_k, ani_min, path, &d_out, &d_nf, &d_milli))) return rc;
+  HG_CUDA(cudaMemcpyAsync(out, d_out, n_out * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaMemcpyAsync(n_found, d_nf, (size_t)Q.n * 4, cudaMemcpyDeviceToHost, c->stream));
+  if (ani_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, n_out * 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
   return HG_OK;
 }
 
@@ -1445,34 +1441,12 @@ extern "C" int hg_search_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t r
                                 const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min,
                                 int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli) {
   if (!c) { hg_set_error("hg_search_packed: NULL argument"); return HG_E_INVALID; }
+  const hg_packed_rows R = {ref_packed, ref_stride, ref_bits, ref_norm, n_ref}, Q = {qry_packed, qry_stride, qry_bits, qry_norm, n_qry};
   int rc;
-  if ((rc = hg_search_packed_check("hg_search_packed", ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits,
-                                   qry_norm, n_qry, hv_d, top_k, path, out, n_found)))
+  if ((rc = hg_packed_args_check("hg_search_packed", R, Q, hv_d)) ||
+      (rc = hg_search_check("hg_search_packed", n_qry, out, n_found, hv_d, top_k, path)))
     return rc;
-  memset(c->search_stats, 0, sizeof(c->search_stats));
-  if (n_qry == 0) return HG_OK;
-  if (n_ref == 0) {
-    memset(out, 0, (size_t)n_qry * top_k * sizeof(hg_hit));
-    memset(n_found, 0, (size_t)n_qry * 4);
-    if (ani_milli) memset(ani_milli, 0, (size_t)n_qry * top_k * 4);
-    return HG_OK;
-  }
-  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
-  uint32_t rmax, qmax;
-  if ((rc = hg_search_packed_bits("hg_search_packed", ref_bits, n_ref, ref_stride, qry_bits, n_qry, qry_stride, same, hv_d, &rmax, &qmax)))
-    return rc;
-  HG_CUDA(cudaSetDevice(c->device));
-  hg_hit *d_out;
-  uint32_t *d_nf, *d_milli;
-  if ((rc = hg_search_packed_run(c, same, ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits, qry_norm,
-                                 n_qry, hv_d, ksize, top_k, ani_min, path, rmax, qmax, &d_out, &d_nf, &d_milli)))
-    return rc;
-  const size_t n_out = (size_t)n_qry * top_k;
-  HG_CUDA(cudaMemcpyAsync(out, d_out, n_out * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
-  HG_CUDA(cudaMemcpyAsync(n_found, d_nf, (size_t)n_qry * 4, cudaMemcpyDeviceToHost, c->stream));
-  if (ani_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, n_out * 4, cudaMemcpyDeviceToHost, c->stream));
-  HG_CUDA(cudaStreamSynchronize(c->stream));
-  return HG_OK;
+  return hg_search_packed_host(c, "hg_search_packed", R, Q, hv_d, ksize, top_k, ani_min, path, out, n_found, ani_milli);
 }
 
 int hg_search_merge(hg_ctx *c, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0, uint32_t n_qry,

@@ -380,19 +380,62 @@ int hg_launch_search_floors(hg_ctx *ctx, const unsigned long long *d_floor_key, 
 // i + i0[m] does not fit 32 bits, |= 2 if some input n_found exceeds top_k (the caller zeroes it before)
 int hg_launch_search_merge(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0,
                            uint32_t n_qry, uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli, uint32_t *d_status);
-// The pieces of hg_search_packed (api.cu) that hg_group_search_packed (peer.cu) shares: the argument checks (`who` names
-// the entry in the error), every row's hv_quant_bits checked -> the largest of the refs and of the queries (0 when
-// `same`), and one search of packed host rows whose result stays on the device (HG_S_TILES of the context).
-int hg_search_packed_check(const char *who, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
-                           const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
-                           const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t top_k, int path, const hg_hit *out,
-                           const uint32_t *n_found);
-int hg_search_packed_bits(const char *who, const uint8_t *ref_bits, uint32_t n_ref, uint64_t ref_stride, const uint8_t *qry_bits,
-                          uint32_t n_qry, uint64_t qry_stride, bool same, uint32_t hv_d, uint32_t *rmax, uint32_t *qmax);
-int hg_search_packed_run(hg_ctx *ctx, bool same, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
-                         const int32_t *ref_norm, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride, const uint8_t *qry_bits,
-                         const int32_t *qry_norm, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, uint32_t top_k, float ani_min, int path,
-                         uint32_t rmax, uint32_t qmax, hg_hit **d_out, uint32_t **d_n_found, uint32_t **d_milli);
+// ---- packed sketch rows from the host (api.cu), shared by the packed dist and search entries and their group forms ----
+
+// One matrix of packed sketch rows in host memory, as the sketch file holds them: row g starts `stride` bytes after row
+// g - 1, has hv_quant_bits bits[g] in 1..16 and bits[g] * hv_d / 8 live bytes.  max_bits: set by hg_packed_rows_check.
+struct hg_packed_rows {
+  const uint8_t *packed;
+  uint64_t stride;
+  const uint8_t *bits;
+  const int32_t *norm;
+  uint32_t n;
+  uint32_t max_bits;
+  uint64_t width(uint32_t hv_d) const { return (uint64_t)max_bits * hv_d / 8; }  // bytes of a row that can be live
+  hg_packed_rows rows(uint32_t a, uint32_t m) const { return {packed + a * stride, stride, bits + a, norm + a, m, max_bits}; }
+};
+// The argument checks of a packed entry (`who` names it in the error): the pointers of a non-empty matrix, hv_d % 256
+// and stride % 4.
+int hg_packed_args_check(const char *who, const hg_packed_rows &R, const hg_packed_rows &Q, uint32_t hv_d);
+// Every row's hv_quant_bits in 1..16 and the live width of each matrix within its stride; sets max_bits.  *same: ref and
+// query are the same rows (same pointers and n); then Q becomes R.
+int hg_packed_rows_check(const char *who, hg_packed_rows *R, hg_packed_rows *Q, uint32_t hv_d, bool *same);
+
+// Host rows on their way to the device, and where they land.
+struct HostRows {
+  const uint8_t *base;  // first row on the host
+  uint64_t stride;      // bytes between host rows
+  uint64_t width;       // bytes of a row that travel (int16 rows: 2 hv_d; packed rows: max hv_quant_bits * hv_d / 8)
+  const uint8_t *bits;  // packed rows: hv_quant_bits per row (host); int16 rows: NULL
+  const int32_t *norm;  // host
+  uint32_t n;
+  uint8_t *d_stage;     // packed rows: where they land (width apart); int16 rows: the matrix itself
+  uint8_t *d_bits;      // packed rows
+  int16_t *d_hv;
+  int32_t *d_norm;
+};
+// Device room for a ref block and a query block of packed rows (one block when `same`): int16 rows in HG_S_HV, each
+// block 256-byte aligned; norms, then bits in HG_S_SMALL; packed bytes in HG_S_TABLES.
+int hg_packed_stage(hg_ctx *ctx, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, HostRows *hr,
+                    HostRows *hq);
+// One block of rows copied whole on ctx->stream (rows, norms, bits), packed rows unpacked to their int16 rows.
+int hg_rows_to_device(hg_ctx *ctx, const HostRows &S, uint32_t hv_d);
+// The output stage of n > 0 hits on the device: sorted into the reference's order if asked (ANI thousandths into
+// ani_milli when it is not NULL), copied to the host; returns when the copies are complete.
+int hg_hits_to_host(hg_ctx *ctx, hg_hit *d_hits, uint64_t n, bool sorted, hg_hit *hits, uint32_t *ani_milli);
+// hg_dist_packed after its checks.
+int hg_dist_packed_run(hg_ctx *ctx, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, uint32_t ksize,
+                       float ani_th, int symmetric, int path, bool sorted, hg_hit *hits, uint32_t *ani_milli, uint64_t cap,
+                       uint64_t *n_hits);
+// The search arguments of a search entry that do not describe rows: out / n_found, hv_d, top_k and path.
+int hg_search_check(const char *who, uint32_t n_qry, const hg_hit *out, const uint32_t *n_found, uint32_t hv_d, uint32_t top_k,
+                    int path);
+// hg_search_packed after its argument checks (`who` names the entry that was called).
+int hg_search_packed_host(hg_ctx *ctx, const char *who, hg_packed_rows R, hg_packed_rows Q, uint32_t hv_d, uint32_t ksize,
+                          uint32_t top_k, float ani_min, int path, hg_hit *out, uint32_t *n_found, uint32_t *ani_milli);
+// One search of checked packed rows whose result stays on the device (HG_S_TILES of the context).
+int hg_search_packed_run(hg_ctx *ctx, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, uint32_t ksize,
+                         uint32_t top_k, float ani_min, int path, hg_hit **d_out, uint32_t **d_n_found, uint32_t **d_milli);
 // hg_search_merge_dev after its argument checks (the context's device is current); returns with the result complete
 int hg_search_merge(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0, uint32_t n_qry,
                     uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli);

@@ -966,16 +966,7 @@ extern "C" int hg_dist_sharded_hits(hg_peer *p, int sorted, hg_hit *hits, uint32
     return HG_OK;
   }
   if (!hits) { hg_set_error("hg_dist_sharded_hits: hits is NULL"); return HG_E_INVALID; }
-  hg_hit *d_hits = (hg_hit *)(p->win[p->rank] + p->gather_off);
-  void *d_milli = nullptr;
-  if (sorted) {
-    if (ani_milli && (rc = hg_scratch(c, HG_S_MISC, cnt * 4 + 256, &d_milli))) return rc;
-    if ((rc = hg_launch_sort_hits(c, d_hits, cnt, (uint32_t *)d_milli))) return rc;
-  }
-  HG_CUDA(cudaMemcpyAsync(hits, d_hits, cnt * sizeof(hg_hit), cudaMemcpyDeviceToHost, c->stream));
-  if (d_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, d_milli, cnt * 4, cudaMemcpyDeviceToHost, c->stream));
-  HG_CUDA(cudaStreamSynchronize(c->stream));
-  return HG_OK;
+  return hg_hits_to_host(c, (hg_hit *)(p->win[p->rank] + p->gather_off), cnt, sorted != 0, hits, ani_milli);
 }
 
 // device pointers of the root's hit list and counter as this member addresses them (benchmarks, callers with their own tail)
@@ -1094,37 +1085,20 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
                                     uint64_t cap, uint64_t *n_hits) {
   if (!g || !n_hits) { hg_set_error("hg_group_dist_packed: NULL argument"); return HG_E_INVALID; }
   *n_hits = 0;
-  if ((n_ref && (!ref_packed || !ref_bits || !ref_norm)) || (n_qry && (!qry_packed || !qry_bits || !qry_norm)) || (cap && !hits)) {
-    hg_set_error("hg_group_dist_packed: NULL argument"); return HG_E_INVALID;
-  }
-  if (hv_d == 0 || hv_d % 256 != 0 || ref_stride % 4 != 0 || qry_stride % 4 != 0) {
-    hg_set_error("hg_group_dist_packed: hv_d %% 256 or row stride %% 4"); return HG_E_INVALID;
-  }
-  if (n_ref == 0 || n_qry == 0) return HG_OK;
-  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
-  // a single GPU, too little work to share, or a shape only the single-GPU entry handles (one matrix against itself
-  // with both orders, the j > i filter over two different matrices): the single-GPU entry
-  if (g->n == 1 || (uint64_t)n_ref * n_qry < 1024ull * 1024ull || hv_d % 512 != 0 || (same && !symmetric) || (!same && symmetric))
-    return hg_dist_packed(g->ctx[0], ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits, qry_norm, n_qry,
-                          hv_d, ksize, ani_th, symmetric, 0, sorted, hits, ani_milli, cap, n_hits);
-  uint32_t rmax = 0, qmax = 0;
-  for (uint32_t i = 0; i < n_ref; ++i) {
-    if (ref_bits[i] < 1 || ref_bits[i] > 16) { hg_set_error("hg_group_dist_packed: ref sketch %u has hv_quant_bits %u", i, (unsigned)ref_bits[i]); return HG_E_INVALID; }
-    rmax = std::max<uint32_t>(rmax, ref_bits[i]);
-  }
-  for (uint32_t i = 0; i < n_qry && !same; ++i) {
-    if (qry_bits[i] < 1 || qry_bits[i] > 16) { hg_set_error("hg_group_dist_packed: query sketch %u has hv_quant_bits %u", i, (unsigned)qry_bits[i]); return HG_E_INVALID; }
-    qmax = std::max<uint32_t>(qmax, qry_bits[i]);
-  }
-  if (same) qmax = rmax;
-  const uint32_t bmax = std::max(rmax, qmax);
-  if (bmax > 13) {  // beyond the limb split: the exact SIMT kernel of the single-GPU entry
-    return hg_dist_packed(g->ctx[0], ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits, qry_norm, n_qry,
-                          hv_d, ksize, ani_th, symmetric, 0, sorted, hits, ani_milli, cap, n_hits);
-  }
-  const size_t rw = (size_t)rmax * hv_d / 8, qw = (size_t)qmax * hv_d / 8;
-  if (rw > ref_stride || qw > qry_stride) { hg_set_error("hg_group_dist_packed: row stride below hv_quant_bits * hv_d / 8"); return HG_E_INVALID; }
+  hg_packed_rows R = {ref_packed, ref_stride, ref_bits, ref_norm, n_ref}, Q = {qry_packed, qry_stride, qry_bits, qry_norm, n_qry};
   int rc;
+  if (cap && !hits) { hg_set_error("hg_group_dist_packed: NULL argument"); return HG_E_INVALID; }
+  if ((rc = hg_packed_args_check("hg_group_dist_packed", R, Q, hv_d))) return rc;
+  if (n_ref == 0 || n_qry == 0) return HG_OK;
+  bool same;
+  if ((rc = hg_packed_rows_check("hg_group_dist_packed", &R, &Q, hv_d, &same))) return rc;
+  const uint32_t bmax = std::max(R.max_bits, Q.max_bits);
+  // a single GPU, too little work to share, a shape only the single-GPU entry handles (one matrix against itself with
+  // both orders, the j > i filter over two different matrices), or rows beyond the limb split (its exact SIMT kernel)
+  if (g->n == 1 || (uint64_t)n_ref * n_qry < 1024ull * 1024ull || hv_d % 512 != 0 || (same && !symmetric) || (!same && symmetric) ||
+      bmax > 13)
+    return hg_dist_packed_run(g->ctx[0], R, Q, same, hv_d, ksize, ani_th, symmetric, HG_PATH_AUTO, sorted != 0, hits, ani_milli, cap,
+                              n_hits);
   const int N = g->n;
   if ((rc = group_windows(g, hg_peer_window_need(n_qry, hv_d, cap)))) return rc;
   // row blocks: multiples of 256 rows when there are enough rows (what the ring ownership of the all-vs-all needs), else of 4
@@ -1133,12 +1107,12 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
     if (n >= 512u * (uint32_t)N) return std::min<uint32_t>(n, 256u * (uint32_t)(((uint64_t)k * ((n + 255) / 256) + N / 2) / N));  // the 256-row tile rows, dealt evenly
     return (uint32_t)(((uint64_t)n * k / N) & ~3ull);
   };
-  struct Member { uint32_t r0, rn, q0, qn; int16_t *d_ref, *d_qry; int32_t *d_rn, *d_qn; };
+  struct Member { uint32_t r0; HostRows r, q; };  // a self-comparison has no ref block: its query rows are all of it
   std::vector<Member> M(N);
   auto make_call = [&](const Member &m) {
     ShardCall a = {};
-    a.d_ref_hv = m.d_ref; a.d_ref_norm = m.d_rn; a.n_ref_local = m.rn; a.ref_row0 = m.r0;
-    a.d_qry_hv = m.d_qry; a.d_qry_norm = m.d_qn;
+    a.d_ref_hv = m.r.d_hv; a.d_ref_norm = m.r.d_norm; a.n_ref_local = m.r.n; a.ref_row0 = m.r0;
+    a.d_qry_hv = m.q.d_hv; a.d_qry_norm = m.q.d_norm;
     for (int k = 0; k <= N; ++k) a.qb[k] = bound(n_qry, k);
     a.hv_d = hv_d; a.ksize = ksize; a.ani_th = ani_th; a.symmetric = symmetric; a.root = 0; a.cap = cap; a.mapped_hits = nullptr;
     return a;
@@ -1147,20 +1121,12 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
   for (int k = 0; k < N; ++k) {
     hg_ctx *c = g->ctx[k];
     Member &m = M[k];
-    m.q0 = bound(n_qry, k); m.qn = bound(n_qry, k + 1) - m.q0;
-    m.r0 = same ? 0 : bound(n_ref, k); m.rn = same ? 0 : bound(n_ref, k + 1) - m.r0;
+    const uint32_t q0 = bound(n_qry, k);
+    m.r0 = same ? 0 : bound(n_ref, k);
+    const uint32_t rn = same ? 0 : bound(n_ref, k + 1) - m.r0;
     HG_CUDA(cudaSetDevice(c->device));
-    void *d_mat, *d_small, *d_pk;
-    const size_t qb = ((size_t)m.qn * hv_d * 2 + 255) & ~(size_t)255, rb = (size_t)m.rn * hv_d * 2;
-    if ((rc = hg_scratch(c, HG_S_HV, qb + rb + 512, &d_mat))) return rc;
-    if ((rc = hg_scratch(c, HG_S_SMALL, ((size_t)m.qn + m.rn) * 5 + 512, &d_small))) return rc;
-    if ((rc = hg_scratch(c, HG_S_TABLES, (size_t)m.qn * qw + (size_t)m.rn * rw + 512, &d_pk))) return rc;
-    m.d_qry = (int16_t *)d_mat;
-    m.d_ref = (int16_t *)((uint8_t *)d_mat + qb);
-    m.d_qn = (int32_t *)d_small;
-    m.d_rn = m.d_qn + m.qn;
-    const ShardCall a = make_call(m);
-    if ((rc = shard_check(g->peer[k], a))) return rc;
+    if ((rc = hg_packed_stage(c, R.rows(m.r0, rn), Q.rows(q0, bound(n_qry, k + 1) - q0), false, hv_d, &m.r, &m.q))) return rc;
+    if ((rc = shard_check(g->peer[k], make_call(m)))) return rc;
   }
   // b-bit values are below 2^(b-1): above 10 bits no row fits the single plane, and up to 13 bits every element fits two limbs
   int used = bmax > 10 ? HG_PATH_TWO_LIMB : HG_PATH_NARROW;
@@ -1178,21 +1144,8 @@ extern "C" int hg_group_dist_packed(hg_group *g, const uint8_t *ref_packed, uint
     return HG_OK;
   };
   for (int k = 0; k < N; ++k) {
-    hg_ctx *c = g->ctx[k];
-    Member &m = M[k];
-    HG_CUDA(cudaSetDevice(c->device));
-    uint8_t *d_pk = (uint8_t *)c->d_scratch[HG_S_TABLES];
-    uint8_t *d_bits = (uint8_t *)c->d_scratch[HG_S_SMALL] + ((size_t)m.qn + m.rn) * 4;
-    auto load = [&](const uint8_t *packed, uint64_t stride, size_t w, const uint8_t *bits, const int32_t *norm, uint32_t r0, uint32_t n,
-                    uint8_t *d_stage, uint8_t *d_b, int32_t *d_n, int16_t *d_hv) -> int {
-      if (n == 0) return HG_OK;
-      HG_CUDA(cudaMemcpy2DAsync(d_stage, w, packed + (size_t)r0 * stride, stride, w, n, cudaMemcpyHostToDevice, c->stream));
-      HG_CUDA(cudaMemcpyAsync(d_b, bits + r0, n, cudaMemcpyHostToDevice, c->stream));
-      HG_CUDA(cudaMemcpyAsync(d_n, norm + r0, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
-      return hg_launch_unpack(c, d_stage, w, d_b, n, hv_d, d_hv);
-    };
-    if ((rc = load(qry_packed, qry_stride, qw, qry_bits, qry_norm, m.q0, m.qn, d_pk, d_bits, m.d_qn, m.d_qry))) return rc;
-    if ((rc = load(ref_packed, ref_stride, rw, ref_bits, ref_norm, m.r0, m.rn, d_pk + (size_t)m.qn * qw, d_bits + m.qn, m.d_rn, m.d_ref))) return rc;
+    HG_CUDA(cudaSetDevice(g->ctx[k]->device));
+    if ((rc = hg_rows_to_device(g->ctx[k], M[k].q, hv_d)) || (rc = hg_rows_to_device(g->ctx[k], M[k].r, hv_d))) return rc;
   }
   int32_t absmax = -1;
   if ((rc = enqueue_all(used))) return rc;
@@ -1235,33 +1188,26 @@ extern "C" int hg_group_search_packed(hg_group *g, const uint8_t *ref_packed, ui
     memset(g->ctx[k]->search_stats, 0, sizeof(g->ctx[k]->search_stats));
     g->ctx[k]->search_ev_used = 0;
   }
-  const int parts = (int)std::min<uint32_t>((uint32_t)g->n, std::max<uint32_t>(1u, n_ref / 1024u));
-  if (parts == 1)
-    return hg_search_packed(g->ctx[0], ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride, qry_bits, qry_norm, n_qry,
-                            hv_d, ksize, top_k, ani_min, path, out, n_found, ani_milli);
+  hg_packed_rows R = {ref_packed, ref_stride, ref_bits, ref_norm, n_ref}, Q = {qry_packed, qry_stride, qry_bits, qry_norm, n_qry};
+  const char *who = "hg_group_search_packed";
   int rc;
-  if ((rc = hg_search_packed_check("hg_group_search_packed", ref_packed, ref_stride, ref_bits, ref_norm, n_ref, qry_packed, qry_stride,
-                                   qry_bits, qry_norm, n_qry, hv_d, top_k, path, out, n_found)))
-    return rc;
+  if ((rc = hg_packed_args_check(who, R, Q, hv_d)) || (rc = hg_search_check(who, n_qry, out, n_found, hv_d, top_k, path))) return rc;
+  const int parts = (int)std::min<uint32_t>((uint32_t)g->n, std::max<uint32_t>(1u, n_ref / 1024u));
+  if (parts == 1) return hg_search_packed_host(g->ctx[0], who, R, Q, hv_d, ksize, top_k, ani_min, path, out, n_found, ani_milli);
   if (n_qry == 0) return HG_OK;
-  const bool same = (ref_packed == qry_packed && ref_bits == qry_bits && ref_norm == qry_norm && n_ref == n_qry);
-  uint32_t rmax, qmax;
-  if ((rc = hg_search_packed_bits("hg_group_search_packed", ref_bits, n_ref, ref_stride, qry_bits, n_qry, qry_stride, same, hv_d, &rmax,
-                                  &qmax)))
-    return rc;
-  if (same) qmax = rmax;  // every member holds a ref block and all queries: two matrices
+  bool same;
+  if ((rc = hg_packed_rows_check(who, &R, &Q, hv_d, &same))) return rc;
   std::vector<uint32_t> b(parts + 1);
   for (int k = 0; k <= parts; ++k) b[k] = (uint32_t)((uint64_t)n_ref * k / parts);
   std::vector<hg_hit *> d_out(parts);
   std::vector<uint32_t *> d_nf(parts), d_milli(parts);
   std::vector<int> rcs(parts, HG_OK);
   std::vector<std::string> msgs(parts);
-  auto member = [&](int m) -> int {
+  auto member = [&](int m) -> int {  // every member holds a ref block and all queries: two matrices, even when `same`
     hg_ctx *c = g->ctx[m];
     HG_CUDA(cudaSetDevice(c->device));
-    return hg_search_packed_run(c, false, ref_packed + (size_t)b[m] * ref_stride, ref_stride, ref_bits + b[m], ref_norm + b[m],
-                                b[m + 1] - b[m], qry_packed, qry_stride, qry_bits, qry_norm, n_qry, hv_d, ksize, top_k, ani_min, path,
-                                rmax, qmax, &d_out[m], &d_nf[m], &d_milli[m]);
+    return hg_search_packed_run(c, R.rows(b[m], b[m + 1] - b[m]), Q, false, hv_d, ksize, top_k, ani_min, path, &d_out[m], &d_nf[m],
+                                &d_milli[m]);
   };
   std::vector<std::thread> th;
   for (int k = 0; k < parts; ++k) {

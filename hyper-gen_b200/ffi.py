@@ -158,21 +158,51 @@ def make_params(k=21, scaled=1500, seed=123, canonical=True, hv_d=4096) -> Sketc
     return SketchParams(scaled=scaled, seed=seed, hv_d=hv_d, ksize=k, canonical=int(bool(canonical)))
 
 
+def _packed_rows(ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2):
+    """the ref and the query rows of an hg_*_packed call as contiguous (packed, bits, norm2) arrays; when qry_packed is
+    ref_packed the query side is the ref's own arrays, so that the library compares one matrix with itself"""
+    r = (np.ascontiguousarray(ref_packed, np.uint8), np.ascontiguousarray(ref_bits, np.uint8), np.ascontiguousarray(ref_norm2, np.int32))
+    if qry_packed is ref_packed:
+        return r, r
+    return r, (np.ascontiguousarray(qry_packed, np.uint8), np.ascontiguousarray(qry_bits, np.uint8),
+               np.ascontiguousarray(qry_norm2, np.int32))
+
+
+def _row_args(rows):
+    """(packed, stride, bits, norm2, n) of one matrix, as the hg_*_packed entries take them"""
+    p, b, n = rows
+    return _ptr(p), p.strides[0] if p.shape[0] else 0, _ptr(b), _ptr(n), p.shape[0]
+
+
+def _dist_packed(fn, h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize, ani_th, mode, sorted_output,
+                 cap):
+    """hg_dist_packed / hg_group_dist_packed (fn) on the context / group h; mode: the arguments between ani_th and
+    sorted ((symmetric, path), or (symmetric,) for the group)"""
+    r, q = _packed_rows(ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2)
+    if cap is None:
+        cap = max(1024, r[0].shape[0] * q[0].shape[0] // 64)
+    while True:
+        hits = np.empty(cap, HIT_DTYPE)
+        milli = np.empty(cap, np.uint32)
+        n_hits = C.c_uint64(0)
+        rc = fn(h, *_row_args(r), *_row_args(q), hv_d, ksize, ani_th, *mode, int(sorted_output), _ptr(hits), _ptr(milli), cap,
+                C.byref(n_hits))
+        if rc == HG_E_CAPACITY and n_hits.value > cap:
+            cap = int(n_hits.value)
+            continue
+        _check(rc)
+        # ani_milli is written by the output-stage sort only (hypergen_b200.h): unsorted calls get None
+        return hits[: n_hits.value].copy(), (milli[: n_hits.value].copy() if sorted_output else None)
+
+
 def _search_packed(fn, h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize, top_k, ani_min, path):
     """hg_search_packed / hg_group_search_packed (fn) on the context / group h"""
-    rp = np.ascontiguousarray(ref_packed, np.uint8)
-    rb = np.ascontiguousarray(ref_bits, np.uint8)
-    rn = np.ascontiguousarray(ref_norm2, np.int32)
-    same = qry_packed is ref_packed
-    qp = rp if same else np.ascontiguousarray(qry_packed, np.uint8)
-    qb = rb if same else np.ascontiguousarray(qry_bits, np.uint8)
-    qn = rn if same else np.ascontiguousarray(qry_norm2, np.int32)
-    R, Q = rp.shape[0], qp.shape[0]
+    r, q = _packed_rows(ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2)
+    Q = q[0].shape[0]
     hits = np.zeros((Q, top_k), HIT_DTYPE)
     n_found = np.zeros(Q, np.uint32)
     milli = np.zeros((Q, top_k), np.uint32)
-    _check(fn(h, _ptr(rp), rp.strides[0] if R else 0, _ptr(rb), _ptr(rn), R, _ptr(qp), qp.strides[0] if Q else 0, _ptr(qb), _ptr(qn),
-              Q, hv_d, ksize, top_k, ani_min, path, _ptr(hits), _ptr(n_found), _ptr(milli)))
+    _check(fn(h, *_row_args(r), *_row_args(q), hv_d, ksize, top_k, ani_min, path, _ptr(hits), _ptr(n_found), _ptr(milli)))
     return hits, n_found, milli
 
 
@@ -391,30 +421,8 @@ class Context:
     def dist_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize=21, ani_th=85.0,
                     symmetric=False, path=0, sorted_output=True, cap=None):
         """hg_dist_packed: packed sketch rows (n x stride uint8) + quant bits + norms -> (hits, ani_milli)."""
-        rp = np.ascontiguousarray(ref_packed, np.uint8)
-        rb = np.ascontiguousarray(ref_bits, np.uint8)
-        rn = np.ascontiguousarray(ref_norm2, np.int32)
-        same = qry_packed is ref_packed
-        qp = rp if same else np.ascontiguousarray(qry_packed, np.uint8)
-        qb = rb if same else np.ascontiguousarray(qry_bits, np.uint8)
-        qn = rn if same else np.ascontiguousarray(qry_norm2, np.int32)
-        R, Q = rp.shape[0], qp.shape[0]
-        if cap is None:
-            cap = max(1024, R * Q // 64)
-        while True:
-            hits = np.empty(cap, HIT_DTYPE)
-            milli = np.empty(cap, np.uint32)
-            n_hits = C.c_uint64(0)
-            rc = load().hg_dist_packed(self._h, _ptr(rp), rp.strides[0] if R else 0, _ptr(rb), _ptr(rn), R, _ptr(qp),
-                                       qp.strides[0] if Q else 0, _ptr(qb), _ptr(qn), Q, hv_d, ksize, ani_th,
-                                       int(symmetric), path, int(sorted_output), _ptr(hits), _ptr(milli), cap,
-                                       C.byref(n_hits))
-            if rc == HG_E_CAPACITY and n_hits.value > cap:
-                cap = int(n_hits.value)
-                continue
-            _check(rc)
-            # ani_milli is written by the output-stage sort only (hypergen_b200.h): unsorted calls get None
-            return hits[: n_hits.value].copy(), (milli[: n_hits.value].copy() if sorted_output else None)
+        return _dist_packed(load().hg_dist_packed, self._h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d,
+                            ksize, ani_th, (int(symmetric), path), sorted_output, cap)
 
     def search_dev(self, d_ref, d_ref_norm2, n_ref, d_qry, d_qry_norm2, n_qry, hv_d, ksize, top_k, ani_min, path, d_out,
                    d_n_found, d_ani_milli=None):
@@ -600,28 +608,9 @@ class Group:
 
     def dist_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize=21, ani_th=85.0,
                     symmetric=False, sorted_output=True, cap=None):
-        rp = np.ascontiguousarray(ref_packed, np.uint8)
-        rb = np.ascontiguousarray(ref_bits, np.uint8)
-        rn = np.ascontiguousarray(ref_norm2, np.int32)
-        same = qry_packed is ref_packed
-        qp = rp if same else np.ascontiguousarray(qry_packed, np.uint8)
-        qb = rb if same else np.ascontiguousarray(qry_bits, np.uint8)
-        qn = rn if same else np.ascontiguousarray(qry_norm2, np.int32)
-        R, Q = rp.shape[0], qp.shape[0]
-        if cap is None:
-            cap = max(1024, R * Q // 64)
-        while True:
-            hits = np.empty(cap, HIT_DTYPE)
-            milli = np.empty(cap, np.uint32)
-            n_hits = C.c_uint64(0)
-            rc = load().hg_group_dist_packed(self._h, _ptr(rp), rp.strides[0] if R else 0, _ptr(rb), _ptr(rn), R, _ptr(qp),
-                                             qp.strides[0] if Q else 0, _ptr(qb), _ptr(qn), Q, hv_d, ksize, ani_th,
-                                             int(symmetric), int(sorted_output), _ptr(hits), _ptr(milli), cap, C.byref(n_hits))
-            if rc == HG_E_CAPACITY and n_hits.value > cap:
-                cap = int(n_hits.value)
-                continue
-            _check(rc)
-            return hits[: n_hits.value].copy(), (milli[: n_hits.value].copy() if sorted_output else None)
+        """hg_group_dist_packed: Context.dist_packed over the GPUs of the group (the group entry takes no path)."""
+        return _dist_packed(load().hg_group_dist_packed, self._h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2,
+                            hv_d, ksize, ani_th, (int(symmetric),), sorted_output, cap)
 
     def search_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize=21, top_k=10,
                       ani_min=0.0, path=0):
