@@ -7,6 +7,7 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <functional>
 #include <vector>
 
 #include "hg_common.cuh"
@@ -52,6 +53,7 @@ extern "C" int hg_init(int device, hg_ctx **out) {
   hg_ctx *c = new hg_ctx();
   memset(c, 0, sizeof(*c));
   c->device = device;
+  hg_cluster_stats_reset(c);
   struct Guard { hg_ctx *c; ~Guard() { if (c) hg_destroy(c); } } guard{c};  // nothing leaks when a step below fails
   cudaDeviceProp prop;
   HG_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -802,6 +804,18 @@ void hg_dist_record(hg_ctx *c, int path, const char *fmt, ...) {
   va_end(ap);
 }
 
+// A window of the pairs of one matrix against itself: ref rows [r0, r0 + h) x query rows [c0, c0 + w), reported with
+// the call's global offsets (i0 + r, j0 + c).
+struct DistWindow { uint32_t r0, h, c0, w; };
+// A dist call that runs only these windows (a cluster run, hg_cluster_*): every row is prepared once, then each window is
+// launched and `after(k)` is enqueued behind the launch of window k - by every kernel branch, the two-limb rerun after a
+// declined single plane included.
+struct DistWindows {
+  std::vector<DistWindow> win;
+  std::function<int(size_t)> after;
+  cudaEvent_t prepared = nullptr;  // if set: recorded once the rows are prepared, before the first window
+};
+
 // one dist call: ref rows [i0, i0 + n_ref) against query rows [j0, j0 + n_qry), both matrices in HBM (or arriving there)
 struct DistOp {
   const int16_t *ref;
@@ -818,6 +832,7 @@ struct DistOp {
   unsigned long long *n_hits;
   const hg_floor *floors = nullptr;  // a search's main pass: per-query thresholds in place of ani_th (hg_floors)
   const float *cfrac_row = nullptr;
+  const DistWindows *windows = nullptr;  // one matrix against itself (ref and query the same rows in HBM): only these windows
 };
 
 // The kernel a dist call tries first, chosen before anything runs.
@@ -967,9 +982,19 @@ static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, H
   for (size_t k = 0; k < chunks.size(); k++) {
     const uint32_t a = chunks[k].first, rows = chunks[k].second;
     if ((!in_q || one) && (rc = prep(hr, Rn, Rl, a, rows, c->ev_chunk[2 + k]))) return rc;
+    if (op.windows) continue;  // they run below, once every row is prepared
     rc = one ? launch(0, a + rows, op.i0, op.ref_norm, a, rows, op.j0 + a, op.qry_norm + a)
              : launch(r_off + a, rows, op.i0 + a, op.ref_norm + a, 0, op.n_qry, op.j0, op.qry_norm);
     if (rc) return rc;
+  }
+  if (op.windows) {
+    if (op.windows->prepared) HG_CUDA(cudaEventRecord(op.windows->prepared, c->stream));
+    for (size_t k = 0; k < op.windows->win.size(); k++) {
+      const DistWindow &w = op.windows->win[k];
+      if ((rc = launch(w.r0, w.h, op.i0 + w.r0, op.ref_norm + w.r0, w.c0, w.w, op.j0 + w.c0, op.qry_norm + w.c0)) ||
+          (rc = op.windows->after(k)))
+        return rc;
+    }
   }
   if (!hr) HG_PROF(c, 5);
   f->chunks = hr ? (uint32_t)chunks.size() : 0;
@@ -1019,8 +1044,16 @@ static int dist_run(hg_ctx *c, const DistOp &op, const DistChoice &ch, HostRows 
   if (ran == HG_PATH_SIMT) {
     HG_PROF(c, 4);
     const hg_floors fl = {op.floors, op.cfrac_row};
-    rc = hg_launch_dist_simt(c, op.ref, op.ref_norm, op.n_ref, op.i0, op.qry, op.qry_norm, op.n_qry, op.j0, op.hv_d, op.ksize, op.ani_th,
-                             op.symmetric, op.hits, op.cap, op.n_hits, op.floors ? &fl : nullptr);
+    const DistWindow all = {0, op.n_ref, 0, op.n_qry};
+    const size_t n_win = op.windows ? op.windows->win.size() : 1;
+    rc = HG_OK;
+    for (size_t k = 0; k < n_win && !rc; k++) {
+      const DistWindow &w = op.windows ? op.windows->win[k] : all;
+      rc = hg_launch_dist_simt(c, op.ref + (size_t)w.r0 * op.hv_d, op.ref_norm + w.r0, w.h, op.i0 + w.r0, op.qry + (size_t)w.c0 * op.hv_d,
+                               op.qry_norm + w.c0, w.w, op.j0 + w.c0, op.hv_d, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits,
+                               op.floors ? &fl : nullptr);
+      if (!rc && op.windows) rc = op.windows->after(k);
+    }
     HG_PROF(c, 5);
     if (rc) return rc;
   }
@@ -1487,5 +1520,219 @@ extern "C" int hg_search_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
     if ((c->search_ev_used >> from[k] & 1) && (c->search_ev_used >> (k + 1) & 1))
       HG_CUDA(cudaEventElapsedTime(&ms[k], c->ev_search[from[k]], c->ev_search[k + 1]));
   }
+  return HG_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// cluster: single-linkage ANI clusters of one sketch set (DESIGN.md §4.9)
+// ---------------------------------------------------------------------------------------
+
+// edge records one window may hold: 2^26 (1 GiB of hg_hit), or HG_CLUSTER_EDGE_CAP, read at every call (at least 256 x 256)
+static uint64_t cluster_edge_cap() {
+  uint64_t cap = 0;
+  if (const char *e = getenv("HG_CLUSTER_EDGE_CAP")) cap = strtoull(e, nullptr, 10);
+  return std::max<uint64_t>(cap ? cap : 1ull << 26, 256ull * 256ull);
+}
+
+// The upper triangle of n rows, columns [c0, n), cut into windows of at most cap pairs j > i.  Column chunks [a, a + w)
+// of a multiple of 256 columns (the last one ends at n) run against refs [0, a + w), each chunk as wide as keeps its
+// a w + w (w - 1) / 2 pairs within cap; where even 256 columns have more, the refs of a 256-column chunk are split into
+// blocks of floor(cap / 256) rows rounded down to a multiple of 256.  So no window's hits can overflow the edge buffer.
+static std::vector<DistWindow> cluster_windows(uint32_t n, uint32_t c0, uint64_t cap) {
+  std::vector<DistWindow> out;
+  auto pairs = [](uint64_t a, uint64_t w) { return a * w + w * (w - 1) / 2; };
+  for (uint32_t a = c0; a < n;) {
+    uint32_t w = std::min<uint32_t>(256, n - a);
+    if (pairs(a, w) <= cap) {
+      while (w < n - a && pairs(a, std::min<uint32_t>(w + 256, n - a)) <= cap) w = std::min<uint32_t>(w + 256, n - a);
+      out.push_back({0, a + w, a, w});
+    } else {
+      const uint32_t h = (uint32_t)std::min<uint64_t>(cap / 256 / 256 * 256, a + w);
+      for (uint32_t r0 = 0; r0 < a + w; r0 += h) out.push_back({r0, std::min(h, a + w - r0), a, w});
+    }
+    a += w;
+  }
+  return out;
+}
+
+void hg_cluster_stats_reset(hg_ctx *c) {
+  memset(c->cluster_stats, 0, sizeof(c->cluster_stats));
+  for (float &m : c->cluster_ms) m = -1.0f;
+}
+
+int hg_cluster_finish(hg_ctx *c, uint32_t *d_rep, uint32_t n, uint32_t *rep, uint32_t *n_clusters, cudaEvent_t flattened) {
+  int rc;
+  void *d_misc;
+  if ((rc = hg_scratch(c, HG_S_MISC, 256, &d_misc))) return rc;
+  uint32_t *d_count = (uint32_t *)d_misc + 1;
+  HG_CUDA(cudaMemsetAsync(d_count, 0, 4, c->stream));
+  if ((rc = hg_launch_cluster_flatten(c, d_rep, n, d_count))) return rc;
+  if (flattened) HG_CUDA(cudaEventRecord(flattened, c->stream));
+  uint32_t count = 0;
+  HG_CUDA(cudaMemcpyAsync(&count, d_count, 4, cudaMemcpyDeviceToHost, c->stream));
+  if (rep && n) HG_CUDA(cudaMemcpyAsync(rep, d_rep, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  if (n_clusters) *n_clusters = count;
+  return HG_OK;
+}
+
+// Device events of a cluster run with profiling on: [0] start, [1] rows prepared, then per window before / after its hook,
+// then the end.  Destroyed with the run.
+struct ClusterEvents {
+  std::vector<cudaEvent_t> ev;
+  ~ClusterEvents() { for (cudaEvent_t e : ev) cudaEventDestroy(e); }
+  int ms(int a, int b, float *out) const {  // both recorded
+    HG_CUDA(cudaEventElapsedTime(out, ev[a], ev[b]));
+    return HG_OK;
+  }
+};
+
+// The single-linkage clusters of rows [0, n) over the linked pairs whose column is in [c0, n) (all of them when c0 = 0):
+// the kernel is chosen once for the whole matrix, every row prepared once, and the windows of cluster_windows launched one
+// after another, each followed on the stream by the hook kernel on its edges and a reset of the edge counter.  d_rep ends
+// as a flattened forest (rep[x] = the smallest index of x's cluster); rep / n_clusters as hg_cluster_finish.  bits: as
+// dist_choose.  Synchronises once, at the end (and where the single-plane verdict is read, as every dist run does).
+static int cluster_run(hg_ctx *c, const int16_t *d_hv, const int32_t *d_norm, uint32_t n, uint32_t c0, uint32_t hv_d, uint32_t ksize,
+                       float ani_th, int path, uint32_t bits, uint32_t *d_rep, uint32_t *rep, uint32_t *n_clusters) {
+  hg_cluster_stats_reset(c);
+  c->pending_stats[0] = c->pending_stats[1] = nullptr;
+  c->ev_used &= ~(3 << 4);
+  if (n == 0) {
+    if (n_clusters) *n_clusters = 0;
+    return HG_OK;
+  }
+  int rc;
+  DistChoice ch;
+  if ((rc = dist_choose(path, n, n, hg_tensor_shape_ok(hv_d, d_hv, d_hv) == HG_OK, bits, &ch))) return rc;
+  const uint64_t cap = cluster_edge_cap();
+  const uint64_t room = std::max<uint64_t>(1, std::min<uint64_t>(cap, (uint64_t)n * (n - 1) / 2));  // no window has more pairs
+  void *d_edges, *d_cnt;
+  if ((rc = hg_scratch(c, HG_S_PACKED, room * sizeof(hg_hit), &d_edges))) return rc;
+  if ((rc = hg_scratch(c, HG_S_COUNTS, 256, &d_cnt))) return rc;
+  unsigned long long *cnt = (unsigned long long *)d_cnt, *linked = cnt + 1;  // edge counter; linked pairs and the largest window's
+  DistWindows W;
+  W.win = cluster_windows(n, c0, cap);
+  ClusterEvents E;
+  if (c->prof) {
+    E.ev.resize(3 + 2 * W.win.size(), nullptr);
+    for (cudaEvent_t &e : E.ev) HG_CUDA(cudaEventCreate(&e));
+    W.prepared = E.ev[1];
+  }
+  auto mark = [&](size_t k) -> int {
+    if (c->prof) HG_CUDA(cudaEventRecord(E.ev[k], c->stream));
+    return HG_OK;
+  };
+  HG_CUDA(cudaMemsetAsync(d_cnt, 0, 3 * sizeof(unsigned long long), c->stream));
+  if ((rc = hg_launch_cluster_iota(c, d_rep, n)) || (rc = mark(0))) return rc;
+  W.after = [&](size_t k) -> int {
+    int r2;
+    if ((r2 = mark(2 + 2 * k)) || (r2 = hg_launch_cluster_hook(c, d_rep, (const hg_hit *)d_edges, cnt, room, linked))) return r2;
+    HG_CUDA(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), c->stream));
+    return mark(3 + 2 * k);
+  };
+  DistOp op = {d_hv, d_norm, n, 0, d_hv, d_norm, n, 0, hv_d, ksize, ani_th, 1, (hg_hit *)d_edges, room, cnt};
+  op.windows = &W;
+  if ((rc = dist_run(c, op, ch, nullptr, nullptr, false))) return rc;
+  unsigned long long h_linked[2] = {0, 0};
+  HG_CUDA(cudaMemcpyAsync(h_linked, linked, sizeof(h_linked), cudaMemcpyDeviceToHost, c->stream));
+  if ((rc = hg_cluster_finish(c, d_rep, n, rep, n_clusters, c->prof ? E.ev.back() : nullptr))) return rc;
+  c->cluster_stats[0] = W.win.size();
+  c->cluster_stats[1] = h_linked[0];
+  c->cluster_stats[2] = h_linked[1];
+  c->cluster_stats[3] = cap;
+  if (c->prof && !W.win.empty()) {
+    const int last = (int)(3 + 2 * (W.win.size() - 1)), end = (int)E.ev.size() - 1;
+    const bool prepared = c->dist_path != HG_PATH_SIMT;  // the SIMT kernel prepares nothing: ms[0] stays -1
+    float hooks = 0.0f, t, windows, flatten, prep = -1.0f;
+    for (size_t k = 0; k < W.win.size(); k++) {
+      if ((rc = E.ms((int)(2 + 2 * k), (int)(3 + 2 * k), &t))) return rc;
+      hooks += t;
+    }
+    if ((prepared && (rc = E.ms(0, 1, &prep))) || (rc = E.ms(prepared ? 1 : 0, last, &windows)) || (rc = E.ms(last, end, &flatten))) return rc;
+    c->cluster_ms[0] = prep;
+    c->cluster_ms[1] = windows - hooks;
+    c->cluster_ms[2] = hooks;
+    c->cluster_ms[3] = flatten;
+  }
+  return HG_OK;
+}
+
+int hg_cluster_check(const char *who, uint32_t n, const uint32_t *rep, uint32_t hv_d, float ani_th, int path) {
+  if (n && !rep) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
+  if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("%s: hv_d %u must be a multiple of 256", who, hv_d); return HG_E_INVALID; }
+  if (path < HG_PATH_AUTO || path > HG_PATH_NARROW) { hg_set_error("%s: path %d", who, path); return HG_E_INVALID; }
+  if (ani_th != ani_th) { hg_set_error("%s: ani_th is NaN", who); return HG_E_INVALID; }
+  return HG_OK;
+}
+
+extern "C" int hg_cluster_dev(hg_ctx *c, const int16_t *d_hv, const int32_t *d_norm2, uint32_t n, uint32_t hv_d, uint32_t ksize,
+                              float ani_th, int path, uint32_t *d_rep, uint32_t *n_clusters) {
+  if (!c || (n && (!d_hv || !d_norm2))) { hg_set_error("hg_cluster_dev: NULL argument"); return HG_E_INVALID; }
+  int rc;
+  if ((rc = hg_cluster_check("hg_cluster_dev", n, d_rep, hv_d, ani_th, path))) return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  return cluster_run(c, d_hv, d_norm2, n, 0, hv_d, ksize, ani_th, path, 0, d_rep, nullptr, n_clusters);
+}
+
+int hg_cluster_packed_run(hg_ctx *c, const hg_packed_rows &R, uint32_t col0, uint32_t hv_d, uint32_t ksize, float ani_th, int path,
+                          uint32_t **d_rep, uint32_t *rep, uint32_t *n_clusters) {
+  int rc;
+  HostRows hr, hq;
+  if ((rc = hg_packed_stage(c, R, R, true, hv_d, &hr, &hq))) return rc;
+  void *d_f;
+  if ((rc = hg_scratch(c, HG_S_TILES, (size_t)R.n * 4, &d_f))) return rc;
+  *d_rep = (uint32_t *)d_f;
+  if ((rc = hg_rows_to_device(c, hr, hv_d))) return rc;
+  return cluster_run(c, hr.d_hv, hr.d_norm, R.n, col0, hv_d, ksize, ani_th, path, R.max_bits, *d_rep, rep, n_clusters);
+}
+
+int hg_cluster_packed_host(hg_ctx *c, const char *who, hg_packed_rows R, uint32_t hv_d, uint32_t ksize, float ani_th, int path,
+                           uint32_t *rep, uint32_t *n_clusters) {
+  hg_cluster_stats_reset(c);
+  if (R.n == 0) {
+    if (n_clusters) *n_clusters = 0;
+    return HG_OK;
+  }
+  int rc;
+  bool same;
+  hg_packed_rows Q = R;
+  if ((rc = hg_packed_rows_check(who, &R, &Q, hv_d, &same))) return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  uint32_t *d_rep;
+  return hg_cluster_packed_run(c, R, 0, hv_d, ksize, ani_th, path, &d_rep, rep, n_clusters);
+}
+
+extern "C" int hg_cluster_packed(hg_ctx *c, const uint8_t *packed, uint64_t stride, const uint8_t *quant_bits, const int32_t *norm2,
+                                 uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th, int path, uint32_t *rep, uint32_t *n_clusters) {
+  if (!c) { hg_set_error("hg_cluster_packed: NULL argument"); return HG_E_INVALID; }
+  const hg_packed_rows R = {packed, stride, quant_bits, norm2, n};
+  int rc;
+  if ((rc = hg_packed_args_check("hg_cluster_packed", R, R, hv_d)) || (rc = hg_cluster_check("hg_cluster_packed", n, rep, hv_d, ani_th, path)))
+    return rc;
+  return hg_cluster_packed_host(c, "hg_cluster_packed", R, hv_d, ksize, ani_th, path, rep, n_clusters);
+}
+
+extern "C" int hg_cluster_union_dev(hg_ctx *c, uint32_t n, uint32_t *d_rep, const hg_hit *d_edges, uint64_t n_edges, uint32_t *n_clusters) {
+  if (!c || (n && !d_rep) || (n_edges && !d_edges)) { hg_set_error("hg_cluster_union_dev: NULL argument"); return HG_E_INVALID; }
+  HG_CUDA(cudaSetDevice(c->device));
+  int rc;
+  void *d_misc;
+  if ((rc = hg_scratch(c, HG_S_MISC, 256, &d_misc))) return rc;
+  uint32_t *d_status = (uint32_t *)d_misc, status = 0;
+  // nothing may reach a find before this: an index >= n would be an access out of bounds, a rep[x] > x a possible cycle
+  HG_CUDA(cudaMemsetAsync(d_status, 0, 4, c->stream));
+  if ((rc = hg_launch_cluster_check(c, d_rep, n, d_edges, n_edges, d_status))) return rc;
+  HG_CUDA(cudaMemcpyAsync(&status, d_status, 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  if (status & 1) { hg_set_error("hg_cluster_union_dev: an edge index is >= n (%u)", n); return HG_E_INVALID; }
+  if (status & 2) { hg_set_error("hg_cluster_union_dev: rep[x] > x for some x: not a forest this union accepts"); return HG_E_INVALID; }
+  if ((rc = hg_launch_cluster_hook(c, d_rep, d_edges, nullptr, n_edges, nullptr))) return rc;
+  return hg_cluster_finish(c, d_rep, n, nullptr, n_clusters);
+}
+
+extern "C" int hg_cluster_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
+  if (!c || !counts || !ms) { hg_set_error("hg_cluster_stats: NULL argument"); return HG_E_INVALID; }
+  memcpy(counts, c->cluster_stats, sizeof(c->cluster_stats));
+  memcpy(ms, c->cluster_ms, sizeof(c->cluster_ms));
   return HG_OK;
 }

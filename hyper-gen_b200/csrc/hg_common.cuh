@@ -165,6 +165,10 @@ struct hg_ctx {
   uint64_t search_stats[4];
   cudaEvent_t ev_search[5];
   int search_ev_used;
+  // the last cluster run (hg_cluster_stats): windows, linked pairs, largest window's pairs, edge capacity; device ms of
+  // its steps (-1: not run or profiling off)
+  uint64_t cluster_stats[4];
+  float cluster_ms[4];
 };
 
 // stage boundaries: 0 start, 1 after staging/memsets, 2 after k-mer hash, 3 after encode,
@@ -191,18 +195,22 @@ enum hg_scratch_slot {
   HG_S_SEQ = 0,        // staged sequence bytes (two halves when the H2D pipeline is active); search: the sample rows
   HG_S_DESC = 1,       // hg_genome_desc[] (+ sentinels); search: the per-query floors
   HG_S_TABLES = 2,     // per-genome hash tables / explicit hash sets
-  HG_S_COUNTS = 3,     // distinct-hash counters; dist: the hit counter of the host entry
+  HG_S_COUNTS = 3,     // distinct-hash counters; dist: the hit counter of the host entry; cluster: the edge counter and
+                       // the run's linked-pair counts
   HG_S_HV = 4,         // int16 HVs (sketch output staging; dist: both matrices of the host entry)
   HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass;
-                       // group search: the members' results gathered on GPU 0
+                       // group search: the members' results gathered on GPU 0; cluster: the edges of one window
   HG_S_SMALL = 6,      // norms / bits / counts per sketch
-  HG_S_MISC = 7,       // CTA -> genome map, |hv| max, probe sink, status word of a search merge
+  HG_S_MISC = 7,       // CTA -> genome map, |hv| max, probe sink, status word of a search merge; cluster: status word
+                       // of a union check, root count of a flatten
   HG_S_REF_LIMBS = 8,  // s8 limb planes of the ref matrix (dist_tc)
   HG_S_QRY_LIMBS = 9,  // s8 limb planes of the query matrix (dist_tc)
-  HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort; search: the per-query segments; group search: the merged result
+  HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort; search: the per-query segments; group search: the merged result;
+                       // group cluster: the merged forest and the members' forests gathered on GPU 0
   HG_S_SORT_CNT = 11,  // digit counters of the hit sort; search: per-query counts and offsets
   HG_S_NARROW_META = 12,  // per-row constants + outlier lists of the single-plane dist path (dist_narrow)
-  HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entries
+  HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entries;
+                          // cluster: the forest of the packed entry
   HG_S_COUNT = 14
 };
 // scratch slot `slot` grown to at least `bytes` (contents not preserved)
@@ -440,3 +448,30 @@ int hg_search_packed_run(hg_ctx *ctx, const hg_packed_rows &R, const hg_packed_r
 int hg_search_merge(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in, const uint32_t *d_in_found, const uint32_t *i0, uint32_t n_qry,
                     uint32_t top_k, hg_hit *d_out, uint32_t *d_n_found, uint32_t *d_milli);
 int hg_launch_absmax(hg_ctx *ctx, const int16_t *d_hv, uint64_t n_elems, int32_t *d_out);
+
+// ---- ANI clustering (cluster.cu, api.cu): union-find over a forest parent[0, n) with parent[x] <= x (DESIGN.md §4.9) ----
+int hg_launch_cluster_iota(hg_ctx *ctx, uint32_t *d_parent, uint32_t n);
+// unites (i, j) of the first min(*d_count, cap) records (d_count NULL: cap records; every index < n of the forest);
+// d_stats (may be NULL): [0] += that number of records, [1] = max([1], it)
+int hg_launch_cluster_hook(hg_ctx *ctx, uint32_t *d_parent, const hg_hit *d_edges, const unsigned long long *d_count, uint64_t cap,
+                           unsigned long long *d_stats);
+// unites (x, d_other[x]) for every x < n; d_other is a forest over at least those n nodes
+int hg_launch_cluster_hook_labels(hg_ctx *ctx, uint32_t *d_parent, const uint32_t *d_other, uint32_t n);
+// after every hook: d_parent[x] = the root of x for every x < n, *d_n_roots += the number of roots (the caller zeroes it)
+int hg_launch_cluster_flatten(hg_ctx *ctx, uint32_t *d_parent, uint32_t n, uint32_t *d_n_roots);
+// *d_status |= 1 if some edge index is >= n, |= 2 if some d_parent[x] > x (the caller zeroes it)
+int hg_launch_cluster_check(hg_ctx *ctx, const uint32_t *d_parent, uint32_t n, const hg_hit *d_edges, uint64_t n_edges,
+                            uint32_t *d_status);
+// The arguments of a cluster entry that do not describe rows (`who` names it): rep, hv_d, ani_th and path.
+int hg_cluster_check(const char *who, uint32_t n, const uint32_t *rep, uint32_t hv_d, float ani_th, int path);
+// hg_cluster_packed after its argument checks (`who` names the entry that was called).
+int hg_cluster_packed_host(hg_ctx *ctx, const char *who, hg_packed_rows R, uint32_t hv_d, uint32_t ksize, float ani_th, int path,
+                           uint32_t *rep, uint32_t *n_clusters);
+// One cluster run over checked packed rows R: the pairs whose column is in [col0, R.n), as a flattened forest over the
+// R.n rows in HG_S_TILES of the context (*d_rep); rep and n_clusters as hg_cluster_finish.
+int hg_cluster_packed_run(hg_ctx *ctx, const hg_packed_rows &R, uint32_t col0, uint32_t hv_d, uint32_t ksize, float ani_th, int path,
+                          uint32_t **d_rep, uint32_t *rep, uint32_t *n_clusters);
+// Flattens the forest d_rep[0, n) and counts its roots; rep (host, may be NULL) receives the labels and n_clusters (may be
+// NULL) the count; `flattened` (may be NULL) is recorded behind the flatten.  Returns with all of it complete.
+int hg_cluster_finish(hg_ctx *ctx, uint32_t *d_rep, uint32_t n, uint32_t *rep, uint32_t *n_clusters, cudaEvent_t flattened = nullptr);
+void hg_cluster_stats_reset(hg_ctx *ctx);

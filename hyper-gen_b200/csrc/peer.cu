@@ -28,6 +28,7 @@
 // Measured on 2 B200s (tools/ipc_probe.cu): push of a 21 MB slice + two barriers 49 us (NCCL all_gather
 // of the same plane 69 us), flag barrier 6.3 us.
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <string>
 #include <thread>
@@ -1247,4 +1248,73 @@ extern "C" int hg_group_search_packed(hg_group *g, const uint8_t *ref_packed, ui
   if (ani_milli) HG_CUDA(cudaMemcpyAsync(ani_milli, r_milli, n_out * 4, cudaMemcpyDeviceToHost, c0->stream));
   HG_CUDA(cudaStreamSynchronize(c0->stream));
   return HG_OK;
+}
+
+// hg_cluster_packed over all GPUs of the group (DESIGN.md §4.9).  The upper triangle is cut by query column into one range
+// per member, b_k = n sqrt(k / parts) rounded to 256, which gives every member about the same number of pairs: member m
+// takes the columns [b_m, b_m+1) against the refs [0, b_m+1).  It copies packed rows [0, b_m+1) over its own PCIe link,
+// unpacks and prepares them, and builds its own forest of those rows with the single-GPU windows and hooks.  As many
+// members as give each at least 2^23 pairs (a 4096-row triangle) take part.  One host thread per GPU drives its members:
+// members that share a device ordinal run one after another (as in hg_group_search_packed).  The forests are copied to
+// GPU 0 and united there into iota(n): the partition of a union of edge sets is the union-find over the members' forests,
+// so the result is the single-GPU one.  The only exchange is one label per row and member, so no windows.
+extern "C" int hg_group_cluster_packed(hg_group *g, const uint8_t *packed, uint64_t stride, const uint8_t *quant_bits, const int32_t *norm2,
+                                       uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th, int path, uint32_t *rep,
+                                       uint32_t *n_clusters) {
+  if (!g) { hg_set_error("hg_group_cluster_packed: NULL argument"); return HG_E_INVALID; }
+  for (int k = 0; k < g->n; ++k) hg_cluster_stats_reset(g->ctx[k]);  // a member without columns reports no run
+  hg_packed_rows R = {packed, stride, quant_bits, norm2, n};
+  const char *who = "hg_group_cluster_packed";
+  int rc;
+  if ((rc = hg_packed_args_check(who, R, R, hv_d)) || (rc = hg_cluster_check(who, n, rep, hv_d, ani_th, path))) return rc;
+  const uint64_t pairs = n ? (uint64_t)n * (n - 1) / 2 : 0;
+  const int parts = (int)std::min<uint64_t>((uint64_t)g->n, std::max<uint64_t>(1, pairs >> 23));
+  if (parts == 1) return hg_cluster_packed_host(g->ctx[0], who, R, hv_d, ksize, ani_th, path, rep, n_clusters);
+  bool same;
+  hg_packed_rows Q = R;
+  if ((rc = hg_packed_rows_check(who, &R, &Q, hv_d, &same))) return rc;
+  std::vector<uint32_t> b(parts + 1, n);
+  b[0] = 0;
+  for (int k = 1; k < parts; ++k) {
+    const uint32_t want = (uint32_t)(std::lround((double)n * std::sqrt((double)k / parts) / 256.0) * 256);
+    b[k] = std::min(n, std::max(b[k - 1], want));
+  }
+  std::vector<uint32_t *> d_rep(parts);
+  std::vector<int> rcs(parts, HG_OK);
+  std::vector<std::string> msgs(parts);
+  auto member = [&](int m) -> int {
+    hg_ctx *c = g->ctx[m];
+    HG_CUDA(cudaSetDevice(c->device));
+    return hg_cluster_packed_run(c, R.rows(0, b[m + 1]), b[m], hv_d, ksize, ani_th, path, &d_rep[m], nullptr, nullptr);
+  };
+  std::vector<std::thread> th;
+  for (int k = 0; k < parts; ++k) {
+    bool first_on_device = true;
+    for (int l = 0; l < k; ++l) first_on_device &= g->ctx[l]->device != g->ctx[k]->device;
+    if (!first_on_device) continue;
+    th.emplace_back([&, k]() {
+      for (int m = k; m < parts; ++m) {
+        if (g->ctx[m]->device != g->ctx[k]->device) continue;
+        if ((rcs[m] = member(m))) msgs[m] = hg_last_error();
+      }
+    });
+  }
+  for (auto &t : th) t.join();
+  for (int k = 0; k < parts; ++k)
+    if (rcs[k]) { hg_set_error("GPU %d (columns %u..%u): %s", g->ctx[k]->device, b[k], b[k + 1], msgs[k].c_str()); return rcs[k]; }
+  // merge on GPU 0: iota(n), then every member's forest gathered next to it and united into it
+  hg_ctx *c0 = g->ctx[0];
+  HG_CUDA(cudaSetDevice(c0->device));
+  uint64_t words = n;
+  for (int k = 0; k < parts; ++k) words += b[k + 1];
+  void *d_buf;
+  if ((rc = hg_scratch(c0, HG_S_SORT_TMP, words * 4, &d_buf))) return rc;
+  uint32_t *merged = (uint32_t *)d_buf, *f = merged + n;
+  if ((rc = hg_launch_cluster_iota(c0, merged, n))) return rc;
+  for (int k = 0; k < parts; ++k) {
+    if (b[k + 1]) HG_CUDA(cudaMemcpyPeerAsync(f, c0->device, d_rep[k], g->ctx[k]->device, (size_t)b[k + 1] * 4, c0->stream));
+    if ((rc = hg_launch_cluster_hook_labels(c0, merged, f, b[k + 1]))) return rc;
+    f += b[k + 1];
+  }
+  return hg_cluster_finish(c0, merged, n, rep, n_clusters);
 }

@@ -22,8 +22,9 @@ EXPORTS = [
     "hg_kmer_hash", "hg_sketch_batch", "hg_sketch_batch_dev", "hg_sketch_status", "hg_unpack", "hg_unpack_dev",
     "hg_dist", "hg_dist_dev", "hg_dist_status", "hg_dist_last_path", "hg_dist_last_reason", "hg_sort_hits_dev", "hg_dist_sorted", "hg_dist_packed",
     "hg_search_dev", "hg_search_packed", "hg_search_stats", "hg_search_merge_dev",
+    "hg_cluster_dev", "hg_cluster_packed", "hg_cluster_union_dev", "hg_cluster_stats",
     "hg_group_create", "hg_group_destroy", "hg_group_size", "hg_group_ctx", "hg_group_sketch_fasta_batch", "hg_group_dist_packed",
-    "hg_group_search_packed",
+    "hg_group_search_packed", "hg_group_cluster_packed",
     "hg_peer_window_need", "hg_peer_create", "hg_peer_connect", "hg_peer_create_local", "hg_peer_destroy", "hg_peer_rank",
     "hg_peer_world", "hg_peer_barrier", "hg_peer_stage_ms", "hg_peer_timeline", "hg_peer_plan_tiles", "hg_peer_plan_push", "hg_dist_sharded_dev", "hg_dist_sharded_hits", "hg_peer_hit_buffers",
 ]
@@ -108,6 +109,12 @@ def load() -> C.CDLL:
     L.hg_search_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, u32, C.c_float, i32, vp, vp, vp]
     L.hg_search_stats.restype = i32; L.hg_search_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
     L.hg_search_merge_dev.restype = i32; L.hg_search_merge_dev.argtypes = [vp, u32, vp, vp, vp, u32, u32, vp, vp, vp]
+    L.hg_cluster_dev.restype = i32
+    L.hg_cluster_dev.argtypes = [vp, vp, vp, u32, u32, u32, C.c_float, i32, vp, C.POINTER(u32)]
+    L.hg_cluster_packed.restype = i32
+    L.hg_cluster_packed.argtypes = [vp, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, vp, C.POINTER(u32)]
+    L.hg_cluster_union_dev.restype = i32; L.hg_cluster_union_dev.argtypes = [vp, u32, vp, vp, u64, C.POINTER(u32)]
+    L.hg_cluster_stats.restype = i32; L.hg_cluster_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
     L.hg_group_create.restype = i32; L.hg_group_create.argtypes = [i32, vp, C.POINTER(vp)]
     L.hg_group_destroy.restype = None; L.hg_group_destroy.argtypes = [vp]
     L.hg_group_size.restype = i32; L.hg_group_size.argtypes = [vp]
@@ -118,6 +125,8 @@ def load() -> C.CDLL:
                                        C.POINTER(u64)]
     L.hg_group_search_packed.restype = i32
     L.hg_group_search_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, u32, C.c_float, i32, vp, vp, vp]
+    L.hg_group_cluster_packed.restype = i32
+    L.hg_group_cluster_packed.argtypes = [vp, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, vp, C.POINTER(u32)]
     L.hg_peer_window_need.restype = u64; L.hg_peer_window_need.argtypes = [u32, u32, u64]
     L.hg_peer_create.restype = i32; L.hg_peer_create.argtypes = [vp, i32, i32, u64, vp, C.POINTER(vp)]
     L.hg_peer_connect.restype = i32; L.hg_peer_connect.argtypes = [vp, vp]
@@ -209,6 +218,21 @@ def _search_packed(fn, h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits,
 def _search_stats(ctx_handle):
     counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
     _check(load().hg_search_stats(ctx_handle, counts, ms))
+    return [int(x) for x in counts], [float(x) for x in ms]
+
+
+def _cluster_packed(fn, h, packed, bits, norm2, hv_d, ksize, ani_th, path):
+    """hg_cluster_packed / hg_group_cluster_packed (fn) on the context / group h"""
+    p, b, nm = _packed_rows(packed, bits, norm2, packed, bits, norm2)[0]
+    rep = np.zeros(p.shape[0], np.uint32)
+    n_clusters = C.c_uint32(0)
+    _check(fn(h, *_row_args((p, b, nm)), hv_d, ksize, ani_th, path, _ptr(rep), C.byref(n_clusters)))
+    return rep, int(n_clusters.value)
+
+
+def _cluster_stats(ctx_handle):
+    counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
+    _check(load().hg_cluster_stats(ctx_handle, counts, ms))
     return [int(x) for x in counts], [float(x) for x in ms]
 
 
@@ -450,6 +474,29 @@ class Context:
         _check(load().hg_search_merge_dev(self._h, n_lists, d_in, d_in_found, _ptr(off), n_qry, top_k, d_out, d_n_found,
                                           d_ani_milli))
 
+    def cluster_dev(self, d_hv, d_norm2, n, hv_d, ksize, ani_th, path, d_rep) -> int:
+        """hg_cluster_dev: device pointers (ints); d_rep receives rep[i] = the smallest index of i's cluster.
+        Returns the number of clusters once the result is complete."""
+        n_clusters = C.c_uint32(0)
+        _check(load().hg_cluster_dev(self._h, d_hv, d_norm2, n, hv_d, ksize, ani_th, path, d_rep, C.byref(n_clusters)))
+        return int(n_clusters.value)
+
+    def cluster_packed(self, packed, bits, norm2, hv_d, ksize=21, ani_th=95.0, path=0):
+        """hg_cluster_packed: packed sketch rows (n x stride uint8) + quant bits + norms -> (rep[n], n_clusters)"""
+        return _cluster_packed(load().hg_cluster_packed, self._h, packed, bits, norm2, hv_d, ksize, ani_th, path)
+
+    def cluster_union_dev(self, n, d_rep, d_edges, n_edges) -> int:
+        """hg_cluster_union_dev: unite n_edges hg_hit records (device) into the forest d_rep[n] (device) and flatten it;
+        returns the number of clusters"""
+        n_clusters = C.c_uint32(0)
+        _check(load().hg_cluster_union_dev(self._h, n, d_rep, d_edges, n_edges, C.byref(n_clusters)))
+        return int(n_clusters.value)
+
+    def cluster_stats(self):
+        """hg_cluster_stats of the last cluster run -> ([windows, linked pairs, largest window's pairs, edge capacity],
+        [ms of preparing the rows, dist windows, hooks, flatten + count] (-1: not run or profiling off))"""
+        return _cluster_stats(self._h)
+
     def sort_hits_dev(self, d_hits, n, d_ani_milli=None):
         """hg_sort_hits_dev: device records to the reference's output order, in place."""
         _check(load().hg_sort_hits_dev(self._h, d_hits, n, d_ani_milli))
@@ -621,3 +668,11 @@ class Group:
     def search_stats(self, i: int = 0):
         """Context.search_stats of member i's part of the last group search"""
         return _search_stats(load().hg_group_ctx(self._h, i))
+
+    def cluster_packed(self, packed, bits, norm2, hv_d, ksize=21, ani_th=95.0, path=0):
+        """hg_group_cluster_packed: Context.cluster_packed over the GPUs of the group; same result."""
+        return _cluster_packed(load().hg_group_cluster_packed, self._h, packed, bits, norm2, hv_d, ksize, ani_th, path)
+
+    def cluster_stats(self, i: int = 0):
+        """Context.cluster_stats of member i's part of the last group cluster run"""
+        return _cluster_stats(load().hg_group_ctx(self._h, i))

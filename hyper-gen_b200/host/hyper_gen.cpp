@@ -16,6 +16,10 @@
 //   hyper-gen search -r <ref sketch> -q <query sketch> -o <out> [-n 10] [-a 0.0]
 //       the -n best refs of every query with ANI >= -a (ties by ascending ref index), one line per result,
 //       queries in file order.  The refs are split over every visible GPU (hg_group_search_packed); HG_GPUS=n limits it.
+//   hyper-gen cluster -r <sketch> -o <out> [-a 95.0]
+//       single-linkage clusters at ANI >= -a, one `representative\tmember` line per sketch: clusters by ascending
+//       representative (the smallest index of the cluster), members ascending, the representative's own line first.
+//       The pairs are split over every visible GPU (hg_group_cluster_packed); HG_GPUS=n limits it.
 // The GPU path is the only path (`-D gpu` is implied): there is no CPU fallback.
 #include <algorithm>
 #include <chrono>
@@ -64,6 +68,11 @@ struct SketchSearch {
   std::string path_ref_sketch, path_query_sketch, out_file;
   uint32_t top_k = 10;
   float ani_min = 0.0f;
+};
+
+struct SketchCluster {
+  std::string path_sketch, out_file;
+  float ani_th = 95.0f;
 };
 
 }  // namespace types
@@ -397,18 +406,49 @@ void search(const types::SketchSearch &ss) {
 
 }  // namespace search
 
+namespace cluster {
+
+void cluster(const types::SketchCluster &sc) {
+  auto sk = utils::load_sketch(sc.path_sketch);
+  if (sk.empty()) die("empty sketch file");
+  const size_t D = sk[0].hv_d, n = sk.size();
+  const dist::Stacked s = dist::stack(sk, D);
+  hg_group *group = open_group();
+  std::vector<uint32_t> rep(n);
+  uint32_t n_clusters = 0;
+  check(hg_group_cluster_packed(group, s.packed.data(), 2 * D, s.bits.data(), s.norm.data(), (uint32_t)n, (uint32_t)D, sk[0].ksize,
+                                sc.ani_th, 0, rep.data(), &n_clusters),
+        "hg_group_cluster_packed");
+  hg_group_destroy(group);
+  std::vector<uint32_t> order(n);
+  for (size_t t = 0; t < n; t++) order[t] = (uint32_t)t;
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return rep[a] < rep[b]; });
+  std::string out;
+  for (uint32_t t : order) {
+    out += sk[rep[t]].file_str; out += '\t'; out += sk[t].file_str; out += '\n';
+  }
+  std::ofstream f(sc.out_file, std::ios::binary);
+  if (!f) die("Dump cluster file failed!");
+  f.write(out.data(), (std::streamsize)out.size());
+  fprintf(stdout, "Output %zu sketches in %u clusters (ANI >= %.1f) to file %s\n", n, n_clusters, (double)sc.ani_th,
+          sc.out_file.c_str());
+}
+
+}  // namespace cluster
+
 int main(int argc, char **argv) {
-  if (argc < 2) die("usage: hyper-gen <sketch|dist|search> ...");
+  if (argc < 2) die("usage: hyper-gen <sketch|dist|search|cluster> ...");
   const std::string mode = argv[1];
   types::SketchParams sp;
   types::SketchDist sd;
   types::SketchSearch ss;
+  types::SketchCluster sc;
   bool ani_given = false;
   for (int i = 2; i + 1 < argc; i += 2) {
     const std::string k = argv[i], v = argv[i + 1];
     if (k == "-p" || k == "--path") sp.path = v;
-    else if (k == "-o" || k == "--out") { sp.out_file = v; sd.out_file = v; ss.out_file = v; }
-    else if (k == "-r" || k == "--path_r") { sd.path_ref_sketch = v; ss.path_ref_sketch = v; }
+    else if (k == "-o" || k == "--out") { sp.out_file = v; sd.out_file = v; ss.out_file = v; sc.out_file = v; }
+    else if (k == "-r" || k == "--path_r") { sd.path_ref_sketch = v; ss.path_ref_sketch = v; sc.path_sketch = v; }
     else if (k == "-q" || k == "--path_q") { sd.path_query_sketch = v; ss.path_query_sketch = v; }
     else if (k == "-n" || k == "--top_k") {
       const long n = atol(v.c_str());
@@ -435,6 +475,10 @@ int main(int argc, char **argv) {
     if (ss.path_ref_sketch.empty() || ss.path_query_sketch.empty() || ss.out_file.empty()) die("search needs -r -q -o");
     if (ani_given) ss.ani_min = sd.ani_threshold;
     search::search(ss);
+  } else if (mode == "cluster") {
+    if (sc.path_sketch.empty() || sc.out_file.empty()) die("cluster needs -r -o");
+    if (ani_given) sc.ani_th = sd.ani_threshold;
+    cluster::cluster(sc);
   } else {
     die("unknown subcommand " + mode);
   }

@@ -399,6 +399,43 @@ HG_API int hg_search_merge_dev(hg_ctx *ctx, uint32_t n_lists, const hg_hit *d_in
                                const uint32_t *i0 /* host, n_lists entries */, uint32_t n_qry, uint32_t top_k, hg_hit *d_out,
                                uint32_t *d_n_found, uint32_t *d_ani_milli /* may be NULL */);
 
+/* ---- ANI clustering: which sketches of one set belong together ---------------------------------------------------
+ * Single linkage over one sketch set of n rows, all against all: sketches i < j are linked when ani(i, j) >= ani_th -
+ * exactly the pairs hg_dist(..., symmetric = 1, ani_th) reports - and a cluster is a connected component of that graph.
+ * rep[i] = the smallest index in i's cluster (so rep[i] <= i, and rep[i] == i marks a representative); *n_clusters
+ * (host, may be NULL) = the number of representatives.  The result does not depend on the kernel, the window plan, the
+ * thread schedule or the number of GPUs.  n == 0: HG_OK with n_clusters = 0; ani_th <= 0 links everything (every ANI
+ * is >= 0); a sketch with norm 0 has ANI 0 to everything; a NaN ani_th is HG_E_INVALID.
+ *   path   as hg_search_dev (0 auto, 1 SIMT, 2 two-limb, 3 single plane) with the same choice and fallbacks;
+ *          hg_dist_last_path / hg_dist_last_reason report the run.
+ * The linked pairs never leave the device: the dist kernels emit them window by window (at most HG_CLUSTER_EDGE_CAP
+ * records each, default 2^26, read at every call) into library scratch, and a lock-free union-find unites each window's
+ * pairs behind it (DESIGN.md §4.9).  Every entry returns with its result complete. */
+HG_API int hg_cluster_dev(hg_ctx *ctx, const int16_t *d_hv, const int32_t *d_norm2, uint32_t n, uint32_t hv_d,
+                          uint32_t ksize, float ani_th, int path, uint32_t *d_rep, uint32_t *n_clusters /* host, may be NULL */);
+/* The same from the rows as the sketch file holds them (as hg_dist_packed: packed bytes + hv_quant_bits + norms,
+ * unpacked on the device); rep in host memory. */
+HG_API int hg_cluster_packed(hg_ctx *ctx, const uint8_t *packed, uint64_t stride, const uint8_t *quant_bits,
+                             const int32_t *norm2, uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th, int path,
+                             uint32_t *rep, uint32_t *n_clusters /* may be NULL */);
+/* hg_cluster_packed over the GPUs of the group: the upper triangle cut by query column into one range per GPU of about
+ * equal pairs (as many GPUs as give each at least 2^23 pairs); each GPU receives the packed rows up to the end of its
+ * range over its own PCIe link and builds a forest of its pairs; the forests are united on GPU 0.  Same arguments,
+ * result identical to hg_cluster_packed.  One GPU in use: hg_cluster_packed on member 0.  Members that share a device
+ * ordinal run one after another.  hg_cluster_stats on hg_group_ctx(g, m) reports member m's run. */
+HG_API int hg_group_cluster_packed(hg_group *g, const uint8_t *packed, uint64_t stride, const uint8_t *quant_bits,
+                                   const int32_t *norm2, uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th, int path,
+                                   uint32_t *rep, uint32_t *n_clusters /* may be NULL */);
+/* Unites the edges (i, j of each record) into an existing forest d_rep (every rep[x] <= x: iota, or a cluster result),
+ * then flattens it, so that rep[x] is the smallest index of x's component; device pointers.  An index >= n or a
+ * rep[x] > x: HG_E_INVALID before anything is written.  The merge step for a host that runs one process per GPU. */
+HG_API int hg_cluster_union_dev(hg_ctx *ctx, uint32_t n, uint32_t *d_rep, const hg_hit *d_edges, uint64_t n_edges,
+                                uint32_t *n_clusters /* host, may be NULL */);
+/* Measurement hook of the last cluster run: counts = {windows, linked pairs, largest window's pairs, edge capacity};
+ * ms = device time of {preparing the rows, the dist windows, the hooks, flatten + count} (-1 where not run or profiling
+ * is off, see hg_set_profiling). */
+HG_API int hg_cluster_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
+
 /* Which path the last hg_dist / hg_dist_dev took (1 SIMT, 2 two-limb tensor, 3 single-plane tensor) and why. */
 HG_API int hg_dist_last_path(hg_ctx *ctx);
 HG_API const char *hg_dist_last_reason(hg_ctx *ctx);

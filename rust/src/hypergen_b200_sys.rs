@@ -40,6 +40,19 @@ extern "C" {
     // the per-block top-k lists (device memory, block m starting at global ref i0[m]) merged into one
     pub fn hg_search_merge_dev(ctx: *mut hg_ctx, n_lists: u32, d_in: *const hg_hit, d_in_found: *const u32, i0: *const u32,
         n_qry: u32, top_k: u32, d_out: *mut hg_hit, d_n_found: *mut u32, d_ani_milli: *mut u32) -> c_int;
+    // single-linkage ANI clusters of one sketch set: rep[i] = the smallest index of i's cluster
+    pub fn hg_cluster_dev(ctx: *mut hg_ctx, d_hv: *const i16, d_norm2: *const i32, n: u32, hv_d: u32, ksize: u32, ani_th: f32,
+        path: c_int, d_rep: *mut u32, n_clusters: *mut u32) -> c_int;
+    pub fn hg_cluster_packed(ctx: *mut hg_ctx, packed: *const u8, stride: u64, quant_bits: *const u8, norm2: *const i32, n: u32,
+        hv_d: u32, ksize: u32, ani_th: f32, path: c_int, rep: *mut u32, n_clusters: *mut u32) -> c_int;
+    // the same with one range of query columns per GPU, the forests united on GPU 0; result identical to hg_cluster_packed
+    pub fn hg_group_cluster_packed(g: *mut hg_group, packed: *const u8, stride: u64, quant_bits: *const u8, norm2: *const i32,
+        n: u32, hv_d: u32, ksize: u32, ani_th: f32, path: c_int, rep: *mut u32, n_clusters: *mut u32) -> c_int;
+    // edge records united into a forest with rep[x] <= x (device memory), then flattened
+    pub fn hg_cluster_union_dev(ctx: *mut hg_ctx, n: u32, d_rep: *mut u32, d_edges: *const hg_hit, n_edges: u64,
+        n_clusters: *mut u32) -> c_int;
+    // counts = {windows, linked pairs, largest window's pairs, edge capacity}; ms of its steps (-1: not run / not profiled)
+    pub fn hg_cluster_stats(ctx: *mut hg_ctx, counts: *mut u64, ms: *mut f32) -> c_int;
 }
 
 /// status -> panic with the library's message, the reference's error style (`unwrap()`, Cargo.toml:67-70)
