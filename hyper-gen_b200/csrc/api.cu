@@ -13,7 +13,6 @@
 #include "hg_common.cuh"
 
 uint32_t hg_kmer_tile_positions();
-uint32_t hg_kmer_tiles_per_cta();
 
 // ---------------------------------------------------------------------------------------
 // errors
@@ -228,6 +227,12 @@ static int check_params(const hg_sketch_params *p) {
   return HG_OK;
 }
 
+static int check_offsets(const uint64_t *off, uint32_t n, const char *name) {
+  for (uint32_t g = 0; g < n; g++)
+    if (off[g + 1] < off[g]) { hg_set_error("%s not monotone at %u", name, g); return HG_E_INVALID; }
+  return HG_OK;
+}
+
 struct SketchPlan {
   std::vector<hg_genome_desc> desc;
   uint64_t total_slots = 0;
@@ -235,32 +240,22 @@ struct SketchPlan {
   uint32_t max_slots = 0;
 };
 
-static int make_plan_bl(const uint64_t *begin, const uint64_t *lens, uint32_t n, const hg_sketch_params *p, SketchPlan &pl);
-
-static int make_plan(const uint64_t *seg_off, uint32_t n, const hg_sketch_params *p, SketchPlan &pl) {
-  std::vector<uint64_t> lens(n);
-  for (uint32_t g = 0; g < n; g++) {
-    if (seg_off[g + 1] < seg_off[g]) { hg_set_error("seg_off not monotone at %u", g); return HG_E_INVALID; }
-    lens[g] = seg_off[g + 1] - seg_off[g];
-  }
-  return make_plan_bl(seg_off, lens.data(), n, p, pl);
-}
-
-// genome g = bytes [begin[g], begin[g] + lens[g]) of the sequence buffer
-static int make_plan_bl(const uint64_t *begin, const uint64_t *lens, uint32_t n, const hg_sketch_params *p, SketchPlan &pl) {
+// genome g = bytes [off[g], off[g + 1]) of a buffer whose byte off[0] sits at byte `base` of the device sequence
+// buffer; off is monotone
+static int make_plan(const uint64_t *off, uint32_t n, uint64_t base, const hg_sketch_params *p, SketchPlan &pl) {
   const uint32_t tile = hg_kmer_tile_positions();
   pl.desc.resize(n + 1);  // + sentinel
   pl.max_slots = 0;
   uint64_t slots_total = 0, tiles_total = 0;
   for (uint32_t g = 0; g < n; g++) {
-    const uint64_t len = lens[g];
+    const uint64_t len = off[g + 1] - off[g];
     const uint64_t n_kmers = len >= p->ksize ? len - p->ksize + 1 : 0;
     // open-addressing table at <= 50 % load for the expected FracMinHash sample size
     uint64_t want = 2 * (len / p->scaled + 1) + 32, slots = 64;
     while (slots < want) slots <<= 1;
     if (slots > (1ull << 31)) { hg_set_error("genome %u too large for one table", g); return HG_E_UNSUPPORTED; }
     hg_genome_desc &d = pl.desc[g];
-    d.seq_begin = begin[g];
+    d.seq_begin = off[g] - off[0] + base;
     d.seq_len = len;
     d.table_begin = slots_total;
     d.table_mask = (uint32_t)(slots - 1);
@@ -297,8 +292,8 @@ static int run_hash_stage(hg_ctx *c, const uint8_t *d_seq, const SketchPlan &pl,
   HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * n, c->stream));
   HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
   HG_PROF(c, 1);
-  if ((rc = hg_launch_kmer_hash(c, d_seq, (const hg_genome_desc *)d_desc, n, pl.n_tiles, p, (uint64_t *)d_tables,
-                                (uint32_t *)d_counts)))
+  if ((rc = hg_launch_kmer_hash(c, d_seq, (const hg_genome_desc *)d_desc, n, pl.n_tiles, p, nullptr,
+                                (uint64_t *)d_tables, (uint32_t *)d_counts)))
     return rc;
   HG_PROF(c, 2);
   *d_desc_out = (hg_genome_desc *)d_desc;
@@ -323,7 +318,7 @@ extern "C" int hg_sketch_batch_dev(hg_ctx *c, const uint8_t *d_seq, const uint64
   if (n == 0) return HG_OK;
   HG_CUDA(cudaSetDevice(c->device));
   SketchPlan pl;
-  if ((rc = make_plan(seg_off, n, p, pl))) return rc;
+  if ((rc = check_offsets(seg_off, n, "seg_off")) || (rc = make_plan(seg_off, n, seg_off[0], p, pl))) return rc;
   hg_genome_desc *d_desc; uint64_t *d_tables; uint32_t *d_counts;
   if ((rc = run_hash_stage(c, d_seq, pl, n, p, &d_desc, &d_tables, &d_counts))) return rc;
   rc = hg_launch_encode(c, d_desc, n, d_tables, d_counts, p->hv_d, d_hv, d_packed, d_quant_bits, d_norm2, d_n_hashes);
@@ -361,6 +356,40 @@ extern "C" int hg_encode_sets_dev(hg_ctx *c, const uint64_t *d_hashes, const uin
   return rc;
 }
 
+// Device staging of the sketches of a host entry: hv and packed in their own slots, norm2 | n_hashes | quant_bits in
+// HG_S_SMALL.  hv and packed exist only when asked for.
+struct SketchOut {
+  int16_t *hv = nullptr;
+  uint8_t *packed = nullptr, *bits = nullptr;
+  int32_t *norm2 = nullptr;
+  uint32_t *n_hashes = nullptr;
+};
+
+static int sketch_out_alloc(hg_ctx *c, uint32_t n, uint32_t hv_d, bool hv, bool packed, SketchOut &o) {
+  void *d_hv = nullptr, *d_packed = nullptr, *d_small;
+  int rc;
+  if (hv && (rc = hg_scratch(c, HG_S_HV, (size_t)n * hv_d * 2, &d_hv))) return rc;
+  if (packed && (rc = hg_scratch(c, HG_S_PACKED, (size_t)n * hv_d * 2, &d_packed))) return rc;
+  if ((rc = hg_scratch(c, HG_S_SMALL, (size_t)n * 12, &d_small))) return rc;
+  o.hv = (int16_t *)d_hv;
+  o.packed = (uint8_t *)d_packed;
+  o.norm2 = (int32_t *)d_small;
+  o.n_hashes = (uint32_t *)d_small + n;
+  o.bits = (uint8_t *)d_small + (size_t)n * 8;
+  return HG_OK;
+}
+
+// D2H of every output the caller passed a buffer for, then the batch's status (synchronises)
+static int sketch_out_fetch(hg_ctx *c, const SketchOut &o, uint32_t n, uint32_t hv_d, int16_t *hv, uint8_t *packed,
+                            uint8_t *quant_bits, int32_t *norm2, uint32_t *n_hashes) {
+  if (hv) HG_CUDA(cudaMemcpyAsync(hv, o.hv, (size_t)n * hv_d * 2, cudaMemcpyDeviceToHost, c->stream));
+  if (packed) HG_CUDA(cudaMemcpyAsync(packed, o.packed, (size_t)n * hv_d * 2, cudaMemcpyDeviceToHost, c->stream));
+  if (quant_bits) HG_CUDA(cudaMemcpyAsync(quant_bits, o.bits, n, cudaMemcpyDeviceToHost, c->stream));
+  if (norm2) HG_CUDA(cudaMemcpyAsync(norm2, o.norm2, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  if (n_hashes) HG_CUDA(cudaMemcpyAsync(n_hashes, o.n_hashes, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  return hg_sketch_status(c);
+}
+
 extern "C" int hg_encode_sets(hg_ctx *c, const uint64_t *hashes, const uint64_t *hash_off, uint32_t n, uint32_t hv_d,
                               int16_t *hv, uint8_t *packed, uint8_t *quant_bits, int32_t *norm2) {
   if (!c || !hash_off) { hg_set_error("hg_encode_sets: NULL argument"); return HG_E_INVALID; }
@@ -370,24 +399,16 @@ extern "C" int hg_encode_sets(hg_ctx *c, const uint64_t *hashes, const uint64_t 
   if (total && !hashes) { hg_set_error("hg_encode_sets: hashes is NULL"); return HG_E_INVALID; }
   HG_CUDA(cudaSetDevice(c->device));
   int rc;
-  void *d_hashes, *d_hv = nullptr, *d_packed = nullptr, *d_small;
+  void *d_hashes;
+  SketchOut o;
   if ((rc = hg_scratch(c, HG_S_TABLES, total * 8 + 64, &d_hashes))) return rc;
-  if (hv && (rc = hg_scratch(c, HG_S_HV, (size_t)n * hv_d * 2, &d_hv))) return rc;
-  if (packed && (rc = hg_scratch(c, HG_S_PACKED, (size_t)n * hv_d * 2, &d_packed))) return rc;
-  if ((rc = hg_scratch(c, HG_S_SMALL, (size_t)n * 12, &d_small))) return rc;
-  uint8_t *d_bits = (uint8_t *)d_small + (size_t)n * 8;
-  int32_t *d_norm = (int32_t *)d_small;
+  if ((rc = sketch_out_alloc(c, n, hv_d, hv != nullptr, packed != nullptr, o))) return rc;
   HG_CUDA(cudaMemcpyAsync(d_hashes, hashes + hash_off[0], total * 8, cudaMemcpyHostToDevice, c->stream));
   std::vector<uint64_t> rel(n + 1);
   for (uint32_t g = 0; g <= n; g++) rel[g] = hash_off[g] - hash_off[0];
-  if ((rc = hg_encode_sets_dev(c, (const uint64_t *)d_hashes, rel.data(), n, hv_d, (int16_t *)d_hv, (uint8_t *)d_packed,
-                               d_bits, d_norm)))
+  if ((rc = hg_encode_sets_dev(c, (const uint64_t *)d_hashes, rel.data(), n, hv_d, o.hv, o.packed, o.bits, o.norm2)))
     return rc;
-  if (hv) HG_CUDA(cudaMemcpyAsync(hv, d_hv, (size_t)n * hv_d * 2, cudaMemcpyDeviceToHost, c->stream));
-  if (packed) HG_CUDA(cudaMemcpyAsync(packed, d_packed, (size_t)n * hv_d * 2, cudaMemcpyDeviceToHost, c->stream));
-  if (quant_bits) HG_CUDA(cudaMemcpyAsync(quant_bits, d_bits, n, cudaMemcpyDeviceToHost, c->stream));
-  if (norm2) HG_CUDA(cudaMemcpyAsync(norm2, d_norm, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  return hg_sketch_status(c);
+  return sketch_out_fetch(c, o, n, hv_d, hv, packed, quant_bits, norm2, nullptr);
 }
 
 extern "C" int hg_sketch_status(hg_ctx *c) {
@@ -397,14 +418,231 @@ extern "C" int hg_sketch_status(hg_ctx *c) {
   return status_to_rc(c->h_status);
 }
 
-// Host-pointer entry: the batch is cut into ~64 MB chunks on genome boundaries and pipelined —
-// chunk c+1 crosses PCIe on a copy stream (double-buffered device staging) while chunk c is hashed
-// and encoded on the compute stream; the sketches come back in one D2H at the end.  (Measured on
-// B200: 32-64 MB chunks sustain the full 55 GB/s PCIe rate; 256 MB chunks drop it to 43 GB/s.)
+// ---------------------------------------------------------------------------------------
+// FASTA file bytes in (fastx_reader::read_merge_seq on the GPU)
+// ---------------------------------------------------------------------------------------
+uint32_t hg_fasta_block_bytes();
+int hg_launch_fasta_merge(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_file_off, const uint64_t *d_blk_off,
+                          uint32_t n_files, uint32_t max_blocks, void *d_sums, uint8_t *d_carry, uint64_t *d_out_off,
+                          uint8_t *d_merged, uint64_t *d_merged_len);
+
+// The merge of files that lie back to back in a device buffer, as in the host buffer (one copy; the kernels take any
+// byte phase): per file (+ end) its offset there and its block prefix.  The merged bytes of a file land at its offset.
+struct MergePlan {
+  std::vector<uint64_t> off, blk;
+  uint64_t max_blocks = 0;
+};
+
+// file_off is monotone
+static int make_merge_plan(const uint64_t *file_off, uint32_t n, MergePlan &mp) {
+  const uint32_t B = hg_fasta_block_bytes();
+  mp.off.assign(n + 1, 0);
+  mp.blk.assign(n + 1, 0);
+  mp.max_blocks = 0;
+  for (uint32_t f = 0; f < n; f++) {
+    const uint64_t len = file_off[f + 1] - file_off[f];
+    mp.off[f + 1] = mp.off[f] + len;
+    const uint64_t nb = (len + B - 1) / B;
+    mp.blk[f + 1] = mp.blk[f] + nb;
+    mp.max_blocks = std::max(mp.max_blocks, nb);
+  }
+  if (mp.max_blocks > 0x7fffffffull) { hg_set_error("file too large"); return HG_E_UNSUPPORTED; }
+  return HG_OK;
+}
+
+// Byte offsets of a merge's device metadata for up to n files and nblk blocks, in one buffer: file offsets (n+1) at 0 |
+// block prefix (n+1) | out_off (nblk) | sums (16 B a block) | carry (1 B a block), then the merged lengths.  The host
+// writes the first two arrays, bytes [0, out).
+struct MergeLayout { size_t blk, out, sums, carry, len; };
+
+static MergeLayout merge_layout(uint32_t n, uint64_t nblk) {
+  MergeLayout L;
+  L.blk = (size_t)(n + 1) * 8;
+  L.out = 2 * L.blk;
+  L.sums = L.out + nblk * 8;
+  L.carry = L.sums + nblk * 16;
+  L.len = (L.carry + nblk + 256 + 15) & ~(size_t)15;
+  return L;
+}
+
+// mp's file offsets and block prefix through pinned h_meta to the head of d_meta, on the compute stream
+static int put_merge_meta(hg_ctx *c, const MergePlan &mp, const MergeLayout &L, uint8_t *h_meta, uint8_t *d_meta) {
+  memcpy(h_meta, mp.off.data(), mp.off.size() * 8);
+  memcpy(h_meta + L.blk, mp.blk.data(), mp.blk.size() * 8);
+  HG_CUDA(cudaMemcpyAsync(d_meta, h_meta, L.out, cudaMemcpyHostToDevice, c->stream));
+  return HG_OK;
+}
+
+static int launch_merge(hg_ctx *c, const uint8_t *d_raw, const MergePlan &mp, const MergeLayout &L, uint8_t *d_meta,
+                        uint8_t *d_merged, uint64_t *d_merged_len) {
+  return hg_launch_fasta_merge(c, d_raw, (const uint64_t *)d_meta, (const uint64_t *)(d_meta + L.blk),
+                               (uint32_t)(mp.off.size() - 1), (uint32_t)mp.max_blocks, d_meta + L.sums,
+                               d_meta + L.carry, (uint64_t *)(d_meta + L.out), d_merged, d_merged_len);
+}
+
+// H2D of the raw files (one copy on the compute stream), merge on the device, lengths back, merged bytes back.
+extern "C" int hg_fasta_merge(hg_ctx *c, const uint8_t *raw, const uint64_t *file_off, uint32_t n, uint8_t *merged,
+                              uint64_t cap, uint64_t *merged_off) {
+  if (!c || !file_off || !merged_off) { hg_set_error("hg_fasta_merge: NULL argument"); return HG_E_INVALID; }
+  merged_off[0] = 0;
+  if (n == 0) return HG_OK;
+  if (!raw && file_off[n] > file_off[0]) { hg_set_error("hg_fasta_merge: raw is NULL"); return HG_E_INVALID; }
+  HG_CUDA(cudaSetDevice(c->device));
+  MergePlan mp;
+  int rc;
+  if ((rc = check_offsets(file_off, n, "file_off")) || (rc = make_merge_plan(file_off, n, mp))) return rc;
+  const uint64_t total = mp.off[n];
+  const MergeLayout L = merge_layout(n, mp.blk[n]);
+  void *d_raw, *d_merged, *d_meta, *h_meta;
+  if ((rc = hg_scratch(c, HG_S_PACKED, total + 64, &d_raw))) return rc;      // raw bytes (free until the sketches are packed)
+  if ((rc = hg_scratch(c, HG_S_SEQ, total + 64, &d_merged))) return rc;      // merged sequences
+  if ((rc = hg_scratch(c, HG_S_MISC, L.len + (size_t)n * 8, &d_meta))) return rc;
+  if ((rc = hg_pinned(c, 1, L.out + (size_t)n * 8, &h_meta))) return rc;
+  uint64_t *h_len = (uint64_t *)((uint8_t *)h_meta + L.out), *d_len = (uint64_t *)((uint8_t *)d_meta + L.len);
+  if ((rc = put_merge_meta(c, mp, L, (uint8_t *)h_meta, (uint8_t *)d_meta))) return rc;
+  if (total) HG_CUDA(cudaMemcpyAsync(d_raw, raw + file_off[0], total, cudaMemcpyHostToDevice, c->stream));
+  if ((rc = launch_merge(c, (const uint8_t *)d_raw, mp, L, (uint8_t *)d_meta, (uint8_t *)d_merged, d_len))) return rc;
+  HG_CUDA(cudaMemcpyAsync(h_len, d_len, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  for (uint32_t f = 0; f < n; f++) merged_off[f + 1] = merged_off[f] + h_len[f];
+  if (merged_off[n] > cap || (!merged && merged_off[n])) { hg_set_error("hg_fasta_merge: need room for %llu bytes", (unsigned long long)merged_off[n]); return HG_E_CAPACITY; }
+  for (uint32_t f = 0; f < n; f++)
+    if (h_len[f])
+      HG_CUDA(cudaMemcpyAsync(merged + merged_off[f], (uint8_t *)d_merged + mp.off[f], h_len[f], cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  return HG_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// host-pointer sketch entries: sequences or raw FASTA files in, sketches out
+// ---------------------------------------------------------------------------------------
+enum class Input { SEQUENCES, FASTA_FILES };
+
+// genomes [g0, g1), whose host bytes [lo, hi) are copied to byte `shift` of a staging slot
+struct Chunk {
+  uint32_t g0, g1;
+  uint64_t lo, hi, shift;
+  SketchPlan pl;
+  MergePlan merge;  // FASTA files only
+};
+
+// The batch cut on genome boundaries into chunks of at most `limit` bytes (or one genome).  Sequences keep the
+// caller's alignment modulo 16; FASTA files go back to back from the start of the slot, and their tiles and tables
+// are planned from the raw sizes, an upper bound of the merged lengths.
+static int plan_chunks(const uint8_t *host, const uint64_t *off, uint32_t n, const hg_sketch_params *p, Input in,
+                       uint64_t limit, std::vector<Chunk> &chunks) {
+  const bool fasta = in == Input::FASTA_FILES;
+  int rc = check_offsets(off, n, fasta ? "file_off" : "seg_off");
+  if (rc) return rc;
+  for (uint32_t g = 0; g < n;) {
+    Chunk ch;
+    ch.g0 = g;
+    ch.lo = off[g];
+    do { ++g; } while (g < n && off[g + 1] - ch.lo <= limit);
+    ch.g1 = g;
+    ch.hi = off[g];
+    ch.shift = fasta ? 0 : (uint64_t)((uintptr_t)(host + ch.lo) & 15);
+    if (fasta && (rc = make_merge_plan(off + ch.g0, ch.g1 - ch.g0, ch.merge))) return rc;
+    if ((rc = make_plan(off + ch.g0, ch.g1 - ch.g0, ch.shift, p, ch.pl))) return rc;
+    chunks.push_back(std::move(ch));
+  }
+  return HG_OK;
+}
+
+// The batch is cut into ~64 MB chunks and pipelined: chunk c+1 crosses PCIe on a copy stream (double-buffered device
+// staging) while chunk c is (merged,) hashed and encoded on the compute stream; the sketches come back in one D2H at
+// the end.  (Measured on B200: 32-64 MB chunks sustain the full 55 GB/s PCIe rate; 256 MB chunks drop it to 43 GB/s.)
 static uint64_t hg_chunk_bytes() {
   const char *e = getenv("HG_CHUNK_MB");
   const uint64_t mb = e ? strtoull(e, nullptr, 10) : 64;
   return (mb ? mb : 64) << 20;
+}
+
+// Nothing comes back to the host between the stages of a FASTA chunk: the hash kernel reads the true merged lengths
+// the merge left in HBM.
+static int sketch_pipeline(hg_ctx *c, const uint8_t *host, const uint64_t *off, uint32_t n, const hg_sketch_params *p,
+                           Input in, int16_t *hv, uint8_t *packed, uint8_t *quant_bits, int32_t *norm2,
+                           uint32_t *n_hashes) {
+  HG_CUDA(cudaSetDevice(c->device));
+  const uint32_t D = p->hv_d;
+  const bool fasta = in == Input::FASTA_FILES;
+  std::vector<Chunk> chunks;
+  int rc = plan_chunks(host, off, n, p, in, hg_chunk_bytes(), chunks);
+  if (rc) return rc;
+  uint64_t max_bytes = 0, max_slots = 0, max_tiles = 0, max_blk = 0;
+  uint32_t max_m = 0;
+  for (const Chunk &ch : chunks) {
+    max_bytes = std::max(max_bytes, ch.hi - ch.lo);
+    max_slots = std::max<uint64_t>(max_slots, ch.pl.total_slots);
+    max_tiles = std::max<uint64_t>(max_tiles, ch.pl.n_tiles);
+    max_m = std::max(max_m, ch.g1 - ch.g0);
+    if (fasta) max_blk = std::max(max_blk, ch.merge.blk.back());
+  }
+  const uint64_t slot_bytes = (max_bytes + 64 + 255) & ~255ull;
+  const size_t n_desc = (size_t)n + chunks.size();  // one sentinel per chunk
+  const MergeLayout L = merge_layout(max_m, max_blk);  // one region for every chunk's merge
+
+  // size every scratch buffer before anything is enqueued (growing one synchronises); FASTA files are staged in
+  // HG_S_REF_LIMBS and merged into HG_S_SEQ
+  void *d_stage, *d_merged = nullptr, *d_meta = nullptr, *d_desc, *d_tables, *d_counts, *d_map, *h_desc, *h_meta = nullptr;
+  SketchOut o;
+  if ((rc = hg_scratch(c, fasta ? HG_S_REF_LIMBS : HG_S_SEQ, 2 * slot_bytes, &d_stage))) return rc;
+  if (fasta && (rc = hg_scratch(c, HG_S_SEQ, slot_bytes, &d_merged))) return rc;
+  if (fasta && (rc = hg_scratch(c, HG_S_QRY_LIMBS, L.len + (size_t)n * 8, &d_meta))) return rc;
+  if ((rc = hg_scratch(c, HG_S_DESC, sizeof(hg_genome_desc) * n_desc, &d_desc))) return rc;
+  if ((rc = hg_scratch(c, HG_S_TABLES, max_slots * 8, &d_tables))) return rc;
+  if ((rc = hg_scratch(c, HG_S_COUNTS, sizeof(uint32_t) * n, &d_counts))) return rc;
+  if ((rc = sketch_out_alloc(c, n, D, hv != nullptr, true, o))) return rc;
+  if ((rc = hg_scratch(c, HG_S_MISC, hg_kmer_map_bytes((uint32_t)max_tiles), &d_map))) return rc;
+  if ((rc = hg_pinned(c, 0, sizeof(hg_genome_desc) * n_desc, &h_desc))) return rc;
+  if (fasta && (rc = hg_pinned(c, 1, L.out * chunks.size(), &h_meta))) return rc;
+  uint64_t *d_len = fasta ? (uint64_t *)((uint8_t *)d_meta + L.len) : nullptr;  // true merged lengths, all files
+  if ((rc = ensure_copy_stream(c))) return rc;
+  c->ev_used = 0;
+  HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
+  HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * n, c->stream));
+  // the copy stream may not overwrite a staging slot before everything already queued is done with it
+  HG_CUDA(cudaEventRecord(c->ev_done[0], c->stream));
+  HG_CUDA(cudaEventRecord(c->ev_done[1], c->stream));
+
+  size_t desc_pos = 0;
+  for (size_t ci = 0; ci < chunks.size(); ci++) {
+    const Chunk &ch = chunks[ci];
+    const int slot = (int)(ci & 1);
+    const uint32_t m = ch.g1 - ch.g0;
+    uint8_t *d_in = (uint8_t *)d_stage + slot * slot_bytes;
+    // ---- copy stream: the chunk in one copy (per-genome copies cost ~6 us each of PCIe idle time), once the slot's
+    // previous tenant has been consumed ----
+    HG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_done[slot], 0));
+    if (ch.hi > ch.lo)
+      HG_CUDA(cudaMemcpyAsync(d_in + ch.shift, host + ch.lo, ch.hi - ch.lo, cudaMemcpyHostToDevice, c->copy_stream));
+    HG_CUDA(cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+    // ---- compute stream: merge metadata, descriptors, table clear, merge, hash, encode ----
+    if (fasta && (rc = put_merge_meta(c, ch.merge, L, (uint8_t *)h_meta + ci * L.out, (uint8_t *)d_meta))) return rc;
+    hg_genome_desc *hd = (hg_genome_desc *)h_desc + desc_pos, *dd = (hg_genome_desc *)d_desc + desc_pos;
+    memcpy(hd, ch.pl.desc.data(), sizeof(hg_genome_desc) * (m + 1));
+    desc_pos += m + 1;
+    HG_CUDA(cudaMemcpyAsync(dd, hd, sizeof(hg_genome_desc) * (m + 1), cudaMemcpyHostToDevice, c->stream));
+    HG_CUDA(cudaMemsetAsync(d_tables, 0xFF, ch.pl.total_slots * 8, c->stream));
+    HG_CUDA(cudaStreamWaitEvent(c->stream, c->ev_copied[slot], 0));
+    const uint8_t *d_seq = d_in;
+    const uint64_t *d_true_len = nullptr;
+    if (fasta) {
+      if ((rc = launch_merge(c, d_in, ch.merge, L, (uint8_t *)d_meta, (uint8_t *)d_merged, d_len + ch.g0))) return rc;
+      HG_CUDA(cudaEventRecord(c->ev_done[slot], c->stream));  // the raw slot may be overwritten now
+      d_seq = (const uint8_t *)d_merged;
+      d_true_len = d_len + ch.g0;
+    }
+    if ((rc = hg_launch_kmer_hash(c, d_seq, dd, m, ch.pl.n_tiles, p, d_true_len, (uint64_t *)d_tables,
+                                  (uint32_t *)d_counts + ch.g0)))
+      return rc;
+    if (!fasta) HG_CUDA(cudaEventRecord(c->ev_done[slot], c->stream));
+    if ((rc = hg_launch_encode(c, dd, m, (const uint64_t *)d_tables, (const uint32_t *)d_counts + ch.g0, D,
+                               o.hv ? o.hv + (size_t)ch.g0 * D : nullptr, o.packed + (size_t)ch.g0 * 2 * D,
+                               o.bits + ch.g0, o.norm2 + ch.g0, o.n_hashes + ch.g0)))
+      return rc;
+  }
+  return sketch_out_fetch(c, o, n, D, hv, packed, quant_bits, norm2, n_hashes);
 }
 
 extern "C" int hg_sketch_batch(hg_ctx *c, const uint8_t *seq, const uint64_t *seg_off, uint32_t n,
@@ -415,105 +653,18 @@ extern "C" int hg_sketch_batch(hg_ctx *c, const uint8_t *seq, const uint64_t *se
   if (rc) return rc;
   if (n == 0) return HG_OK;
   if (!seq && seg_off[n] > seg_off[0]) { hg_set_error("hg_sketch_batch: seq is NULL"); return HG_E_INVALID; }
-  HG_CUDA(cudaSetDevice(c->device));
-  const uint32_t D = p->hv_d;
+  return sketch_pipeline(c, seq, seg_off, n, p, Input::SEQUENCES, hv, packed, quant_bits, norm2, n_hashes);
+}
 
-  const uint64_t chunk_bytes = hg_chunk_bytes();
-  struct Chunk { uint32_t g0, g1; uint64_t lo, hi, shift; SketchPlan pl; };
-  std::vector<Chunk> chunks;
-  for (uint32_t g = 0; g < n;) {
-    Chunk ch;
-    ch.g0 = g;
-    ch.lo = seg_off[g];
-    do { ++g; } while (g < n && seg_off[g + 1] - ch.lo <= chunk_bytes);
-    ch.g1 = g;
-    ch.hi = seg_off[g];
-    ch.shift = (uint64_t)((uintptr_t)(seq + ch.lo) & 15);  // keep the caller's alignment modulo 16
-    std::vector<uint64_t> rel(ch.g1 - ch.g0 + 1);
-    for (uint32_t t = 0; t <= ch.g1 - ch.g0; t++) {
-      if (seg_off[ch.g0 + t] < ch.lo) { hg_set_error("seg_off not monotone"); return HG_E_INVALID; }
-      rel[t] = seg_off[ch.g0 + t] - ch.lo + ch.shift;
-    }
-    if ((rc = make_plan(rel.data(), ch.g1 - ch.g0, p, ch.pl))) return rc;
-    chunks.push_back(std::move(ch));
-  }
-  uint64_t max_bytes = 0, max_slots = 0, max_tiles = 0;
-  for (const Chunk &ch : chunks) {
-    max_bytes = std::max(max_bytes, ch.hi - ch.lo);
-    max_slots = std::max<uint64_t>(max_slots, ch.pl.total_slots);
-    max_tiles = std::max<uint64_t>(max_tiles, ch.pl.n_tiles);
-  }
-  const uint64_t slot_bytes = (max_bytes + 64 + 255) & ~255ull;
-  const size_t n_desc = (size_t)n + chunks.size();  // one sentinel per chunk
-
-  // size every scratch buffer before anything is enqueued (growing one synchronises)
-  void *d_seq, *d_desc, *d_tables, *d_counts, *d_hv = nullptr, *d_packed, *d_small, *d_map, *h_desc;
-  if ((rc = hg_scratch(c, HG_S_SEQ, 2 * slot_bytes, &d_seq))) return rc;
-  if ((rc = hg_scratch(c, HG_S_DESC, sizeof(hg_genome_desc) * n_desc, &d_desc))) return rc;
-  if ((rc = hg_scratch(c, HG_S_TABLES, max_slots * 8, &d_tables))) return rc;
-  if ((rc = hg_scratch(c, HG_S_COUNTS, sizeof(uint32_t) * n, &d_counts))) return rc;
-  if (hv && (rc = hg_scratch(c, HG_S_HV, (size_t)n * D * 2, &d_hv))) return rc;
-  if ((rc = hg_scratch(c, HG_S_PACKED, (size_t)n * D * 2, &d_packed))) return rc;
-  if ((rc = hg_scratch(c, HG_S_SMALL, (size_t)n * 12, &d_small))) return rc;
-  if ((rc = hg_scratch(c, HG_S_MISC, (max_tiles / hg_kmer_tiles_per_cta() + 2) * 4 + 256, &d_map))) return rc;
-  if ((rc = hg_pinned(c, 0, sizeof(hg_genome_desc) * n_desc, &h_desc))) return rc;
-  uint8_t *d_bits = (uint8_t *)d_small + (size_t)n * 8;
-  int32_t *d_norm = (int32_t *)d_small;
-  uint32_t *d_nh = (uint32_t *)d_small + n;
-  if ((rc = ensure_copy_stream(c))) return rc;
-  c->ev_used = 0;
-  HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
-  HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * n, c->stream));
-  // the copy stream may not overwrite a staging slot before everything already queued is done with it
-  HG_CUDA(cudaEventRecord(c->ev_done[0], c->stream));
-  HG_CUDA(cudaEventRecord(c->ev_done[1], c->stream));
-
-  const bool dbg = getenv("HG_DEBUG_PIPE") != nullptr;
-  cudaEvent_t t0 = nullptr, t1 = nullptr, t2 = nullptr;
-  if (dbg) {
-    cudaEventCreate(&t0); cudaEventCreate(&t1); cudaEventCreate(&t2);
-    cudaEventRecord(t0, c->stream);
-  }
-  size_t desc_pos = 0;
-  for (size_t ci = 0; ci < chunks.size(); ci++) {
-    const Chunk &ch = chunks[ci];
-    const int slot = (int)(ci & 1);
-    const uint32_t m = ch.g1 - ch.g0;
-    uint8_t *d_slot = (uint8_t *)d_seq + slot * slot_bytes;
-    // ---- copy stream: H2D of this chunk once the slot's previous tenant has been consumed ----
-    HG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_done[slot], 0));
-    if (ch.hi > ch.lo)
-      HG_CUDA(cudaMemcpyAsync(d_slot + ch.shift, seq + ch.lo, ch.hi - ch.lo, cudaMemcpyHostToDevice, c->copy_stream));
-    HG_CUDA(cudaEventRecord(c->ev_copied[slot], c->copy_stream));
-    // ---- compute stream: descriptors, table clear, hash, encode ----
-    hg_genome_desc *hd = (hg_genome_desc *)h_desc + desc_pos, *dd = (hg_genome_desc *)d_desc + desc_pos;
-    memcpy(hd, ch.pl.desc.data(), sizeof(hg_genome_desc) * (m + 1));
-    desc_pos += m + 1;
-    HG_CUDA(cudaMemcpyAsync(dd, hd, sizeof(hg_genome_desc) * (m + 1), cudaMemcpyHostToDevice, c->stream));
-    HG_CUDA(cudaMemsetAsync(d_tables, 0xFF, ch.pl.total_slots * 8, c->stream));
-    HG_CUDA(cudaStreamWaitEvent(c->stream, c->ev_copied[slot], 0));
-    if ((rc = hg_launch_kmer_hash(c, d_slot, dd, m, ch.pl.n_tiles, p, (uint64_t *)d_tables, (uint32_t *)d_counts + ch.g0)))
-      return rc;
-    HG_CUDA(cudaEventRecord(c->ev_done[slot], c->stream));
-    if ((rc = hg_launch_encode(c, dd, m, (const uint64_t *)d_tables, (const uint32_t *)d_counts + ch.g0, D,
-                               d_hv ? (int16_t *)d_hv + (size_t)ch.g0 * D : nullptr,
-                               (uint8_t *)d_packed + (size_t)ch.g0 * 2 * D, d_bits + ch.g0, d_norm + ch.g0, d_nh + ch.g0)))
-      return rc;
-  }
-  if (dbg) { cudaEventRecord(t1, c->copy_stream); cudaEventRecord(t2, c->stream); }
-  if (hv) HG_CUDA(cudaMemcpyAsync(hv, d_hv, (size_t)n * D * 2, cudaMemcpyDeviceToHost, c->stream));
-  if (packed) HG_CUDA(cudaMemcpyAsync(packed, d_packed, (size_t)n * D * 2, cudaMemcpyDeviceToHost, c->stream));
-  if (quant_bits) HG_CUDA(cudaMemcpyAsync(quant_bits, d_bits, n, cudaMemcpyDeviceToHost, c->stream));
-  if (norm2) HG_CUDA(cudaMemcpyAsync(norm2, d_norm, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  if (n_hashes) HG_CUDA(cudaMemcpyAsync(n_hashes, d_nh, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  rc = hg_sketch_status(c);
-  if (dbg) {
-    float a = 0, b = 0;
-    cudaEventElapsedTime(&a, t0, t1); cudaEventElapsedTime(&b, t0, t2);
-    fprintf(stderr, "[hg pipe] chunks=%zu copies done at %.2f ms, compute done at %.2f ms\n", chunks.size(), a, b);
-    cudaEventDestroy(t0); cudaEventDestroy(t1); cudaEventDestroy(t2);
-  }
-  return rc;
+extern "C" int hg_sketch_fasta_batch(hg_ctx *c, const uint8_t *raw, const uint64_t *file_off, uint32_t n,
+                                     const hg_sketch_params *p, int16_t *hv, uint8_t *packed, uint8_t *quant_bits,
+                                     int32_t *norm2, uint32_t *n_hashes) {
+  if (!c || !file_off) { hg_set_error("hg_sketch_fasta_batch: NULL argument"); return HG_E_INVALID; }
+  int rc = check_params(p);
+  if (rc) return rc;
+  if (n == 0) return HG_OK;
+  if (!raw && file_off[n] > file_off[0]) { hg_set_error("hg_sketch_fasta_batch: raw is NULL"); return HG_E_INVALID; }
+  return sketch_pipeline(c, raw, file_off, n, p, Input::FASTA_FILES, hv, packed, quant_bits, norm2, n_hashes);
 }
 
 extern "C" int hg_kmer_hash(hg_ctx *c, const uint8_t *seq, const uint64_t *seg_off, uint32_t n,
@@ -525,18 +676,15 @@ extern "C" int hg_kmer_hash(hg_ctx *c, const uint8_t *seq, const uint64_t *seg_o
   if (n == 0) return HG_OK;
   if (!seq && seg_off[n] > 0) { hg_set_error("hg_kmer_hash: seq is NULL"); return HG_E_INVALID; }
   HG_CUDA(cudaSetDevice(c->device));
-  const uint64_t lo = seg_off[0], hi = seg_off[n];
+  std::vector<Chunk> one;  // the whole batch, staged at once
+  if ((rc = plan_chunks(seq, seg_off, n, p, Input::SEQUENCES, UINT64_MAX, one))) return rc;
+  const Chunk &ch = one[0];
   void *d_seq;
-  if ((rc = hg_scratch(c, HG_S_SEQ, hi - lo + 64, &d_seq))) return rc;
-  const uint64_t shift = (uint64_t)((uintptr_t)(seq + lo) & 15);
-  HG_CUDA(cudaMemcpyAsync((uint8_t *)d_seq + shift, seq + lo, hi - lo, cudaMemcpyHostToDevice, c->stream));
-  std::vector<uint64_t> rel(n + 1);
-  for (uint32_t g = 0; g <= n; g++) rel[g] = seg_off[g] - lo + shift;
-  SketchPlan pl;
-  if ((rc = make_plan(rel.data(), n, p, pl))) return rc;
+  if ((rc = hg_scratch(c, HG_S_SEQ, ch.hi - ch.lo + 64, &d_seq))) return rc;
+  HG_CUDA(cudaMemcpyAsync((uint8_t *)d_seq + ch.shift, seq + ch.lo, ch.hi - ch.lo, cudaMemcpyHostToDevice, c->stream));
   hg_genome_desc *d_desc; uint64_t *d_tables; uint32_t *d_counts;
-  if ((rc = run_hash_stage(c, (const uint8_t *)d_seq, pl, n, p, &d_desc, &d_tables, &d_counts))) return rc;
-  if ((rc = hg_launch_sort_tables(c, d_desc, n, d_tables, pl.max_slots))) return rc;
+  if ((rc = run_hash_stage(c, (const uint8_t *)d_seq, ch.pl, n, p, &d_desc, &d_tables, &d_counts))) return rc;
+  if ((rc = hg_launch_sort_tables(c, d_desc, n, d_tables, ch.pl.max_slots))) return rc;
   std::vector<uint32_t> counts(n);
   HG_CUDA(cudaMemcpyAsync(counts.data(), d_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   if ((rc = hg_sketch_status(c))) return rc;  // synchronises
@@ -545,218 +693,10 @@ extern "C" int hg_kmer_hash(hg_ctx *c, const uint8_t *seq, const uint64_t *seg_o
   if (total > cap || (!hashes && total)) { hg_set_error("hg_kmer_hash: need room for %llu hashes", (unsigned long long)total); return HG_E_CAPACITY; }
   for (uint32_t g = 0; g < n; g++)
     if (counts[g])
-      HG_CUDA(cudaMemcpyAsync(hashes + hash_off[g], d_tables + pl.desc[g].table_begin, (size_t)counts[g] * 8,
+      HG_CUDA(cudaMemcpyAsync(hashes + hash_off[g], d_tables + ch.pl.desc[g].table_begin, (size_t)counts[g] * 8,
                               cudaMemcpyDeviceToHost, c->stream));
   HG_CUDA(cudaStreamSynchronize(c->stream));
   return HG_OK;
-}
-
-// ---------------------------------------------------------------------------------------
-// FASTA file bytes in (fastx_reader::read_merge_seq on the GPU)
-// ---------------------------------------------------------------------------------------
-uint32_t hg_fasta_block_bytes();
-int hg_launch_fasta_merge(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_file_off, const uint64_t *d_blk_off,
-                          uint32_t n_files, uint32_t max_blocks, void *d_sums, uint8_t *d_carry, uint64_t *d_out_off,
-                          uint8_t *d_merged, uint64_t *d_merged_len);
-
-struct FastaStage {
-  std::vector<uint64_t> dev_off;   // device offset of every file (+ end)
-  std::vector<uint64_t> merged_len;
-  uint8_t *d_merged = nullptr;
-};
-
-// H2D of the raw files (one copy, files back to back), merge on the device, lengths back.
-static int fasta_stage(hg_ctx *c, const uint8_t *raw, const uint64_t *file_off, uint32_t n, FastaStage &st) {
-  const uint32_t B = hg_fasta_block_bytes();
-  st.dev_off.assign(n + 1, 0);
-  std::vector<uint64_t> blk_off(n + 1, 0);
-  uint64_t max_blocks = 0;
-  for (uint32_t f = 0; f < n; f++) {
-    if (file_off[f + 1] < file_off[f]) { hg_set_error("file_off not monotone at %u", f); return HG_E_INVALID; }
-    const uint64_t len = file_off[f + 1] - file_off[f];
-    st.dev_off[f + 1] = st.dev_off[f] + len;  // files back to back, as in the host buffer: one copy (the kernels take any byte phase)
-    const uint64_t nb = (len + B - 1) / B;
-    blk_off[f + 1] = blk_off[f] + nb;
-    max_blocks = std::max(max_blocks, nb);
-  }
-  if (max_blocks > 0x7fffffffull) { hg_set_error("file too large"); return HG_E_UNSUPPORTED; }
-  const uint64_t total = st.dev_off[n], nblk = blk_off[n];
-  void *d_raw, *d_merged, *d_meta, *d_sums, *h_meta;
-  int rc;
-  // device layout of the small arrays: file_off (n+1) | blk_off (n+1) | merged_len (n) | out_off (nblk) | carry (nblk bytes)
-  const size_t meta_words = (size_t)(3 * n + 2) + nblk;
-  if ((rc = hg_scratch(c, HG_S_PACKED, total + 64, &d_raw))) return rc;      // raw bytes (free until the sketches are packed)
-  if ((rc = hg_scratch(c, HG_S_SEQ, total + 64, &d_merged))) return rc;      // merged sequences
-  if ((rc = hg_scratch(c, HG_S_MISC, meta_words * 8 + nblk + 256, &d_meta))) return rc;
-  if ((rc = hg_scratch(c, HG_S_TABLES, nblk * 16 + 256, &d_sums))) return rc;
-  if ((rc = hg_pinned(c, 1, (size_t)(2 * n + 2) * 8 + (size_t)n * 8, &h_meta))) return rc;
-  uint64_t *h_off = (uint64_t *)h_meta, *h_blk = h_off + (n + 1), *h_len = h_blk + (n + 1);
-  memcpy(h_off, st.dev_off.data(), (n + 1) * 8);
-  memcpy(h_blk, blk_off.data(), (n + 1) * 8);
-  uint64_t *d_off = (uint64_t *)d_meta, *d_blk = d_off + (n + 1), *d_len = d_blk + (n + 1), *d_out = d_len + n;
-  uint8_t *d_carry = (uint8_t *)(d_out + nblk);
-  HG_CUDA(cudaMemcpyAsync(d_off, h_off, (size_t)(2 * n + 2) * 8, cudaMemcpyHostToDevice, c->stream));
-  if (total) HG_CUDA(cudaMemcpyAsync(d_raw, raw + file_off[0], total, cudaMemcpyHostToDevice, c->stream));
-  if ((rc = hg_launch_fasta_merge(c, (const uint8_t *)d_raw, d_off, d_blk, n, (uint32_t)max_blocks, d_sums, d_carry, d_out,
-                                  (uint8_t *)d_merged, d_len)))
-    return rc;
-  HG_CUDA(cudaMemcpyAsync(h_len, d_len, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
-  HG_CUDA(cudaStreamSynchronize(c->stream));
-  st.merged_len.assign(h_len, h_len + n);
-  st.d_merged = (uint8_t *)d_merged;
-  return HG_OK;
-}
-
-extern "C" int hg_fasta_merge(hg_ctx *c, const uint8_t *raw, const uint64_t *file_off, uint32_t n, uint8_t *merged,
-                              uint64_t cap, uint64_t *merged_off) {
-  if (!c || !file_off || !merged_off) { hg_set_error("hg_fasta_merge: NULL argument"); return HG_E_INVALID; }
-  merged_off[0] = 0;
-  if (n == 0) return HG_OK;
-  if (!raw && file_off[n] > file_off[0]) { hg_set_error("hg_fasta_merge: raw is NULL"); return HG_E_INVALID; }
-  HG_CUDA(cudaSetDevice(c->device));
-  FastaStage st;
-  int rc = fasta_stage(c, raw, file_off, n, st);
-  if (rc) return rc;
-  for (uint32_t f = 0; f < n; f++) merged_off[f + 1] = merged_off[f] + st.merged_len[f];
-  if (merged_off[n] > cap || (!merged && merged_off[n])) { hg_set_error("hg_fasta_merge: need room for %llu bytes", (unsigned long long)merged_off[n]); return HG_E_CAPACITY; }
-  for (uint32_t f = 0; f < n; f++)
-    if (st.merged_len[f])
-      HG_CUDA(cudaMemcpyAsync(merged + merged_off[f], st.d_merged + st.dev_off[f], st.merged_len[f], cudaMemcpyDeviceToHost, c->stream));
-  HG_CUDA(cudaStreamSynchronize(c->stream));
-  return HG_OK;
-}
-
-// Raw FASTA files in, sketches out.  Same ~64 MB chunk pipeline as hg_sketch_batch (copy stream +
-// double-buffered staging), with the merge kernels in front of the hash kernel.  Nothing comes back
-// to the host between the stages: tiles and tables are planned from the raw file sizes (an upper
-// bound of the merged lengths) and the hash kernel reads the true lengths the merge left in HBM.
-extern "C" int hg_sketch_fasta_batch(hg_ctx *c, const uint8_t *raw, const uint64_t *file_off, uint32_t n,
-                                     const hg_sketch_params *p, int16_t *hv, uint8_t *packed, uint8_t *quant_bits,
-                                     int32_t *norm2, uint32_t *n_hashes) {
-  if (!c || !file_off) { hg_set_error("hg_sketch_fasta_batch: NULL argument"); return HG_E_INVALID; }
-  int rc = check_params(p);
-  if (rc) return rc;
-  if (n == 0) return HG_OK;
-  if (!raw && file_off[n] > file_off[0]) { hg_set_error("hg_sketch_fasta_batch: raw is NULL"); return HG_E_INVALID; }
-  HG_CUDA(cudaSetDevice(c->device));
-  const uint32_t D = p->hv_d, B = hg_fasta_block_bytes();
-  const uint64_t chunk_bytes = hg_chunk_bytes();
-
-  struct Chunk {
-    uint32_t g0, g1;
-    std::vector<uint64_t> dev_off, blk_off;  // per file of the chunk (+ end): offset in the slot, block prefix
-    uint64_t max_blocks = 0;
-    SketchPlan pl;
-  };
-  std::vector<Chunk> chunks;
-  for (uint32_t g = 0; g < n;) {
-    Chunk ch;
-    ch.g0 = g;
-    const uint64_t lo = file_off[g];
-    do {
-      if (file_off[g + 1] < file_off[g]) { hg_set_error("file_off not monotone at %u", g); return HG_E_INVALID; }
-      ++g;
-    } while (g < n && file_off[g + 1] - lo <= chunk_bytes);
-    ch.g1 = g;
-    const uint32_t m = ch.g1 - ch.g0;
-    ch.dev_off.assign(m + 1, 0);
-    ch.blk_off.assign(m + 1, 0);
-    std::vector<uint64_t> lens(m);
-    for (uint32_t t = 0; t < m; t++) {
-      lens[t] = file_off[ch.g0 + t + 1] - file_off[ch.g0 + t];
-      ch.dev_off[t + 1] = ch.dev_off[t] + lens[t];  // back to back, as in the host buffer
-      const uint64_t nb = (lens[t] + B - 1) / B;
-      ch.blk_off[t + 1] = ch.blk_off[t] + nb;
-      ch.max_blocks = std::max(ch.max_blocks, nb);
-    }
-    if (ch.max_blocks > 0x7fffffffull) { hg_set_error("file too large"); return HG_E_UNSUPPORTED; }
-    if ((rc = make_plan_bl(ch.dev_off.data(), lens.data(), m, p, ch.pl))) return rc;  // upper bounds
-    chunks.push_back(std::move(ch));
-  }
-  uint64_t max_bytes = 0, max_slots = 0, max_tiles = 0, max_blk = 0;
-  uint32_t max_m = 0;
-  for (const Chunk &ch : chunks) {
-    max_bytes = std::max(max_bytes, ch.dev_off.back());
-    max_slots = std::max<uint64_t>(max_slots, ch.pl.total_slots);
-    max_tiles = std::max<uint64_t>(max_tiles, ch.pl.n_tiles);
-    max_blk = std::max(max_blk, ch.blk_off.back());
-    max_m = std::max(max_m, ch.g1 - ch.g0);
-  }
-  const uint64_t slot_bytes = (max_bytes + 64 + 255) & ~255ull;
-  const size_t n_desc = (size_t)n + chunks.size();
-  // per-chunk merge metadata in one buffer: file_off | blk_off | out_off | sums | carry
-  const size_t meta_bytes = ((size_t)(2 * (max_m + 1)) * 8 + max_blk * 8 + max_blk * 16 + max_blk + 256 + 15) & ~(size_t)15;
-  const size_t h_meta_per_chunk = (size_t)(2 * (max_m + 1)) * 8;
-
-  void *d_rawbuf, *d_merged, *d_meta, *d_desc, *d_tables, *d_counts, *d_hv = nullptr, *d_packed, *d_small, *d_map, *h_desc,
-      *h_meta;
-  if ((rc = hg_scratch(c, HG_S_REF_LIMBS, 2 * slot_bytes, &d_rawbuf))) return rc;  // raw files, double buffered
-  if ((rc = hg_scratch(c, HG_S_SEQ, slot_bytes, &d_merged))) return rc;
-  if ((rc = hg_scratch(c, HG_S_QRY_LIMBS, meta_bytes + (size_t)n * 8, &d_meta))) return rc;
-  if ((rc = hg_scratch(c, HG_S_DESC, sizeof(hg_genome_desc) * n_desc, &d_desc))) return rc;
-  if ((rc = hg_scratch(c, HG_S_TABLES, max_slots * 8, &d_tables))) return rc;
-  if ((rc = hg_scratch(c, HG_S_COUNTS, sizeof(uint32_t) * n, &d_counts))) return rc;
-  if (hv && (rc = hg_scratch(c, HG_S_HV, (size_t)n * D * 2, &d_hv))) return rc;
-  if ((rc = hg_scratch(c, HG_S_PACKED, (size_t)n * D * 2, &d_packed))) return rc;
-  if ((rc = hg_scratch(c, HG_S_SMALL, (size_t)n * 12, &d_small))) return rc;
-  if ((rc = hg_scratch(c, HG_S_MISC, (max_tiles / hg_kmer_tiles_per_cta() + 2) * 4 + 256, &d_map))) return rc;
-  if ((rc = hg_pinned(c, 0, sizeof(hg_genome_desc) * n_desc, &h_desc))) return rc;
-  if ((rc = hg_pinned(c, 1, h_meta_per_chunk * chunks.size(), &h_meta))) return rc;
-  uint8_t *d_bits = (uint8_t *)d_small + (size_t)n * 8;
-  int32_t *d_norm = (int32_t *)d_small;
-  uint32_t *d_nh = (uint32_t *)d_small + n;
-  uint64_t *d_len = (uint64_t *)((uint8_t *)d_meta + meta_bytes);  // true merged lengths, all files
-  uint64_t *dm_off = (uint64_t *)d_meta, *dm_blk = dm_off + (max_m + 1), *dm_out = dm_blk + (max_m + 1);
-  uint8_t *dm_sums = (uint8_t *)(dm_out + max_blk);
-  uint8_t *dm_carry = dm_sums + max_blk * 16;
-  if ((rc = ensure_copy_stream(c))) return rc;
-  c->ev_used = 0;
-  HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
-  HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * n, c->stream));
-  HG_CUDA(cudaEventRecord(c->ev_done[0], c->stream));
-  HG_CUDA(cudaEventRecord(c->ev_done[1], c->stream));
-
-  size_t desc_pos = 0;
-  for (size_t ci = 0; ci < chunks.size(); ci++) {
-    const Chunk &ch = chunks[ci];
-    const int slot = (int)(ci & 1);
-    const uint32_t m = ch.g1 - ch.g0;
-    uint8_t *d_raw = (uint8_t *)d_rawbuf + slot * slot_bytes;
-    // ---- copy stream: the chunk's files in one copy (per-file copies cost ~6 us each of PCIe idle time) ----
-    HG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_done[slot], 0));
-    if (ch.dev_off[m]) HG_CUDA(cudaMemcpyAsync(d_raw, raw + file_off[ch.g0], ch.dev_off[m], cudaMemcpyHostToDevice, c->copy_stream));
-    HG_CUDA(cudaEventRecord(c->ev_copied[slot], c->copy_stream));
-    // ---- compute stream ----
-    uint64_t *hm = (uint64_t *)((uint8_t *)h_meta + ci * h_meta_per_chunk);
-    memcpy(hm, ch.dev_off.data(), (m + 1) * 8);
-    memcpy(hm + (max_m + 1), ch.blk_off.data(), (m + 1) * 8);
-    HG_CUDA(cudaMemcpyAsync(dm_off, hm, h_meta_per_chunk, cudaMemcpyHostToDevice, c->stream));
-    hg_genome_desc *hd = (hg_genome_desc *)h_desc + desc_pos, *dd = (hg_genome_desc *)d_desc + desc_pos;
-    memcpy(hd, ch.pl.desc.data(), sizeof(hg_genome_desc) * (m + 1));
-    desc_pos += m + 1;
-    HG_CUDA(cudaMemcpyAsync(dd, hd, sizeof(hg_genome_desc) * (m + 1), cudaMemcpyHostToDevice, c->stream));
-    HG_CUDA(cudaMemsetAsync(d_tables, 0xFF, ch.pl.total_slots * 8, c->stream));
-    HG_CUDA(cudaStreamWaitEvent(c->stream, c->ev_copied[slot], 0));
-    if ((rc = hg_launch_fasta_merge(c, d_raw, dm_off, dm_blk, m, (uint32_t)ch.max_blocks, dm_sums, dm_carry, dm_out,
-                                    (uint8_t *)d_merged, d_len + ch.g0)))
-      return rc;
-    HG_CUDA(cudaEventRecord(c->ev_done[slot], c->stream));  // the raw slot may be overwritten now
-    c->d_actual_len = d_len + ch.g0;
-    rc = hg_launch_kmer_hash(c, (const uint8_t *)d_merged, dd, m, ch.pl.n_tiles, p, (uint64_t *)d_tables,
-                             (uint32_t *)d_counts + ch.g0);
-    c->d_actual_len = nullptr;
-    if (rc) return rc;
-    if ((rc = hg_launch_encode(c, dd, m, (const uint64_t *)d_tables, (const uint32_t *)d_counts + ch.g0, D,
-                               d_hv ? (int16_t *)d_hv + (size_t)ch.g0 * D : nullptr,
-                               (uint8_t *)d_packed + (size_t)ch.g0 * 2 * D, d_bits + ch.g0, d_norm + ch.g0, d_nh + ch.g0)))
-      return rc;
-  }
-  if (hv) HG_CUDA(cudaMemcpyAsync(hv, d_hv, (size_t)n * D * 2, cudaMemcpyDeviceToHost, c->stream));
-  if (packed) HG_CUDA(cudaMemcpyAsync(packed, d_packed, (size_t)n * D * 2, cudaMemcpyDeviceToHost, c->stream));
-  if (quant_bits) HG_CUDA(cudaMemcpyAsync(quant_bits, d_bits, n, cudaMemcpyDeviceToHost, c->stream));
-  if (norm2) HG_CUDA(cudaMemcpyAsync(norm2, d_norm, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  if (n_hashes) HG_CUDA(cudaMemcpyAsync(n_hashes, d_nh, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  return hg_sketch_status(c);
 }
 
 // ---------------------------------------------------------------------------------------

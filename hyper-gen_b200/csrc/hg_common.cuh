@@ -153,8 +153,7 @@ struct hg_ctx {
   // H2D pipeline of the host-pointer sketch entry
   int tc_attr_set;
   int n1_attr_set;
-  const uint64_t *d_actual_len;  // optional per-genome true lengths for the next k-mer launch (raw-FASTA path)
-  cudaStream_t copy_stream;      // created on first use, with the events below
+  cudaStream_t copy_stream;  // created on first use, with the events below
   cudaEvent_t ev_copied[2], ev_done[2];
   cudaEvent_t ev_chunk[10];  // dist streaming: fork + query matrix + one per row chunk
   // hg_dist_dev with the single-plane path forced: the pre-pass verdict is not waited for (hg_dist_status reads it)
@@ -247,9 +246,13 @@ struct hg_genome_desc {   // per genome, device-visible
   uint32_t pad_;
 };
 
+// d_true_len (optional): per genome the bases to hash when fewer than desc.seq_len (the merged length of a FASTA file
+// whose tiles were planned from its raw size)
 int hg_launch_kmer_hash(hg_ctx *ctx, const uint8_t *d_seq, const hg_genome_desc *d_desc,
                         uint32_t n_genomes, uint32_t n_tiles, const hg_sketch_params *p,
-                        uint64_t *d_tables, uint32_t *d_counts);
+                        const uint64_t *d_true_len, uint64_t *d_tables, uint32_t *d_counts);
+// bytes of HG_S_MISC that hg_launch_kmer_hash over n_tiles tiles takes for its CTA -> genome map
+size_t hg_kmer_map_bytes(uint32_t n_tiles);
 int hg_launch_sort_tables(hg_ctx *ctx, const hg_genome_desc *d_desc, uint32_t n_genomes,
                           uint64_t *d_tables, uint32_t max_slots);
 int hg_launch_encode(hg_ctx *ctx, const hg_genome_desc *d_desc, uint32_t n_genomes,

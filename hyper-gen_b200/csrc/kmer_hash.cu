@@ -395,15 +395,15 @@ __global__ void tile_map_kernel(const hg_genome_desc *__restrict__ desc, uint32_
 
 template <int K, bool CANON>
 int launch_kc(hg_ctx *ctx, uint32_t n_tiles, const uint8_t *d_seq, const hg_genome_desc *d_desc, uint32_t n_genomes,
-              uint64_t threshold, uint64_t seed, uint64_t *d_tables, uint32_t *d_counts) {
+              const uint64_t *d_true_len, uint64_t threshold, uint64_t seed, uint64_t *d_tables, uint32_t *d_counts) {
   const uint32_t grid = (n_tiles + KH_WARPS - 1) / KH_WARPS;
   void *d_map;
-  int rc = hg_scratch(ctx, HG_S_MISC, (size_t)grid * 4 + 256, &d_map);
+  int rc = hg_scratch(ctx, HG_S_MISC, hg_kmer_map_bytes(n_tiles), &d_map);
   if (rc) return rc;
   tile_map_kernel<<<(n_genomes * 32 + 127) / 128, 128, 0, ctx->stream>>>(d_desc, n_genomes, (uint32_t *)d_map);
   kmer_hash_kernel<K, CANON><<<grid, KH_THREADS, 0, ctx->stream>>>(d_seq, d_desc, n_genomes, n_tiles, threshold, seed,
                                                                    d_tables, d_counts, ctx->d_status, 0x47434100u,
-                                                                   0x00000054u, (const uint32_t *)d_map, ctx->d_actual_len,
+                                                                   0x00000054u, (const uint32_t *)d_map, d_true_len,
                                                                    make_uint2(0xDFDFDFDFu, 0x15060200u));
   ctx->launches += 2;
   HG_CUDA(cudaGetLastError());
@@ -412,24 +412,27 @@ int launch_kc(hg_ctx *ctx, uint32_t n_tiles, const uint8_t *d_seq, const hg_geno
 
 template <int K>
 int launch_k(hg_ctx *ctx, bool canon, uint32_t n_tiles, const uint8_t *d_seq, const hg_genome_desc *d_desc,
-             uint32_t n_genomes, uint64_t threshold, uint64_t seed, uint64_t *d_tables, uint32_t *d_counts) {
-  return canon ? launch_kc<K, true>(ctx, n_tiles, d_seq, d_desc, n_genomes, threshold, seed, d_tables, d_counts)
-               : launch_kc<K, false>(ctx, n_tiles, d_seq, d_desc, n_genomes, threshold, seed, d_tables, d_counts);
+             uint32_t n_genomes, const uint64_t *d_true_len, uint64_t threshold, uint64_t seed, uint64_t *d_tables,
+             uint32_t *d_counts) {
+  return canon ? launch_kc<K, true>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed, d_tables, d_counts)
+               : launch_kc<K, false>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed, d_tables, d_counts);
 }
 
 }  // namespace
 
 uint32_t hg_kmer_tile_positions() { return KH_TILE; }
-uint32_t hg_kmer_tiles_per_cta() { return KH_WARPS; }
+size_t hg_kmer_map_bytes(uint32_t n_tiles) { return (size_t)((n_tiles + KH_WARPS - 1) / KH_WARPS) * 4 + 256; }
 
 int hg_launch_kmer_hash(hg_ctx *ctx, const uint8_t *d_seq, const hg_genome_desc *d_desc, uint32_t n_genomes,
-                        uint32_t n_tiles, const hg_sketch_params *p, uint64_t *d_tables, uint32_t *d_counts) {
+                        uint32_t n_tiles, const hg_sketch_params *p, const uint64_t *d_true_len, uint64_t *d_tables,
+                        uint32_t *d_counts) {
   if (n_tiles == 0) return HG_OK;
   const uint64_t threshold = UINT64_MAX / p->scaled;  // sketch.rs:73
   const bool canon = p->canonical != 0;
   switch (p->ksize) {
 #define HG_K(KK) \
-  case KK: return launch_k<KK>(ctx, canon, n_tiles, d_seq, d_desc, n_genomes, threshold, p->seed, d_tables, d_counts);
+  case KK: return launch_k<KK>(ctx, canon, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, p->seed, d_tables, \
+                               d_counts);
 #ifdef HG_KMER_ONLY_K21  // (development: one instantiation, for reading its SASS)
     HG_K(21)
 #else

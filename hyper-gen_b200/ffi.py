@@ -163,6 +163,16 @@ def _ptr(a) -> int:
     return a.ctypes.data
 
 
+def _sketch_out(n: int, hv_d: int, want_hv: bool, n_hashes: bool = True) -> dict:
+    """The host arrays of n sketches, in the order the C entries take them: hv (None unless wanted), packed,
+    quant_bits, norm2 and, unless n_hashes is False, n_hashes.  Pass them on as *map(_ptr, out.values())."""
+    out = dict(hv=np.empty((n, hv_d), np.int16) if want_hv else None, packed=np.empty((n, 2 * hv_d), np.uint8),
+               quant_bits=np.empty(n, np.uint8), norm2=np.empty(n, np.int32))
+    if n_hashes:
+        out["n_hashes"] = np.empty(n, np.uint32)
+    return out
+
+
 def make_params(k=21, scaled=1500, seed=123, canonical=True, hv_d=4096) -> SketchParams:
     return SketchParams(scaled=scaled, seed=seed, hv_d=hv_d, ksize=k, canonical=int(bool(canonical)))
 
@@ -317,15 +327,10 @@ class Context:
         seq = np.ascontiguousarray(seq, np.uint8)
         off = np.ascontiguousarray(seg_off, np.uint64)
         n = off.size - 1
-        D = int(params.hv_d)
-        hv = np.empty((n, D), np.int16) if want_hv else None
-        packed = np.empty((n, 2 * D), np.uint8)
-        qb = np.empty(n, np.uint8)
-        norm2 = np.empty(n, np.int32)
-        nh = np.empty(n, np.uint32)
+        out = _sketch_out(n, int(params.hv_d), want_hv)
         _check(load().hg_sketch_batch(self._h, _ptr(seq) if seq.size else None, _ptr(off), n, C.byref(params),
-                                      _ptr(hv), _ptr(packed), _ptr(qb), _ptr(norm2), _ptr(nh)))
-        return dict(hv=hv, packed=packed, quant_bits=qb, norm2=norm2, n_hashes=nh)
+                                      *map(_ptr, out.values())))
+        return out
 
     def sketch_batch_dev(self, d_seq: int, seg_off: np.ndarray, params: SketchParams, d_hv, d_packed,
                          d_quant_bits: int, d_norm2: int, d_n_hashes: int):
@@ -340,13 +345,10 @@ class Context:
         off = np.zeros(n + 1, np.uint64)
         off[1:] = np.cumsum([len(x) for x in sets])
         hashes = np.ascontiguousarray(np.concatenate(sets) if n and int(off[-1]) else np.zeros(0), np.uint64)
-        hv = np.empty((n, hv_d), np.int16) if want_hv else None
-        packed = np.empty((n, 2 * hv_d), np.uint8)
-        qb = np.empty(n, np.uint8)
-        norm2 = np.empty(n, np.int32)
-        _check(load().hg_encode_sets(self._h, _ptr(hashes) if hashes.size else None, _ptr(off), n, hv_d, _ptr(hv),
-                                     _ptr(packed), _ptr(qb), _ptr(norm2)))
-        return dict(hv=hv, packed=packed, quant_bits=qb, norm2=norm2)
+        out = _sketch_out(n, hv_d, want_hv, n_hashes=False)
+        _check(load().hg_encode_sets(self._h, _ptr(hashes) if hashes.size else None, _ptr(off), n, hv_d,
+                                     *map(_ptr, out.values())))
+        return out
 
     def encode_sets_dev(self, d_hashes: int, hash_off: np.ndarray, hv_d: int, d_hv, d_packed, d_quant_bits, d_norm2):
         off = np.ascontiguousarray(hash_off, np.uint64)
@@ -375,15 +377,10 @@ class Context:
         """hg_sketch_fasta_batch: raw FASTA file contents in, sketches out (as sketch_batch)."""
         raw, off = self._concat_files(files)
         n = len(files)
-        D = int(params.hv_d)
-        hv = np.empty((n, D), np.int16) if want_hv else None
-        packed = np.empty((n, 2 * D), np.uint8)
-        qb = np.empty(n, np.uint8)
-        norm2 = np.empty(n, np.int32)
-        nh = np.empty(n, np.uint32)
+        out = _sketch_out(n, int(params.hv_d), want_hv)
         _check(load().hg_sketch_fasta_batch(self._h, _ptr(raw) if raw.size else None, _ptr(off), n, C.byref(params),
-                                            _ptr(hv), _ptr(packed), _ptr(qb), _ptr(norm2), _ptr(nh)))
-        return dict(hv=hv, packed=packed, quant_bits=qb, norm2=norm2, n_hashes=nh)
+                                            *map(_ptr, out.values())))
+        return out
 
     def sketch_status(self):
         _check(load().hg_sketch_status(self._h))
@@ -643,15 +640,10 @@ class Group:
     def sketch_fasta_batch(self, files, params: SketchParams, want_hv: bool = True):
         raw, off = Context._concat_files(files)
         n = len(files)
-        D = int(params.hv_d)
-        hv = np.empty((n, D), np.int16) if want_hv else None
-        packed = np.empty((n, 2 * D), np.uint8)
-        qb = np.empty(n, np.uint8)
-        norm2 = np.empty(n, np.int32)
-        nh = np.empty(n, np.uint32)
+        out = _sketch_out(n, int(params.hv_d), want_hv)
         _check(load().hg_group_sketch_fasta_batch(self._h, _ptr(raw) if raw.size else None, _ptr(off), n, C.byref(params),
-                                                  _ptr(hv), _ptr(packed), _ptr(qb), _ptr(norm2), _ptr(nh)))
-        return dict(hv=hv, packed=packed, quant_bits=qb, norm2=norm2, n_hashes=nh)
+                                                  *map(_ptr, out.values())))
+        return out
 
     def dist_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize=21, ani_th=85.0,
                     symmetric=False, sorted_output=True, cap=None):

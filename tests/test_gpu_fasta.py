@@ -22,6 +22,15 @@ def _fasta(seq, name=b"g", width=80, eol=b"\n", records=1, final_eol=True):
     return bytes(out)
 
 
+def _assert_sketches_equal(got, want, hv_d):
+    assert np.array_equal(got["n_hashes"], want["n_hashes"])
+    assert np.array_equal(got["hv"], want["hv"]) and np.array_equal(got["norm2"], want["norm2"])
+    assert np.array_equal(got["quant_bits"], want["quant_bits"])
+    for g in range(want["quant_bits"].size):  # the live bytes of each packed row
+        nb = int(want["quant_bits"][g]) * hv_d // 8
+        assert np.array_equal(got["packed"][g, :nb], want["packed"][g, :nb]), g
+
+
 def test_fasta_merge_matches_reference_reader(ctx, hg, oracle):
     rng = np.random.default_rng(8)
     s = random_dna(rng, 30_000, p_n=0.01, p_lower=0.1)
@@ -52,18 +61,14 @@ def test_sketch_from_raw_fasta_equals_sketch_from_merged(ctx, hg, oracle):
     seqs = [oracle.read_merge_seq(f) for f in files]
     off = np.cumsum([0] + [s.size for s in seqs]).astype(np.uint64)
     want = oracle.sketch_batch(np.concatenate(seqs), off, scaled=300, hv_d=1024)
-    assert np.array_equal(got["n_hashes"], want["n_hashes"])
-    assert np.array_equal(got["hv"], want["hv"]) and np.array_equal(got["norm2"], want["norm2"])
-    assert np.array_equal(got["quant_bits"], want["quant_bits"])
-    for g in range(len(files)):
-        nb = int(want["quant_bits"][g]) * 1024 // 8
-        assert np.array_equal(got["packed"][g, :nb], want["packed"][g, :nb])
+    _assert_sketches_equal(got, want, 1024)
 
 
 def test_raw_fasta_chunk_pipeline(ctx, hg, oracle, monkeypatch):
     """Several 1 MB chunks through the double-buffered copy/merge/hash/encode pipeline, with files
     whose merged length is far below the raw size the tiles were planned from (long headers, a file
-    that is all header, a merged length below k)."""
+    that is all header, a merged length below k); then the merged sequences of the same files through
+    the sequence entry's chunks, which start at several alignments modulo 16."""
     from hypergen_b200 import synth
     monkeypatch.setenv("HG_CHUNK_MB", "1")
     rng = np.random.default_rng(77)
@@ -80,8 +85,18 @@ def test_raw_fasta_chunk_pipeline(ctx, hg, oracle, monkeypatch):
     seqs = [oracle.read_merge_seq(f) for f in files]
     off = np.cumsum([0] + [s.size for s in seqs]).astype(np.uint64)
     want = oracle.sketch_batch(np.concatenate(seqs), off, scaled=200, hv_d=2048)
-    assert np.array_equal(got["n_hashes"], want["n_hashes"])
-    assert np.array_equal(got["hv"], want["hv"]) and np.array_equal(got["norm2"], want["norm2"])
-    assert np.array_equal(got["quant_bits"], want["quant_bits"])
+    _assert_sketches_equal(got, want, 2048)
     again = ctx.sketch_fasta_batch(files, p)                                # scratch reuse across calls
     assert np.array_equal(again["hv"], want["hv"])
+
+    lead = 5                                                                # bytes before the first genome
+    buf = np.concatenate([np.full(lead, ord("N"), np.uint8)] + seqs)
+    seq_off = off + np.uint64(lead)
+    starts, g = [], 0                                                       # chunk starts: genome boundaries, <= 1 MB a chunk
+    while g < len(seqs):
+        starts.append(int(seq_off[g]))
+        g += 1
+        while g < len(seqs) and int(seq_off[g + 1]) - starts[-1] <= 1 << 20:
+            g += 1
+    assert len(starts) > 2 and len({(buf.ctypes.data + s) % 16 for s in starts}) > 1
+    _assert_sketches_equal(ctx.sketch_batch(buf, seq_off, p), want, 2048)
