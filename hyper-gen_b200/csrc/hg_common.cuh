@@ -47,16 +47,35 @@ __device__ __forceinline__ uint64_t final64(uint64_t a, uint64_t b) {
 }
 
 // NW = ceil(K / 8) words; word m holds bytes 8m..8m+7 of the k-mer, little-endian, the last
-// one zero-extended (tail64_le_unaligned, cuda_kernel.cu:155-194).
+// one zero-extended (tail64_le_unaligned, cuda_kernel.cu:155-194).  Word m is mixed with prime
+// p_(NW-m), alternately into (a, b) and (b, a), starting from a = seed, b = K.
+//
+// Round 1 (word 0) is mixup64(X, Y, w[0], P): which of a, b plays X (xored) and which Y (added
+// to) depends on NW alone.  kmer_hash.cu takes this round from product tables built from these
+// roles; rounds 2.. and final64 are t1ha2_kmer_rest for every caller.
+template <int K>
+struct t1ha2_round1 {
+  static constexpr int NW = (K + 7) / 8;
+  static constexpr bool x_is_seed = NW % 2 == 0;  // mixup64(a, b, ...): X = a = seed, Y = b = K
+  static constexpr uint64_t prime = NW == 4 ? t1_p4() : NW == 3 ? t1_p3() : NW == 2 ? t1_p2() : t1_p1();
+};
+
+// words 1..NW-1 and final64, from the state (a, b) after round 1
+template <int K>
+__device__ __forceinline__ uint64_t t1ha2_kmer_rest(uint64_t a, uint64_t b, const uint64_t (&w)[(K + 7) / 8]) {
+  constexpr int NW = (K + 7) / 8;
+  if (NW > 3) mixup64(b, a, w[NW > 3 ? NW - 3 : 0], t1_p3());
+  if (NW > 2) mixup64(a, b, w[NW > 2 ? NW - 2 : 0], t1_p2());
+  if (NW > 1) mixup64(b, a, w[NW - 1], t1_p1());
+  return final64(a, b);
+}
+
 template <int K>
 __device__ __forceinline__ uint64_t t1ha2_kmer(const uint64_t (&w)[(K + 7) / 8], uint64_t seed) {
   uint64_t a = seed, b = (uint64_t)K;
-  int m = 0;
-  if (K > 24) mixup64(a, b, w[m++], t1_p4());
-  if (K > 16) mixup64(b, a, w[m++], t1_p3());
-  if (K > 8) mixup64(a, b, w[m++], t1_p2());
-  if (K > 0) mixup64(b, a, w[m++], t1_p1());
-  return final64(a, b);
+  if (t1ha2_round1<K>::x_is_seed) mixup64(a, b, w[0], t1ha2_round1<K>::prime);
+  else mixup64(b, a, w[0], t1ha2_round1<K>::prime);
+  return t1ha2_kmer_rest<K>(a, b, w);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -200,7 +219,7 @@ enum hg_scratch_slot {
   HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass;
                        // group search: the members' results gathered on GPU 0; cluster: the edges of one window
   HG_S_SMALL = 6,      // norms / bits / counts per sketch
-  HG_S_MISC = 7,       // CTA -> genome map, |hv| max, probe sink, status word of a search merge; cluster: status word
+  HG_S_MISC = 7,       // CTA -> genome map + round-1 tables, |hv| max, probe sink, status word of a search merge; cluster: status word
                        // of a union check, root count of a flatten
   HG_S_REF_LIMBS = 8,  // s8 limb planes of the ref matrix (dist_tc)
   HG_S_QRY_LIMBS = 9,  // s8 limb planes of the query matrix (dist_tc)
@@ -251,7 +270,7 @@ struct hg_genome_desc {   // per genome, device-visible
 int hg_launch_kmer_hash(hg_ctx *ctx, const uint8_t *d_seq, const hg_genome_desc *d_desc,
                         uint32_t n_genomes, uint32_t n_tiles, const hg_sketch_params *p,
                         const uint64_t *d_true_len, uint64_t *d_tables, uint32_t *d_counts);
-// bytes of HG_S_MISC that hg_launch_kmer_hash over n_tiles tiles takes for its CTA -> genome map
+// bytes of HG_S_MISC that hg_launch_kmer_hash over n_tiles tiles takes for its CTA -> genome map and t1ha2 round-1 tables
 size_t hg_kmer_map_bytes(uint32_t n_tiles);
 int hg_launch_sort_tables(hg_ctx *ctx, const hg_genome_desc *d_desc, uint32_t n_genomes,
                           uint64_t *d_tables, uint32_t max_slots);

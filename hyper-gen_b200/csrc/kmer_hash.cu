@@ -21,7 +21,8 @@
 //     canonical = lexicographic min via ONE multi-word unsigned compare of the two states (same
 //     choice as the reference's byte compare, cuda_kernel.cu:84-89,306-311), and the chosen k-mer becomes
 //     its upper-case ASCII bytes with two PRMT table lookups per 8 bases (the hash is defined
-//     over the ASCII k-mer, sketch.rs:90); t1ha2_atonce in registers; threshold compare;
+//     over the ASCII k-mer, sketch.rs:90); t1ha2_atonce in registers, its first round (K >= 8) from
+//     two product tables in shared memory indexed by the first 8 bases; threshold compare;
 //   * the rare survivors (1/scaled) are inserted into the genome's open-addressing table in
 //     HBM with atomicCAS, which both removes duplicates (the reference keeps a set) and has
 //     no per-thread capacity cliff (the reference drops hits beyond 8 per thread,
@@ -141,17 +142,55 @@ __device__ __noinline__ void table_insert(uint64_t *__restrict__ table, uint32_t
   atomicOr(status, 1u);  // table full: reported by hg_sketch_status, never silently dropped
 }
 
-template <int K, bool CANON>
+// ---- t1ha2's first round from product tables (K >= 8) ----
+// Word 0 of a k-mer with K >= 8 is the ASCII of its first 8 bases: 4^8 values.  Round 1 is
+// mixup64(X, Y, w0, P) (roles and prime: hg::t1ha2_round1), i.e. t = Y + w0 mod 2^64, X ^= lo64(t P),
+// Y += hi64(t P).  With w0 = w_lo + 2^32 w_hi (w_lo = bases 0-3, w_hi = bases 4-7) and c = [Y + w0 >= 2^64]:
+//   t P = (Y + w_lo) P + w_hi P 2^32 - c P 2^64   (mod 2^128)
+// so the round is two lookups and a 128-bit add:
+//   L[i] = (Y + w_lo(i)) P mod 2^128, with X_lo xored into word 0 and Y added to the high 64 bits;
+//   H[j] = w_hi(j) P (96 bits: words 1-3 of the sum; word 0 of the sum is word 0 of L).
+// i, j are the base-4 numbers of bases 0-3 and 4-7 (base 0 least significant, A < C < G < T).  w0 grows
+// with j * 256 + i, so c is a threshold test on that index; it can only be 1 when Y is the seed and the
+// seed is above 2^64 - w0(TTTTTTTT), which the host decides per launch (the WRAP instantiations).
+constexpr int KH_TAB_ENTRIES = 512;                        // L[256] | H[256], 16 bytes each
+constexpr size_t KH_TAB_BYTES = KH_TAB_ENTRIES * sizeof(uint4);
+constexpr int KH_TAB_COPIES = 2;  // in shared memory (measured: 20.85 ms per 1000 genomes vs 20.94 with one copy)
+
+// ASCII of the 4 bases of a base-4 number e (base 0 in the low 2 bits and the low byte)
+__host__ __device__ inline uint32_t ascii4(uint32_t e) {
+  uint32_t w = 0;
+  for (int k = 0; k < 4; ++k) w |= ((0x54474341u >> (8 * ((e >> (2 * k)) & 3u))) & 0xFFu) << (8 * k);
+  return w;
+}
+
+template <int K, bool CANON, bool WRAP>
 __global__ void __launch_bounds__(KH_THREADS, KH_MIN_CTAS)
 kmer_hash_kernel(const uint8_t *__restrict__ seq, const hg_genome_desc *__restrict__ desc,
                  uint32_t n_genomes, uint32_t n_tiles, uint64_t threshold, uint64_t seed,
                  uint64_t *__restrict__ tables, uint32_t *__restrict__ counts,
                  uint32_t *__restrict__ status, uint32_t lut_lo, uint32_t lut_hi,
-                 const uint32_t *__restrict__ cta_genome, const uint64_t *__restrict__ actual_len, uint2 consts) {
+                 const uint32_t *__restrict__ cta_genome, const uint64_t *__restrict__ actual_len, uint2 consts,
+                 const uint4 *__restrict__ round1_tab, uint32_t wrap_at) {
   constexpr int NW = (K + 7) / 8;          // nibble words == t1ha2 input words (8 bases each)
   constexpr int LASTN = K - 8 * (NW - 1);  // bases in the last word, 1..8
   constexpr uint32_t LASTMASK = LASTN == 8 ? 0xFFFFFFFFu : ((1u << (4 * LASTN)) - 1u);
-  // every warp owns a private staging area and runs on its own: no CTA-wide barrier anywhere
+  constexpr bool TAB = K >= 8;             // round 1 from the product tables
+  using R1 = hg::t1ha2_round1<K>;
+  // The round-1 tables, copied into shared memory once per CTA: the kernel's only CTA-wide barrier, ahead of every
+  // return.  Two copies, entry e of copy r at 2 e + r, and the lane's parity picks the copy: the 8 lanes of an LDS.128
+  // phase then hit each half of the bank groups with 4 random indices instead of all of them with 8 (fewer conflicts).
+  __shared__ uint4 s_tab[TAB ? KH_TAB_COPIES * KH_TAB_ENTRIES : 1];
+  if (TAB) {
+#pragma unroll
+    for (int e = threadIdx.x; e < KH_TAB_ENTRIES; e += KH_THREADS) {
+      const uint4 v = round1_tab[e];
+      s_tab[2 * e] = v;
+      s_tab[2 * e + 1] = v;
+    }
+    __syncthreads();
+  }
+  // apart from that every warp owns a private staging area and runs on its own
   __shared__ __align__(8) uint32_t s_nib_all[KH_WARPS][KH_CHUNKS * 2 + 8];    // 8 bases per word
   __shared__ uint32_t s_valid_all[KH_WARPS][KH_CHUNKS / 2 + 4];  // 16 bits per chunk
   // survivors are queued here and inserted together at the end of the tile, so the round trip
@@ -350,13 +389,32 @@ kmer_hash_kernel(const uint8_t *__restrict__ seq, const hg_genome_desc *__restri
       }
       // ---- ASCII expansion: each nibble is a PRMT selector into {0,'A','C','G','T',0,0,0} ----
       uint64_t w[NW];
+      w[0] = 0;  // (read by t1ha2_kmer only)
 #pragma unroll
-      for (int m = 0; m < NW; ++m) {
+      for (int m = TAB ? 1 : 0; m < NW; ++m) {
         const uint32_t lo = prmt(lut_lo, lut_hi, C[m]);
         const uint32_t hi = prmt(lut_lo, lut_hi, C[m] >> 16);
         w[m] = (uint64_t)lo | ((uint64_t)hi << 32);
       }
-      const uint64_t h = hg::t1ha2_kmer<K>(w, seed);
+      uint64_t h;
+      if (TAB) {
+        // table indices from the nibble codes: code - 1 is the 2-bit base value; x * 5 puts the values of nibbles
+        // 2n and 2n + 1 side by side at bits 2-5 of byte n, and * 0x44 gathers i at bits 8-15 and j at bits 24-31
+        const uint32_t z = (((C[0] - 0x11111111u) * 5u) & 0x3C3C3C3Cu) * 0x44u;
+        const char *tab = reinterpret_cast<const char *>(s_tab) + (threadIdx.x & 1u) * sizeof(uint4);  // this lane's copy
+        const uint4 l = *reinterpret_cast<const uint4 *>(tab + ((z >> 3) & 0x1FE0u));                 // L[i]: 32 i
+        const uint4 hh = *reinterpret_cast<const uint4 *>(tab + 256 * 32 + ((z >> 19) & 0x1FE0u));    // H[j]: 32 j
+        uint32_t x_w1, y_lo, y_hi;  // word 1 of the sum carries into Y1 = words 2-3 (+ Y, folded into L)
+        asm("add.cc.u32 %0, %3, %4; addc.cc.u32 %1, %5, %6; addc.u32 %2, %7, %8;"
+            : "=r"(x_w1), "=r"(y_lo), "=r"(y_hi) : "r"(l.y), "r"(hh.x), "r"(l.z), "r"(hh.y), "r"(l.w), "r"(hh.z));
+        if (R1::x_is_seed) x_w1 ^= (uint32_t)(seed >> 32);  // X_lo is in L; X_hi is 0 when X = K
+        const uint64_t x1 = (uint64_t)l.x | ((uint64_t)x_w1 << 32);
+        uint64_t y1 = (uint64_t)y_lo | ((uint64_t)y_hi << 32);
+        if (WRAP && (z & 0xFF00FF00u) >= wrap_at) y1 -= R1::prime;  // Y + w0 wrapped: t P is P 2^64 less
+        h = R1::x_is_seed ? hg::t1ha2_kmer_rest<K>(x1, y1, w) : hg::t1ha2_kmer_rest<K>(y1, x1, w);
+      } else {
+        h = hg::t1ha2_kmer<K>(w, seed);
+      }
       hs[jj % KH_GROUP] = h;
       min_hi = min(min_hi, (uint32_t)(h >> 32));
       if ((jj % KH_GROUP) == KH_GROUP - 1) {
@@ -383,9 +441,23 @@ kmer_hash_kernel(const uint8_t *__restrict__ seq, const hg_genome_desc *__restri
   }
 }
 
-// cta_genome[c] = genome that owns tile c * KH_WARPS: one warp per genome fills its range.
+// cta_genome[c] = genome that owns tile c * KH_WARPS: one warp per genome fills its range.  The CTAs from
+// tab_cta on build the round-1 tables (one L and one H entry per thread) for X, Y, P.
 __global__ void tile_map_kernel(const hg_genome_desc *__restrict__ desc, uint32_t n_genomes,
-                                uint32_t *__restrict__ cta_genome) {
+                                uint32_t *__restrict__ cta_genome, uint32_t tab_cta, uint4 *__restrict__ tab,
+                                uint64_t X, uint64_t Y, uint64_t P) {
+  if (blockIdx.x >= tab_cta) {
+    const uint32_t e = (blockIdx.x - tab_cta) * blockDim.x + threadIdx.x;
+    if (e >= 256) return;
+    // L[e] = (Y + w_lo(e)) P mod 2^128; the add may carry out of 64 bits, and that carry is worth P 2^64
+    const uint64_t t = Y + ascii4(e);
+    const uint64_t lo = t * P, hi = __umul64hi(t, P) + (t < Y ? P : 0ull) + Y;
+    tab[e] = make_uint4((uint32_t)lo ^ (uint32_t)X, (uint32_t)(lo >> 32), (uint32_t)hi, (uint32_t)(hi >> 32));
+    // H[e] = w_hi(e) P < 2^96
+    const uint64_t wh = ascii4(e), hlo = wh * P;
+    tab[256 + e] = make_uint4((uint32_t)hlo, (uint32_t)(hlo >> 32), (uint32_t)__umul64hi(wh, P), 0u);
+    return;
+  }
   const uint32_t g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (g >= n_genomes) return;
   const uint32_t c0 = (desc[g].first_tile + KH_WARPS - 1) / KH_WARPS;
@@ -393,18 +465,41 @@ __global__ void tile_map_kernel(const hg_genome_desc *__restrict__ desc, uint32_
   for (uint32_t c = c0 + lane; c < c1; c += 32) cta_genome[c] = g;
 }
 
-template <int K, bool CANON>
+// byte offset of the round-1 tables in HG_S_MISC, behind the CTA -> genome map
+size_t kh_tab_offset(uint32_t n_tiles) { return ((size_t)(n_tiles + KH_WARPS - 1) / KH_WARPS * 4 + 255) & ~(size_t)255; }
+
+// The smallest index j * 256 + i whose word 0 wraps Y + w0 past 2^64, in the (z & 0xFF00FF00) form the kernel
+// compares (j at bits 24-31, i at bits 8-15); KH_NO_WRAP when Y + w0 wraps for no word 0.
+constexpr uint32_t KH_NO_WRAP = 0xFFFFFFFFu;  // above every (z & 0xFF00FF00)
+uint32_t kh_wrap_at(uint64_t Y) {
+  auto w0 = [](uint32_t idx) { return (uint64_t)ascii4(idx & 0xFFu) | ((uint64_t)ascii4(idx >> 8) << 32); };
+  if (Y + w0(0xFFFFu) >= Y) return KH_NO_WRAP;
+  uint32_t lo = 0, hi = 0xFFFFu;  // w0 grows with the index: bisect for the first wrapping one, which is <= hi
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) / 2;
+    if (Y + w0(mid) < Y) hi = mid;
+    else lo = mid + 1;
+  }
+  return ((lo >> 8) << 24) | ((lo & 0xFFu) << 8);
+}
+
+template <int K, bool CANON, bool WRAP>
 int launch_kc(hg_ctx *ctx, uint32_t n_tiles, const uint8_t *d_seq, const hg_genome_desc *d_desc, uint32_t n_genomes,
-              const uint64_t *d_true_len, uint64_t threshold, uint64_t seed, uint64_t *d_tables, uint32_t *d_counts) {
+              const uint64_t *d_true_len, uint64_t threshold, uint64_t seed, uint64_t *d_tables, uint32_t *d_counts,
+              uint32_t wrap_at) {
+  using R1 = hg::t1ha2_round1<K>;
   const uint32_t grid = (n_tiles + KH_WARPS - 1) / KH_WARPS;
   void *d_map;
   int rc = hg_scratch(ctx, HG_S_MISC, hg_kmer_map_bytes(n_tiles), &d_map);
   if (rc) return rc;
-  tile_map_kernel<<<(n_genomes * 32 + 127) / 128, 128, 0, ctx->stream>>>(d_desc, n_genomes, (uint32_t *)d_map);
-  kmer_hash_kernel<K, CANON><<<grid, KH_THREADS, 0, ctx->stream>>>(d_seq, d_desc, n_genomes, n_tiles, threshold, seed,
-                                                                   d_tables, d_counts, ctx->d_status, 0x47434100u,
-                                                                   0x00000054u, (const uint32_t *)d_map, d_true_len,
-                                                                   make_uint2(0xDFDFDFDFu, 0x15060200u));
+  uint4 *d_tab = (uint4 *)((uint8_t *)d_map + kh_tab_offset(n_tiles));
+  const uint32_t map_ctas = (n_genomes * 32 + 127) / 128, tab_ctas = K >= 8 ? 2 : 0;
+  const uint64_t X = R1::x_is_seed ? seed : (uint64_t)K, Y = R1::x_is_seed ? (uint64_t)K : seed;
+  tile_map_kernel<<<map_ctas + tab_ctas, 128, 0, ctx->stream>>>(d_desc, n_genomes, (uint32_t *)d_map, map_ctas, d_tab,
+                                                                X, Y, R1::prime);
+  kmer_hash_kernel<K, CANON, WRAP><<<grid, KH_THREADS, 0, ctx->stream>>>(
+      d_seq, d_desc, n_genomes, n_tiles, threshold, seed, d_tables, d_counts, ctx->d_status, 0x47434100u, 0x00000054u,
+      (const uint32_t *)d_map, d_true_len, make_uint2(0xDFDFDFDFu, 0x15060200u), d_tab, wrap_at);
   ctx->launches += 2;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
@@ -414,14 +509,25 @@ template <int K>
 int launch_k(hg_ctx *ctx, bool canon, uint32_t n_tiles, const uint8_t *d_seq, const hg_genome_desc *d_desc,
              uint32_t n_genomes, const uint64_t *d_true_len, uint64_t threshold, uint64_t seed, uint64_t *d_tables,
              uint32_t *d_counts) {
-  return canon ? launch_kc<K, true>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed, d_tables, d_counts)
-               : launch_kc<K, false>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed, d_tables, d_counts);
+  // only a seed in the Y role can wrap (K = 8 and 17..24), and only a seed near 2^64: a kernel of its own
+  if constexpr (K >= 8 && !hg::t1ha2_round1<K>::x_is_seed) {
+    const uint32_t wrap_at = kh_wrap_at(seed);
+    if (wrap_at != KH_NO_WRAP)
+      return canon ? launch_kc<K, true, true>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed,
+                                              d_tables, d_counts, wrap_at)
+                   : launch_kc<K, false, true>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed,
+                                               d_tables, d_counts, wrap_at);
+  }
+  return canon ? launch_kc<K, true, false>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed, d_tables,
+                                           d_counts, KH_NO_WRAP)
+               : launch_kc<K, false, false>(ctx, n_tiles, d_seq, d_desc, n_genomes, d_true_len, threshold, seed, d_tables,
+                                            d_counts, KH_NO_WRAP);
 }
 
 }  // namespace
 
 uint32_t hg_kmer_tile_positions() { return KH_TILE; }
-size_t hg_kmer_map_bytes(uint32_t n_tiles) { return (size_t)((n_tiles + KH_WARPS - 1) / KH_WARPS) * 4 + 256; }
+size_t hg_kmer_map_bytes(uint32_t n_tiles) { return kh_tab_offset(n_tiles) + KH_TAB_BYTES; }
 
 int hg_launch_kmer_hash(hg_ctx *ctx, const uint8_t *d_seq, const hg_genome_desc *d_desc, uint32_t n_genomes,
                         uint32_t n_tiles, const hg_sketch_params *p, const uint64_t *d_true_len, uint64_t *d_tables,
