@@ -21,10 +21,13 @@ class SketchCluster:
 
 def format_cluster_lines(names, rep) -> str:
     """One `rep_name\\tmember_name` line per sketch (galah's representative / member layout): clusters in ascending
-    representative index, members in ascending index within a cluster, so a representative's own line comes first."""
+    representative index, the representative's own line first, then the members in ascending index - the key
+    (rep, t != rep, t).  A greedy representative (derep) need not be the smallest index of its cluster; a single-linkage
+    one (cluster) always is, so there the key is (rep, t)."""
     rep = np.asarray(rep, np.int64)
-    order = np.lexsort((np.arange(rep.size), rep))
-    return "".join("%s\t%s\n" % (names[rep[t]], names[t]) for t in order)
+    t = np.arange(rep.size)
+    order = np.lexsort((t, t != rep, rep))
+    return "".join("%s\t%s\n" % (names[rep[k]], names[k]) for k in order)
 
 
 def cluster(sc: SketchCluster, ctx: Context | None = None, path: int = 0, group: Group | None = None) -> str:

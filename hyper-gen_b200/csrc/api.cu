@@ -747,13 +747,17 @@ void hg_dist_record(hg_ctx *c, int path, const char *fmt, ...) {
 // A window of the pairs of one matrix against itself: ref rows [r0, r0 + h) x query rows [c0, c0 + w), reported with
 // the call's global offsets (i0 + r, j0 + c).
 struct DistWindow { uint32_t r0, h, c0, w; };
-// A dist call that runs only these windows (a cluster run, hg_cluster_*): every row is prepared once, then each window is
-// launched and `after(k)` is enqueued behind the launch of window k - by every kernel branch, the two-limb rerun after a
-// declined single plane included.
+// A dist call that runs only these windows (a cluster or derep run, hg_cluster_* / hg_derep_*): every row is prepared
+// once, then each window is launched and `after(k)` is enqueued behind the launch of window k - by every kernel branch,
+// the two-limb rerun after a declined single plane included.
 struct DistWindows {
   std::vector<DistWindow> win;
   std::function<int(size_t)> after;
   cudaEvent_t prepared = nullptr;  // if set: recorded once the rows are prepared, before the first window
+  // The single plane's verdict is read once the rows are prepared, before the first window: a declined plane then
+  // launches no window and no `after`, and the rerun starts from the state the caller left.  For hooks that are not
+  // idempotent (the greedy steps of a derep run); without it the declined windows run their hooks on empty edge lists.
+  bool decide_first = false;
 };
 
 // one dist call: ref rows [i0, i0 + n_ref) against query rows [j0, j0 + n_qry), both matrices in HBM (or arriving there)
@@ -927,8 +931,10 @@ static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, H
              : launch(r_off + a, rows, op.i0 + a, op.ref_norm + a, 0, op.n_qry, op.j0, op.qry_norm);
     if (rc) return rc;
   }
+  const bool first = narrow && op.windows && op.windows->decide_first;
   if (op.windows) {
     if (op.windows->prepared) HG_CUDA(cudaEventRecord(op.windows->prepared, c->stream));
+    if (first && (rc = hg_narrow_verdict(c, &Qm, in_q ? nullptr : &Rm, &f->absmax, &f->outliers))) return rc;
     for (size_t k = 0; k < op.windows->win.size(); k++) {
       const DistWindow &w = op.windows->win[k];
       if ((rc = launch(w.r0, w.h, op.i0 + w.r0, op.ref_norm + w.r0, w.c0, w.w, op.j0 + w.c0, op.qry_norm + w.c0)) ||
@@ -938,7 +944,7 @@ static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, H
   }
   if (!hr) HG_PROF(c, 5);
   f->chunks = hr ? (uint32_t)chunks.size() : 0;
-  if (!narrow) return HG_OK;
+  if (!narrow || first) return HG_OK;
   if (defer) {  // the kernel itself honours the pre-pass's verdict (it does nothing when the rows are not narrow)
     c->pending_stats[0] = Qm.stats_all;
     c->pending_nsets[0] = Qm.n_sets;
@@ -1467,7 +1473,8 @@ extern "C" int hg_search_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
 // cluster: single-linkage ANI clusters of one sketch set (DESIGN.md §4.9)
 // ---------------------------------------------------------------------------------------
 
-// edge records one window may hold: 2^26 (1 GiB of hg_hit), or HG_CLUSTER_EDGE_CAP, read at every call (at least 256 x 256)
+// edge records one window of a cluster or derep run may hold: 2^26 (1 GiB of hg_hit), or HG_CLUSTER_EDGE_CAP, read at
+// every call (at least 256 x 256)
 static uint64_t cluster_edge_cap() {
   uint64_t cap = 0;
   if (const char *e = getenv("HG_CLUSTER_EDGE_CAP")) cap = strtoull(e, nullptr, 10);
@@ -1476,15 +1483,17 @@ static uint64_t cluster_edge_cap() {
 
 // The upper triangle of n rows, columns [c0, n), cut into windows of at most cap pairs j > i.  Column chunks [a, a + w)
 // of a multiple of 256 columns (the last one ends at n) run against refs [0, a + w), each chunk as wide as keeps its
-// a w + w (w - 1) / 2 pairs within cap; where even 256 columns have more, the refs of a 256-column chunk are split into
-// blocks of floor(cap / 256) rows rounded down to a multiple of 256.  So no window's hits can overflow the edge buffer.
-static std::vector<DistWindow> cluster_windows(uint32_t n, uint32_t c0, uint64_t cap) {
+// a w + w (w - 1) / 2 pairs within cap and w within max_w (a multiple of 256); where even 256 columns have more, the
+// refs of a 256-column chunk are split into blocks of floor(cap / 256) rows rounded down to a multiple of 256.  So no
+// window's hits can overflow the edge buffer.
+static std::vector<DistWindow> cluster_windows(uint32_t n, uint32_t c0, uint64_t cap, uint64_t max_w = UINT32_MAX) {
   std::vector<DistWindow> out;
   auto pairs = [](uint64_t a, uint64_t w) { return a * w + w * (w - 1) / 2; };
   for (uint32_t a = c0; a < n;) {
     uint32_t w = std::min<uint32_t>(256, n - a);
     if (pairs(a, w) <= cap) {
-      while (w < n - a && pairs(a, std::min<uint32_t>(w + 256, n - a)) <= cap) w = std::min<uint32_t>(w + 256, n - a);
+      while (w < n - a && (uint64_t)w + 256 <= max_w && pairs(a, std::min<uint32_t>(w + 256, n - a)) <= cap)
+        w = std::min<uint32_t>(w + 256, n - a);
       out.push_back({0, a + w, a, w});
     } else {
       const uint32_t h = (uint32_t)std::min<uint64_t>(cap / 256 / 256 * 256, a + w);
@@ -1674,5 +1683,231 @@ extern "C" int hg_cluster_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
   if (!c || !counts || !ms) { hg_set_error("hg_cluster_stats: NULL argument"); return HG_E_INVALID; }
   memcpy(counts, c->cluster_stats, sizeof(c->cluster_stats));
   memcpy(ms, c->cluster_ms, sizeof(c->cluster_ms));
+  return HG_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// derep: greedy ANI dereplication of one sketch set (DESIGN.md §4.10)
+// ---------------------------------------------------------------------------------------
+
+static void derep_stats_reset(hg_ctx *c) {
+  memset(c->derep_stats, 0, sizeof(c->derep_stats));
+  for (float &m : c->derep_ms) m = -1.0f;
+}
+
+// The state of a derep run, carved from HG_S_TILES (which neither the dist windows nor the internal search touch):
+// per row of the permuted space is_rep, the rep list (ascending), the order, the search's top-1 result and the labels;
+// the covered flags and adjacency bitmap of one column chunk; the rep count, a status word and the linked pairs.
+struct DerepState {
+  uint8_t *is_rep, *covered;
+  uint32_t *rep_list, *order, *n_found, *rep, *adj;
+  uint32_t *count;  // [0] representatives so far, [1] status
+  hg_hit *out;
+  unsigned long long *linked;
+};
+
+static int derep_state(hg_ctx *c, uint32_t n, DerepState *S) {
+  const size_t sizes[] = {(size_t)n, (size_t)HG_DEREP_CHUNK, (size_t)n * 4, (size_t)n * 4, (size_t)n * 4, (size_t)n * 4,
+                          (size_t)HG_DEREP_CHUNK * HG_DEREP_CHUNK / 8, 16, (size_t)n * sizeof(hg_hit), 8};
+  size_t off[10], total = 0;
+  for (int k = 0; k < 10; k++) {
+    off[k] = total;
+    total += (sizes[k] + 255) & ~(size_t)255;
+  }
+  void *p;
+  int rc;
+  if ((rc = hg_scratch(c, HG_S_TILES, total, &p))) return rc;
+  uint8_t *b = (uint8_t *)p;
+  *S = {b + off[0], b + off[1], (uint32_t *)(b + off[2]), (uint32_t *)(b + off[3]), (uint32_t *)(b + off[4]), (uint32_t *)(b + off[5]),
+        (uint32_t *)(b + off[6]), (uint32_t *)(b + off[7]), (hg_hit *)(b + off[8]), (unsigned long long *)(b + off[9])};
+  // the chunk state starts clear (each greedy step leaves it so), and the counters at 0
+  HG_CUDA(cudaMemsetAsync(S->covered, 0, HG_DEREP_CHUNK, c->stream));
+  HG_CUDA(cudaMemsetAsync(S->adj, 0, (size_t)HG_DEREP_CHUNK * HG_DEREP_CHUNK / 8, c->stream));
+  HG_CUDA(cudaMemsetAsync(S->count, 0, 16, c->stream));
+  HG_CUDA(cudaMemsetAsync(S->linked, 0, 8, c->stream));
+  return HG_OK;
+}
+
+// Greedy dereplication of rows [0, n) at ani_th in the priority order `order` (host; NULL: file order), in two phases.
+//   1. Representatives: the rows in priority order (gathered into HG_S_DEREP_ROWS when an order is given), the kernel
+//      chosen once and every row prepared once, then the upper triangle in the windows of cluster_windows with column
+//      chunks of at most HG_DEREP_CHUNK; behind each window a mark hook, behind a chunk's last window its greedy step.
+//      The single plane's verdict is read before the first window (DistWindows::decide_first): a greedy step marks
+//      every uncovered node of its chunk, so it must never run on the empty edges of a declined plane.
+//   2. Assignment: the representatives' rows gathered (ascending, so in priority order) into HG_S_DEREP_REPS, a top-1
+//      search of every row against them at ani_min = ani_th (ties to the smaller ref index: the first in the order),
+//      and the finalize kernel, which maps the labels back to file indices in d_rep.
+// hg_dist_last_path / reason report phase 1; hg_search_stats the search of phase 2 (zeros when every row is a
+// representative and no search runs).  bits: as dist_choose.  d_rep: the labels on the device (NULL: in the state);
+// rep (host, may be NULL) receives them.
+static int derep_run(hg_ctx *c, const int16_t *d_hv, const int32_t *d_norm, uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th,
+                     int path, uint32_t bits, const uint32_t *order, uint32_t *d_rep, uint32_t *rep, uint32_t *n_reps) {
+  derep_stats_reset(c);
+  memset(c->search_stats, 0, sizeof(c->search_stats));
+  c->search_ev_used = 0;
+  c->pending_stats[0] = c->pending_stats[1] = nullptr;
+  c->ev_used &= ~(3 << 4);
+  if (n == 0) {
+    if (n_reps) *n_reps = 0;
+    return HG_OK;
+  }
+  int rc;
+  DerepState S;
+  if ((rc = derep_state(c, n, &S))) return rc;
+  if (!d_rep) d_rep = S.rep;  // the packed entry: labels on the device before their copy to `rep`
+  const int16_t *W = d_hv;
+  const int32_t *Wn = d_norm;
+  ClusterEvents E;  // [0] start, [1] permuted, [2] rows prepared, per window before / after its hook, phase 2 start, end
+  DistWindows DW;
+  DW.win = cluster_windows(n, 0, cluster_edge_cap(), HG_DEREP_CHUNK);
+  DW.decide_first = true;
+  const size_t n_ev = 5 + 2 * DW.win.size();
+  if (c->prof) {
+    E.ev.resize(n_ev, nullptr);
+    for (cudaEvent_t &e : E.ev) HG_CUDA(cudaEventCreate(&e));
+    DW.prepared = E.ev[2];
+  }
+  auto mark = [&](size_t k) -> int {
+    if (c->prof) HG_CUDA(cudaEventRecord(E.ev[k], c->stream));
+    return HG_OK;
+  };
+  if ((rc = mark(0))) return rc;
+  if (order) {
+    const size_t mb = ((size_t)n * hv_d * 2 + 255) & ~(size_t)255;
+    void *d_w;
+    if ((rc = hg_scratch(c, HG_S_DEREP_ROWS, mb + (size_t)n * 4, &d_w))) return rc;
+    HG_CUDA(cudaMemcpyAsync(S.order, order, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
+    W = (const int16_t *)d_w;
+    Wn = (const int32_t *)((uint8_t *)d_w + mb);
+    if ((rc = hg_launch_derep_gather(c, d_hv, d_norm, S.order, n, hv_d, (int16_t *)W, (int32_t *)Wn))) return rc;
+  }
+  if ((rc = mark(1))) return rc;
+
+  // ---- phase 1: the representatives ----
+  DistChoice ch;
+  if ((rc = dist_choose(path, n, n, hg_tensor_shape_ok(hv_d, W, W) == HG_OK, bits, &ch))) return rc;
+  const uint64_t room = std::max<uint64_t>(1, std::min<uint64_t>(cluster_edge_cap(), (uint64_t)n * (n - 1) / 2));
+  void *d_edges, *d_cnt;
+  if ((rc = hg_scratch(c, HG_S_PACKED, room * sizeof(hg_hit), &d_edges))) return rc;
+  if ((rc = hg_scratch(c, HG_S_COUNTS, 256, &d_cnt))) return rc;
+  unsigned long long *cnt = (unsigned long long *)d_cnt;
+  HG_CUDA(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), c->stream));
+  DW.after = [&](size_t k) -> int {
+    const DistWindow &w = DW.win[k];
+    int r2;
+    if ((r2 = mark(3 + 2 * k)) ||
+        (r2 = hg_launch_derep_mark(c, (const hg_hit *)d_edges, cnt, room, w.c0, w.w, S.is_rep, S.covered, S.adj, S.linked)))
+      return r2;
+    HG_CUDA(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), c->stream));
+    const bool last = k + 1 == DW.win.size() || DW.win[k + 1].c0 != w.c0;  // the chunk's refs may span several windows
+    if (last && (r2 = hg_launch_derep_greedy(c, w.c0, w.w, S.covered, S.adj, S.is_rep, S.rep_list, S.count))) return r2;
+    return mark(4 + 2 * k);
+  };
+  DistOp op = {W, Wn, n, 0, W, Wn, n, 0, hv_d, ksize, ani_th, 1, (hg_hit *)d_edges, room, cnt};
+  op.windows = &DW;
+  if ((rc = dist_run(c, op, ch, nullptr, nullptr, false))) return rc;
+  const int p1_path = c->dist_path;
+  char p1_reason[sizeof(c->dist_reason)];
+  memcpy(p1_reason, c->dist_reason, sizeof(p1_reason));
+  uint32_t h_count[2] = {0, 0};
+  unsigned long long linked = 0;
+  HG_CUDA(cudaMemcpyAsync(h_count, S.count, 8, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaMemcpyAsync(&linked, S.linked, 8, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  const uint32_t k_reps = h_count[0];
+
+  // ---- phase 2: every other row to its closest representative ----
+  if ((rc = mark(n_ev - 2))) return rc;
+  if (k_reps < n) {  // (all rows representatives: nothing to assign)
+    const size_t rb = ((size_t)k_reps * hv_d * 2 + 255) & ~(size_t)255;
+    void *d_r;
+    if ((rc = hg_scratch(c, HG_S_DEREP_REPS, rb + (size_t)k_reps * 4, &d_r))) return rc;
+    int16_t *R = (int16_t *)d_r;
+    int32_t *Rn = (int32_t *)((uint8_t *)d_r + rb);
+    if ((rc = hg_launch_derep_gather(c, W, Wn, S.rep_list, k_reps, hv_d, R, Rn))) return rc;
+    rc = search_run(c, R, Rn, k_reps, W, Wn, n, hv_d, ksize, 1, ani_th, path, bits, S.out, S.n_found, nullptr);
+    hg_dist_record(c, p1_path, "%s", p1_reason);  // in auto mode a small rep set may have made the search pick SIMT
+    if (rc) return rc;
+  }
+  if ((rc = hg_launch_derep_finalize(c, S.is_rep, S.rep_list, S.out, S.n_found, order ? S.order : nullptr, n, d_rep, S.count + 1)) ||
+      (rc = mark(n_ev - 1)))
+    return rc;
+  HG_CUDA(cudaMemcpyAsync(h_count + 1, S.count + 1, 4, cudaMemcpyDeviceToHost, c->stream));
+  if (rep) HG_CUDA(cudaMemcpyAsync(rep, d_rep, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  if (h_count[1]) {
+    hg_set_error("hg_derep: internal error: a sketch that is not a representative matched none at ANI >= %g", (double)ani_th);
+    return HG_E_CUDA;
+  }
+  if (n_reps) *n_reps = k_reps;
+  uint64_t chunks = 0;
+  for (size_t k = 0; k < DW.win.size(); k++) chunks += k == 0 || DW.win[k].c0 != DW.win[k - 1].c0;
+  c->derep_stats[0] = chunks;
+  c->derep_stats[1] = DW.win.size();
+  c->derep_stats[2] = linked;
+  c->derep_stats[3] = k_reps;
+  if (c->prof) {
+    const int last = (int)(4 + 2 * (DW.win.size() - 1)), p2 = (int)n_ev - 2, end = (int)n_ev - 1;
+    const int prep_end = p1_path != HG_PATH_SIMT ? 2 : 1;  // the SIMT kernel prepares nothing
+    float hooks = 0.0f, t, windows;
+    for (size_t k = 0; k < DW.win.size(); k++) {
+      if ((rc = E.ms((int)(3 + 2 * k), (int)(4 + 2 * k), &t))) return rc;
+      hooks += t;
+    }
+    if ((rc = E.ms(0, prep_end, &c->derep_ms[0])) || (rc = E.ms(prep_end, last, &windows)) || (rc = E.ms(p2, end, &c->derep_ms[3])))
+      return rc;
+    c->derep_ms[1] = windows - hooks;
+    c->derep_ms[2] = hooks;
+  }
+  return HG_OK;
+}
+
+// order: NULL, or a permutation of [0, n) - checked whole before anything runs
+static int derep_order_check(const char *who, const uint32_t *order, uint32_t n) {
+  if (!order) return HG_OK;
+  std::vector<uint8_t> seen(n, 0);
+  for (uint32_t t = 0; t < n; t++) {
+    if (order[t] >= n) { hg_set_error("%s: order[%u] = %u is not below n = %u", who, t, order[t], n); return HG_E_INVALID; }
+    if (seen[order[t]]++) { hg_set_error("%s: order[%u] = %u repeats an earlier entry", who, t, order[t]); return HG_E_INVALID; }
+  }
+  return HG_OK;
+}
+
+extern "C" int hg_derep_dev(hg_ctx *c, const int16_t *d_hv, const int32_t *d_norm2, uint32_t n, uint32_t hv_d, uint32_t ksize,
+                            float ani_th, int path, const uint32_t *order, uint32_t *d_rep, uint32_t *n_reps) {
+  if (!c || (n && (!d_hv || !d_norm2))) { hg_set_error("hg_derep_dev: NULL argument"); return HG_E_INVALID; }
+  int rc;
+  if ((rc = hg_cluster_check("hg_derep_dev", n, d_rep, hv_d, ani_th, path)) || (rc = derep_order_check("hg_derep_dev", order, n)))
+    return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  return derep_run(c, d_hv, d_norm2, n, hv_d, ksize, ani_th, path, 0, order, d_rep, nullptr, n_reps);
+}
+
+extern "C" int hg_derep_packed(hg_ctx *c, const uint8_t *packed, uint64_t stride, const uint8_t *quant_bits, const int32_t *norm2,
+                               uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th, int path, const uint32_t *order, uint32_t *rep,
+                               uint32_t *n_reps) {
+  if (!c) { hg_set_error("hg_derep_packed: NULL argument"); return HG_E_INVALID; }
+  hg_packed_rows R = {packed, stride, quant_bits, norm2, n}, Q = R;
+  int rc;
+  if ((rc = hg_packed_args_check("hg_derep_packed", R, R, hv_d)) || (rc = hg_cluster_check("hg_derep_packed", n, rep, hv_d, ani_th, path)) ||
+      (rc = derep_order_check("hg_derep_packed", order, n)))
+    return rc;
+  if (n == 0) {
+    derep_stats_reset(c);
+    if (n_reps) *n_reps = 0;
+    return HG_OK;
+  }
+  bool same;
+  if ((rc = hg_packed_rows_check("hg_derep_packed", &R, &Q, hv_d, &same))) return rc;
+  HG_CUDA(cudaSetDevice(c->device));
+  HostRows hr, hq;
+  if ((rc = hg_packed_stage(c, R, R, true, hv_d, &hr, &hq)) || (rc = hg_rows_to_device(c, hr, hv_d))) return rc;
+  return derep_run(c, hr.d_hv, hr.d_norm, n, hv_d, ksize, ani_th, path, R.max_bits, order, nullptr, rep, n_reps);
+}
+
+extern "C" int hg_derep_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
+  if (!c || !counts || !ms) { hg_set_error("hg_derep_stats: NULL argument"); return HG_E_INVALID; }
+  memcpy(counts, c->derep_stats, sizeof(c->derep_stats));
+  memcpy(ms, c->derep_ms, sizeof(c->derep_ms));
   return HG_OK;
 }

@@ -154,8 +154,8 @@ struct hg_ctx {
   cudaStream_t stream;
   unsigned long long launches;
   // grow-only device scratch
-  void *d_scratch[14];        // indexed by hg_scratch_slot
-  size_t d_scratch_bytes[14];
+  void *d_scratch[16];        // indexed by hg_scratch_slot
+  size_t d_scratch_bytes[16];
   // pinned host scratch
   void *h_pinned[4];
   size_t h_pinned_bytes[4];
@@ -187,6 +187,10 @@ struct hg_ctx {
   // its steps (-1: not run or profiling off)
   uint64_t cluster_stats[4];
   float cluster_ms[4];
+  // the last derep run (hg_derep_stats): column chunks, windows, linked pairs, representatives; device ms of its
+  // phases (-1: not run or profiling off)
+  uint64_t derep_stats[4];
+  float derep_ms[4];
 };
 
 // stage boundaries: 0 start, 1 after staging/memsets, 2 after k-mer hash, 3 after encode,
@@ -214,10 +218,11 @@ enum hg_scratch_slot {
   HG_S_DESC = 1,       // hg_genome_desc[] (+ sentinels); search: the per-query floors
   HG_S_TABLES = 2,     // per-genome hash tables / explicit hash sets
   HG_S_COUNTS = 3,     // distinct-hash counters; dist: the hit counter of the host entry; cluster: the edge counter and
-                       // the run's linked-pair counts
+                       // the run's linked-pair counts; derep (phase 1): the same
   HG_S_HV = 4,         // int16 HVs (sketch output staging; dist: both matrices of the host entry)
   HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass;
-                       // group search: the members' results gathered on GPU 0; cluster: the edges of one window
+                       // group search: the members' results gathered on GPU 0; cluster, derep (phase 1): the edges of
+                       // one window
   HG_S_SMALL = 6,      // norms / bits / counts per sketch
   HG_S_MISC = 7,       // CTA -> genome map + round-1 tables, |hv| max, probe sink, status word of a search merge; cluster: status word
                        // of a union check, root count of a flatten
@@ -228,8 +233,13 @@ enum hg_scratch_slot {
   HG_S_SORT_CNT = 11,  // digit counters of the hit sort; search: per-query counts and offsets
   HG_S_NARROW_META = 12,  // per-row constants + outlier lists of the single-plane dist path (dist_narrow)
   HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entries;
-                          // cluster: the forest of the packed entry
-  HG_S_COUNT = 14
+                          // cluster: the forest of the packed entry; derep: its state (is_rep, rep list, order, the
+                          // search result, covered flags, bitmap, counters) and the labels of the packed entry
+  // derep: what the internal search (HG_S_SEQ, DESC, PACKED, COUNTS, SORT_*, MISC and the dist slots) and the packed
+  // staging (HV, SMALL, TABLES) leave alone
+  HG_S_DEREP_ROWS = 14,   // the working matrix in priority order, and its norms (when an order is given)
+  HG_S_DEREP_REPS = 15,   // the representatives' rows in priority order, and their norms: the refs of the search
+  HG_S_COUNT = 16
 };
 // scratch slot `slot` grown to at least `bytes` (contents not preserved)
 int hg_scratch(hg_ctx *ctx, int slot, size_t bytes, void **out);
@@ -497,3 +507,22 @@ int hg_cluster_packed_run(hg_ctx *ctx, const hg_packed_rows &R, uint32_t col0, u
 // NULL) the count; `flattened` (may be NULL) is recorded behind the flatten.  Returns with all of it complete.
 int hg_cluster_finish(hg_ctx *ctx, uint32_t *d_rep, uint32_t n, uint32_t *rep, uint32_t *n_clusters, cudaEvent_t flattened = nullptr);
 void hg_cluster_stats_reset(hg_ctx *ctx);
+
+// ---- greedy ANI dereplication (derep.cu, api.cu): DESIGN.md §4.10 ----
+// The widest column chunk of the representative phase: one greedy step per chunk, w x w bits of adjacency (128 KB)
+constexpr uint32_t HG_DEREP_CHUNK = 1024;
+// row t of d_dst (and its norm) = row d_idx[t] of d_src, for t < m (hv_d % 256 == 0)
+int hg_launch_derep_gather(hg_ctx *ctx, const int16_t *d_src, const int32_t *d_src_norm, const uint32_t *d_idx, uint32_t m,
+                           uint32_t hv_d, int16_t *d_dst, int32_t *d_dst_norm);
+// the first min(*d_count, cap) edges of a window of column chunk [a, a + w): covered[j - a] = 1 for an edge from an earlier
+// representative i < a; bit i - a of bitmap row j - a for i >= a.  d_linked (may be NULL) += that number of edges
+int hg_launch_derep_mark(hg_ctx *ctx, const hg_hit *d_edges, const unsigned long long *d_count, uint64_t cap, uint32_t a, uint32_t w,
+                         const uint8_t *d_is_rep, uint8_t *d_covered, uint32_t *d_adj, unsigned long long *d_linked);
+// the greedy step of chunk [a, a + w), w <= HG_DEREP_CHUNK, after its last window's marks: is_rep[a, a + w), the chunk's
+// representatives appended to d_rep_list (ascending) and counted in *d_n_reps; covered and the bitmap cleared
+int hg_launch_derep_greedy(hg_ctx *ctx, uint32_t a, uint32_t w, uint8_t *d_covered, uint32_t *d_adj, uint8_t *d_is_rep,
+                           uint32_t *d_rep_list, uint32_t *d_n_reps);
+// d_rep[order[t]] = order[t's representative] from is_rep, the rep list and a top-1 search result (d_out, d_n_found) of
+// every row against the rep matrix (d_order NULL: the identity); *d_status |= 1 if a non-representative found none
+int hg_launch_derep_finalize(hg_ctx *ctx, const uint8_t *d_is_rep, const uint32_t *d_rep_list, const hg_hit *d_out,
+                             const uint32_t *d_n_found, const uint32_t *d_order, uint32_t n, uint32_t *d_rep, uint32_t *d_status);

@@ -23,6 +23,7 @@ EXPORTS = [
     "hg_dist", "hg_dist_dev", "hg_dist_status", "hg_dist_last_path", "hg_dist_last_reason", "hg_sort_hits_dev", "hg_dist_sorted", "hg_dist_packed",
     "hg_search_dev", "hg_search_packed", "hg_search_stats", "hg_search_merge_dev",
     "hg_cluster_dev", "hg_cluster_packed", "hg_cluster_union_dev", "hg_cluster_stats",
+    "hg_derep_dev", "hg_derep_packed", "hg_derep_stats",
     "hg_group_create", "hg_group_destroy", "hg_group_size", "hg_group_ctx", "hg_group_sketch_fasta_batch", "hg_group_dist_packed",
     "hg_group_search_packed", "hg_group_cluster_packed",
     "hg_peer_window_need", "hg_peer_create", "hg_peer_connect", "hg_peer_create_local", "hg_peer_destroy", "hg_peer_rank",
@@ -115,6 +116,11 @@ def load() -> C.CDLL:
     L.hg_cluster_packed.argtypes = [vp, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, vp, C.POINTER(u32)]
     L.hg_cluster_union_dev.restype = i32; L.hg_cluster_union_dev.argtypes = [vp, u32, vp, vp, u64, C.POINTER(u32)]
     L.hg_cluster_stats.restype = i32; L.hg_cluster_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
+    L.hg_derep_dev.restype = i32
+    L.hg_derep_dev.argtypes = [vp, vp, vp, u32, u32, u32, C.c_float, i32, vp, vp, C.POINTER(u32)]
+    L.hg_derep_packed.restype = i32
+    L.hg_derep_packed.argtypes = [vp, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, vp, vp, C.POINTER(u32)]
+    L.hg_derep_stats.restype = i32; L.hg_derep_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
     L.hg_group_create.restype = i32; L.hg_group_create.argtypes = [i32, vp, C.POINTER(vp)]
     L.hg_group_destroy.restype = None; L.hg_group_destroy.argtypes = [vp]
     L.hg_group_size.restype = i32; L.hg_group_size.argtypes = [vp]
@@ -244,6 +250,16 @@ def _cluster_stats(ctx_handle):
     counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
     _check(load().hg_cluster_stats(ctx_handle, counts, ms))
     return [int(x) for x in counts], [float(x) for x in ms]
+
+
+def _order(order, n):
+    """a priority order as the hg_derep_* entries take it: None, or n uint32 entries (kept alive by the caller)"""
+    if order is None:
+        return None
+    order = np.ascontiguousarray(order, np.uint32)
+    if order.shape != (n,):
+        raise ValueError("order must have one entry per sketch (%d), got shape %s" % (n, order.shape))
+    return order
 
 
 class Context:
@@ -493,6 +509,33 @@ class Context:
         """hg_cluster_stats of the last cluster run -> ([windows, linked pairs, largest window's pairs, edge capacity],
         [ms of preparing the rows, dist windows, hooks, flatten + count] (-1: not run or profiling off))"""
         return _cluster_stats(self._h)
+
+    def derep_dev(self, d_hv, d_norm2, n, hv_d, ksize, ani_th, path, d_rep, order=None) -> int:
+        """hg_derep_dev: device pointers (ints); d_rep receives rep[i] = the index of i's representative; order (host
+        array of n entries, or None for file order) is the priority.  Returns the number of representatives once the
+        result is complete."""
+        o = _order(order, n)
+        n_reps = C.c_uint32(0)
+        _check(load().hg_derep_dev(self._h, d_hv, d_norm2, n, hv_d, ksize, ani_th, path, _ptr(o), d_rep,
+                                   C.byref(n_reps)))
+        return int(n_reps.value)
+
+    def derep_packed(self, packed, bits, norm2, hv_d, ksize=21, ani_th=95.0, path=0, order=None):
+        """hg_derep_packed: packed sketch rows (n x stride uint8) + quant bits + norms -> (rep[n], n_reps)"""
+        p, b, nm = _packed_rows(packed, bits, norm2, packed, bits, norm2)[0]
+        o = _order(order, p.shape[0])
+        rep = np.zeros(p.shape[0], np.uint32)
+        n_reps = C.c_uint32(0)
+        _check(load().hg_derep_packed(self._h, *_row_args((p, b, nm)), hv_d, ksize, ani_th, path, _ptr(o),
+                                      _ptr(rep), C.byref(n_reps)))
+        return rep, int(n_reps.value)
+
+    def derep_stats(self):
+        """hg_derep_stats of the last derep run -> ([column chunks, windows, linked pairs, representatives], [ms of
+        preparing the rows, dist windows, mark hooks + greedy steps, assignment] (-1: not run or profiling off))"""
+        counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
+        _check(load().hg_derep_stats(self._h, counts, ms))
+        return [int(x) for x in counts], [float(x) for x in ms]
 
     def sort_hits_dev(self, d_hits, n, d_ani_milli=None):
         """hg_sort_hits_dev: device records to the reference's output order, in place."""

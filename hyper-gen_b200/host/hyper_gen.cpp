@@ -20,6 +20,10 @@
 //       single-linkage clusters at ANI >= -a, one `representative\tmember` line per sketch: clusters by ascending
 //       representative (the smallest index of the cluster), members ascending, the representative's own line first.
 //       The pairs are split over every visible GPU (hg_group_cluster_packed); HG_GPUS=n limits it.
+//   hyper-gen derep -r <sketch> -o <out> [-a 95.0] [-O file|size]
+//       greedy dereplication at ANI >= -a: representatives taken in priority order (-O file: file order; -O size:
+//       descending hv_norm_2, ties by file index), every other sketch with its closest representative; the lines of
+//       `cluster`, each cluster's representative line first.  On one GPU (hg_derep_packed).
 // The GPU path is the only path (`-D gpu` is implied): there is no CPU fallback.
 #include <algorithm>
 #include <chrono>
@@ -32,6 +36,7 @@
 #include <string>
 #include <functional>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "../../include/hypergen_b200.h"
@@ -73,6 +78,12 @@ struct SketchSearch {
 struct SketchCluster {
   std::string path_sketch, out_file;
   float ani_th = 95.0f;
+};
+
+struct SketchDerep {
+  std::string path_sketch, out_file;
+  float ani_th = 95.0f;
+  std::string order = "file";
 };
 
 }  // namespace types
@@ -408,6 +419,23 @@ void search(const types::SketchSearch &ss) {
 
 namespace cluster {
 
+// One `representative\tmember` line per sketch: clusters by ascending representative, the representative's own line
+// first, then the members ascending - the key (rep, t != rep, t).
+void write_lines(const std::vector<types::FileSketch> &sk, const std::vector<uint32_t> &rep, const std::string &out_file) {
+  std::vector<uint32_t> order(rep.size());
+  for (size_t t = 0; t < rep.size(); t++) order[t] = (uint32_t)t;
+  std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
+    return std::make_tuple(rep[a], a != rep[a], a) < std::make_tuple(rep[b], b != rep[b], b);
+  });
+  std::string out;
+  for (uint32_t t : order) {
+    out += sk[rep[t]].file_str; out += '\t'; out += sk[t].file_str; out += '\n';
+  }
+  std::ofstream f(out_file, std::ios::binary);
+  if (!f) die("Dump cluster file failed!");
+  f.write(out.data(), (std::streamsize)out.size());
+}
+
 void cluster(const types::SketchCluster &sc) {
   auto sk = utils::load_sketch(sc.path_sketch);
   if (sk.empty()) die("empty sketch file");
@@ -420,35 +448,59 @@ void cluster(const types::SketchCluster &sc) {
                                 sc.ani_th, 0, rep.data(), &n_clusters),
         "hg_group_cluster_packed");
   hg_group_destroy(group);
-  std::vector<uint32_t> order(n);
-  for (size_t t = 0; t < n; t++) order[t] = (uint32_t)t;
-  std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return rep[a] < rep[b]; });
-  std::string out;
-  for (uint32_t t : order) {
-    out += sk[rep[t]].file_str; out += '\t'; out += sk[t].file_str; out += '\n';
-  }
-  std::ofstream f(sc.out_file, std::ios::binary);
-  if (!f) die("Dump cluster file failed!");
-  f.write(out.data(), (std::streamsize)out.size());
+  write_lines(sk, rep, sc.out_file);
   fprintf(stdout, "Output %zu sketches in %u clusters (ANI >= %.1f) to file %s\n", n, n_clusters, (double)sc.ani_th,
           sc.out_file.c_str());
 }
 
 }  // namespace cluster
 
+namespace derep {
+
+void derep(const types::SketchDerep &sd) {
+  auto sk = utils::load_sketch(sd.path_sketch);
+  if (sk.empty()) die("empty sketch file");
+  const size_t D = sk[0].hv_d, n = sk.size();
+  const dist::Stacked s = dist::stack(sk, D);
+  std::vector<uint32_t> order;  // empty: file order
+  if (sd.order == "size") {  // descending hv_norm_2 (about hv_d times the sampled hashes: larger genomes first)
+    order.resize(n);
+    for (size_t t = 0; t < n; t++) order[t] = (uint32_t)t;
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return s.norm[a] > s.norm[b]; });
+  }
+  hg_ctx *ctx = nullptr;
+  check(hg_init(0, &ctx), "hg_init");
+  std::vector<uint32_t> rep(n);
+  uint32_t n_reps = 0;
+  check(hg_derep_packed(ctx, s.packed.data(), 2 * D, s.bits.data(), s.norm.data(), (uint32_t)n, (uint32_t)D, sk[0].ksize, sd.ani_th, 0,
+                        order.empty() ? nullptr : order.data(), rep.data(), &n_reps),
+        "hg_derep_packed");
+  hg_destroy(ctx);
+  cluster::write_lines(sk, rep, sd.out_file);
+  fprintf(stdout, "Output %zu sketches in %u clusters (greedy, ANI >= %.1f) to file %s\n", n, n_reps, (double)sd.ani_th,
+          sd.out_file.c_str());
+}
+
+}  // namespace derep
+
 int main(int argc, char **argv) {
-  if (argc < 2) die("usage: hyper-gen <sketch|dist|search|cluster> ...");
+  if (argc < 2) die("usage: hyper-gen <sketch|dist|search|cluster|derep> ...");
   const std::string mode = argv[1];
   types::SketchParams sp;
   types::SketchDist sd;
   types::SketchSearch ss;
   types::SketchCluster sc;
+  types::SketchDerep sr;
   bool ani_given = false;
   for (int i = 2; i + 1 < argc; i += 2) {
     const std::string k = argv[i], v = argv[i + 1];
     if (k == "-p" || k == "--path") sp.path = v;
-    else if (k == "-o" || k == "--out") { sp.out_file = v; sd.out_file = v; ss.out_file = v; sc.out_file = v; }
-    else if (k == "-r" || k == "--path_r") { sd.path_ref_sketch = v; ss.path_ref_sketch = v; sc.path_sketch = v; }
+    else if (k == "-o" || k == "--out") { sp.out_file = v; sd.out_file = v; ss.out_file = v; sc.out_file = v; sr.out_file = v; }
+    else if (k == "-r" || k == "--path_r") { sd.path_ref_sketch = v; ss.path_ref_sketch = v; sc.path_sketch = v; sr.path_sketch = v; }
+    else if (k == "-O" || k == "--order") {
+      if (v != "file" && v != "size") die("-O must be file or size");
+      sr.order = v;
+    }
     else if (k == "-q" || k == "--path_q") { sd.path_query_sketch = v; ss.path_query_sketch = v; }
     else if (k == "-n" || k == "--top_k") {
       const long n = atol(v.c_str());
@@ -479,6 +531,10 @@ int main(int argc, char **argv) {
     if (sc.path_sketch.empty() || sc.out_file.empty()) die("cluster needs -r -o");
     if (ani_given) sc.ani_th = sd.ani_threshold;
     cluster::cluster(sc);
+  } else if (mode == "derep") {
+    if (sr.path_sketch.empty() || sr.out_file.empty()) die("derep needs -r -o");
+    if (ani_given) sr.ani_th = sd.ani_threshold;
+    derep::derep(sr);
   } else {
     die("unknown subcommand " + mode);
   }

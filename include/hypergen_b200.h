@@ -436,6 +436,36 @@ HG_API int hg_cluster_union_dev(hg_ctx *ctx, uint32_t n, uint32_t *d_rep, const 
  * is off, see hg_set_profiling). */
 HG_API int hg_cluster_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
 
+/* ---- greedy ANI dereplication: one representative per group, every other sketch assigned to one -----------------
+ * Over one sketch set of n rows at ani_th, in the priority order `order` (host, n entries, a permutation of [0, n);
+ * NULL: file order, order[t] = t).  Every ANI is the exact value hg_dist computes.
+ *   1. Sketch order[t] is a representative iff no earlier representative order[s] (s < t) has
+ *      ani(order[s], order[t]) >= ani_th.
+ *   2. A representative's rep is itself.  Any other sketch g goes to the representative r with the largest ani(r, g)
+ *      among those with ani(r, g) >= ani_th (never empty: the one that excluded g is there); ties go to the
+ *      representative first in `order`.  It may come before or after g in the order.
+ * rep[i] = the index of sketch i's representative (rep[r] == r exactly for representatives); *n_reps (host, may be
+ * NULL) = the number of representatives.  The result does not depend on the kernel, the window plan or the thread
+ * schedule.  n == 0: HG_OK with n_reps = 0; ani_th <= 0: order[0] is the only representative; a sketch with norm 0 is
+ * its own representative when ani_th > 0.  A NaN ani_th, or an order with an index >= n or a repeat, is HG_E_INVALID
+ * before anything runs; HG_E_CUDA with "internal error" if a non-representative matched no representative.
+ *   path   as hg_cluster_dev; hg_dist_last_path / hg_dist_last_reason report the representative phase, and
+ *          hg_search_stats the top-1 search of the assignment phase (zeros when every sketch is a representative).
+ * On one GPU: the representatives come from the dist windows of hg_cluster_dev (at most HG_CLUSTER_EDGE_CAP pairs
+ * each, and at most 1024 columns) with a greedy step on the device behind each column chunk; then one top-1 search of
+ * every sketch against the representatives (DESIGN.md §4.10).  Every entry returns with its result complete. */
+HG_API int hg_derep_dev(hg_ctx *ctx, const int16_t *d_hv, const int32_t *d_norm2, uint32_t n, uint32_t hv_d, uint32_t ksize,
+                        float ani_th, int path, const uint32_t *order /* host, n entries, may be NULL */,
+                        uint32_t *d_rep, uint32_t *n_reps /* host, may be NULL */);
+/* The same from the rows as the sketch file holds them (as hg_cluster_packed); rep in host memory. */
+HG_API int hg_derep_packed(hg_ctx *ctx, const uint8_t *packed, uint64_t stride, const uint8_t *quant_bits, const int32_t *norm2,
+                           uint32_t n, uint32_t hv_d, uint32_t ksize, float ani_th, int path, const uint32_t *order,
+                           uint32_t *rep, uint32_t *n_reps /* may be NULL */);
+/* Measurement hook of the last derep run: counts = {column chunks, windows, linked pairs, representatives};
+ * ms = device time of {preparing the rows (the permutation included), the dist windows, the mark hooks + greedy
+ * steps, the assignment (gather + search + finalize)} (-1 where not run or profiling is off, see hg_set_profiling). */
+HG_API int hg_derep_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
+
 /* Which path the last hg_dist / hg_dist_dev took (1 SIMT, 2 two-limb tensor, 3 single-plane tensor) and why. */
 HG_API int hg_dist_last_path(hg_ctx *ctx);
 HG_API const char *hg_dist_last_reason(hg_ctx *ctx);

@@ -53,6 +53,14 @@ extern "C" {
         n_clusters: *mut u32) -> c_int;
     // counts = {windows, linked pairs, largest window's pairs, edge capacity}; ms of its steps (-1: not run / not profiled)
     pub fn hg_cluster_stats(ctx: *mut hg_ctx, counts: *mut u64, ms: *mut f32) -> c_int;
+    // greedy ANI dereplication: representatives in priority order (order: n entries, or null for file order), every
+    // other sketch with its closest representative; rep[i] = the index of i's representative
+    pub fn hg_derep_dev(ctx: *mut hg_ctx, d_hv: *const i16, d_norm2: *const i32, n: u32, hv_d: u32, ksize: u32, ani_th: f32,
+        path: c_int, order: *const u32, d_rep: *mut u32, n_reps: *mut u32) -> c_int;
+    pub fn hg_derep_packed(ctx: *mut hg_ctx, packed: *const u8, stride: u64, quant_bits: *const u8, norm2: *const i32, n: u32,
+        hv_d: u32, ksize: u32, ani_th: f32, path: c_int, order: *const u32, rep: *mut u32, n_reps: *mut u32) -> c_int;
+    // counts = {column chunks, windows, linked pairs, representatives}; ms of its phases (-1: not run / not profiled)
+    pub fn hg_derep_stats(ctx: *mut hg_ctx, counts: *mut u64, ms: *mut f32) -> c_int;
 }
 
 /// status -> panic with the library's message, the reference's error style (`unwrap()`, Cargo.toml:67-70)
