@@ -1030,6 +1030,19 @@ extern "C" int hg_dist_dev(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref
   return dist_run(c, op, ch, nullptr, nullptr, path == HG_PATH_NARROW);
 }
 
+extern "C" int hg_dist_norm_flags(hg_ctx *c, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int path, uint32_t *d_flags) {
+  if (!c || (n_rows && (!d_hv || !d_flags))) { hg_set_error("hg_dist_norm_flags: NULL argument"); return HG_E_INVALID; }
+  if (path != HG_PATH_TWO_LIMB && path != HG_PATH_NARROW) { hg_set_error("hg_dist_norm_flags: path %d (2 or 3)", path); return HG_E_INVALID; }
+  HG_CUDA(cudaSetDevice(c->device));
+  if (n_rows == 0) return HG_OK;
+  int rc;
+  if ((rc = hg_tensor_shape_ok(hv_d, d_hv, d_hv))) return rc;
+  rc = path == HG_PATH_NARROW ? hg_narrow_norm_flags(c, d_hv, n_rows, hv_d, d_flags) : hg_tc_norm_flags(c, d_hv, n_rows, hv_d, d_flags);
+  if (rc) return rc;
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  return HG_OK;
+}
+
 // After hg_dist_dev(path = 3): the pre-pass verdict that call did not wait for.
 extern "C" int hg_dist_status(hg_ctx *c) {
   if (!c) { hg_set_error("ctx is NULL"); return HG_E_INVALID; }

@@ -15,7 +15,7 @@ struct DistEpilogue {
   uint32_t i0, j0;  // global index offsets of this shard
   float ksize_f;
   float ani_th;
-  float jmin;  // conservative Jaccard pre-filter (0 = off): pairs below it cannot reach ani_th
+  float jmin;  // conservative Jaccard pre-filter (0 = off): pairs below it (and above -1) cannot reach ani_th
   float cfrac; // jmin / (1 + jmin): dot >= cfrac * (norm_r + norm_q) is the same bound, division-free
   int symmetric;
   hg_hit *__restrict__ hits;
@@ -44,7 +44,8 @@ __device__ __forceinline__ void dist_emit(const DistEpilogue &e, bool live, uint
       bool cand = true;
       if (jmin > 0.0f) {  // cheap monotone bound first; the exact f32 sequence decides
         const int32_t den = (int32_t)((uint32_t)nr + (uint32_t)nq - (uint32_t)dot);
-        cand = den <= 0 || __int2float_rn(dot) >= jmin * __int2float_rn(den);
+        const float fd = __int2float_rn(dot), fn = __int2float_rn(den);
+        cand = den <= 0 || fd >= jmin * fn || fd <= -fn;  // the last: J <= -1, ANI 100 (DESIGN.md, dist epilogue)
       }
       if (cand) {
         ani = ani_from_dot(dot, nr, nq, e.ksize_f);
@@ -84,7 +85,8 @@ __device__ __forceinline__ bool dist_eval(const DistEpilogue &e, bool live, uint
   if constexpr (QF) { const hg_floor f = fl.q[lj]; th = f.ani; jmin = f.jmin; imax = f.imax; }
   if (jmin > 0.0f) {
     const int32_t den = (int32_t)((uint32_t)nr + (uint32_t)nq - (uint32_t)dot);
-    if (!(den <= 0 || __int2float_rn(dot) >= jmin * __int2float_rn(den))) return false;
+    const float fd = __int2float_rn(dot), fn = __int2float_rn(den);
+    if (!(den <= 0 || fd >= jmin * fn || fd <= -fn)) return false;
   }
   const float ani = ani_from_dot(dot, nr, nq, e.ksize_f);
   *ani_out = ani;

@@ -62,7 +62,7 @@ constexpr int32_t COL_NEVER = INT32_MAX;       // column past the last query
 struct NarrowSide {  // per-row constants of one matrix, already offset to the first row of the launch
   const int32_t *s;         // centre
   const int32_t *a2;        // 2 * sum_d a[d]
-  const uint32_t *e;        // sum_d |eps[d]|  (0: the row is exactly 2 a + s)
+  const uint32_t *e;        // sum_d |eps[d]|  (0: the row is exactly 2 a + s; E_ALWAYS: its true norm reaches HG_NORM_WRAP_CUT)
   const uint32_t *out_off;  // first outlier entry
   const uint32_t *out_cnt;
 };
@@ -107,11 +107,15 @@ __device__ __forceinline__ uint32_t warp_sum(uint32_t v) {
   return v;
 }
 
+// e of a row whose true norm sum x^2 reaches HG_NORM_WRAP_CUT: its i32 norm, dots and denominators may wrap, so the
+// row / column bound is off (n1_loosen) and every pair with it takes the exact path
+constexpr uint32_t E_ALWAYS = 0xFFFFFFFFu;
+
 constexpr int PREP_THREADS = 256;  // 8 warps, one row per warp
 
 // One warp per row, no block-level synchronisation, two int16 per instruction (VIMNMX.S16x2, VIADD.16x2,
 // IDP.2A).  Pass 1: range, sum, parity count.  Pass 2 re-reads the row (L1/L2): plane, 2 sum(a), residual
-// statistics.  Pass 3, rows with outliers only: their entries.  Four 16-byte loads in flight per lane and 48
+// statistics, and the row's true norm sum x^2 from sum a^2 (IDP.4A on the plane bytes) and the residuals.  Pass 3, rows with outliers only: their entries.  Four 16-byte loads in flight per lane and 48
 // warps per SM measured best (4.6 TB/s of HBM traffic on the 820 MB config-4 matrix); keeping the row in
 // registers between the passes (116 registers, 16 warps per SM) was 8 % slower there and equal on config 3.
 constexpr int PF = 4;
@@ -166,7 +170,7 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
   // pass 2
   const uint32_t ns2 = (uint32_t)(-s & 0xFFFF) * 0x00010001u;  // -s in both halves
   uint32_t cnt = 0, sum_e = 0;
-  int sum_2a = 0;
+  int sum_2a = 0, sum_aa = 0;  // sum a^2 <= 32768 * 128^2 = 2^29
   uint2 *dst = reinterpret_cast<uint2 *>(o.plane + (size_t)row * hv_d) + lane;
   auto pass2 = [&](const uint4 &v, uint2 *out) {
     const uint32_t w[4] = {v.x, v.y, v.z, v.w};
@@ -186,7 +190,9 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
         }
       }
     }
-    *out = make_uint2(__byte_perm(r[0], r[1], 0x6420), __byte_perm(r[2], r[3], 0x6420));
+    const uint2 a8 = make_uint2(__byte_perm(r[0], r[1], 0x6420), __byte_perm(r[2], r[3], 0x6420));
+    sum_aa = __dp4a((int)a8.x, (int)a8.x, __dp4a((int)a8.y, (int)a8.y, sum_aa));  // signed bytes: IDP.4A.S8.S8
+    *out = a8;
   };
   for (uint32_t t0 = 0; t0 < nt; t0 += PF) {
     uint4 v[PF];
@@ -205,7 +211,10 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
     if (lane >= (uint32_t)d) inc += y;
   }
   const uint32_t tot_c = __shfl_sync(0xffffffffu, inc, 31);
-  const uint32_t tot_2a = warp_sum((uint32_t)sum_2a), tot_e = warp_sum(sum_e);
+  const uint32_t tot_2a = warp_sum((uint32_t)sum_2a), tot_e = warp_sum(sum_e), tot_aa = warp_sum((uint32_t)sum_aa);
+  // the row's true norm: sum x^2 = sum x~^2 + sum (x^2 - x~^2), sum x~^2 = 4 sum a^2 + 2 s sum 2a + D s^2; the second
+  // term (residuals only) is added in pass 3, before the row's `e` is written
+  long long xx = 4ll * tot_aa + 2ll * s * (int32_t)tot_2a + (long long)hv_d * s * s;
   uint32_t base = 0, kept = tot_c;
   if (lane == 0) {
     if (bad) { atomicExch(&o.stats[3], 1u); kept = 0; }
@@ -215,7 +224,7 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
     }
     o.s[row] = s;
     o.a2[row] = (int32_t)tot_2a;
-    o.e[row] = tot_e;
+    if (!kept) o.e[row] = xx >= (long long)HG_NORM_WRAP_CUT ? E_ALWAYS : tot_e;  // no residuals (or declined)
     o.out_off[row] = base;
     o.out_cnt[row] = kept;
     const uint32_t am = (uint32_t)max(abs(lo), abs(hi)), tm = (uint32_t)abs(s) + 256u;
@@ -227,6 +236,7 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
   if (kept == 0) return;
   // pass 3 (rows with outliers only): write the entries, lane by lane in scan order
   uint32_t pos = base + inc - cnt;
+  long long d_xx = 0;
   for (uint32_t t = 0; t < nt; ++t) {
     const uint4 v = __ldg(src + 32 * t);
     const uint32_t w[4] = {v.x, v.y, v.z, v.w};
@@ -235,9 +245,15 @@ narrow_prep_kernel(const int16_t *__restrict__ hv, uint32_t n_rows, uint32_t hv_
       const int tt = (int)(int16_t)(w[e >> 1] >> (16 * (e & 1))) - s;
       const int a = max(-128, min(127, tt >> 1));
       const int eps = tt - 2 * a;
-      if (eps != 0) o.entries[pos++] = ((8u * (lane + 32 * t) + (uint32_t)e) << 16) | ((uint32_t)eps & 0xFFFFu);
+      if (eps != 0) {
+        o.entries[pos++] = ((8u * (lane + 32 * t) + (uint32_t)e) << 16) | ((uint32_t)eps & 0xFFFFu);
+        d_xx += (long long)eps * (tt + 2 * a + 2 * s);  // x^2 - x~^2 = eps (x + x~)
+      }
     }
   }
+#pragma unroll
+  for (int m = 16; m; m >>= 1) d_xx += __shfl_xor_sync(0xffffffffu, d_xx, m);
+  if (lane == 0) o.e[row] = xx + d_xx >= (long long)HG_NORM_WRAP_CUT ? E_ALWAYS : tot_e;
 }
 
 // ---- tile walk: non-empty 256 x 256 tiles, row-block major ------------------------------------------
@@ -287,8 +303,9 @@ struct N1Tiles {
   }
 };
 
-// bound of a row / column lowered by the largest correction its outliers can contribute
+// bound of a row / column lowered by the largest correction its outliers can contribute (off for an E_ALWAYS row)
 __device__ __forceinline__ int32_t n1_loosen(int32_t t, uint32_t e, uint32_t m, int32_t always) {
+  if (e == E_ALWAYS) return always;
   if (t == always || e == 0) return t;
   const uint64_t M = (uint64_t)e * m;
   if (M > (1ull << 29)) return always;
@@ -336,7 +353,8 @@ __device__ __forceinline__ void n1_process(const hg::DistEpilogue &ep, const hg_
     int32_t dot = (int32_t)c.y;
     if (live) {
       const uint32_t er = na.r.e[li], eq = na.q.e[lj];
-      if (er | eq) dot = (int32_t)((uint32_t)dot + (uint32_t)n1_correction(na, li, lj, er, eq));
+      // (e alone does not say there are entries: an E_ALWAYS row may have none)
+      if ((er | eq) && (na.r.out_cnt[li] | na.q.out_cnt[lj])) dot = (int32_t)((uint32_t)dot + (uint32_t)n1_correction(na, li, lj, er, eq));
     }
     float ani = 0.0f;
     const bool keep = hg::dist_eval<QF>(ep, live, li, lj, dot, &ani, fl);
@@ -677,6 +695,11 @@ __global__ void narrow_stats_init_kernel(uint32_t *stats, uint32_t entry_base) {
   if (threadIdx.x < 4) stats[threadIdx.x] = threadIdx.x == 2 ? entry_base : 0u;
 }
 
+__global__ void narrow_flags_kernel(const uint32_t *__restrict__ e, uint32_t n, uint32_t *__restrict__ flags) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) flags[i] = e[i] == E_ALWAYS;
+}
+
 uint32_t narrow_budget() {  // outlier entries per row on average (HG_NARROW_BUDGET overrides; tests use it to force the correction path)
   uint32_t per_row = 4;
   if (const char *e = getenv("HG_NARROW_BUDGET")) per_row = (uint32_t)std::max(0, atoi(e));
@@ -848,6 +871,21 @@ int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32
   ctx->launches++;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
+}
+
+// flags[i] = 1 if the pre-pass marks row i E_ALWAYS (its true norm reaches HG_NORM_WRAP_CUT); HG_E_UNSUPPORTED if the
+// pre-pass declines the rows (synchronises the stream)
+int hg_narrow_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, uint32_t *d_flags) {
+  void *meta;
+  int rc;
+  hg_narrow_mat m;
+  if ((rc = hg_scratch(ctx, HG_S_NARROW_META, hg_narrow_meta_bytes(n_rows), &meta))) return rc;
+  if ((rc = hg_narrow_setup(ctx, d_hv, n_rows, hv_d, HG_S_QRY_LIMBS, meta, &m))) return rc;
+  if ((rc = hg_narrow_prep_rows(ctx, &m, 0, n_rows))) return rc;
+  narrow_flags_kernel<<<(n_rows + 255) / 256, 256, 0, ctx->stream>>>(m.e, n_rows, d_flags);
+  ctx->launches++;
+  HG_CUDA(cudaGetLastError());
+  return hg_narrow_verdict(ctx, &m, nullptr, nullptr, nullptr);
 }
 
 // Reads the pre-pass statistics (synchronises the stream): HG_OK if every row prepared so far fits the single

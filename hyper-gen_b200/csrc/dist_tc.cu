@@ -47,20 +47,21 @@ constexpr uint32_t TC_TMEM_COLS = 512;
 // and the compacted append.
 
 // per-column bound of query column lj (INT32_MIN = always take the exact path).  QF (a search pass): the column's own
-// cfrac, and the launch's smallest positive one for the rows (hg_floors).
+// cfrac, and the launch's smallest positive one for the rows (hg_floors).  The bound holds only while nothing of the
+// pair wraps i32: a row whose true norm (qry_sq / ref_sq, 64 bits) reaches HG_NORM_WRAP_CUT is always a candidate.
 template <bool QF>
-__device__ __forceinline__ int32_t tc_col_bound(const hg::DistEpilogue &ep, const hg_floors &fl, uint32_t lj) {
+__device__ __forceinline__ int32_t tc_col_bound(const hg::DistEpilogue &ep, const hg_floors &fl, const unsigned long long *qry_sq, uint32_t lj) {
   float cfrac = ep.cfrac;
   if constexpr (QF) cfrac = lj < ep.n_qry ? fl.q[lj].cfrac : 0.0f;
-  if (!(cfrac > 0.0f) || lj >= ep.n_qry) return INT32_MIN;
+  if (!(cfrac > 0.0f) || lj >= ep.n_qry || qry_sq[lj] >= HG_NORM_WRAP_CUT) return INT32_MIN;
   const int32_t nq = ep.qry_norm[lj];
   return nq > 0 ? __float2int_rd(cfrac * __int2float_rz(nq)) - 1 : INT32_MIN;
 }
 template <bool QF>
-__device__ __forceinline__ int32_t tc_row_bound(const hg::DistEpilogue &ep, const hg_floors &fl, uint32_t li) {
+__device__ __forceinline__ int32_t tc_row_bound(const hg::DistEpilogue &ep, const hg_floors &fl, const unsigned long long *ref_sq, uint32_t li) {
   float cfrac = ep.cfrac;
   if constexpr (QF) cfrac = *fl.cfrac_row;
-  if (!(cfrac > 0.0f) || li >= ep.n_ref) return INT32_MIN / 2;
+  if (!(cfrac > 0.0f) || li >= ep.n_ref || ref_sq[li] >= HG_NORM_WRAP_CUT) return INT32_MIN / 2;
   const int32_t nr = ep.ref_norm[li];
   return nr > 0 ? __float2int_rd(cfrac * __int2float_rz(nr)) - 1 : INT32_MIN / 2;
 }
@@ -253,8 +254,8 @@ template <int PUSHW, bool QF = false>
 __global__ void __launch_bounds__(TC_THREADS + 32 * PUSHW, 1)
 dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
                 uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len,
-                hg::DistEpilogue ep, uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan,
-                hg_floors fl) {
+                hg::DistEpilogue ep, const unsigned long long *__restrict__ ref_sq, const unsigned long long *__restrict__ qry_sq,
+                uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan, hg_floors fl) {
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
   if (feed.seq_ptr) feed.seq = *feed.seq_ptr;
@@ -403,9 +404,9 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
       int32_t tr = 0;
       auto bounds = [&]() {
         const int t = threadIdx.x - 64;
-        if (t < TC_BN) s_tq[t] = tc_col_bound<QF>(ep, fl, col0 + t);
+        if (t < TC_BN) s_tq[t] = tc_col_bound<QF>(ep, fl, qry_sq, col0 + t);
         asm volatile("bar.sync 1, %0;" ::"r"(32 * TC_EPI_WARPS) : "memory");
-        tr = tc_row_bound<QF>(ep, fl, li);
+        tr = tc_row_bound<QF>(ep, fl, ref_sq, li);
       };
       if (early) bounds();
       // my 128 x 128 part of the tile may be empty (below the diagonal, or past the last ref row)
@@ -436,15 +437,24 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
   }
 }
 
-// i16 -> two s8 limb planes: out[0][r][d] = h, out[1][r][d] = l  (plane stride = rows * hv_d)
 // i16 -> two s8 limb planes: plane 0 = h, plane 1 = l, `plane_stride` bytes apart; `out` points at the first element
-// of plane 0 that belongs to `hv`
-__global__ void split_limbs_kernel(const int16_t *__restrict__ hv, uint64_t n_elems, int8_t *__restrict__ out, uint64_t plane_stride) {
-  const uint64_t n8 = n_elems / 8;
-  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (uint64_t)gridDim.x * blockDim.x) {
+// of plane 0 that belongs to `hv`.  Also adds every row's sum x^2 into sq[row] (zeroed before): 16 consecutive lanes
+// cover 128 elements, which lie in one row (hv_d % 128 == 0), and add them with one atomic.
+__global__ void split_limbs_kernel(const int16_t *__restrict__ hv, uint64_t n_elems, int8_t *__restrict__ out, uint64_t plane_stride,
+                                   uint32_t hv_d, unsigned long long *__restrict__ sq) {
+  const uint64_t n8 = n_elems / 8;  // a multiple of 16, and so is the stride: a half-warp is in or out of the loop together
+  const uint32_t lane = threadIdx.x & 31, half = 0xFFFFu << (lane & 16);
+  const uint64_t i0 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (uint64_t)gridDim.x * blockDim.x;
+  // row / column of element 8 i, advanced by the stride without a division per step
+  uint64_t row = i0 * 8 / hv_d;
+  uint32_t col = (uint32_t)(i0 * 8 - row * hv_d);
+  const uint64_t drow = stride * 8 / hv_d;
+  const uint32_t dcol = (uint32_t)(stride * 8 - drow * hv_d);
+  for (uint64_t i = i0; i < n8; i += stride) {
     const uint4 v = reinterpret_cast<const uint4 *>(hv)[i];
     const uint32_t w[4] = {v.x, v.y, v.z, v.w};
     uint32_t hi[2] = {0, 0}, lo[2] = {0, 0};
+    unsigned long long s = 0;
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int x = (int)(int16_t)(w[e >> 1] >> (16 * (e & 1)));
@@ -452,10 +462,22 @@ __global__ void split_limbs_kernel(const int16_t *__restrict__ hv, uint64_t n_el
       const int h = (x - l) >> 7;
       hi[e >> 2] |= (uint32_t)(h & 0xFF) << (8 * (e & 3));
       lo[e >> 2] |= (uint32_t)(l & 0xFF) << (8 * (e & 3));
+      s += (uint32_t)(x * x);
     }
     reinterpret_cast<uint2 *>(out)[i] = make_uint2(hi[0], hi[1]);
     reinterpret_cast<uint2 *>(out + plane_stride)[i] = make_uint2(lo[0], lo[1]);
+#pragma unroll
+    for (int o = 8; o; o >>= 1) s += __shfl_xor_sync(half, s, o);
+    if ((lane & 15) == 0) atomicAdd(sq + row, s);
+    row += drow;
+    col += dcol;
+    if (col >= hv_d) { col -= hv_d; ++row; }
   }
+}
+
+__global__ void tc_flags_kernel(const unsigned long long *__restrict__ sq, uint32_t n, uint32_t *__restrict__ flags) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) flags[i] = sq[i] >= HG_NORM_WRAP_CUT;
 }
 
 }  // namespace
@@ -484,17 +506,15 @@ int hg_tensor_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b) {
   return HG_OK;
 }
 
-// ---- one matrix as two s8 limb planes [2][n_rows][hv_d]; its rows may be split piecewise, as they arrive ----
+// ---- one matrix as two s8 limb planes [2][n_rows][hv_d] and its row sums; its rows may be split piecewise, as they arrive ----
+
+uint64_t hg_tc_mat_bytes(uint32_t n_rows, uint32_t hv_d) { return 2 * (uint64_t)n_rows * hv_d + 8 * (uint64_t)n_rows; }
 
 int hg_tc_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int plane_slot, hg_tc_mat *m) {
   void *p;
   int rc;
-  if ((rc = hg_scratch(ctx, plane_slot, 2 * (uint64_t)n_rows * hv_d + 1024, &p))) return rc;
-  m->hv = d_hv;
-  m->planes = (int8_t *)p;
-  m->n_rows = n_rows;
-  m->hv_d = hv_d;
-  return tc_attrs(ctx);
+  if ((rc = hg_scratch(ctx, plane_slot, hg_tc_mat_bytes(n_rows, hv_d) + 1024, &p))) return rc;
+  return hg_tc_attach(ctx, d_hv, n_rows, hv_d, (int8_t *)p, m);
 }
 
 // limb split of rows [row0, row0 + rows) (asynchronous)
@@ -503,8 +523,21 @@ int hg_tc_split_rows(hg_ctx *ctx, const hg_tc_mat *m, uint32_t row0, uint32_t ro
   const uint64_t elems = (uint64_t)rows * m->hv_d;
   uint64_t blocks = (elems / 8 + 255) / 256;
   if (blocks > (uint64_t)ctx->sm_count * 16) blocks = (uint64_t)ctx->sm_count * 16;
+  HG_CUDA(cudaMemsetAsync(m->sq + row0, 0, (size_t)rows * 8, ctx->stream));
   split_limbs_kernel<<<(unsigned)blocks, 256, 0, ctx->stream>>>(m->hv + (size_t)row0 * m->hv_d, elems, m->planes + (size_t)row0 * m->hv_d,
-                                                                (uint64_t)m->n_rows * m->hv_d);
+                                                                (uint64_t)m->n_rows * m->hv_d, m->hv_d, m->sq + row0);
+  ctx->launches++;
+  HG_CUDA(cudaGetLastError());
+  return HG_OK;
+}
+
+// flags[i] = 1 if the limb split finds row i's true norm at or above HG_NORM_WRAP_CUT (asynchronous)
+int hg_tc_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, uint32_t *d_flags) {
+  hg_tc_mat m;
+  int rc;
+  if ((rc = hg_tc_setup(ctx, d_hv, n_rows, hv_d, HG_S_QRY_LIMBS, &m))) return rc;
+  if ((rc = hg_tc_split_rows(ctx, &m, 0, n_rows))) return rc;
+  tc_flags_kernel<<<(n_rows + 255) / 256, 256, 0, ctx->stream>>>(m.sq, n_rows, d_flags);
   ctx->launches++;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
@@ -521,6 +554,7 @@ int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, u
 int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int8_t *planes, hg_tc_mat *m) {
   m->hv = d_hv;
   m->planes = planes;
+  m->sq = reinterpret_cast<unsigned long long *>(planes + 2 * (uint64_t)n_rows * hv_d);
   m->n_rows = n_rows;
   m->hv_d = hv_d;
   return tc_attrs(ctx);
@@ -576,16 +610,17 @@ int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref
   cfg.dynamicSmemBytes = T2_SMEM_BYTES;
   cfg.stream = ctx->stream;
   static const hg_push_plan no_push = {};
+  const unsigned long long *rsq = R->sq + r0, *qsq = Q->sq + q0;  // indexed like the norms
   if (push) {  // a member of several GPUs: pusher warps send my limb-plane rows while the tiles are computed
     cfg.blockDim = dim3(TC_THREADS + 32 * TC_PUSH_WARPS, 1, 1);
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<TC_PUSH_WARPS>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul,
-                               walk_add, fd, *push, hg_floors{}));
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<TC_PUSH_WARPS>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, rsq, qsq,
+                               walk_mul, walk_add, fd, *push, hg_floors{}));
   } else if (floors) {
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0, true>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul,
-                               walk_add, fd, no_push, *floors));
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0, true>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, rsq, qsq,
+                               walk_mul, walk_add, fd, no_push, *floors));
   } else {
-    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul, walk_add, fd,
-                               no_push, hg_floors{}));
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<0>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, rsq, qsq, walk_mul,
+                               walk_add, fd, no_push, hg_floors{}));
   }
   ctx->launches++;
   HG_CUDA(cudaGetLastError());

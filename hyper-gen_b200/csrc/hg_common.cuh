@@ -248,6 +248,10 @@ int hg_pinned(hg_ctx *ctx, int slot, size_t bytes, void **out);
 // The dist kernels, numbered as the `path` argument of the dist entries (include/hypergen_b200.h).
 enum hg_dist_path { HG_PATH_AUTO = 0, HG_PATH_SIMT = 1, HG_PATH_TWO_LIMB = 2, HG_PATH_NARROW = 3 };
 constexpr int32_t HG_LIMB_MAX_ABS = 8127;  // the largest |x| that splits into two s8 limbs x = 128 h + l (13 bits)
+// ceil(2^31 / 3): while both rows' true norms sum x^2 stay below it, no i32 norm, dot or denominator of the pair wraps,
+// and the tensor kernels' per-row / per-column candidate bounds are exact.  A row at or above it is a candidate against
+// every column (DESIGN.md, dist epilogue).
+constexpr uint64_t HG_NORM_WRAP_CUT = 715827883ull;
 // sets what hg_dist_last_path / hg_dist_last_reason report
 void hg_dist_record(hg_ctx *ctx, int path, const char *fmt, ...);
 
@@ -349,15 +353,20 @@ int hg_tensor_shape_ok(uint32_t hv_d, const void *d_a, const void *d_b);
 // two s8 limb planes of one matrix (dist_tc.cu), split piecewise or at once
 struct hg_tc_mat {
   const int16_t *hv;
-  int8_t *planes;  // [2][n_rows][hv_d]
+  int8_t *planes;  // [2][n_rows][hv_d], followed by sq
+  unsigned long long *sq;  // [n_rows]: sum x^2 of every row in 64 bits (the split writes it; HG_NORM_WRAP_CUT)
   uint32_t n_rows, hv_d;
 };
+// bytes of the planes and the row sums of an n_rows x hv_d matrix
+uint64_t hg_tc_mat_bytes(uint32_t n_rows, uint32_t hv_d);
 int hg_tc_setup(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int plane_slot, hg_tc_mat *m);
 int hg_tc_split_rows(hg_ctx *ctx, const hg_tc_mat *m, uint32_t row0, uint32_t rows);
+int hg_tc_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, uint32_t *d_flags);
 int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                  const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
                  float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits,
                  const hg_floors *floors = nullptr);
+// `planes` holds hg_tc_mat_bytes(n_rows, hv_d)
 int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int8_t *planes, hg_tc_mat *m);
 int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                     const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
@@ -391,6 +400,7 @@ int hg_narrow_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t
                      uint32_t *entries, uint32_t *stats_all, uint32_t n_sets, uint32_t my_set, uint32_t entry_base,
                      uint32_t set_cap, hg_narrow_mat *m, bool init_stats = true);
 int hg_narrow_prep_rows(hg_ctx *ctx, const hg_narrow_mat *m, uint32_t row0, uint32_t rows);
+int hg_narrow_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, uint32_t *d_flags);
 int hg_narrow_launch(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                      const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                      uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,

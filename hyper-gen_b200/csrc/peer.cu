@@ -201,7 +201,7 @@ ShardLayout make_layout(int world, uint32_t n_total, uint32_t hv_d, uint64_t cap
   l.set_cap = n_planes == 1 ? hg_narrow_set_cap(n_total) : 0;
   l.entries = align_up(l.arrays + (n_planes == 1 ? hg_narrow_arrays_bytes(n_total) : 0), 256);
   l.plane = align_up(l.entries + (uint64_t)world * l.set_cap * 4, 1024);
-  l.end = l.plane + (uint64_t)n_planes * n_total * hv_d + 1024;
+  l.end = l.plane + (n_planes == 1 ? (uint64_t)n_total * hv_d : hg_tc_mat_bytes(n_total, hv_d)) + 1024;  // two limb planes: + row sums
   return l;
 }
 
@@ -613,7 +613,7 @@ static int shard_reserve(hg_peer *p, const ShardCall &a, int use_path) {
   void *x;
   int rc;
   if (!a.symmetric && a.n_ref_local) {
-    if ((rc = hg_scratch(c, HG_S_REF_LIMBS, 2 * (uint64_t)a.n_ref_local * a.hv_d + 1024, &x))) return rc;
+    if ((rc = hg_scratch(c, HG_S_REF_LIMBS, hg_tc_mat_bytes(a.n_ref_local, a.hv_d) + 1024, &x))) return rc;
     if ((rc = hg_scratch(c, HG_S_NARROW_META, hg_narrow_arrays_bytes(a.n_ref_local) + (uint64_t)hg_narrow_set_cap(a.n_ref_local) * 4 + 256, &x))) return rc;
   }
   if (p->world > 1) {
@@ -724,7 +724,10 @@ static int shard_enqueue(hg_peer *p, const ShardCall &a, int use_path) {
     add(ch, lay.norm + lo * 4, n * 4);
     add(ch, lay.plane + lo * a.hv_d, n * a.hv_d);
     if (use_path == HG_PATH_NARROW) for (int k = 0; k < 5; ++k) add(ch, lay.arrays + ((uint64_t)k * n_total + lo) * 4, n * 4);
-    else add(ch, lay.plane + ((uint64_t)n_total + lo) * a.hv_d, n * a.hv_d);
+    else {
+      add(ch, lay.plane + ((uint64_t)n_total + lo) * a.hv_d, n * a.hv_d);
+      add(ch, lay.plane + 2 * (uint64_t)n_total * a.hv_d + lo * 8, n * 8);  // their row sums (hg_tc_mat::sq)
+    }
   }
   if (use_path == HG_PATH_NARROW && world > 1) {  // the statistics and the outlier entries of ALL my rows (the pre-pass above is complete)
     if (nl) {  // (range 0 of the start set: the pushers cut it down to the entries the pre-pass actually wrote)

@@ -17,7 +17,7 @@ HG_OK, HG_E_INVALID, HG_E_CUDA, HG_E_CAPACITY, HG_E_RANGE, HG_E_UNSUPPORTED = 0,
 
 EXPORTS = [
     "hg_init", "hg_destroy", "hg_sync", "hg_host_alloc", "hg_host_free", "hg_host_register", "hg_host_unregister", "hg_last_error", "hg_version", "hg_stream_handle", "hg_launch_count",
-    "hg_set_profiling", "hg_stage_ms", "hg_int_peak", "hg_tensor_peak", "hg_encode_sets", "hg_encode_sets_dev",
+    "hg_set_profiling", "hg_stage_ms", "hg_int_peak", "hg_tensor_peak", "hg_dist_norm_flags", "hg_encode_sets", "hg_encode_sets_dev",
     "hg_fasta_merge", "hg_sketch_fasta_batch",
     "hg_kmer_hash", "hg_sketch_batch", "hg_sketch_batch_dev", "hg_sketch_status", "hg_unpack", "hg_unpack_dev",
     "hg_dist", "hg_dist_dev", "hg_dist_status", "hg_dist_last_path", "hg_dist_last_reason", "hg_sort_hits_dev", "hg_dist_sorted", "hg_dist_packed",
@@ -83,6 +83,7 @@ def load() -> C.CDLL:
     L.hg_stage_ms.restype = i32; L.hg_stage_ms.argtypes = [vp, C.POINTER(C.c_float)]
     L.hg_int_peak.restype = i32; L.hg_int_peak.argtypes = [vp, i32, C.POINTER(C.c_double)]
     L.hg_tensor_peak.restype = i32; L.hg_tensor_peak.argtypes = [vp, C.POINTER(C.c_double)]
+    L.hg_dist_norm_flags.restype = i32; L.hg_dist_norm_flags.argtypes = [vp, vp, u32, u32, i32, vp]
     L.hg_encode_sets.restype = i32; L.hg_encode_sets.argtypes = [vp, vp, vp, u32, u32, vp, vp, vp, vp]
     L.hg_encode_sets_dev.restype = i32; L.hg_encode_sets_dev.argtypes = [vp, vp, vp, u32, u32, vp, vp, vp, vp]
     L.hg_fasta_merge.restype = i32; L.hg_fasta_merge.argtypes = [vp, vp, vp, u32, vp, u64, vp]
@@ -317,6 +318,11 @@ class Context:
         v = C.c_double(0)
         _check(load().hg_tensor_peak(self._h, C.byref(v)))
         return v.value
+
+    def dist_norm_flags(self, d_hv, n_rows, hv_d, path, d_flags):
+        """hg_dist_norm_flags (device pointers as ints): per row 1 if tensor kernel `path` takes it as a row whose true
+        norm reaches ceil(2^31 / 3)"""
+        _check(load().hg_dist_norm_flags(self._h, d_hv, n_rows, hv_d, path, d_flags))
 
     # -- stage 1 --
     def kmer_hash(self, seq: np.ndarray, seg_off: np.ndarray, params: SketchParams):

@@ -103,6 +103,11 @@ HG_API int hg_int_peak(hg_ctx *ctx, int which, double *lane_ops_per_s);
  * 256 x 256 x 32) back to back from resident shared-memory operands on every TPC.  Returns integer ops / s (2 per MAC).
  * Both probes are measurement hooks of this build, not part of the interface a host binds. */
 HG_API int hg_tensor_peak(hg_ctx *ctx, double *ops_per_s);
+/* Which rows of d_hv (n_rows x hv_d, on the device) the tensor kernel `path` (2 two-limb, 3 single plane) takes as
+ * rows whose true norm sum x^2 reaches ceil(2^31 / 3), i.e. rows whose every pair skips the candidate bound:
+ * d_flags[i] = 1 or 0, from the kernel's own row preparation.  HG_E_UNSUPPORTED for path 3 if its pre-pass declines
+ * the rows.  Synchronous.  A measurement hook like the probes above. */
+HG_API int hg_dist_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int path, uint32_t *d_flags);
 
 /* ---- stage 1: sketch -------------------------------------------------------------- */
 

@@ -67,3 +67,17 @@ def test_identity_holds_in_wrapping_i32():
     dot = w(4 * (ax @ ay.T) + sy[None, :] * (2 * ax.sum(1) + d * sx)[:, None] + sx[:, None] * (2 * ay.sum(1))[None, :]
             + ex @ y.T + (2 * ax + sx[:, None]) @ ey.T)
     assert np.array_equal(dot, w(x @ y.T))
+
+
+def test_true_norm_from_the_plane_and_the_residuals():
+    """narrow_prep_kernel's sum x^2 (HG_NORM_WRAP_CUT): 4 sum a^2 + 2 s sum 2a + D s^2 + sum eps (x - s + 2a + 2s)"""
+    rng = np.random.default_rng(4)
+    d = 2048
+    x = sketch_like(rng, 30, d, 200)
+    x[2, [1, 9, 700]] = [29001, -30999, 4001]
+    x[5, 3] += 1
+    x[7] = 255 - 2 * (np.arange(d) % 256)  # spans exactly 510
+    s, a, eps = prep(x)
+    t = x - s[:, None]
+    xx = 4 * (a * a).sum(1) + 2 * s * (2 * a).sum(1) + d * s * s + (eps * (t + 2 * a + 2 * s[:, None])).sum(1)
+    assert np.array_equal(xx, (x * x).sum(1))
