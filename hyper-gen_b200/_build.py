@@ -18,7 +18,7 @@ OBJ = os.path.join(ROOT, "build", "obj")
 LIB = os.path.join(HERE, "libhypergen_b200.so")
 
 SOURCES = ["api.cu", "kmer_hash.cu", "encode.cu", "dist_simt.cu", "dist_tc.cu", "dist_narrow.cu", "probe.cu", "fasta.cu", "sort.cu", "peer.cu",
-           "search.cu", "cluster.cu", "derep.cu"]
+           "search.cu", "cluster.cu", "derep.cu", "matrix.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC,-fvisibility=hidden", "-diag-suppress", "177",

@@ -744,8 +744,8 @@ void hg_dist_record(hg_ctx *c, int path, const char *fmt, ...) {
   va_end(ap);
 }
 
-// A window of the pairs of one matrix against itself: ref rows [r0, r0 + h) x query rows [c0, c0 + w), reported with
-// the call's global offsets (i0 + r, j0 + c).
+// A window of a dist call's pairs: ref rows [r0, r0 + h) x query rows [c0, c0 + w) (indices into the call's ref and
+// query blocks), reported with the call's global offsets (i0 + r, j0 + c).
 struct DistWindow { uint32_t r0, h, c0, w; };
 // A dist call that runs only these windows (a cluster or derep run, hg_cluster_* / hg_derep_*): every row is prepared
 // once, then each window is launched and `after(k)` is enqueued behind the launch of window k - by every kernel branch,
@@ -758,6 +758,10 @@ struct DistWindows {
   // launches no window and no `after`, and the rerun starts from the state the caller left.  For hooks that are not
   // idempotent (the greedy steps of a derep run); without it the declined windows run their hooks on empty edge lists.
   bool decide_first = false;
+  // An ANI matrix run (hg_ani_matrix_*): window k writes the exact dot of every pair to dense[k] (hg_dense) instead of
+  // appending hits, and `before(k)` is enqueued ahead of its launch.
+  const hg_dense *dense = nullptr;
+  std::function<int(size_t)> before;
 };
 
 // one dist call: ref rows [i0, i0 + n_ref) against query rows [j0, j0 + n_qry), both matrices in HBM (or arriving there)
@@ -776,7 +780,7 @@ struct DistOp {
   unsigned long long *n_hits;
   const hg_floor *floors = nullptr;  // a search's main pass: per-query thresholds in place of ani_th (hg_floors)
   const float *cfrac_row = nullptr;
-  const DistWindows *windows = nullptr;  // one matrix against itself (ref and query the same rows in HBM): only these windows
+  const DistWindows *windows = nullptr;  // only these windows (the ref block may lie inside the query matrix, as anywhere)
 };
 
 // The kernel a dist call tries first, chosen before anything runs.
@@ -916,11 +920,12 @@ static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, H
     }
     return narrow ? hg_narrow_prep_rows(c, M, a, rows) : hg_tc_split_rows(c, T, a, rows);
   };
-  auto launch = [&](uint32_t r0, uint32_t nr, uint32_t i0, const int32_t *rn, uint32_t q0, uint32_t nq, uint32_t j0, const int32_t *qn) {
+  auto launch = [&](uint32_t r0, uint32_t nr, uint32_t i0, const int32_t *rn, uint32_t q0, uint32_t nq, uint32_t j0, const int32_t *qn,
+                    const hg_dense *dn = nullptr) {
     const hg_floors fl = {op.floors ? op.floors + q0 : nullptr, op.cfrac_row};  // indexed like qn = qry_norm + q0
     const hg_floors *flp = op.floors ? &fl : nullptr;
-    return narrow ? hg_narrow_launch(c, Rn, r0, nr, i0, rn, &Qm, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits, flp)
-                  : hg_tc_launch(c, Rl, r0, nr, i0, rn, &Qt, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits, flp);
+    return narrow ? hg_narrow_launch(c, Rn, r0, nr, i0, rn, &Qm, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits, flp, dn)
+                  : hg_tc_launch(c, Rl, r0, nr, i0, rn, &Qt, q0, nq, j0, qn, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits, flp, dn);
   };
   if (!one && (rc = prep(hq, &Qm, &Qt, 0, op.n_qry, c->ev_chunk[1]))) return rc;
   for (size_t k = 0; k < chunks.size(); k++) {
@@ -937,7 +942,9 @@ static int dist_tensor(hg_ctx *c, const DistOp &op, bool narrow, HostRows *hr, H
     if (first && (rc = hg_narrow_verdict(c, &Qm, in_q ? nullptr : &Rm, &f->absmax, &f->outliers))) return rc;
     for (size_t k = 0; k < op.windows->win.size(); k++) {
       const DistWindow &w = op.windows->win[k];
-      if ((rc = launch(w.r0, w.h, op.i0 + w.r0, op.ref_norm + w.r0, w.c0, w.w, op.j0 + w.c0, op.qry_norm + w.c0)) ||
+      if ((op.windows->before && (rc = op.windows->before(k))) ||
+          (rc = launch(r_off + w.r0, w.h, op.i0 + w.r0, op.ref_norm + w.r0, w.c0, w.w, op.j0 + w.c0, op.qry_norm + w.c0,
+                       op.windows->dense ? &op.windows->dense[k] : nullptr)) ||
           (rc = op.windows->after(k)))
         return rc;
     }
@@ -995,9 +1002,10 @@ static int dist_run(hg_ctx *c, const DistOp &op, const DistChoice &ch, HostRows 
     rc = HG_OK;
     for (size_t k = 0; k < n_win && !rc; k++) {
       const DistWindow &w = op.windows ? op.windows->win[k] : all;
+      if (op.windows && op.windows->before && (rc = op.windows->before(k))) break;
       rc = hg_launch_dist_simt(c, op.ref + (size_t)w.r0 * op.hv_d, op.ref_norm + w.r0, w.h, op.i0 + w.r0, op.qry + (size_t)w.c0 * op.hv_d,
                                op.qry_norm + w.c0, w.w, op.j0 + w.c0, op.hv_d, op.ksize, op.ani_th, op.symmetric, op.hits, op.cap, op.n_hits,
-                               op.floors ? &fl : nullptr);
+                               op.floors ? &fl : nullptr, op.windows && op.windows->dense ? &op.windows->dense[k] : nullptr);
       if (!rc && op.windows) rc = op.windows->after(k);
     }
     HG_PROF(c, 5);
@@ -1922,5 +1930,233 @@ extern "C" int hg_derep_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
   if (!c || !counts || !ms) { hg_set_error("hg_derep_stats: NULL argument"); return HG_E_INVALID; }
   memcpy(counts, c->derep_stats, sizeof(c->derep_stats));
   memcpy(ms, c->derep_ms, sizeof(c->derep_ms));
+  return HG_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// ANI matrix: every pair, dense (DESIGN.md §4.11)
+// ---------------------------------------------------------------------------------------
+
+// output bytes one band may hold: 64 MiB (16 M cells: a 256-row band of 65 536 columns, and far more than the 74 CTA
+// pairs' 4.8 M cells of one wave of tiles), or HG_MATRIX_BAND_BYTES, read at every call
+static uint64_t matrix_band_bytes() {
+  uint64_t b = 0;
+  if (const char *e = getenv("HG_MATRIX_BAND_BYTES")) b = strtoull(e, nullptr, 10);
+  return b ? b : 64ull << 20;
+}
+
+// cell offset of row i's first cell (hg_dense_row of the caller's layout)
+static uint64_t matrix_row(bool lower, uint64_t ld, uint32_t i) { return lower ? (uint64_t)i * ((uint64_t)i - 1) / 2 : (uint64_t)i * ld; }
+
+// Bands of ref rows [first, n_ref): rows [a, a + h) against the query columns [0, a + h) (lower) or [0, n_qry), each
+// the most rows whose cells fit `bytes` (at least one row), cut to a multiple of 256 rows where that many fit.
+static std::vector<DistWindow> matrix_bands(uint32_t first, uint32_t n_ref, uint32_t n_qry, bool lower, uint64_t bytes) {
+  const uint64_t cap = std::max<uint64_t>(1, bytes / 4);
+  std::vector<DistWindow> out;
+  for (uint32_t a = first; a < n_ref;) {
+    auto cells = [&](uint64_t h) { return lower ? h * a + h * (h - 1) / 2 : h * n_qry; };
+    uint64_t lo = 1, hi = n_ref - a;
+    while (lo < hi) {
+      const uint64_t m = (lo + hi + 1) / 2;
+      if (cells(m) <= cap) lo = m; else hi = m - 1;
+    }
+    if (lo >= 256 && lo < n_ref - a) lo &= ~255ull;
+    out.push_back({a, (uint32_t)lo, 0, lower ? a + (uint32_t)lo : n_qry});
+    a += (uint32_t)lo;
+  }
+  return out;
+}
+
+static void matrix_stats_reset(hg_ctx *c) {
+  memset(c->matrix_stats, 0, sizeof(c->matrix_stats));
+  for (float &m : c->matrix_ms) m = -1.0f;
+}
+
+// The matrix cells of ref rows [first, n_ref) - of the one matrix ref = qry in lower mode, else against every query row:
+// the kernel chosen once and every row prepared once, then the bands of matrix_bands, each launched in dense mode and
+// converted in place behind its launch (DistWindows::after).  d_out: the bands write straight into the caller's device
+// matrix.  h_out: they alternate between two band buffers; band k is copied to the host on the copy stream under band
+// k + 1's kernel, and band k + 2 (same buffer) waits for that copy.  The single plane's verdict is read before band 0
+// (decide_first), so a declined attempt writes and copies nothing.  d_out / h_out hold row `first` at offset 0.
+// `upload` (may be empty) brings the rows to the device first; profiling counts it with the row preparation.  Returns
+// with everything complete.
+static int matrix_run(hg_ctx *c, const int16_t *d_ref, const int32_t *d_rn, uint32_t n_ref, const int16_t *d_qry, const int32_t *d_qn,
+                      uint32_t n_qry, uint32_t hv_d, uint32_t ksize, int path, uint32_t bits, bool lower, uint32_t first, float *d_out,
+                      float *h_out, uint64_t ld, const std::function<int()> &upload = nullptr) {
+  int rc;
+  DistChoice ch;
+  if ((rc = dist_choose(path, n_ref, n_qry, hg_tensor_shape_ok(hv_d, d_ref, d_qry) == HG_OK, bits, &ch))) return rc;
+  DistWindows W;
+  W.win = matrix_bands(first, n_ref, n_qry, lower, matrix_band_bytes());
+  W.decide_first = true;
+  const size_t nb = W.win.size();
+  auto cells = [&](const DistWindow &w) { return matrix_row(lower, n_qry, w.r0 + w.h) - matrix_row(lower, n_qry, w.r0); };
+  uint64_t band_max = 0;
+  for (const DistWindow &w : W.win) band_max = std::max(band_max, cells(w));
+  int32_t *buf[2] = {nullptr, nullptr};
+  if (h_out) {
+    void *p;
+    const uint64_t bb = (band_max * 4 + 255) & ~255ull;
+    if ((rc = hg_scratch(c, HG_S_PACKED, 2 * bb, &p)) || (rc = ensure_copy_stream(c))) return rc;
+    buf[0] = (int32_t *)p;
+    buf[1] = (int32_t *)((uint8_t *)p + bb);
+  }
+  std::vector<hg_dense> D(nb);
+  for (size_t k = 0; k < nb; k++)
+    D[k] = h_out ? hg_dense{buf[k & 1], lower ? 0 : (uint64_t)n_qry, W.win[k].r0} : hg_dense{(int32_t *)d_out, lower ? 0 : ld, first};
+  W.dense = D.data();
+  // [0] converted, [1..2] band buffer copied; then with profiling: [3] start, [4] rows prepared, per band: kernel start,
+  // kernel end, converted, copy start, copy end
+  ClusterEvents E;
+  E.ev.resize(c->prof ? 5 + 5 * nb : 3, nullptr);
+  for (size_t t = 0; t < E.ev.size(); t++) HG_CUDA(cudaEventCreateWithFlags(&E.ev[t], t < 3 ? cudaEventDisableTiming : cudaEventDefault));
+  auto mark = [&](size_t t, cudaStream_t s) -> int {
+    if (c->prof) HG_CUDA(cudaEventRecord(E.ev[t], s));
+    return HG_OK;
+  };
+  if (c->prof) W.prepared = E.ev[4];
+  uint64_t entries = 0, bytes = 0;
+  W.before = [&](size_t k) -> int {
+    if (h_out && k >= 2) HG_CUDA(cudaStreamWaitEvent(c->stream, E.ev[1 + (k & 1)], 0));  // its buffer's last band is on the host
+    return mark(5 + 5 * k, c->stream);
+  };
+  W.after = [&](size_t k) -> int {
+    const DistWindow &w = W.win[k];
+    int r2;
+    if ((r2 = mark(6 + 5 * k, c->stream)) || (r2 = hg_launch_ani_convert(c, D[k], w.r0, w.h, n_qry, d_rn, d_qn, ksize)) ||
+        (r2 = mark(7 + 5 * k, c->stream)))
+      return r2;
+    const uint64_t n_cells = cells(w);
+    entries += n_cells;
+    if (!h_out) return HG_OK;
+    HG_CUDA(cudaEventRecord(E.ev[0], c->stream));
+    HG_CUDA(cudaStreamWaitEvent(c->copy_stream, E.ev[0], 0));
+    if ((r2 = mark(8 + 5 * k, c->copy_stream))) return r2;
+    float *dst = h_out + (matrix_row(lower, ld, w.r0) - matrix_row(lower, ld, first));
+    if (lower || ld == n_qry)
+      HG_CUDA(cudaMemcpyAsync(dst, buf[k & 1], n_cells * 4, cudaMemcpyDeviceToHost, c->copy_stream));
+    else
+      HG_CUDA(cudaMemcpy2DAsync(dst, ld * 4, buf[k & 1], (size_t)n_qry * 4, (size_t)n_qry * 4, w.h, cudaMemcpyDeviceToHost, c->copy_stream));
+    HG_CUDA(cudaEventRecord(E.ev[1 + (k & 1)], c->copy_stream));
+    bytes += n_cells * 4;
+    return mark(9 + 5 * k, c->copy_stream);
+  };
+  void *d_cnt;
+  if ((rc = hg_scratch(c, HG_S_COUNTS, 256, &d_cnt))) return rc;  // (no hits: the counter a declined attempt resets)
+  if ((rc = mark(3, c->stream)) || (upload && (rc = upload()))) return rc;
+  DistOp op = {d_ref, d_rn, n_ref, 0, d_qry, d_qn, n_qry, 0, hv_d, ksize, 0.0f, 0, nullptr, 0, (unsigned long long *)d_cnt};
+  op.windows = &W;
+  rc = dist_run(c, op, ch, nullptr, nullptr, false);
+  if (h_out) HG_CUDA(cudaStreamSynchronize(c->copy_stream));  // (also on an error: no copy may outlive the call)
+  HG_CUDA(cudaStreamSynchronize(c->stream));
+  if (rc) return rc;
+  c->matrix_stats[0] = nb;
+  c->matrix_stats[1] = entries;
+  c->matrix_stats[2] = bytes;
+  c->matrix_stats[3] = (uint64_t)c->dist_path;
+  if (c->prof && nb) {
+    float t, kern = 0.0f, conv = 0.0f, copy = 0.0f;
+    for (size_t k = 0; k < nb; k++) {
+      if ((rc = E.ms((int)(5 + 5 * k), (int)(6 + 5 * k), &t))) return rc;
+      kern += t;
+      if ((rc = E.ms((int)(6 + 5 * k), (int)(7 + 5 * k), &t))) return rc;
+      conv += t;
+      if (h_out) {
+        if ((rc = E.ms((int)(8 + 5 * k), (int)(9 + 5 * k), &t))) return rc;
+        copy += t;
+      }
+    }
+    if (c->dist_path != HG_PATH_SIMT && (rc = E.ms(3, 4, &c->matrix_ms[0]))) return rc;  // the SIMT kernel prepares nothing
+    c->matrix_ms[1] = kern;
+    c->matrix_ms[2] = conv;
+    if (h_out) c->matrix_ms[3] = copy;
+  }
+  return HG_OK;
+}
+
+int hg_matrix_check(const char *who, bool same, uint32_t n_ref, uint32_t n_qry, uint32_t hv_d, int path, int lower, const void *out,
+                    uint64_t ld) {
+  if (hv_d == 0 || hv_d % 256 != 0) { hg_set_error("%s: hv_d %u must be a multiple of 256", who, hv_d); return HG_E_INVALID; }
+  if (path < HG_PATH_AUTO || path > HG_PATH_NARROW) { hg_set_error("%s: path %d", who, path); return HG_E_INVALID; }
+  if (lower != 0 && lower != 1) { hg_set_error("%s: lower %d (0 or 1)", who, lower); return HG_E_INVALID; }
+  if (lower && !same) { hg_set_error("%s: the lower triangle needs the same rows as ref and query", who); return HG_E_INVALID; }
+  if (!lower && ld < n_qry) { hg_set_error("%s: ld %llu < n_qry %u", who, (unsigned long long)ld, n_qry); return HG_E_INVALID; }
+  if (!out && hg_matrix_entries(n_ref, n_qry, lower)) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
+  return HG_OK;
+}
+
+uint64_t hg_matrix_entries(uint32_t n_ref, uint32_t n_qry, int lower) {
+  return lower ? (n_ref ? (uint64_t)n_ref * (n_ref - 1) / 2 : 0) : (uint64_t)n_ref * n_qry;
+}
+
+int HostPin::pin(void *p, uint64_t bytes) {
+  cudaPointerAttributes a;
+  const uint8_t *last = (const uint8_t *)p + bytes - 1;
+  bool locked = cudaPointerGetAttributes(&a, p) == cudaSuccess && a.type == cudaMemoryTypeHost;
+  locked = locked && cudaPointerGetAttributes(&a, last) == cudaSuccess && a.type == cudaMemoryTypeHost;
+  cudaGetLastError();  // (an unregistered pointer is not an error to keep)
+  if (locked || bytes == 0) return HG_OK;
+  HG_CUDA(cudaHostRegister(p, bytes, cudaHostRegisterPortable));
+  ptr = p;
+  return HG_OK;
+}
+HostPin::~HostPin() {
+  if (ptr) cudaHostUnregister(ptr);
+}
+
+int hg_matrix_packed_run(hg_ctx *c, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, uint32_t ksize, int path,
+                         bool lower, uint32_t first, float *out, uint64_t ld) {
+  HG_CUDA(cudaSetDevice(c->device));
+  matrix_stats_reset(c);
+  int rc;
+  HostRows hr, hq;
+  if ((rc = hg_packed_stage(c, R, Q, same, hv_d, &hr, &hq))) return rc;
+  auto upload = [&]() -> int {
+    int r2 = hg_rows_to_device(c, hr, hv_d);
+    return r2 || same ? r2 : hg_rows_to_device(c, hq, hv_d);
+  };
+  return matrix_run(c, hr.d_hv, hr.d_norm, R.n, hq.d_hv, hq.d_norm, Q.n, hv_d, ksize, path, std::max(R.max_bits, Q.max_bits), lower, first,
+                    nullptr, out, ld, upload);
+}
+
+extern "C" int hg_ani_matrix_dev(hg_ctx *c, const int16_t *d_ref, const int32_t *d_ref_norm2, uint32_t n_ref, const int16_t *d_qry,
+                                 const int32_t *d_qry_norm2, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, int path, int lower,
+                                 float *d_out, uint64_t ld) {
+  const char *who = "hg_ani_matrix_dev";
+  if (!c || (n_ref && (!d_ref || !d_ref_norm2)) || (n_qry && (!d_qry || !d_qry_norm2))) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
+  const bool same = d_ref == d_qry && d_ref_norm2 == d_qry_norm2 && n_ref == n_qry;
+  int rc;
+  if ((rc = hg_matrix_check(who, same, n_ref, n_qry, hv_d, path, lower, d_out, ld))) return rc;
+  matrix_stats_reset(c);
+  if (hg_matrix_entries(n_ref, n_qry, lower) == 0) return HG_OK;
+  HG_CUDA(cudaSetDevice(c->device));
+  return matrix_run(c, d_ref, d_ref_norm2, n_ref, d_qry, d_qry_norm2, n_qry, hv_d, ksize, path, 0, lower != 0, 0, d_out, nullptr, ld);
+}
+
+extern "C" int hg_ani_matrix_packed(hg_ctx *c, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                                    const int32_t *ref_norm2, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                                    const uint8_t *qry_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d, uint32_t ksize,
+                                    int path, int lower, float *out, uint64_t ld) {
+  const char *who = "hg_ani_matrix_packed";
+  if (!c) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
+  hg_packed_rows R = {ref_packed, ref_stride, ref_bits, ref_norm2, n_ref}, Q = {qry_packed, qry_stride, qry_bits, qry_norm2, n_qry};
+  const bool same = R.packed == Q.packed && R.bits == Q.bits && R.norm == Q.norm && R.n == Q.n;
+  int rc;
+  if ((rc = hg_packed_args_check(who, R, Q, hv_d)) || (rc = hg_matrix_check(who, same, n_ref, n_qry, hv_d, path, lower, out, ld))) return rc;
+  matrix_stats_reset(c);
+  const uint64_t entries = hg_matrix_entries(n_ref, n_qry, lower);
+  if (entries == 0) return HG_OK;
+  bool same2;
+  if ((rc = hg_packed_rows_check(who, &R, &Q, hv_d, &same2))) return rc;
+  HostPin pin;
+  const uint64_t span = lower ? entries : (uint64_t)(n_ref - 1) * ld + n_qry;
+  if ((rc = pin.pin(out, span * 4))) return rc;
+  return hg_matrix_packed_run(c, R, Q, same2, hv_d, ksize, path, lower != 0, 0, out, ld);
+}
+
+extern "C" int hg_ani_matrix_stats(hg_ctx *c, uint64_t counts[4], float ms[4]) {
+  if (!c || !counts || !ms) { hg_set_error("hg_ani_matrix_stats: NULL argument"); return HG_E_INVALID; }
+  memcpy(counts, c->matrix_stats, sizeof(c->matrix_stats));
+  memcpy(ms, c->matrix_ms, sizeof(c->matrix_ms));
   return HG_OK;
 }

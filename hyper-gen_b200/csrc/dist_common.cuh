@@ -94,6 +94,30 @@ __device__ __forceinline__ bool dist_eval(const DistEpilogue &e, bool live, uint
   return ani >= th;
 }
 
+// ---- dense output (hg_dense): the exact dot of every live pair, no threshold ----
+// cells of global row gi owned by query columns gj, gj + 1, ... up to 16: how many are live (inside the launch's
+// columns, and below the diagonal in a lower triangle)
+__device__ __forceinline__ uint32_t dense_live(const hg_dense &d, const DistEpilogue &e, uint32_t gi, uint32_t gj) {
+  uint32_t end = e.j0 + e.n_qry;
+  if (!d.ld && gi < end) end = gi;
+  return gj >= end ? 0u : min(16u, end - gj);
+}
+__device__ __forceinline__ int32_t *dense_cell(const hg_dense &d, uint32_t gi, uint32_t gj) {
+  return d.base + (hg_dense_row(d, gi) - hg_dense_row(d, d.row_base)) + gj;
+}
+// the first n of 16 consecutive cells of row gi from column gj: four 16-byte stores when all 16 are live and aligned
+__device__ __forceinline__ void dense_store16(const hg_dense &d, uint32_t gi, uint32_t gj, uint32_t n, const int32_t (&v)[16]) {
+  int32_t *p = dense_cell(d, gi, gj);
+  if (n == 16 && ((uintptr_t)p & 15) == 0) {
+#pragma unroll
+    for (int t = 0; t < 4; ++t) reinterpret_cast<int4 *>(p)[t] = make_int4(v[4 * t], v[4 * t + 1], v[4 * t + 2], v[4 * t + 3]);
+    return;
+  }
+#pragma unroll
+  for (int j = 0; j < 16; ++j)
+    if ((uint32_t)j < n) p[j] = v[j];
+}
+
 // ---- arrival flags of a multi-GPU launch (hg_tile_feed) ----
 __device__ __forceinline__ unsigned long long feed_ns() {
   unsigned long long t;

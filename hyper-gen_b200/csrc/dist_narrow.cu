@@ -459,12 +459,45 @@ __device__ __forceinline__ uint32_t n1_drain(const hg::DistEpilogue &ep, const h
   return n_list;
 }
 
-// QF: per-query thresholds (a search pass, PUSHW = 0 only); `fl` is not read otherwise
-template <int PUSHW, bool QF = false>
-__global__ void __launch_bounds__(N1_THREADS + 32 * PUSHW, 1)
-dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry, uint32_t ref_row_base,
-               uint32_t qry_row_base, hg::DistEpilogue ep, NarrowArgs na, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan,
-               hg_floors fl) {
+// Dense mode (hg_dense): the same drain without the bound; every live element gets its outlier correction when its row
+// or column has entries (`rcorr`, and the column flags in place of the bounds in s_col), and the exact dot goes to its cell.
+__device__ __forceinline__ void n1_drain_dense(const hg::DistEpilogue &ep, const hg_dense &dn, const NarrowArgs &na, uint32_t taddr,
+                                               int c_begin, int c_end, const int32_t *s_col, int32_t sr, int32_t xr, bool row_live,
+                                               bool rcorr, uint32_t li, uint32_t col0) {
+  const uint32_t gi = ep.i0 + li;
+  uint32_t nx[16];
+  tmem_ld16(taddr + c_begin, nx);
+#pragma unroll 1
+  for (int c = c_begin; c < c_end; c += 16) {
+    uint32_t ac[16];
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    tmem_ld_fence(nx);
+#pragma unroll
+    for (int j = 0; j < 16; ++j) ac[j] = nx[j];
+    if (c + 16 < c_end) tmem_ld16(taddr + c + 16, nx);
+    const uint32_t gj = ep.j0 + col0 + c;
+    const uint32_t n = row_live ? hg::dense_live(dn, ep, gi, gj) : 0u;
+    if (n) {  // (no `continue`: the warp stays converged for the next tcgen05.wait)
+      int32_t dot[16];
+#pragma unroll
+      for (int j = 0; j < 16; ++j) {
+        dot[j] = (int32_t)(4u * ac[j] + (uint32_t)s_col[N1_BN + c + j] * (uint32_t)xr + (uint32_t)sr * (uint32_t)s_col[2 * N1_BN + c + j]);
+        if ((uint32_t)j < n && (rcorr || s_col[c + j])) {
+          const uint32_t lj = col0 + c + j;
+          dot[j] = (int32_t)((uint32_t)dot[j] + (uint32_t)n1_correction(na, li, lj, na.r.e[li], na.q.e[lj]));
+        }
+      }
+      hg::dense_store16(dn, gi, gj, n, dot);
+    }
+  }
+}
+
+// QF: per-query thresholds (a search pass, PUSHW = 0 only); `fl` is not read otherwise.  DENSE (PUSHW = 0, no QF): every
+// live pair's dot to its cell of `dn` (hg_dense) instead of the bound, the exact epilogue and the append.
+template <int PUSHW, bool QF, bool DENSE>
+__device__ __forceinline__ void n1_body(const CUtensorMap &tm_ref, const CUtensorMap &tm_qry, uint32_t ref_row_base, uint32_t qry_row_base,
+                                        const hg::DistEpilogue &ep, const NarrowArgs &na, hg_tile_feed feed, const hg_push_plan &plan,
+                                        const hg_floors &fl, const hg_dense &dn) {
   constexpr int STAGES = N1_STAGES, STAGE_BYTES = N1_STAGE_BYTES;
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
@@ -602,12 +635,15 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
       }
       int32_t *s_col = s_col_all + (tile_n & 1u) * N1_COL_WORDS;  // double buffered: one barrier per tile is enough
       int32_t tr, sr, xr;
-      bool live;
+      bool live, rcorr;
       auto constants = [&]() {
         {
           const uint32_t t = threadIdx.x - 64, lj = col0 + t;  // one column per epilogue thread
           int32_t tq = COL_NEVER, sq = 0, tt = 0;
-          if (lj < ep.n_qry) {
+          if (DENSE) {  // the column's outlier flag
+            tq = lj < ep.n_qry && na.q.e[lj] && na.q.out_cnt[lj];
+            if (lj < ep.n_qry) { sq = na.q.s[lj]; tt = na.q.a2[lj]; }
+          } else if (lj < ep.n_qry) {
             tq = COL_ALWAYS;
             float cq = ep.cfrac;
             if constexpr (QF) cq = fl.q[lj].cfrac;
@@ -627,6 +663,7 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
         const uint32_t li = row0 + q * 32 + lane;
         tr = ROW_ALWAYS; sr = 0; xr = 0;
         live = li < ep.n_ref;
+        rcorr = DENSE && live && na.r.e[li] && na.r.out_cnt[li];
         if (live) {
           float cr = ep.cfrac;
           if constexpr (QF) cr = *fl.cfrac_row;
@@ -648,9 +685,14 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
       uint32_t n_list = 0;
       // my 128 x 256 part of the tile may be empty (below the diagonal, or past the last ref row)
       const bool mine_empty = row0 >= ep.n_ref || (ep.symmetric && (uint64_t)ep.j0 + col0 + N1_BN - 1 <= (uint64_t)ep.i0 + row0);
-      if (!mine_empty)
+      if constexpr (DENSE) {
+        if (!mine_empty)
+          n1_drain_dense(ep, dn, na, tmem_base + ((q * 32u) << 16) + b * N1_BN, half * (N1_BN / 2), (half + 1) * (N1_BN / 2), s_col, sr, xr,
+                         live, rcorr, row0 + q * 32 + lane, col0);
+      } else if (!mine_empty) {
         n_list = n1_drain<QF>(ep, fl, na, tmem_base + ((q * 32u) << 16) + b * N1_BN, half * (N1_BN / 2), (half + 1) * (N1_BN / 2), s_col, tr,
                           sr, xr, live, q * 32 + lane, row0, col0, list, anis, 0u);
+      }
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(mapa_u32(tmem_empty_bar(b), 0));  // this warp's TMEM reads of buffer b are done
@@ -665,6 +707,21 @@ dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(N1_TMEM_COLS) : "memory");
   }
+}
+
+template <int PUSHW, bool QF = false>
+__global__ void __launch_bounds__(N1_THREADS + 32 * PUSHW, 1)
+dist_n1_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry, uint32_t ref_row_base,
+               uint32_t qry_row_base, hg::DistEpilogue ep, NarrowArgs na, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan,
+               hg_floors fl) {
+  n1_body<PUSHW, QF, false>(tm_ref, tm_qry, ref_row_base, qry_row_base, ep, na, feed, plan, fl, hg_dense{});
+}
+
+__global__ void __launch_bounds__(N1_THREADS, 1)
+dist_n1_dense_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry, uint32_t ref_row_base,
+                     uint32_t qry_row_base, hg::DistEpilogue ep, NarrowArgs na, hg_tile_feed feed,
+                     const __grid_constant__ hg_push_plan plan, hg_dense dn) {
+  n1_body<0, false, true>(tm_ref, tm_qry, ref_row_base, qry_row_base, ep, na, feed, plan, hg_floors{}, dn);
 }
 
 void carve_arrays(hg_narrow_mat &m, void *arrays) {
@@ -722,6 +779,7 @@ static int narrow_attrs(hg_ctx *ctx) {
     HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
     HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<N1_PUSH_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
     HG_CUDA(cudaFuncSetAttribute(dist_n1_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_n1_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, N1_SMEM_BYTES));
     ctx->n1_attr_set = 1;
   }
   return HG_OK;
@@ -789,18 +847,19 @@ int hg_narrow_prep_rows(hg_ctx *ctx, const hg_narrow_mat *m, uint32_t row0, uint
 int hg_narrow_launch(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                      const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                      uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                     unsigned long long *d_n_hits, const hg_floors *floors) {
+                     unsigned long long *d_n_hits, const hg_floors *floors, const hg_dense *dense) {
   return hg_narrow_launch_ex(ctx, R, r0, n_ref, i0, d_ref_norm, Q, q0, n_qry, j0, d_qry_norm, ksize, ani_th, symmetric, d_hits, cap,
-                             d_n_hits, 1, 0, nullptr, nullptr, floors);
+                             d_n_hits, 1, 0, nullptr, nullptr, floors, dense);
 }
 
 int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                         const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                         uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
                         unsigned long long *d_n_hits, uint32_t walk_mul, uint32_t walk_add, const hg_tile_feed *feed,
-                        const hg_push_plan *push, const hg_floors *floors) {
+                        const hg_push_plan *push, const hg_floors *floors, const hg_dense *dense) {
   if (n_ref == 0 || n_qry == 0) return HG_OK;
   if (floors && push) { hg_set_error("hg_narrow_launch: per-query thresholds on a multi-GPU member"); return HG_E_UNSUPPORTED; }
+  if (dense && (floors || push)) { hg_set_error("hg_narrow_launch: dense output of a search pass or a multi-GPU member"); return HG_E_UNSUPPORTED; }
   if (walk_mul == 0 || walk_add >= walk_mul) { hg_set_error("hg_narrow_launch: tile walk %u / %u", walk_add, walk_mul); return HG_E_INVALID; }
   int rc;
   const uint32_t hv_d = R->hv_d;
@@ -860,7 +919,9 @@ int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32
   cfg.gridDim = dim3(2 * n_pairs, 1, 1);
   cfg.dynamicSmemBytes = N1_SMEM_BYTES;
   static const hg_push_plan no_push = {};
-  if (push) {  // a member of several GPUs: the launch carries pusher warps that send my operand rows while the tiles are computed
+  if (dense) {
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_dense_kernel, tm_ref, tm_qry, r0, q0, ep, na, fd, no_push, *dense));
+  } else if (push) {  // a member of several GPUs: the launch carries pusher warps that send my operand rows while the tiles are computed
     cfg.blockDim = dim3(N1_THREADS + 32 * N1_PUSH_WARPS, 1, 1);
     HG_CUDA(cudaLaunchKernelEx(&cfg, dist_n1_kernel<N1_PUSH_WARPS>, tm_ref, tm_qry, r0, q0, ep, na, fd, *push, hg_floors{}));
   } else if (floors) {

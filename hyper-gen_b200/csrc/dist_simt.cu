@@ -30,17 +30,19 @@ __device__ __forceinline__ void mac8(int32_t &acc, const uint4 &a, const uint4 &
   }
 }
 
-// QF: per-query thresholds (a search pass); `fl` is not read otherwise
-template <bool QF>
-__global__ void __launch_bounds__(DS_THREADS)
-dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qry, uint32_t hv_d,
-                 hg::DistEpilogue ep, hg_floors fl) {
+// QF: per-query thresholds (a search pass); `fl` is not read otherwise.  DENSE: every live pair's dot to its cell of `dn`
+// (hg_dense), no threshold; `fl` and the hit fields of `ep` are not read.
+template <bool QF, bool DENSE>
+__device__ __forceinline__ void simt_body(const int16_t *__restrict__ ref, const int16_t *__restrict__ qry, uint32_t hv_d,
+                                          hg::DistEpilogue ep, hg_floors fl, hg_dense dn) {
   __shared__ __align__(16) unsigned char s_a[DS_TILE * DS_ROW_BYTES];
   __shared__ __align__(16) unsigned char s_b[DS_TILE * DS_ROW_BYTES];
 
   const uint32_t row0 = blockIdx.y * DS_TILE, col0 = blockIdx.x * DS_TILE;
   // symmetric: a tile whose largest global j is not above its smallest global i is empty
   if (ep.symmetric && (uint64_t)ep.j0 + col0 + DS_TILE - 1 <= (uint64_t)ep.i0 + row0) return;
+  // lower triangle: a tile with no j < i
+  if (DENSE && !dn.ld && (uint64_t)ep.j0 + col0 >= (uint64_t)ep.i0 + row0 + DS_TILE - 1) return;
 
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
   int32_t acc[4][4];
@@ -85,8 +87,26 @@ dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qr
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const uint32_t li = row0 + ty + 16 * i, lj = col0 + tx + 16 * j;
-      hg::dist_emit<QF>(ep, li < ep.n_ref && lj < ep.n_qry, li, lj, acc[i][j], fl);
+      if constexpr (DENSE) {
+        const uint32_t gi = ep.i0 + li, gj = ep.j0 + lj;
+        if (li < ep.n_ref && lj < ep.n_qry && (dn.ld || gj < gi)) *hg::dense_cell(dn, gi, gj) = acc[i][j];
+      } else {
+        hg::dist_emit<QF>(ep, li < ep.n_ref && lj < ep.n_qry, li, lj, acc[i][j], fl);
+      }
     }
+}
+
+template <bool QF>
+__global__ void __launch_bounds__(DS_THREADS)
+dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qry, uint32_t hv_d,
+                 hg::DistEpilogue ep, hg_floors fl) {
+  simt_body<QF, false>(ref, qry, hv_d, ep, fl, hg_dense{});
+}
+
+__global__ void __launch_bounds__(DS_THREADS)
+dist_simt_dense_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qry, uint32_t hv_d, hg::DistEpilogue ep,
+                       hg_dense dn) {
+  simt_body<false, true>(ref, qry, hv_d, ep, hg_floors{}, dn);
 }
 
 }  // namespace
@@ -94,7 +114,7 @@ dist_simt_kernel(const int16_t *__restrict__ ref, const int16_t *__restrict__ qr
 int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref, uint32_t i0,
                         const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry, uint32_t j0,
                         uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                        unsigned long long *d_n_hits, const hg_floors *floors) {
+                        unsigned long long *d_n_hits, const hg_floors *floors, const hg_dense *dense) {
   if (n_ref == 0 || n_qry == 0) return HG_OK;
   if (hv_d % DS_KS != 0) {
     hg_set_error("hv_d %u must be a multiple of %d", hv_d, DS_KS);
@@ -115,7 +135,9 @@ int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_
     e2.ref_norm = d_ref_norm + (size_t)y0 * DS_TILE;
     e2.n_ref = n_ref - y0 * DS_TILE;
     e2.i0 = i0 + y0 * DS_TILE;
-    if (floors)
+    if (dense)
+      dist_simt_dense_kernel<<<dim3(gx, gy), DS_THREADS, 0, ctx->stream>>>(d_ref + (size_t)y0 * DS_TILE * hv_d, d_qry, hv_d, e2, *dense);
+    else if (floors)
       dist_simt_kernel<true><<<dim3(gx, gy), DS_THREADS, 0, ctx->stream>>>(d_ref + (size_t)y0 * DS_TILE * hv_d, d_qry, hv_d, e2,
                                                                            *floors);
     else

@@ -189,6 +189,35 @@ __device__ __forceinline__ uint32_t tc_drain(const hg::DistEpilogue &ep, const h
   return n_list;
 }
 
+// Dense mode (hg_dense): the same drain without the bound, the exact dot of each of my 16 columns stored to its cell.
+__device__ __forceinline__ void tc_drain_dense(const hg::DistEpilogue &ep, const hg_dense &dn, uint32_t taddr, int c_begin, int c_end,
+                                               bool row_live, uint32_t gi, uint32_t gj0) {
+  uint32_t nh[16], nc[16], nl[16];
+  tmem_ld16(taddr + 0 * TC_BN + c_begin, nh);
+  tmem_ld16(taddr + 1 * TC_BN + c_begin, nc);
+  tmem_ld16(taddr + 2 * TC_BN + c_begin, nl);
+#pragma unroll 1
+  for (int c = c_begin; c < c_end; c += 16) {
+    uint32_t hh[16], cr[16], ll[16];
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    tmem_ld_fence(nh);
+    tmem_ld_fence(nc);
+    tmem_ld_fence(nl);
+#pragma unroll
+    for (int j = 0; j < 16; ++j) { hh[j] = nh[j]; cr[j] = nc[j]; ll[j] = nl[j]; }
+    if (c + 16 < c_end) {
+      tmem_ld16(taddr + 0 * TC_BN + c + 16, nh);
+      tmem_ld16(taddr + 1 * TC_BN + c + 16, nc);
+      tmem_ld16(taddr + 2 * TC_BN + c + 16, nl);
+    }
+    int32_t dot[16];
+#pragma unroll
+    for (int j = 0; j < 16; ++j) dot[j] = (int32_t)((((hh[j] << 7) + cr[j]) << 7) + ll[j]);  // wrapping i32, as dist.rs:147-151
+    const uint32_t n = row_live ? hg::dense_live(dn, ep, gi, gj0 + c) : 0u;
+    if (n) hg::dense_store16(dn, gi, gj0 + c, n, dot);
+  }
+}
+
 // ---- the kernel: persistent CTA pairs, cta_group::2, 256 x 128 tiles ---------------------------
 constexpr int T2_STAGES = 4;
 constexpr int T2_A_BYTES = 128 * TC_BK;               // my 128 ref rows, one limb plane
@@ -249,13 +278,14 @@ struct PairTiles {
   }
 };
 
-// QF: per-query thresholds (a search pass, PUSHW = 0 only); `fl` is not read otherwise
-template <int PUSHW, bool QF = false>
-__global__ void __launch_bounds__(TC_THREADS + 32 * PUSHW, 1)
-dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
-                uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len,
-                hg::DistEpilogue ep, const unsigned long long *__restrict__ ref_sq, const unsigned long long *__restrict__ qry_sq,
-                uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan, hg_floors fl) {
+// QF: per-query thresholds (a search pass, PUSHW = 0 only); `fl` is not read otherwise.  DENSE (PUSHW = 0, no QF): every
+// live pair's dot to its cell of `dn` (hg_dense) instead of the bound, the exact epilogue and the append.
+template <int PUSHW, bool QF, bool DENSE>
+__device__ __forceinline__ void tc2_body(const CUtensorMap &tm_ref, const CUtensorMap &tm_qry, uint32_t ref_plane_rows, uint32_t ref_row_base,
+                                         uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len, const hg::DistEpilogue &ep,
+                                         const unsigned long long *ref_sq, const unsigned long long *qry_sq,
+                                         uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const hg_push_plan &plan,
+                                         const hg_floors &fl, const hg_dense &dn) {
   uint32_t rank;  // 0 = leader (issues the MMAs, owns the full / tmem-empty barriers), 1 = peer
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
   if (feed.seq_ptr) feed.seq = *feed.seq_ptr;
@@ -408,19 +438,24 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
         asm volatile("bar.sync 1, %0;" ::"r"(32 * TC_EPI_WARPS) : "memory");
         tr = tc_row_bound<QF>(ep, fl, ref_sq, li);
       };
-      if (early) bounds();
+      if (!DENSE && early) bounds();
       // my 128 x 128 part of the tile may be empty (below the diagonal, or past the last ref row)
       const bool mine_empty = row0 >= ep.n_ref || (ep.symmetric && (uint64_t)ep.j0 + col0 + TC_BN - 1 <= (uint64_t)ep.i0 + row0);
       mbar_wait_cluster(accum_bar, tile_n & 1u);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       if (!early) {  // the producer has seen this tile's arrival flags; so do we now (an acquire, returns at once)
         hg::feed_wait(feed, tiles.need, have_l);
-        bounds();
+        if (!DENSE) bounds();
       }
       uint32_t n_list = 0;
-      if (!mine_empty)
+      if constexpr (DENSE) {
+        if (!mine_empty)
+          tc_drain_dense(ep, dn, tmem_base + ((q * 32u) << 16), half * (TC_BN / 2), (half + 1) * (TC_BN / 2), li < ep.n_ref, ep.i0 + li,
+                         ep.j0 + col0);
+      } else if (!mine_empty) {
         n_list = tc_drain<QF>(ep, fl, tmem_base + ((q * 32u) << 16), half * (TC_BN / 2), (half + 1) * (TC_BN / 2), s_tq, tr,
                           li < ep.n_ref, q * 32 + lane, row0, col0, list, anis, 0u);
+      }
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(te);  // this warp's TMEM reads are done: the next tile's MMAs may start
@@ -435,6 +470,25 @@ dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constan
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
   }
+}
+
+template <int PUSHW, bool QF = false>
+__global__ void __launch_bounds__(TC_THREADS + 32 * PUSHW, 1)
+dist_tc2_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
+                uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len,
+                hg::DistEpilogue ep, const unsigned long long *__restrict__ ref_sq, const unsigned long long *__restrict__ qry_sq,
+                uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed, const __grid_constant__ hg_push_plan plan, hg_floors fl) {
+  tc2_body<PUSHW, QF, false>(tm_ref, tm_qry, ref_plane_rows, ref_row_base, qry_plane_rows, qry_row_base, k_len, ep, ref_sq, qry_sq, walk_mul,
+                             walk_add, feed, plan, fl, hg_dense{});
+}
+
+__global__ void __launch_bounds__(TC_THREADS, 1)
+dist_tc2_dense_kernel(const __grid_constant__ CUtensorMap tm_ref, const __grid_constant__ CUtensorMap tm_qry,
+                      uint32_t ref_plane_rows, uint32_t ref_row_base, uint32_t qry_plane_rows, uint32_t qry_row_base, uint32_t k_len,
+                      hg::DistEpilogue ep, uint32_t walk_mul, uint32_t walk_add, hg_tile_feed feed,
+                      const __grid_constant__ hg_push_plan plan, hg_dense dn) {
+  tc2_body<0, false, true>(tm_ref, tm_qry, ref_plane_rows, ref_row_base, qry_plane_rows, qry_row_base, k_len, ep, nullptr, nullptr, walk_mul,
+                           walk_add, feed, plan, hg_floors{}, dn);
 }
 
 // i16 -> two s8 limb planes: plane 0 = h, plane 1 = l, `plane_stride` bytes apart; `out` points at the first element
@@ -489,6 +543,7 @@ static int tc_attrs(hg_ctx *ctx) {
     HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
     HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<TC_PUSH_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
     HG_CUDA(cudaFuncSetAttribute(dist_tc2_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
+    HG_CUDA(cudaFuncSetAttribute(dist_tc2_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM_BYTES));
     ctx->tc_attr_set = 1;
   }
   return HG_OK;
@@ -546,9 +601,10 @@ int hg_tc_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t
 // rows [r0, r0 + n_ref) of R against rows [q0, q0 + n_qry) of Q (both split); norms point at the windows' first rows
 int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                  const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
-                 float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, const hg_floors *floors) {
+                 float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, const hg_floors *floors,
+                 const hg_dense *dense) {
   return hg_tc_launch_ex(ctx, R, r0, n_ref, i0, d_ref_norm, Q, q0, n_qry, j0, d_qry_norm, ksize, ani_th, symmetric, d_hits, cap,
-                         d_n_hits, 1, 0, nullptr, nullptr, floors);
+                         d_n_hits, 1, 0, nullptr, nullptr, floors, dense);
 }
 
 int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int8_t *planes, hg_tc_mat *m) {
@@ -563,9 +619,10 @@ int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_
 int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                     const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
                     float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, uint32_t walk_mul,
-                    uint32_t walk_add, const hg_tile_feed *feed, const hg_push_plan *push, const hg_floors *floors) {
+                    uint32_t walk_add, const hg_tile_feed *feed, const hg_push_plan *push, const hg_floors *floors, const hg_dense *dense) {
   if (n_ref == 0 || n_qry == 0) return HG_OK;
   if (floors && push) { hg_set_error("hg_tc_launch: per-query thresholds on a multi-GPU member"); return HG_E_UNSUPPORTED; }
+  if (dense && (floors || push)) { hg_set_error("hg_tc_launch: dense output of a search pass or a multi-GPU member"); return HG_E_UNSUPPORTED; }
   hg_tile_feed fd = {};
   if (feed) fd = *feed;
   if (walk_mul == 0 || walk_add >= walk_mul) { hg_set_error("hg_tc_launch: tile walk %u / %u", walk_add, walk_mul); return HG_E_INVALID; }
@@ -611,7 +668,10 @@ int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref
   cfg.stream = ctx->stream;
   static const hg_push_plan no_push = {};
   const unsigned long long *rsq = R->sq + r0, *qsq = Q->sq + q0;  // indexed like the norms
-  if (push) {  // a member of several GPUs: pusher warps send my limb-plane rows while the tiles are computed
+  if (dense) {
+    HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_dense_kernel, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, walk_mul, walk_add, fd,
+                               no_push, *dense));
+  } else if (push) {  // a member of several GPUs: pusher warps send my limb-plane rows while the tiles are computed
     cfg.blockDim = dim3(TC_THREADS + 32 * TC_PUSH_WARPS, 1, 1);
     HG_CUDA(cudaLaunchKernelEx(&cfg, dist_tc2_kernel<TC_PUSH_WARPS>, tm_ref, tm_qry, R->n_rows, r0, Q->n_rows, q0, k_len, ep, rsq, qsq,
                                walk_mul, walk_add, fd, *push, hg_floors{}));

@@ -191,6 +191,10 @@ struct hg_ctx {
   // phases (-1: not run or profiling off)
   uint64_t derep_stats[4];
   float derep_ms[4];
+  // the last ANI matrix run (hg_ani_matrix_stats): bands, entries, bytes copied to the host, kernel path; device ms of
+  // its stages (-1: not run or profiling off)
+  uint64_t matrix_stats[4];
+  float matrix_ms[4];
 };
 
 // stage boundaries: 0 start, 1 after staging/memsets, 2 after k-mer hash, 3 after encode,
@@ -267,6 +271,19 @@ struct hg_floors {
   const float *cfrac_row;  // device scalar (0: no positive cfrac)
 };
 
+// Dense output of a dist launch (hg_ani_matrix_*): the exact i32 dot of every live pair goes to its cell, in place of
+// the threshold and the append (a conversion kernel turns the cells into ANI afterwards).  Cell (i, j) of global ref row
+// i and query column j lies at base + hg_dense_row(i) - hg_dense_row(row_base) + j: base holds row `row_base` first.
+// ld > 0: a rectangle with rows ld apart; ld == 0: the strict lower triangle (row i at i (i - 1) / 2, only j < i written).
+struct hg_dense {
+  int32_t *base;
+  uint64_t ld;
+  uint32_t row_base;
+};
+__host__ __device__ inline uint64_t hg_dense_row(const hg_dense &d, uint32_t i) {
+  return d.ld ? (uint64_t)i * d.ld : (uint64_t)i * ((uint64_t)i - 1) / 2;
+}
+
 // ---- kernel launchers (all asynchronous on ctx->stream) ----
 
 struct hg_genome_desc {   // per genome, device-visible
@@ -297,7 +314,12 @@ int hg_launch_unpack(hg_ctx *ctx, const uint8_t *d_packed, uint64_t row_stride,
 int hg_launch_dist_simt(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm, uint32_t n_ref,
                         uint32_t i0, const int16_t *d_qry, const int32_t *d_qry_norm, uint32_t n_qry,
                         uint32_t j0, uint32_t hv_d, uint32_t ksize, float ani_th, int symmetric,
-                        hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, const hg_floors *floors = nullptr);
+                        hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, const hg_floors *floors = nullptr,
+                        const hg_dense *dense = nullptr);
+// rows [a, a + h) of a dense output (every cell the launches wrote): dot -> ani_from_dot in place, f32 bits over i32.
+// Rectangle rows hold n_cols cells, lower-triangle row i holds i.  Norms are indexed by global row / column.
+int hg_launch_ani_convert(hg_ctx *ctx, const hg_dense &d, uint32_t a, uint32_t h, uint32_t n_cols, const int32_t *d_ref_norm,
+                          const int32_t *d_qry_norm, uint32_t ksize);
 // A dist launch that is one member of several GPUs (csrc/peer.cu) walks a host-built list of ITS tiles instead of the
 // arithmetic enumeration, ordered by when the rows they read arrive, and its TMA producer waits for the arrival flags
 // of those rows: the operand exchange over NVLink overlaps the tile computation.
@@ -365,14 +387,14 @@ int hg_tc_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t
 int hg_tc_launch(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                  const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
                  float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits,
-                 const hg_floors *floors = nullptr);
+                 const hg_floors *floors = nullptr, const hg_dense *dense = nullptr);
 // `planes` holds hg_tc_mat_bytes(n_rows, hv_d)
 int hg_tc_attach(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint32_t hv_d, int8_t *planes, hg_tc_mat *m);
 int hg_tc_launch_ex(hg_ctx *ctx, const hg_tc_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                     const hg_tc_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm, uint32_t ksize,
                     float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap, unsigned long long *d_n_hits, uint32_t walk_mul,
                     uint32_t walk_add, const hg_tile_feed *feed = nullptr, const hg_push_plan *push = nullptr,
-                    const hg_floors *floors = nullptr);
+                    const hg_floors *floors = nullptr, const hg_dense *dense = nullptr);
 void hg_tc_tile_shape(uint32_t *rows, uint32_t *cols);
 // single s8 plane (x = 2a + s) + sparse outlier corrections (dist_narrow.cu): one matrix in that form, prepared
 // piecewise (rows as they arrive over PCIe) or at once
@@ -404,13 +426,13 @@ int hg_narrow_norm_flags(hg_ctx *ctx, const int16_t *d_hv, uint32_t n_rows, uint
 int hg_narrow_launch(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                      const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                      uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
-                     unsigned long long *d_n_hits, const hg_floors *floors = nullptr);
+                     unsigned long long *d_n_hits, const hg_floors *floors = nullptr, const hg_dense *dense = nullptr);
 // as hg_narrow_launch for one member of `walk_mul` GPUs sharing the tile enumeration (takes tiles walk_add, walk_add + walk_mul, ...)
 int hg_narrow_launch_ex(hg_ctx *ctx, const hg_narrow_mat *R, uint32_t r0, uint32_t n_ref, uint32_t i0, const int32_t *d_ref_norm,
                         const hg_narrow_mat *Q, uint32_t q0, uint32_t n_qry, uint32_t j0, const int32_t *d_qry_norm,
                         uint32_t ksize, float ani_th, int symmetric, hg_hit *d_hits, uint64_t cap,
                         unsigned long long *d_n_hits, uint32_t walk_mul, uint32_t walk_add, const hg_tile_feed *feed = nullptr,
-                        const hg_push_plan *push = nullptr, const hg_floors *floors = nullptr);
+                        const hg_push_plan *push = nullptr, const hg_floors *floors = nullptr, const hg_dense *dense = nullptr);
 void hg_narrow_tile_shape(uint32_t *rows, uint32_t *cols);
 int hg_narrow_verdict(hg_ctx *ctx, const hg_narrow_mat *A, const hg_narrow_mat *B, int32_t *absmax_out, uint64_t *outliers_out);
 int hg_launch_int_peak(hg_ctx *ctx, int which, uint32_t iters, uint32_t *d_sink, uint32_t blocks);
@@ -536,3 +558,22 @@ int hg_launch_derep_greedy(hg_ctx *ctx, uint32_t a, uint32_t w, uint8_t *d_cover
 // every row against the rep matrix (d_order NULL: the identity); *d_status |= 1 if a non-representative found none
 int hg_launch_derep_finalize(hg_ctx *ctx, const uint8_t *d_is_rep, const uint32_t *d_rep_list, const hg_hit *d_out,
                              const uint32_t *d_n_found, const uint32_t *d_order, uint32_t n, uint32_t *d_rep, uint32_t *d_status);
+
+// ---- the all-vs-all ANI matrix (api.cu, matrix.cu): DESIGN.md §4.11 ----
+// cells of a matrix run: n_ref x n_qry, or n_ref (n_ref - 1) / 2 in lower mode
+uint64_t hg_matrix_entries(uint32_t n_ref, uint32_t n_qry, int lower);
+// The arguments of a matrix entry that do not describe rows (`who` names it): hv_d, path, lower (and `same` rows for it),
+// ld >= n_qry for a rectangle, out when there is something to write.
+int hg_matrix_check(const char *who, bool same, uint32_t n_ref, uint32_t n_qry, uint32_t hv_d, int path, int lower, const void *out,
+                    uint64_t ld);
+// A host output buffer page-locked for the call: kept as it is when it already is (hg_host_alloc, registered), else
+// registered (portable: every context's copies see it) and unregistered when this goes out of scope.
+struct HostPin {
+  void *ptr = nullptr;
+  int pin(void *p, uint64_t bytes);
+  ~HostPin();
+};
+// The matrix cells of checked packed rows: ref rows [first, R.n) against Q (lower: R == Q, the strict lower triangle),
+// into the page-locked host matrix `out`, which holds row `first` at offset 0 (rectangle: rows ld apart).
+int hg_matrix_packed_run(hg_ctx *ctx, const hg_packed_rows &R, const hg_packed_rows &Q, bool same, uint32_t hv_d, uint32_t ksize, int path,
+                         bool lower, uint32_t first, float *out, uint64_t ld);

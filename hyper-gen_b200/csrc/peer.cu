@@ -1321,3 +1321,69 @@ extern "C" int hg_group_cluster_packed(hg_group *g, const uint8_t *packed, uint6
   }
   return hg_cluster_finish(c0, merged, n, rep, n_clusters);
 }
+
+// hg_ani_matrix_packed over all GPUs of the group (DESIGN.md §4.11).  The ref rows are cut into one contiguous range per
+// member with about the same number of output entries: b_k = n sqrt(k / parts) in lower mode, n_ref k / parts for a
+// rectangle.  Member m copies the packed rows it reads over its own PCIe link (lower: rows [0, b_m+1); rectangle: its
+// range and every query row), computes its bands and copies them straight into its part of `out`, which is page-locked
+// once for all members.  As many members as give each at least 2^23 entries take part (cluster's rule).  One host thread
+// per GPU drives its members; members that share a device ordinal run one after another.  Every cell is the exact value
+// whatever the kernel, so the result is byte-identical to hg_ani_matrix_packed.
+extern "C" int hg_group_ani_matrix_packed(hg_group *g, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                                          const int32_t *ref_norm2, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                                          const uint8_t *qry_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d,
+                                          uint32_t ksize, int path, int lower, float *out, uint64_t ld) {
+  const char *who = "hg_group_ani_matrix_packed";
+  if (!g) { hg_set_error("%s: NULL argument", who); return HG_E_INVALID; }
+  hg_packed_rows R = {ref_packed, ref_stride, ref_bits, ref_norm2, n_ref}, Q = {qry_packed, qry_stride, qry_bits, qry_norm2, n_qry};
+  const bool same = R.packed == Q.packed && R.bits == Q.bits && R.norm == Q.norm && R.n == Q.n;
+  int rc;
+  if ((rc = hg_packed_args_check(who, R, Q, hv_d)) || (rc = hg_matrix_check(who, same, n_ref, n_qry, hv_d, path, lower, out, ld))) return rc;
+  const uint64_t entries = hg_matrix_entries(n_ref, n_qry, lower);
+  const int parts = (int)std::min<uint64_t>((uint64_t)g->n, std::max<uint64_t>(1, entries >> 23));
+  if (parts == 1)
+    return hg_ani_matrix_packed(g->ctx[0], ref_packed, ref_stride, ref_bits, ref_norm2, n_ref, qry_packed, qry_stride, qry_bits, qry_norm2,
+                                n_qry, hv_d, ksize, path, lower, out, ld);
+  bool same2;
+  if ((rc = hg_packed_rows_check(who, &R, &Q, hv_d, &same2))) return rc;
+  std::vector<uint32_t> b(parts + 1, n_ref);
+  b[0] = 0;
+  for (int k = 1; k < parts; ++k) {
+    const uint32_t want = lower ? (uint32_t)std::lround((double)n_ref * std::sqrt((double)k / parts))
+                                : (uint32_t)((uint64_t)n_ref * k / parts);
+    b[k] = std::min(n_ref, std::max(b[k - 1], want));
+  }
+  HostPin pin;
+  HG_CUDA(cudaSetDevice(g->ctx[0]->device));
+  if ((rc = pin.pin(out, (lower ? entries : (uint64_t)(n_ref - 1) * ld + n_qry) * 4))) return rc;
+  std::vector<int> rcs(parts, HG_OK);
+  std::vector<std::string> msgs(parts);
+  auto member = [&](int m) -> int {
+    hg_ctx *c = g->ctx[m];
+    if (b[m] == b[m + 1]) return HG_OK;
+    if (lower)
+      return hg_matrix_packed_run(c, R.rows(0, b[m + 1]), R.rows(0, b[m + 1]), true, hv_d, ksize, path, true, b[m],
+                                  out + (uint64_t)b[m] * ((uint64_t)b[m] - 1) / 2, ld);
+    return hg_matrix_packed_run(c, R.rows(b[m], b[m + 1] - b[m]), Q, false, hv_d, ksize, path, false, 0, out + (uint64_t)b[m] * ld, ld);
+  };
+  for (int k = 0; k < g->n; ++k) {  // a member without rows reports no run
+    memset(g->ctx[k]->matrix_stats, 0, sizeof(g->ctx[k]->matrix_stats));
+    for (float &t : g->ctx[k]->matrix_ms) t = -1.0f;
+  }
+  std::vector<std::thread> th;
+  for (int k = 0; k < parts; ++k) {
+    bool first_on_device = true;
+    for (int l = 0; l < k; ++l) first_on_device &= g->ctx[l]->device != g->ctx[k]->device;
+    if (!first_on_device) continue;
+    th.emplace_back([&, k]() {
+      for (int m = k; m < parts; ++m) {
+        if (g->ctx[m]->device != g->ctx[k]->device) continue;
+        if ((rcs[m] = member(m))) msgs[m] = hg_last_error();
+      }
+    });
+  }
+  for (auto &t : th) t.join();
+  for (int k = 0; k < parts; ++k)
+    if (rcs[k]) { hg_set_error("GPU %d (rows %u..%u): %s", g->ctx[k]->device, b[k], b[k + 1], msgs[k].c_str()); return rcs[k]; }
+  return HG_OK;
+}

@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 
 import numpy as np
 
@@ -24,6 +25,7 @@ EXPORTS = [
     "hg_search_dev", "hg_search_packed", "hg_search_stats", "hg_search_merge_dev",
     "hg_cluster_dev", "hg_cluster_packed", "hg_cluster_union_dev", "hg_cluster_stats",
     "hg_derep_dev", "hg_derep_packed", "hg_derep_stats",
+    "hg_ani_matrix_dev", "hg_ani_matrix_packed", "hg_group_ani_matrix_packed", "hg_ani_matrix_stats",
     "hg_group_create", "hg_group_destroy", "hg_group_size", "hg_group_ctx", "hg_group_sketch_fasta_batch", "hg_group_dist_packed",
     "hg_group_search_packed", "hg_group_cluster_packed",
     "hg_peer_window_need", "hg_peer_create", "hg_peer_connect", "hg_peer_create_local", "hg_peer_destroy", "hg_peer_rank",
@@ -122,6 +124,13 @@ def load() -> C.CDLL:
     L.hg_derep_packed.restype = i32
     L.hg_derep_packed.argtypes = [vp, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, vp, vp, C.POINTER(u32)]
     L.hg_derep_stats.restype = i32; L.hg_derep_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
+    L.hg_ani_matrix_dev.restype = i32
+    L.hg_ani_matrix_dev.argtypes = [vp, vp, vp, u32, vp, vp, u32, u32, u32, i32, i32, vp, u64]
+    L.hg_ani_matrix_packed.restype = i32
+    L.hg_ani_matrix_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, i32, i32, vp, u64]
+    L.hg_group_ani_matrix_packed.restype = i32
+    L.hg_group_ani_matrix_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, i32, i32, vp, u64]
+    L.hg_ani_matrix_stats.restype = i32; L.hg_ani_matrix_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
     L.hg_group_create.restype = i32; L.hg_group_create.argtypes = [i32, vp, C.POINTER(vp)]
     L.hg_group_destroy.restype = None; L.hg_group_destroy.argtypes = [vp]
     L.hg_group_size.restype = i32; L.hg_group_size.argtypes = [vp]
@@ -250,6 +259,52 @@ def _cluster_packed(fn, h, packed, bits, norm2, hv_d, ksize, ani_th, path):
 def _cluster_stats(ctx_handle):
     counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
     _check(load().hg_cluster_stats(ctx_handle, counts, ms))
+    return [int(x) for x in counts], [float(x) for x in ms]
+
+
+def pinned_empty(shape, dtype) -> np.ndarray:
+    """an uninitialised numpy array in page-locked host memory (hg_host_alloc), freed (hg_host_free) with its last view:
+    the GPU copies into it at link rate, where a pageable array has to be page-locked for every call"""
+    dtype = np.dtype(dtype)
+    count = int(np.prod(shape))
+    nbytes = max(1, count * dtype.itemsize)
+    p = C.c_void_p()
+    _check(load().hg_host_alloc(nbytes, C.byref(p)))
+    raw = (C.c_uint8 * nbytes).from_address(p.value)
+    weakref.finalize(raw, load().hg_host_free, p.value).atexit = False  # the numpy array below keeps `raw` alive
+    return np.frombuffer(raw, np.uint8, count * dtype.itemsize).view(dtype).reshape(shape)
+
+
+def _ani_matrix_packed(fn, h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize, path, lower, out):
+    """hg_ani_matrix_packed / hg_group_ani_matrix_packed (fn) on the context / group h.  lower: the strict lower triangle
+    of the ref rows (the query must be the same arrays; n (n - 1) / 2 float32), else the n_ref x n_qry rectangle.  out: None, or a float32
+    array to write into (lower: 1-D, at least n (n - 1) / 2 entries; rectangle: 1-D with rows n_qry apart, or 2-D with
+    n_ref rows of at least n_qry contiguous entries, rows its ld apart).  None: a new page-locked array (pinned_empty)."""
+    r, q = _packed_rows(ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2)
+    n_ref, n_qry = r[0].shape[0], q[0].shape[0]
+    if out is None:
+        out = pinned_empty(n_ref * (n_ref - 1) // 2 if lower else (n_ref, n_qry), np.float32)
+    if out.dtype != np.float32 or not (out.flags.c_contiguous or (out.ndim == 2 and out.strides[1] == 4)):
+        raise ValueError("out must be float32 with contiguous rows")
+    if lower:
+        if out.ndim != 1 or out.size < n_ref * (n_ref - 1) // 2:
+            raise ValueError("out must be 1-D with at least %d entries" % (n_ref * (n_ref - 1) // 2))
+        ld = 0
+    elif out.ndim == 2:
+        ld = out.strides[0] // 4
+        if out.shape[0] < n_ref or out.shape[1] < n_qry or out.strides[0] % 4 or out.strides[0] < 0:
+            raise ValueError("out must have at least %d rows of %d entries" % (n_ref, n_qry))
+    else:
+        ld = n_qry
+        if out.ndim != 1 or out.size < n_ref * n_qry:
+            raise ValueError("out must be 1-D with at least %d entries, or 2-D" % (n_ref * n_qry))
+    _check(fn(h, *_row_args(r), *_row_args(q), hv_d, ksize, path, int(lower), _ptr(out), ld))
+    return out
+
+
+def _ani_matrix_stats(ctx_handle):
+    counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
+    _check(load().hg_ani_matrix_stats(ctx_handle, counts, ms))
     return [int(x) for x in counts], [float(x) for x in ms]
 
 
@@ -536,6 +591,26 @@ class Context:
                                       _ptr(rep), C.byref(n_reps)))
         return rep, int(n_reps.value)
 
+    def ani_matrix_dev(self, d_ref, d_ref_norm2, n_ref, d_qry, d_qry_norm2, n_qry, hv_d, ksize, path, lower, d_out, ld=0):
+        """hg_ani_matrix_dev: device pointers (ints); d_out (float32) receives the strict lower triangle (lower) or the
+        n_ref x n_qry rectangle with rows ld apart.  Returns when the result is complete."""
+        _check(load().hg_ani_matrix_dev(self._h, d_ref, d_ref_norm2, n_ref, d_qry, d_qry_norm2, n_qry, hv_d, ksize, path, int(lower),
+                                        d_out, ld))
+
+    def ani_matrix_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed=None, qry_bits=None, qry_norm2=None, hv_d=4096, ksize=21,
+                          path=0, lower=True, out=None):
+        """hg_ani_matrix_packed: packed sketch rows -> float32 ANI of every pair: the strict lower triangle of the ref rows
+        (lower, n (n - 1) / 2 entries in PHYLIP order) or the ref x query rectangle (a square when qry_packed is None)."""
+        if qry_packed is None:
+            qry_packed, qry_bits, qry_norm2 = ref_packed, ref_bits, ref_norm2
+        return _ani_matrix_packed(load().hg_ani_matrix_packed, self._h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2,
+                                  hv_d, ksize, path, lower, out)
+
+    def ani_matrix_stats(self):
+        """hg_ani_matrix_stats of the last matrix run -> ([bands, entries, bytes copied to the host, path], [ms of row
+        preparation, band kernels, conversion, copies to the host])"""
+        return _ani_matrix_stats(self._h)
+
     def derep_stats(self):
         """hg_derep_stats of the last derep run -> ([column chunks, windows, linked pairs, representatives], [ms of
         preparing the rows, dist windows, mark hooks + greedy steps, assignment] (-1: not run or profiling off))"""
@@ -717,3 +792,15 @@ class Group:
     def cluster_stats(self, i: int = 0):
         """Context.cluster_stats of member i's part of the last group cluster run"""
         return _cluster_stats(load().hg_group_ctx(self._h, i))
+
+    def ani_matrix_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed=None, qry_bits=None, qry_norm2=None, hv_d=4096, ksize=21,
+                          path=0, lower=True, out=None):
+        """hg_group_ani_matrix_packed: Context.ani_matrix_packed with the ref rows split over the GPUs; same bytes."""
+        if qry_packed is None:
+            qry_packed, qry_bits, qry_norm2 = ref_packed, ref_bits, ref_norm2
+        return _ani_matrix_packed(load().hg_group_ani_matrix_packed, self._h, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits,
+                                  qry_norm2, hv_d, ksize, path, lower, out)
+
+    def ani_matrix_stats(self, i: int = 0):
+        """Context.ani_matrix_stats of member i's part of the last group matrix run"""
+        return _ani_matrix_stats(load().hg_group_ctx(self._h, i))

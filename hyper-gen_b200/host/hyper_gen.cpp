@@ -24,9 +24,14 @@
 //       greedy dereplication at ANI >= -a: representatives taken in priority order (-O file: file order; -O size:
 //       descending hv_norm_2, ties by file index), every other sketch with its closest representative; the lines of
 //       `cluster`, each cluster's representative line first.  On one GPU (hg_derep_packed).
+//   hyper-gen triangle -r <sketch> -o <out>
+//       the ANI of every pair in the PHYLIP lower-triangular layout mash and skani print: n on the first line, then
+//       per sketch its name and, tab-separated, its ANI with every earlier sketch (`dist`'s %u.%03u).  The rows are
+//       split over every visible GPU (hg_group_ani_matrix_packed); HG_GPUS=n limits it.
 // The GPU path is the only path (`-D gpu` is implied): there is no CPU fallback.
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -455,6 +460,65 @@ void cluster(const types::SketchCluster &sc) {
 
 }  // namespace cluster
 
+namespace triangle {
+
+// Rows [r0, r1) of the text: sketch i's name, then a tab and ANI(i, j) for every j < i, as `dist` prints it
+// (thousandths rounded to nearest even, as ani_milli_kernel rounds them).
+static void format_rows(const std::vector<types::FileSketch> &sk, const float *tri, size_t r0, size_t r1, std::string &out) {
+  char buf[32];
+  for (size_t i = r0; i < r1; i++) {
+    out += sk[i].file_str;
+    const float *row = tri + i * (i - 1) / 2;
+    for (size_t j = 0; j < i; j++) {
+      const uint32_t m = (uint32_t)llrint((double)row[j] * 1000.0);
+      const int len = snprintf(buf, sizeof(buf), "\t%u.%03u", m / 1000u, m % 1000u);
+      out.append(buf, (size_t)len);
+    }
+    out += '\n';
+  }
+}
+
+void triangle(const std::string &path_sketch, const std::string &out_file) {
+  using clk = std::chrono::steady_clock;
+  auto ms = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
+  const auto t0 = clk::now();
+  auto sk = utils::load_sketch(path_sketch);
+  if (sk.empty()) die("empty sketch file");
+  const size_t D = sk[0].hv_d, n = sk.size();
+  const dist::Stacked s = dist::stack(sk, D);
+  const uint64_t entries = (uint64_t)n * (n - 1) / 2;
+  float *tri = nullptr;  // page-locked: the bands are copied straight into it
+  if (entries) check(hg_host_alloc(entries * 4, (void **)&tri), "hg_host_alloc");
+  const auto t1 = clk::now();
+  hg_group *group = open_group();
+  check(hg_group_ani_matrix_packed(group, s.packed.data(), 2 * D, s.bits.data(), s.norm.data(), (uint32_t)n, s.packed.data(), 2 * D,
+                                   s.bits.data(), s.norm.data(), (uint32_t)n, (uint32_t)D, sk[0].ksize, 0, 1, tri, 0),
+        "hg_group_ani_matrix_packed");
+  hg_group_destroy(group);
+  const auto t2 = clk::now();
+  // formatting: row ranges of about equal text per thread (row i has i entries)
+  const size_t n_th = std::max<size_t>(1, std::min<size_t>(std::thread::hardware_concurrency(), n / 64 + 1));
+  std::vector<size_t> cut(n_th + 1, n);
+  cut[0] = 0;
+  for (size_t k = 1; k < n_th; k++) cut[k] = std::max(cut[k - 1], (size_t)llround((double)n * std::sqrt((double)k / (double)n_th)));
+  std::vector<std::string> part(n_th);
+  part[0] = std::to_string(n) + "\n";
+  std::vector<std::thread> th;
+  for (size_t k = 0; k < n_th; k++) th.emplace_back([&, k]() { format_rows(sk, tri, cut[k], cut[k + 1], part[k]); });
+  for (auto &t : th) t.join();
+  const auto t3 = clk::now();
+  std::ofstream f(out_file, std::ios::binary);
+  if (!f) die("Dump triangle file failed!");
+  for (const std::string &p : part) f.write(p.data(), (std::streamsize)p.size());
+  f.close();
+  if (tri) hg_host_free(tri);
+  const auto t4 = clk::now();
+  fprintf(stdout, "Output %zu sketches, %llu ANIs to file %s (ms: load %.1f, GPU %.1f, format %.1f on %zu threads, write %.1f)\n", n,
+          (unsigned long long)entries, out_file.c_str(), ms(t0, t1), ms(t1, t2), ms(t2, t3), n_th, ms(t3, t4));
+}
+
+}  // namespace triangle
+
 namespace derep {
 
 void derep(const types::SketchDerep &sd) {
@@ -484,7 +548,7 @@ void derep(const types::SketchDerep &sd) {
 }  // namespace derep
 
 int main(int argc, char **argv) {
-  if (argc < 2) die("usage: hyper-gen <sketch|dist|search|cluster|derep> ...");
+  if (argc < 2) die("usage: hyper-gen <sketch|dist|search|cluster|derep|triangle> ...");
   const std::string mode = argv[1];
   types::SketchParams sp;
   types::SketchDist sd;
@@ -535,6 +599,9 @@ int main(int argc, char **argv) {
     if (sr.path_sketch.empty() || sr.out_file.empty()) die("derep needs -r -o");
     if (ani_given) sr.ani_th = sd.ani_threshold;
     derep::derep(sr);
+  } else if (mode == "triangle") {
+    if (sc.path_sketch.empty() || sc.out_file.empty()) die("triangle needs -r -o");
+    triangle::triangle(sc.path_sketch, sc.out_file);
   } else {
     die("unknown subcommand " + mode);
   }

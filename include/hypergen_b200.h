@@ -471,6 +471,49 @@ HG_API int hg_derep_packed(hg_ctx *ctx, const uint8_t *packed, uint64_t stride, 
  * steps, the assignment (gather + search + finalize)} (-1 where not run or profiling is off, see hg_set_profiling). */
 HG_API int hg_derep_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
 
+/* ---- the all-vs-all ANI matrix ----------------------------------------------------------------------------------
+ * Entry (i, j) is bit for bit the `ani` that hg_dist(..., ani_th = 0, symmetric = 0) reports for ref row i and query row
+ * j (clamped to [0, 100], NaN as 0: that call reports every pair), through every kernel and where the i32 norms and
+ * denominators wrap.  f32 values.  Two layouts, chosen by `lower`:
+ *   lower = 0, rectangle: out[i * ld + j] for every i < n_ref, j < n_qry, with ld >= n_qry; the cells between rows are
+ *     never written.  With the same rows as ref and query it is the full square; the diagonal is whatever the kernel
+ *     gives the self pair.
+ *   lower = 1, strict lower triangle of one set: ref and query must be the same rows (same pointers and n), else
+ *     HG_E_INVALID.  Row i holds j < i at out[i (i - 1) / 2 + j]: n (n - 1) / 2 entries, the PHYLIP lower-triangular
+ *     order.  Only these pairs are copied, and only the band's diagonal block computes more.
+ * n = 0, n = 1 in lower mode, or an empty rectangle: HG_OK, nothing written.  Every offset is 64-bit.
+ *   path   as hg_cluster_dev (0 auto, 1 SIMT, 2 two-limb, 3 single plane) with the same choice and fallbacks;
+ *          hg_dist_last_path / hg_dist_last_reason report the run.
+ * The rows are computed in bands of ref rows (HG_MATRIX_BAND_BYTES of output each, read at every call; default 64 MiB):
+ * band k + 1's kernel runs while band k's cells are converted and copied (DESIGN.md §4.11).  Every entry returns with
+ * its result complete. */
+/* Rows, norms and output in HBM; the whole output must fit on the device. */
+HG_API int hg_ani_matrix_dev(hg_ctx *ctx, const int16_t *d_ref, const int32_t *d_ref_norm2, uint32_t n_ref, const int16_t *d_qry,
+                             const int32_t *d_qry_norm2, uint32_t n_qry, uint32_t hv_d, uint32_t ksize, int path, int lower,
+                             float *d_out, uint64_t ld);
+/* Rows as the sketch file holds them (as hg_dist_packed), output in host memory; the output never has to fit on the
+ * device.  A page-locked `out` (hg_host_alloc or registered) is copied into directly; any other is registered for the
+ * call. */
+HG_API int hg_ani_matrix_packed(hg_ctx *ctx, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                                const int32_t *ref_norm2, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                                const uint8_t *qry_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d, uint32_t ksize,
+                                int path, int lower, float *out, uint64_t ld);
+/* hg_ani_matrix_packed over the GPUs of the group: the ref rows cut into one contiguous range per member with about the
+ * same number of output entries (in lower mode the boundaries grow like sqrt).  A member copies the packed rows it needs
+ * over its own link (lower: rows [0, end of its range); rectangle: its range and every query row) and writes its bands
+ * straight into `out`.  As many members as give each at least 2^23 entries take part; with one, hg_ani_matrix_packed on
+ * member 0.  Members that share a device ordinal run one after another.  The result is byte-identical to
+ * hg_ani_matrix_packed; hg_ani_matrix_stats on hg_group_ctx(g, m) reports member m's part. */
+HG_API int hg_group_ani_matrix_packed(hg_group *g, const uint8_t *ref_packed, uint64_t ref_stride, const uint8_t *ref_bits,
+                                      const int32_t *ref_norm2, uint32_t n_ref, const uint8_t *qry_packed, uint64_t qry_stride,
+                                      const uint8_t *qry_bits, const int32_t *qry_norm2, uint32_t n_qry, uint32_t hv_d,
+                                      uint32_t ksize, int path, int lower, float *out, uint64_t ld);
+/* Measurement hook of the last matrix run: counts = {bands, entries written, bytes copied to the host, the kernel path
+ * that produced them}; ms = device time of {row preparation (the packed entries: with the rows' upload and unpack), band
+ * kernels, dot-to-ANI conversion, copies to the host}
+ * (-1 where a stage did not run or profiling is off, see hg_set_profiling). */
+HG_API int hg_ani_matrix_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4]);
+
 /* Which path the last hg_dist / hg_dist_dev took (1 SIMT, 2 two-limb tensor, 3 single-plane tensor) and why. */
 HG_API int hg_dist_last_path(hg_ctx *ctx);
 HG_API const char *hg_dist_last_reason(hg_ctx *ctx);

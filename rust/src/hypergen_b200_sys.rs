@@ -61,6 +61,18 @@ extern "C" {
         hv_d: u32, ksize: u32, ani_th: f32, path: c_int, order: *const u32, rep: *mut u32, n_reps: *mut u32) -> c_int;
     // counts = {column chunks, windows, linked pairs, representatives}; ms of its phases (-1: not run / not profiled)
     pub fn hg_derep_stats(ctx: *mut hg_ctx, counts: *mut u64, ms: *mut f32) -> c_int;
+    // the ANI of every pair as f32: lower = 1 the strict lower triangle of one set (row i at i (i - 1) / 2), lower = 0
+    // the n_ref x n_qry rectangle with rows ld apart; bit for bit hg_dist's ani at ani_th = 0
+    pub fn hg_ani_matrix_dev(ctx: *mut hg_ctx, d_ref: *const i16, d_ref_norm2: *const i32, n_ref: u32, d_qry: *const i16,
+        d_qry_norm2: *const i32, n_qry: u32, hv_d: u32, ksize: u32, path: c_int, lower: c_int, d_out: *mut f32, ld: u64) -> c_int;
+    pub fn hg_ani_matrix_packed(ctx: *mut hg_ctx, ref_packed: *const u8, ref_stride: u64, ref_bits: *const u8, ref_norm2: *const i32,
+        n_ref: u32, qry_packed: *const u8, qry_stride: u64, qry_bits: *const u8, qry_norm2: *const i32, n_qry: u32, hv_d: u32,
+        ksize: u32, path: c_int, lower: c_int, out: *mut f32, ld: u64) -> c_int;
+    pub fn hg_group_ani_matrix_packed(g: *mut hg_group, ref_packed: *const u8, ref_stride: u64, ref_bits: *const u8,
+        ref_norm2: *const i32, n_ref: u32, qry_packed: *const u8, qry_stride: u64, qry_bits: *const u8, qry_norm2: *const i32,
+        n_qry: u32, hv_d: u32, ksize: u32, path: c_int, lower: c_int, out: *mut f32, ld: u64) -> c_int;
+    // counts = {bands, entries, bytes copied to the host, kernel path}; ms of its stages (-1: not run / not profiled)
+    pub fn hg_ani_matrix_stats(ctx: *mut hg_ctx, counts: *mut u64, ms: *mut f32) -> c_int;
 }
 
 /// status -> panic with the library's message, the reference's error style (`unwrap()`, Cargo.toml:67-70)
