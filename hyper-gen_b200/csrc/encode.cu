@@ -66,6 +66,7 @@ encode_kernel(const hg_genome_desc *__restrict__ desc, const uint64_t *__restric
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
   for (uint32_t d = tid; d < 64 * CP; d += EN_THREADS) s_cnt[d] = 0;
+  __syncthreads();  // an empty set never enters the batch loop: the read-out below sees other threads' cells
 
   // work split: chunk-blocks of 32 chunks x strided hash subsets
   const uint32_t nCB = (C + 31) / 32;
@@ -78,7 +79,7 @@ encode_kernel(const hg_genome_desc *__restrict__ desc, const uint64_t *__restric
     const uint32_t lim = min(base + EN_BATCH, (slots + 31u) & ~31u);  // warp-uniform trip count
     for (uint32_t s = base + tid; s < lim; s += EN_THREADS) {
       const uint64_t h = s < slots ? table[s] : HG_EMPTY_SLOT;
-      const bool have = h != HG_EMPTY_SLOT;
+      const bool have = s < slots && (!counts || h != HG_EMPTY_SLOT);  // dense list mode: u64::MAX is a hash too
       const uint32_t bal = __ballot_sync(0xffffffffu, have);
       uint32_t pos = 0;
       if (lane == 0 && bal) pos = atomicAdd(&s_m, (uint32_t)__popc(bal));
@@ -294,8 +295,8 @@ int hg_launch_encode(hg_ctx *ctx, const hg_genome_desc *d_desc, uint32_t n_genom
                      uint8_t *d_quant_bits, int32_t *d_norm2, uint32_t *d_n_hashes) {
   if (n_genomes == 0) return HG_OK;
   const size_t smem = (size_t)hv_d * 6 + 264 + (size_t)EN_BATCH * 8;
-  if (smem > 220 * 1024) {  // 6 B per dimension + the hash batch: hv_d <= 31744
-    hg_set_error("hv_d %u too large for the on-chip encoder (max 31744; dist accepts up to 32768)", hv_d);
+  if (smem > 220 * 1024) {  // 6 B per dimension + the hash batch: hv_d <= 32000 (a multiple of 256)
+    hg_set_error("hv_d %u too large for the on-chip encoder (max 32000; dist accepts up to 32768)", hv_d);
     return HG_E_UNSUPPORTED;
   }
   HG_CUDA(cudaFuncSetAttribute(encode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));

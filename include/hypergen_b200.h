@@ -146,6 +146,7 @@ HG_API int hg_sketch_status(hg_ctx *ctx);
 /* Stage hook = hd::encode_hash_hd_avx2 + compute_hv_l2_norm + compress_hd_sketch
  * (src/hd.rs:15-92,116-157, src/dist.rs:132-137) from explicit hash SETS (unique values,
  * as the reference's HashSet argument): set g = hashes[hash_off[g] .. hash_off[g+1]).
+ * Every element is a hash, 0 and u64::MAX included.  hv_d <= 32000 (HG_E_UNSUPPORTED above).
  * Host pointers; outputs as hg_sketch_batch. */
 HG_API int hg_encode_sets(hg_ctx *ctx, const uint64_t *hashes, const uint64_t *hash_off, uint32_t n_sets,
                           uint32_t hv_d, int16_t *hv, uint8_t *packed, uint8_t *quant_bits, int32_t *norm2);
