@@ -53,6 +53,7 @@ extern "C" int hg_init(int device, hg_ctx **out) {
   memset(c, 0, sizeof(*c));
   c->device = device;
   hg_cluster_stats_reset(c);
+  for (int i = 0; i < 5; i++) c->records_ms[i] = -1.0f;
   struct Guard { hg_ctx *c; ~Guard() { if (c) hg_destroy(c); } } guard{c};  // nothing leaks when a step below fails
   cudaDeviceProp prop;
   HG_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -186,6 +187,21 @@ int hg_scratch(hg_ctx *c, int slot, size_t bytes, void **out) {
   return HG_OK;
 }
 
+int hg_scratch_keep(hg_ctx *c, int slot, size_t bytes, size_t keep, void **out) {
+  if (c->d_scratch_bytes[slot] < bytes) {
+    void *p = nullptr;
+    const size_t want = bytes + bytes / 2 + 4096;
+    HG_CUDA(cudaMalloc(&p, want));
+    if (keep) HG_CUDA(cudaMemcpyAsync(p, c->d_scratch[slot], keep, cudaMemcpyDeviceToDevice, c->stream));
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+    if (c->d_scratch[slot]) HG_CUDA(cudaFree(c->d_scratch[slot]));
+    c->d_scratch[slot] = p;
+    c->d_scratch_bytes[slot] = want;
+  }
+  *out = c->d_scratch[slot];
+  return HG_OK;
+}
+
 int hg_pinned(hg_ctx *c, int slot, size_t bytes, void **out) {
   if (bytes == 0) bytes = 256;
   if (c->h_pinned_bytes[slot] < bytes) {
@@ -240,22 +256,31 @@ struct SketchPlan {
   uint32_t max_slots = 0;
 };
 
-// genome g = bytes [off[g], off[g + 1]) of a buffer whose byte off[0] sits at byte `base` of the device sequence
-// buffer; off is monotone
-static int make_plan(const uint64_t *off, uint32_t n, uint64_t base, const hg_sketch_params *p, SketchPlan &pl) {
+// genome g = bytes [r[g].begin, r[g].begin + r[g].len) of the device sequence buffer
+struct SeqRange { uint64_t begin, len; };
+
+// the ranges of genomes that lie back to back: genome g = bytes [off[g], off[g + 1]) of a buffer whose byte off[0] sits
+// at byte `base` of the device sequence buffer; off is monotone
+static std::vector<SeqRange> back_to_back(const uint64_t *off, uint32_t n, uint64_t base) {
+  std::vector<SeqRange> r(n);
+  for (uint32_t g = 0; g < n; g++) r[g] = {off[g] - off[0] + base, off[g + 1] - off[g]};
+  return r;
+}
+
+static int make_plan(const SeqRange *r, uint32_t n, const hg_sketch_params *p, SketchPlan &pl) {
   const uint32_t tile = hg_kmer_tile_positions();
   pl.desc.resize(n + 1);  // + sentinel
   pl.max_slots = 0;
   uint64_t slots_total = 0, tiles_total = 0;
   for (uint32_t g = 0; g < n; g++) {
-    const uint64_t len = off[g + 1] - off[g];
+    const uint64_t len = r[g].len;
     const uint64_t n_kmers = len >= p->ksize ? len - p->ksize + 1 : 0;
     // open-addressing table at <= 50 % load for the expected FracMinHash sample size
     uint64_t want = 2 * (len / p->scaled + 1) + 32, slots = 64;
     while (slots < want) slots <<= 1;
     if (slots > (1ull << 31)) { hg_set_error("genome %u too large for one table", g); return HG_E_UNSUPPORTED; }
     hg_genome_desc &d = pl.desc[g];
-    d.seq_begin = off[g] - off[0] + base;
+    d.seq_begin = r[g].begin;
     d.seq_len = len;
     d.table_begin = slots_total;
     d.table_mask = (uint32_t)(slots - 1);
@@ -318,7 +343,8 @@ extern "C" int hg_sketch_batch_dev(hg_ctx *c, const uint8_t *d_seq, const uint64
   if (n == 0) return HG_OK;
   HG_CUDA(cudaSetDevice(c->device));
   SketchPlan pl;
-  if ((rc = check_offsets(seg_off, n, "seg_off")) || (rc = make_plan(seg_off, n, seg_off[0], p, pl))) return rc;
+  if ((rc = check_offsets(seg_off, n, "seg_off")) || (rc = make_plan(back_to_back(seg_off, n, seg_off[0]).data(), n, p, pl)))
+    return rc;
   hg_genome_desc *d_desc; uint64_t *d_tables; uint32_t *d_counts;
   if ((rc = run_hash_stage(c, d_seq, pl, n, p, &d_desc, &d_tables, &d_counts))) return rc;
   rc = hg_launch_encode(c, d_desc, n, d_tables, d_counts, p->hv_d, d_hv, d_packed, d_quant_bits, d_norm2, d_n_hashes);
@@ -516,7 +542,7 @@ extern "C" int hg_fasta_merge(hg_ctx *c, const uint8_t *raw, const uint64_t *fil
 // ---------------------------------------------------------------------------------------
 // host-pointer sketch entries: sequences or raw FASTA files in, sketches out
 // ---------------------------------------------------------------------------------------
-enum class Input { SEQUENCES, FASTA_FILES };
+enum class Input { SEQUENCES, FASTA_FILES, FASTA_RECORDS };  // records: planned per chunk, once its records are known
 
 // genomes [g0, g1), whose host bytes [lo, hi) are copied to byte `shift` of a staging slot
 struct Chunk {
@@ -531,7 +557,7 @@ struct Chunk {
 // are planned from the raw sizes, an upper bound of the merged lengths.
 static int plan_chunks(const uint8_t *host, const uint64_t *off, uint32_t n, const hg_sketch_params *p, Input in,
                        uint64_t limit, std::vector<Chunk> &chunks) {
-  const bool fasta = in == Input::FASTA_FILES;
+  const bool fasta = in != Input::SEQUENCES;
   int rc = check_offsets(off, n, fasta ? "file_off" : "seg_off");
   if (rc) return rc;
   for (uint32_t g = 0; g < n;) {
@@ -543,7 +569,8 @@ static int plan_chunks(const uint8_t *host, const uint64_t *off, uint32_t n, con
     ch.hi = off[g];
     ch.shift = fasta ? 0 : (uint64_t)((uintptr_t)(host + ch.lo) & 15);
     if (fasta && (rc = make_merge_plan(off + ch.g0, ch.g1 - ch.g0, ch.merge))) return rc;
-    if ((rc = make_plan(off + ch.g0, ch.g1 - ch.g0, ch.shift, p, ch.pl))) return rc;
+    if (in != Input::FASTA_RECORDS && (rc = make_plan(back_to_back(off + ch.g0, ch.g1 - ch.g0, ch.shift).data(), ch.g1 - ch.g0, p, ch.pl)))
+      return rc;
     chunks.push_back(std::move(ch));
   }
   return HG_OK;
@@ -665,6 +692,222 @@ extern "C" int hg_sketch_fasta_batch(hg_ctx *c, const uint8_t *raw, const uint64
   if (n == 0) return HG_OK;
   if (!raw && file_off[n] > file_off[0]) { hg_set_error("hg_sketch_fasta_batch: raw is NULL"); return HG_E_INVALID; }
   return sketch_pipeline(c, raw, file_off, n, p, Input::FASTA_FILES, hv, packed, quant_bits, norm2, n_hashes);
+}
+
+// ---------------------------------------------------------------------------------------
+// FASTA records in: one sketch per record
+// ---------------------------------------------------------------------------------------
+int hg_launch_fasta_rec_count(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_file_off, const uint64_t *d_blk_off,
+                              uint32_t n_files, uint32_t max_blocks, uint64_t n_blocks, uint32_t *d_cnt, uint64_t *d_first);
+int hg_launch_fasta_rec_table(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_file_off, const uint64_t *d_blk_off,
+                              uint32_t n_files, uint32_t max_blocks, const uint8_t *d_carry, const uint64_t *d_out_off,
+                              const uint64_t *d_merged_len, const uint32_t *d_cnt, const uint64_t *d_first, uint64_t n_slots,
+                              hg_fasta_record *d_rec, uint64_t *d_rec_n);
+
+// The chunked pipeline of the per-file entry with the record index behind the merge.  A chunk's hash plan needs its
+// records, so each chunk makes two round trips to the host (the header count, then the record table); the next
+// chunk's H2D is queued on the copy stream before them, so PCIe stays busy.  The raw slot is released after the index
+// pass, which reads the raw bytes too.  A record's range starts at its header's 'N', which adds no k-mer.
+int hg_records_run(hg_ctx *c, const uint8_t *raw, const uint64_t *off, uint32_t n, const hg_sketch_params *p,
+                   uint64_t rec_cap, hg_records_part &out) {
+  out = hg_records_part();
+  int rc = check_params(p);
+  if (rc) return rc;
+  for (int i = 0; i < 4; i++) c->records_stats[i] = 0;
+  for (int i = 0; i < 5; i++) c->records_ms[i] = -1.0f;
+  HG_CUDA(cudaSetDevice(c->device));
+  const uint32_t D = p->hv_d;
+  std::vector<Chunk> chunks;
+  if ((rc = plan_chunks(raw, off, n, p, Input::FASTA_RECORDS, hg_chunk_bytes(), chunks))) return rc;
+  uint64_t max_bytes = 0, max_blk = 0;
+  uint32_t max_m = 0;
+  for (const Chunk &ch : chunks) {
+    max_bytes = std::max(max_bytes, ch.hi - ch.lo);
+    max_m = std::max(max_m, ch.g1 - ch.g0);
+    max_blk = std::max(max_blk, ch.merge.blk.back());
+  }
+  const uint64_t slot_bytes = (max_bytes + 64 + 255) & ~255ull;
+  const MergeLayout L = merge_layout(max_m, max_blk);
+  void *d_stage, *d_merged, *d_meta, *d_idx, *h_meta;
+  if ((rc = hg_scratch(c, HG_S_REF_LIMBS, 2 * slot_bytes, &d_stage))) return rc;
+  if ((rc = hg_scratch(c, HG_S_SEQ, slot_bytes, &d_merged))) return rc;
+  if ((rc = hg_scratch(c, HG_S_QRY_LIMBS, L.len + (size_t)n * 8, &d_meta))) return rc;
+  if ((rc = hg_scratch(c, HG_S_NARROW_META, (max_blk + 1) * 8 + max_blk * 4, &d_idx))) return rc;
+  if ((rc = hg_pinned(c, 1, L.out * chunks.size(), &h_meta))) return rc;
+  if ((rc = ensure_copy_stream(c))) return rc;
+  uint8_t *meta = (uint8_t *)d_meta;
+  const uint64_t *d_foff = (const uint64_t *)meta, *d_boff = (const uint64_t *)(meta + L.blk);
+  uint64_t *d_len = (uint64_t *)(meta + L.len);  // merged lengths, all files
+  uint64_t *d_first = (uint64_t *)d_idx;
+  uint32_t *d_cnt = (uint32_t *)(d_first + max_blk + 1);
+  c->ev_used = 0;
+  HG_CUDA(cudaMemsetAsync(c->d_status, 0, 4 * sizeof(uint32_t), c->stream));
+  HG_CUDA(cudaEventRecord(c->ev_done[0], c->stream));
+  HG_CUDA(cudaEventRecord(c->ev_done[1], c->stream));
+  auto copy = [&](size_t ci) -> int {
+    const Chunk &ch = chunks[ci];
+    const int slot = (int)(ci & 1);
+    HG_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_done[slot], 0));
+    if (ch.hi > ch.lo)
+      HG_CUDA(cudaMemcpyAsync((uint8_t *)d_stage + slot * slot_bytes, raw + ch.lo, ch.hi - ch.lo, cudaMemcpyHostToDevice, c->copy_stream));
+    HG_CUDA(cudaEventRecord(c->ev_copied[slot], c->copy_stream));
+    return HG_OK;
+  };
+  // Profiling: ev[0] merge [1] count pass [2] (host) [3] table pass [4] (host) [5] hash [6] encode [7].  A chunk's
+  // hash and encode are read at the next chunk's first synchronisation.
+  const bool prof = c->prof != 0;
+  float ms[5] = {0, 0, 0, 0, 0};  // merge, index, hash, encode, host gap
+  bool hash_pending = false;
+  auto mark = [&](int i) { if (prof) cudaEventRecord(c->ev[i], c->stream); };
+  auto span = [&](int a, int b) { float t = 0; cudaEventElapsedTime(&t, c->ev[a], c->ev[b]); return t; };
+  auto read_hash = [&]() {
+    if (!hash_pending) return;
+    ms[4] += span(4, 5); ms[2] += span(5, 6); ms[3] += span(6, 7);
+    hash_pending = false;
+  };
+
+  if ((rc = copy(0))) return rc;
+  uint64_t rows = 0, slots = 0;
+  std::vector<SeqRange> rng;
+  for (size_t ci = 0; ci < chunks.size(); ci++) {
+    const Chunk &ch = chunks[ci];
+    const int slot = (int)(ci & 1);
+    const uint32_t m = ch.g1 - ch.g0, max_blocks = (uint32_t)ch.merge.max_blocks;
+    const uint64_t nblk = ch.merge.blk.back();
+    const uint8_t *d_in = (const uint8_t *)d_stage + slot * slot_bytes;
+    if (ci + 1 < chunks.size() && (rc = copy(ci + 1))) return rc;
+    // ---- merge and index pass 1; the header count to the host ----
+    if ((rc = put_merge_meta(c, ch.merge, L, (uint8_t *)h_meta + ci * L.out, meta))) return rc;
+    HG_CUDA(cudaStreamWaitEvent(c->stream, c->ev_copied[slot], 0));
+    mark(0);
+    if ((rc = launch_merge(c, d_in, ch.merge, L, meta, (uint8_t *)d_merged, d_len + ch.g0))) return rc;
+    mark(1);
+    if ((rc = hg_launch_fasta_rec_count(c, d_in, d_foff, d_boff, m, max_blocks, nblk, d_cnt, d_first))) return rc;
+    mark(2);
+    void *h_x;
+    if ((rc = hg_pinned(c, 3, 64, &h_x))) return rc;
+    HG_CUDA(cudaMemcpyAsync(h_x, d_first + nblk, 8, cudaMemcpyDeviceToHost, c->stream));
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+    read_hash();
+    const uint64_t n_slots = *(const uint64_t *)h_x + m;
+    // ---- index pass 2; the table to the host ----
+    void *d_tab, *h_tab;
+    if ((rc = hg_scratch(c, HG_S_TILES, n_slots * (sizeof(hg_fasta_record) + 8), &d_tab))) return rc;
+    if ((rc = hg_pinned(c, 3, n_slots * sizeof(hg_fasta_record), &h_tab))) return rc;
+    hg_fasta_record *d_rec = (hg_fasta_record *)d_tab;
+    mark(3);
+    if ((rc = hg_launch_fasta_rec_table(c, d_in, d_foff, d_boff, m, max_blocks, meta + L.carry, (const uint64_t *)(meta + L.out),
+                                        d_len + ch.g0, d_cnt, d_first, n_slots, d_rec, (uint64_t *)(d_rec + n_slots))))
+      return rc;
+    mark(4);
+    HG_CUDA(cudaEventRecord(c->ev_done[slot], c->stream));  // the raw slot may be overwritten now
+    HG_CUDA(cudaMemcpyAsync(h_tab, d_rec, n_slots * sizeof(hg_fasta_record), cudaMemcpyDeviceToHost, c->stream));
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+    if (prof) { ms[0] += span(0, 1); ms[1] += span(1, 2) + span(3, 4); ms[4] += span(2, 3); }
+    slots += n_slots;
+    // ---- the chunk's records (empty leading slots dropped) and their ranges in the merged bytes ----
+    rng.clear();
+    const hg_fasta_record *hr = (const hg_fasta_record *)h_tab;
+    uint64_t pos = 0;  // merged offset of the slot inside its file
+    for (uint64_t s = 0; s < n_slots; s++) {
+      hg_fasta_record r = hr[s];
+      if (!r.has_header) pos = 0;
+      const uint64_t begin = ch.merge.off[r.file] + pos, len = r.seq_len + r.has_header;
+      pos += len;
+      if (!r.has_header && r.seq_len == 0) continue;
+      r.file += ch.g0;
+      r.name_off += ch.lo;
+      out.rec.push_back(r);
+      rng.push_back({begin, len});
+    }
+    if (out.rec.size() > 0xFFFFFFFFull) { hg_set_error("more than 2^32 - 1 records in one call"); return HG_E_UNSUPPORTED; }
+    const uint32_t mr = (uint32_t)rng.size();
+    if (out.rec.size() > rec_cap || mr == 0) continue;  // over capacity: count the rest, sketch nothing more
+    // ---- hash and encode the chunk's records into rows [rows, rows + mr) ----
+    SketchPlan pl;
+    if ((rc = make_plan(rng.data(), mr, p, pl))) return rc;
+    const uint64_t need = rows + mr;
+    void *d_packed, *d_norm2, *d_nh, *d_bits, *d_desc, *d_tables, *d_counts, *h_desc;
+    if ((rc = hg_scratch_keep(c, HG_S_PACKED, need * 2 * D, rows * 2 * D, &d_packed))) return rc;
+    if ((rc = hg_scratch_keep(c, HG_S_SMALL, need * 4, rows * 4, &d_norm2))) return rc;
+    if ((rc = hg_scratch_keep(c, HG_S_SORT_CNT, need * 4, rows * 4, &d_nh))) return rc;
+    if ((rc = hg_scratch_keep(c, HG_S_SORT_TMP, need, rows, &d_bits))) return rc;
+    if ((rc = hg_scratch(c, HG_S_DESC, sizeof(hg_genome_desc) * (mr + 1), &d_desc))) return rc;
+    if ((rc = hg_scratch(c, HG_S_TABLES, pl.total_slots * 8, &d_tables))) return rc;
+    if ((rc = hg_scratch(c, HG_S_COUNTS, sizeof(uint32_t) * mr, &d_counts))) return rc;
+    if ((rc = hg_pinned(c, 0, sizeof(hg_genome_desc) * (mr + 1), &h_desc))) return rc;
+    memcpy(h_desc, pl.desc.data(), sizeof(hg_genome_desc) * (mr + 1));
+    mark(5);
+    HG_CUDA(cudaMemcpyAsync(d_desc, h_desc, sizeof(hg_genome_desc) * (mr + 1), cudaMemcpyHostToDevice, c->stream));
+    HG_CUDA(cudaMemsetAsync(d_tables, 0xFF, pl.total_slots * 8, c->stream));
+    HG_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(uint32_t) * mr, c->stream));
+    const hg_genome_desc *dd = (const hg_genome_desc *)d_desc;
+    if ((rc = hg_launch_kmer_hash(c, (const uint8_t *)d_merged, dd, mr, pl.n_tiles, p, nullptr, (uint64_t *)d_tables,
+                                  (uint32_t *)d_counts)))
+      return rc;
+    mark(6);
+    if ((rc = hg_launch_encode(c, dd, mr, (const uint64_t *)d_tables, (const uint32_t *)d_counts, D, nullptr,
+                               (uint8_t *)d_packed + rows * 2 * D, (uint8_t *)d_bits + rows, (int32_t *)d_norm2 + rows,
+                               (uint32_t *)d_nh + rows)))
+      return rc;
+    mark(7);
+    hash_pending = prof;
+    rows = need;
+  }
+  if (prof) {
+    HG_CUDA(cudaStreamSynchronize(c->stream));
+    read_hash();
+    for (int i = 0; i < 5; i++) c->records_ms[i] = ms[i];
+  }
+  c->records_stats[0] = chunks.size();
+  c->records_stats[1] = out.rec.size();
+  c->records_stats[2] = slots;
+  if (rows) {  // the slots hold this call's rows until the context's next entry
+    out.packed = (const uint8_t *)c->d_scratch[HG_S_PACKED];
+    out.norm2 = (const int32_t *)c->d_scratch[HG_S_SMALL];
+    out.n_hashes = (const uint32_t *)c->d_scratch[HG_S_SORT_CNT];
+    out.bits = (const uint8_t *)c->d_scratch[HG_S_SORT_TMP];
+  }
+  return HG_OK;
+}
+
+int hg_records_fetch(hg_ctx *c, const hg_records_part &o, uint32_t D, uint8_t *packed, uint8_t *quant_bits, int32_t *norm2,
+                     uint32_t *n_hashes) {
+  HG_CUDA(cudaSetDevice(c->device));
+  const size_t n = o.rec.size();
+  if (n && packed) HG_CUDA(cudaMemcpyAsync(packed, o.packed, n * 2 * D, cudaMemcpyDeviceToHost, c->stream));
+  if (n && quant_bits) HG_CUDA(cudaMemcpyAsync(quant_bits, o.bits, n, cudaMemcpyDeviceToHost, c->stream));
+  if (n && norm2) HG_CUDA(cudaMemcpyAsync(norm2, o.norm2, n * 4, cudaMemcpyDeviceToHost, c->stream));
+  if (n && n_hashes) HG_CUDA(cudaMemcpyAsync(n_hashes, o.n_hashes, n * 4, cudaMemcpyDeviceToHost, c->stream));
+  return hg_sketch_status(c);
+}
+
+extern "C" int hg_sketch_fasta_records(hg_ctx *c, const uint8_t *raw, const uint64_t *file_off, uint32_t n,
+                                       const hg_sketch_params *p, uint32_t rec_cap, hg_fasta_record *records,
+                                       uint8_t *packed, uint8_t *quant_bits, int32_t *norm2, uint32_t *n_hashes,
+                                       uint32_t *n_records) {
+  if (!c || !file_off || !n_records) { hg_set_error("hg_sketch_fasta_records: NULL argument"); return HG_E_INVALID; }
+  *n_records = 0;
+  int rc = check_params(p);
+  if (rc) return rc;
+  if (n == 0) return HG_OK;
+  if (!raw && file_off[n] > file_off[0]) { hg_set_error("hg_sketch_fasta_records: raw is NULL"); return HG_E_INVALID; }
+  hg_records_part part;
+  if ((rc = hg_records_run(c, raw, file_off, n, p, rec_cap, part))) return rc;
+  *n_records = (uint32_t)part.rec.size();
+  if (part.rec.size() > rec_cap) {
+    hg_set_error("hg_sketch_fasta_records: %u records, rec_cap is %u", *n_records, rec_cap);
+    return HG_E_CAPACITY;
+  }
+  if (records && !part.rec.empty()) memcpy(records, part.rec.data(), part.rec.size() * sizeof(hg_fasta_record));
+  return hg_records_fetch(c, part, p->hv_d, packed, quant_bits, norm2, n_hashes);
+}
+
+extern "C" int hg_fasta_records_stats(hg_ctx *c, uint64_t counts[4], float ms[4], float *host_gap_ms) {
+  if (!c || !counts || !ms || !host_gap_ms) { hg_set_error("hg_fasta_records_stats: NULL argument"); return HG_E_INVALID; }
+  for (int i = 0; i < 4; i++) { counts[i] = c->records_stats[i]; ms[i] = c->records_ms[i]; }
+  *host_gap_ms = c->records_ms[4];
+  return HG_OK;
 }
 
 extern "C" int hg_kmer_hash(hg_ctx *c, const uint8_t *seq, const uint64_t *seg_off, uint32_t n,

@@ -340,6 +340,160 @@ fasta_emit_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ 
   }
 }
 
+// ---- record index (hg_sketch_fasta_records): runs after the merge, on the same raw bytes ----
+// Every header start emitted exactly one 'N', so a record is located by its header's raw index and the merged offset
+// of that 'N'.  Table layout of a merge: file f owns slots [first[blk_off[f]] + f, first[blk_off[f + 1]] + f + 1): one
+// leading slot, then its headers in file order; the host drops a leading slot whose sequence is empty.
+
+// sum over the CTA (every thread passes its value; the result is valid in thread 0)
+__device__ __forceinline__ uint32_t block_sum(uint32_t v) {
+  __shared__ uint32_t s_c[FA_THREADS / 32];
+  v = __reduce_add_sync(0xffffffffu, v);
+  if ((threadIdx.x & 31) == 0) s_c[threadIdx.x >> 5] = v;
+  __syncthreads();
+  uint32_t t = 0;
+  if (threadIdx.x == 0)
+#pragma unroll
+    for (int w = 0; w < FA_THREADS / 32; ++w) t += s_c[w];
+  return t;
+}
+
+// header starts per 4 KB block (the header test needs no carried state: a '>' at a line start always opens one)
+__global__ void __launch_bounds__(FA_THREADS)
+fasta_rec_count_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ file_off, const uint64_t *__restrict__ blk_off,
+                       uint32_t *__restrict__ cnt) {
+  const uint32_t f = blockIdx.y;
+  const uint64_t len = file_off[f + 1] - file_off[f];
+  const uint64_t nb = (len + FA_BLOCK - 1) / FA_BLOCK, blk = blockIdx.x;
+  if (blk >= nb) return;
+  const uint64_t p0 = blk * FA_BLOCK + (uint64_t)threadIdx.x * FA_BPT;
+  const Lane L = classify(load_raw(raw + file_off[f], len, p0), len, p0);
+  const uint32_t t = block_sum(__popc(L.hdr_start));
+  if (threadIdx.x == 0) cnt[blk_off[f] + blk] = t;
+}
+
+// one CTA: first[b] = header starts in blocks before b (all files of the merge), first[nblk] = all of them
+__global__ void __launch_bounds__(1024) fasta_rec_prefix_kernel(const uint32_t *__restrict__ cnt, uint64_t nblk,
+                                                                uint64_t *__restrict__ first) {
+  __shared__ uint64_t s_w[32];
+  __shared__ uint64_t s_carry;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (threadIdx.x == 0) s_carry = 0;
+  __syncthreads();
+  for (uint64_t base = 0; base < nblk; base += 1024) {
+    const uint64_t i = base + threadIdx.x;
+    const uint64_t v = i < nblk ? cnt[i] : 0;
+    uint64_t x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint64_t y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) s_w[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+      uint64_t y = s_w[lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint64_t z = __shfl_up_sync(0xffffffffu, y, o);
+        if (lane >= o) y += z;
+      }
+      s_w[lane] = y;
+    }
+    __syncthreads();
+    const uint64_t incl = s_carry + (warp ? s_w[warp - 1] : 0) + x;
+    if (i < nblk) first[i] = incl - v;
+    __syncthreads();  // s_carry and s_w are read by every thread before they change
+    if (threadIdx.x == 1023) s_carry = incl;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) first[nblk] = s_carry;
+}
+
+// the leading slot of every file: its sequence starts at merged offset 0 (rec_n = -1 stands for a virtual 'N' before it)
+__global__ void fasta_rec_lead_kernel(const uint64_t *__restrict__ file_off, const uint64_t *__restrict__ blk_off, uint32_t n_files,
+                                      const uint64_t *__restrict__ first, hg_fasta_record *__restrict__ rec,
+                                      uint64_t *__restrict__ rec_n) {
+  const uint32_t f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n_files) return;
+  const uint64_t s = first[blk_off[f]] + f;
+  hg_fasta_record r;
+  r.name_off = file_off[f];
+  r.name_len = 0;
+  r.seq_len = 0;
+  r.file = f;
+  r.has_header = 0;
+  rec[s] = r;
+  rec_n[s] = ~0ull;
+}
+
+// Per block with a header start: the merged offset of every header's 'N' (the emit kernel's offsets) and its slot.
+// Files f0 .. f0 + gridDim.y - 1 (file_off / blk_off index all files of the merge).
+__global__ void __launch_bounds__(FA_THREADS)
+fasta_rec_emit_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ file_off, const uint64_t *__restrict__ blk_off,
+                      uint32_t f0, const uint8_t *__restrict__ carry, const uint64_t *__restrict__ out_off,
+                      const uint32_t *__restrict__ cnt, const uint64_t *__restrict__ first, hg_fasta_record *__restrict__ rec,
+                      uint64_t *__restrict__ rec_n) {
+  __shared__ uint32_t s_h[FA_THREADS / 32];
+  const uint32_t f = f0 + blockIdx.y;
+  const uint64_t len = file_off[f + 1] - file_off[f];
+  const uint64_t nb = (len + FA_BLOCK - 1) / FA_BLOCK, blk = blockIdx.x;
+  if (blk >= nb) return;
+  const uint64_t gb = blk_off[f] + blk;
+  if (cnt[gb] == 0) return;  // most blocks of a genome hold no header
+  const uint64_t p0 = blk * FA_BLOCK + (uint64_t)threadIdx.x * FA_BPT;
+  const Lane L = classify(load_raw(raw + file_off[f], len, p0), len, p0);
+  const bool carry_in = carry[gb] != 0;
+  uint32_t m0, total;
+  const uint32_t ex = block_seg_scan(lane_seg(L, m0), total);
+  bool oh;
+  const uint32_t m = emit_mask(L, seg_has(ex) ? (seg_hdr(ex) != 0) : carry_in, oh);
+  const uint64_t pos = out_off[gb] + (carry_in ? seg_c1(ex) : seg_c0(ex));
+  // the thread's headers are preceded by those of lower threads: exclusive scan of the per-thread counts
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const uint32_t h = __popc(L.hdr_start);
+  uint32_t x = h;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) s_h[warp] = x;
+  __syncthreads();
+  uint32_t before = x - h;
+  for (int w = 0; w < warp; ++w) before += s_h[w];
+  uint64_t s = first[gb] + f + 1 + before;
+  for (uint32_t bits = L.hdr_start; bits; bits &= bits - 1, ++s) {
+    const int i = __ffs(bits) - 1;
+    hg_fasta_record r;
+    r.name_off = file_off[f] + p0 + i + 1;
+    r.name_len = 0;
+    r.seq_len = 0;
+    r.file = f;
+    r.has_header = 1;
+    rec[s] = r;
+    rec_n[s] = pos + __popc(m & ((1u << i) - 1u));
+  }
+}
+
+// One thread per slot: seq_len from the next slot's 'N' (or the file's merged length), and the header's name span by a
+// forward search for the end of its line (headers are short; a long one costs its own thread only).
+__global__ void fasta_rec_finish_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ file_off,
+                                        const uint64_t *__restrict__ merged_len, uint64_t n_slots, hg_fasta_record *__restrict__ rec,
+                                        const uint64_t *__restrict__ rec_n) {
+  const uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n_slots) return;
+  const uint32_t f = rec[s].file;
+  const uint64_t next = s + 1 < n_slots && rec[s + 1].file == f ? rec_n[s + 1] : merged_len[f];
+  rec[s].seq_len = next - rec_n[s] - 1;
+  if (rec[s].has_header) {
+    const uint64_t a = rec[s].name_off, end = file_off[f + 1];
+    uint64_t q = a;
+    while (q < end && raw[q] != '\n') ++q;
+    rec[s].name_len = q - a - (q < end && q > a && raw[q - 1] == '\r' ? 1 : 0);
+  }
+}
+
 }  // namespace
 
 uint32_t hg_fasta_block_bytes() { return FA_BLOCK; }
@@ -367,6 +521,43 @@ int hg_launch_fasta_merge(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_f
                                                                              d_carry, d_out_off, d_merged);
     ctx->launches++;
   }
+  HG_CUDA(cudaGetLastError());
+  return HG_OK;
+}
+
+// Record index, pass 1 (after hg_launch_fasta_merge, same arguments): d_cnt (n_blocks) and d_first (n_blocks + 1, the
+// last entry the header count of the merge).  The host reads d_first[n_blocks] back: the table has that + n_files slots.
+int hg_launch_fasta_rec_count(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_file_off, const uint64_t *d_blk_off,
+                              uint32_t n_files, uint32_t max_blocks, uint64_t n_blocks, uint32_t *d_cnt, uint64_t *d_first) {
+  for (uint32_t f0 = 0; f0 < n_files && max_blocks; f0 += 65535) {
+    const uint32_t nf = n_files - f0 < 65535 ? n_files - f0 : 65535;
+    fasta_rec_count_kernel<<<dim3(max_blocks, nf), FA_THREADS, 0, ctx->stream>>>(d_raw, d_file_off + f0, d_blk_off + f0, d_cnt);
+    ctx->launches++;
+  }
+  fasta_rec_prefix_kernel<<<1, 1024, 0, ctx->stream>>>(d_cnt, n_blocks, d_first);
+  ctx->launches++;
+  HG_CUDA(cudaGetLastError());
+  return HG_OK;
+}
+
+// Pass 2: the n_slots-entry table (rec; rec_n the 'N' offsets) from pass 1 and the merge's carry / out_off / lengths.
+// name_off is an index into d_raw; file is the index in this merge.
+int hg_launch_fasta_rec_table(hg_ctx *ctx, const uint8_t *d_raw, const uint64_t *d_file_off, const uint64_t *d_blk_off,
+                              uint32_t n_files, uint32_t max_blocks, const uint8_t *d_carry, const uint64_t *d_out_off,
+                              const uint64_t *d_merged_len, const uint32_t *d_cnt, const uint64_t *d_first, uint64_t n_slots,
+                              hg_fasta_record *d_rec, uint64_t *d_rec_n) {
+  if (n_files == 0) return HG_OK;
+  fasta_rec_lead_kernel<<<(n_files + 255) / 256, 256, 0, ctx->stream>>>(d_file_off, d_blk_off, n_files, d_first, d_rec, d_rec_n);
+  ctx->launches++;
+  for (uint32_t f0 = 0; f0 < n_files && max_blocks; f0 += 65535) {
+    const uint32_t nf = n_files - f0 < 65535 ? n_files - f0 : 65535;
+    fasta_rec_emit_kernel<<<dim3(max_blocks, nf), FA_THREADS, 0, ctx->stream>>>(d_raw, d_file_off, d_blk_off, f0, d_carry, d_out_off,
+                                                                               d_cnt, d_first, d_rec, d_rec_n);
+    ctx->launches++;
+  }
+  fasta_rec_finish_kernel<<<(unsigned)((n_slots + 255) / 256), 256, 0, ctx->stream>>>(d_raw, d_file_off, d_merged_len, n_slots,
+                                                                                      d_rec, d_rec_n);
+  ctx->launches++;
   HG_CUDA(cudaGetLastError());
   return HG_OK;
 }

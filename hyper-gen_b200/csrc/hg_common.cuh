@@ -6,6 +6,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <vector>
+
 #include "../../include/hypergen_b200.h"
 
 #define HG_EMPTY_SLOT 0xFFFFFFFFFFFFFFFFull
@@ -195,6 +197,10 @@ struct hg_ctx {
   // its stages (-1: not run or profiling off)
   uint64_t matrix_stats[4];
   float matrix_ms[4];
+  // the last FASTA records call (hg_fasta_records_stats): chunks, records, table slots; device ms of merge, index, hash,
+  // encode and the host gap (-1: profiling off)
+  uint64_t records_stats[4];
+  float records_ms[5];
 };
 
 // stage boundaries: 0 start, 1 after staging/memsets, 2 after k-mer hash, 3 after encode,
@@ -217,6 +223,9 @@ int hg_cuda_fail(cudaError_t e, const char *what, const char *file, int line);
 
 // Grow-only device scratch slots.  A slot has one tenant per entry point; entry points of one
 // context never run concurrently (one stream), so slots may be shared between them.
+// The FASTA records entry (hg_sketch_fasta_records) stages like the per-file one (REF_LIMBS raw, SEQ merged,
+// QRY_LIMBS merge metadata, DESC, TABLES, COUNTS, MISC per chunk) and keeps its outputs for the whole call in PACKED,
+// SMALL, SORT_TMP and SORT_CNT, which grow between chunks with their contents kept (hg_scratch_keep).
 enum hg_scratch_slot {
   HG_S_SEQ = 0,        // staged sequence bytes (two halves when the H2D pipeline is active); search: the sample rows
   HG_S_DESC = 1,       // hg_genome_desc[] (+ sentinels); search: the per-query floors
@@ -226,19 +235,23 @@ enum hg_scratch_slot {
   HG_S_HV = 4,         // int16 HVs (sketch output staging; dist: both matrices of the host entry)
   HG_S_PACKED = 5,     // packed sketches; dist: hit records of the host entry; search: the candidates of a pass;
                        // group search: the members' results gathered on GPU 0; cluster, derep (phase 1): the edges of
-                       // one window
-  HG_S_SMALL = 6,      // norms / bits / counts per sketch
+                       // one window; records: the packed row of every record
+  HG_S_SMALL = 6,      // norms / bits / counts per sketch; records: norm2 of every record
   HG_S_MISC = 7,       // CTA -> genome map + round-1 tables, |hv| max, probe sink, status word of a search merge; cluster: status word
                        // of a union check, root count of a flatten
   HG_S_REF_LIMBS = 8,  // s8 limb planes of the ref matrix (dist_tc)
   HG_S_QRY_LIMBS = 9,  // s8 limb planes of the query matrix (dist_tc)
   HG_S_SORT_TMP = 10,  // ping-pong buffer of the hit sort; search: the per-query segments; group search: the merged result;
-                       // group cluster: the merged forest and the members' forests gathered on GPU 0
-  HG_S_SORT_CNT = 11,  // digit counters of the hit sort; search: per-query counts and offsets
-  HG_S_NARROW_META = 12,  // per-row constants + outlier lists of the single-plane dist path (dist_narrow)
+                       // group cluster: the merged forest and the members' forests gathered on GPU 0; records: the
+                       // quant bits of every record
+  HG_S_SORT_CNT = 11,  // digit counters of the hit sort; search: per-query counts and offsets; records: n_hashes of
+                       // every record
+  HG_S_NARROW_META = 12,  // per-row constants + outlier lists of the single-plane dist path (dist_narrow); records:
+                          // the index pass's header count per block and their prefix
   HG_S_TILES = 13,        // tile list of a multi-GPU dist launch (peer.cu); search: the results of the host entries;
                           // cluster: the forest of the packed entry; derep: its state (is_rep, rep list, order, the
-                          // search result, covered flags, bitmap, counters) and the labels of the packed entry
+                          // search result, covered flags, bitmap, counters) and the labels of the packed entry;
+                          // records: one chunk's record table and the merged offsets of its headers' 'N'
   // derep: what the internal search (HG_S_SEQ, DESC, PACKED, COUNTS, SORT_*, MISC and the dist slots) and the packed
   // staging (HV, SMALL, TABLES) leave alone
   HG_S_DEREP_ROWS = 14,   // the working matrix in priority order, and its norms (when an order is given)
@@ -247,6 +260,25 @@ enum hg_scratch_slot {
 };
 // scratch slot `slot` grown to at least `bytes` (contents not preserved)
 int hg_scratch(hg_ctx *ctx, int slot, size_t bytes, void **out);
+// the same with the slot's first `keep` bytes preserved across a growth (grows by half again, so a slot that grows a
+// little per chunk is copied a logarithmic number of times)
+int hg_scratch_keep(hg_ctx *ctx, int slot, size_t bytes, size_t keep, void **out);
+
+// One context's part of a FASTA records call (api.cu): the record table on the host (file indices relative to the
+// part's first file), the sketch rows in that context's HBM until hg_records_fetch copies them out.
+struct hg_records_part {
+  std::vector<hg_fasta_record> rec;
+  const uint8_t *packed = nullptr, *bits = nullptr;
+  const int32_t *norm2 = nullptr;
+  const uint32_t *n_hashes = nullptr;
+};
+// the records of files file_off[0 .. n_files) (monotone, checked here); stops sketching once more than rec_cap
+// records are found but counts them all
+int hg_records_run(hg_ctx *ctx, const uint8_t *raw, const uint64_t *file_off, uint32_t n_files, const hg_sketch_params *p,
+                   uint64_t rec_cap, hg_records_part &out);
+// part's rows to the host outputs (any may be NULL), then the sketch status of the call (synchronises)
+int hg_records_fetch(hg_ctx *ctx, const hg_records_part &part, uint32_t hv_d, uint8_t *packed, uint8_t *quant_bits,
+                     int32_t *norm2, uint32_t *n_hashes);
 int hg_pinned(hg_ctx *ctx, int slot, size_t bytes, void **out);
 
 // The dist kernels, numbered as the `path` argument of the dist entries (include/hypergen_b200.h).

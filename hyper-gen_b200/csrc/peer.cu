@@ -30,6 +30,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <thread>
 #include <vector>
@@ -1077,6 +1078,59 @@ extern "C" int hg_group_sketch_fasta_batch(hg_group *g, const uint8_t *raw, cons
   for (int k = 0; k < parts; ++k)
     if (rcs[k]) { hg_set_error("GPU %d (files %u..%u): %s", g->ctx[k]->device, b[k], b[k + 1], msgs[k].c_str()); return rcs[k]; }
   return HG_OK;
+}
+
+// hg_sketch_fasta_records over all GPUs of the group: the files split as above.  Each member sketches its run and keeps
+// the rows on its device; once the total is known to fit rec_cap, each member copies its rows to its prefix offset.
+extern "C" int hg_group_sketch_fasta_records(hg_group *g, const uint8_t *raw, const uint64_t *file_off, uint32_t n_files,
+                                             const hg_sketch_params *p, uint32_t rec_cap, hg_fasta_record *records,
+                                             uint8_t *packed, uint8_t *quant_bits, int32_t *norm2, uint32_t *n_hashes,
+                                             uint32_t *n_records) {
+  if (!g || !file_off || !p || !n_records) { hg_set_error("hg_group_sketch_fasta_records: NULL argument"); return HG_E_INVALID; }
+  *n_records = 0;
+  if (n_files == 0) return HG_OK;
+  if (!raw && file_off[n_files] > file_off[0]) { hg_set_error("hg_group_sketch_fasta_records: raw is NULL"); return HG_E_INVALID; }
+  for (uint32_t f = 0; f < n_files; ++f)
+    if (file_off[f + 1] < file_off[f]) { hg_set_error("file_off not monotone at %u", f); return HG_E_INVALID; }
+  const int parts = (int)std::min<uint32_t>((uint32_t)g->n, n_files);
+  const std::vector<uint32_t> b = split_by_weight(file_off, n_files, parts);
+  std::vector<hg_records_part> part(parts);
+  std::vector<int> rcs(parts, HG_OK);
+  std::vector<std::string> msgs(parts);
+  auto run_all = [&](const std::function<int(int)> &fn) {  // one host thread per member with files
+    std::vector<std::thread> th;
+    for (int k = 0; k < parts; ++k)
+      if (b[k + 1] > b[k])
+        th.emplace_back([&, k]() {
+          rcs[k] = fn(k);
+          if (rcs[k]) msgs[k] = hg_last_error();
+        });
+    for (auto &t : th) t.join();
+    for (int k = 0; k < parts; ++k)
+      if (rcs[k]) { hg_set_error("GPU %d (files %u..%u): %s", g->ctx[k]->device, b[k], b[k + 1], msgs[k].c_str()); return rcs[k]; }
+    return (int)HG_OK;
+  };
+  int rc = run_all([&](int k) { return hg_records_run(g->ctx[k], raw, file_off + b[k], b[k + 1] - b[k], p, rec_cap, part[k]); });
+  if (rc) return rc;
+  std::vector<uint64_t> pre(parts + 1, 0);
+  for (int k = 0; k < parts; ++k) pre[k + 1] = pre[k] + part[k].rec.size();
+  if (pre[parts] > 0xFFFFFFFFull) { hg_set_error("more than 2^32 - 1 records in one call"); return HG_E_UNSUPPORTED; }
+  *n_records = (uint32_t)pre[parts];
+  if (pre[parts] > rec_cap) {
+    hg_set_error("hg_group_sketch_fasta_records: %u records, rec_cap is %u", *n_records, rec_cap);
+    return HG_E_CAPACITY;
+  }
+  const size_t D = p->hv_d;
+  return run_all([&](int k) {
+    const uint64_t r0 = pre[k];
+    if (records)
+      for (size_t r = 0; r < part[k].rec.size(); ++r) {
+        records[r0 + r] = part[k].rec[r];
+        records[r0 + r].file += b[k];
+      }
+    return hg_records_fetch(g->ctx[k], part[k], p->hv_d, packed ? packed + r0 * 2 * D : nullptr, quant_bits ? quant_bits + r0 : nullptr,
+                            norm2 ? norm2 + r0 : nullptr, n_hashes ? n_hashes + r0 : nullptr);
+  });
 }
 
 // hg_dist_packed over all GPUs of the group.  Every GPU receives a contiguous block of the packed ref rows and of the

@@ -19,14 +19,15 @@ HG_OK, HG_E_INVALID, HG_E_CUDA, HG_E_CAPACITY, HG_E_RANGE, HG_E_UNSUPPORTED = 0,
 EXPORTS = [
     "hg_init", "hg_destroy", "hg_sync", "hg_host_alloc", "hg_host_free", "hg_host_register", "hg_host_unregister", "hg_last_error", "hg_version", "hg_stream_handle", "hg_launch_count",
     "hg_set_profiling", "hg_stage_ms", "hg_int_peak", "hg_tensor_peak", "hg_dist_norm_flags", "hg_encode_sets", "hg_encode_sets_dev",
-    "hg_fasta_merge", "hg_sketch_fasta_batch",
+    "hg_fasta_merge", "hg_sketch_fasta_batch", "hg_sketch_fasta_records", "hg_fasta_records_stats",
     "hg_kmer_hash", "hg_sketch_batch", "hg_sketch_batch_dev", "hg_sketch_status", "hg_unpack", "hg_unpack_dev",
     "hg_dist", "hg_dist_dev", "hg_dist_status", "hg_dist_last_path", "hg_dist_last_reason", "hg_sort_hits_dev", "hg_dist_sorted", "hg_dist_packed",
     "hg_search_dev", "hg_search_packed", "hg_search_stats", "hg_search_merge_dev",
     "hg_cluster_dev", "hg_cluster_packed", "hg_cluster_union_dev", "hg_cluster_stats",
     "hg_derep_dev", "hg_derep_packed", "hg_derep_stats",
     "hg_ani_matrix_dev", "hg_ani_matrix_packed", "hg_group_ani_matrix_packed", "hg_ani_matrix_stats",
-    "hg_group_create", "hg_group_destroy", "hg_group_size", "hg_group_ctx", "hg_group_sketch_fasta_batch", "hg_group_dist_packed",
+    "hg_group_create", "hg_group_destroy", "hg_group_size", "hg_group_ctx", "hg_group_sketch_fasta_batch", "hg_group_sketch_fasta_records",
+    "hg_group_dist_packed",
     "hg_group_search_packed", "hg_group_cluster_packed",
     "hg_peer_window_need", "hg_peer_create", "hg_peer_connect", "hg_peer_create_local", "hg_peer_destroy", "hg_peer_rank",
     "hg_peer_world", "hg_peer_barrier", "hg_peer_stage_ms", "hg_peer_timeline", "hg_peer_plan_tiles", "hg_peer_plan_push", "hg_dist_sharded_dev", "hg_dist_sharded_hits", "hg_peer_hit_buffers",
@@ -41,6 +42,9 @@ class SketchParams(C.Structure):
 
 
 HIT_DTYPE = np.dtype([("i", np.uint32), ("j", np.uint32), ("dot", np.int32), ("ani", np.float32)])
+# struct hg_fasta_record
+RECORD_DTYPE = np.dtype([("name_off", np.uint64), ("name_len", np.uint64), ("seq_len", np.uint64), ("file", np.uint32),
+                         ("has_header", np.uint32)])
 
 
 class HyperGenError(RuntimeError):
@@ -90,6 +94,10 @@ def load() -> C.CDLL:
     L.hg_encode_sets_dev.restype = i32; L.hg_encode_sets_dev.argtypes = [vp, vp, vp, u32, u32, vp, vp, vp, vp]
     L.hg_fasta_merge.restype = i32; L.hg_fasta_merge.argtypes = [vp, vp, vp, u32, vp, u64, vp]
     L.hg_sketch_fasta_batch.restype = i32; L.hg_sketch_fasta_batch.argtypes = [vp, vp, vp, u32, pp, vp, vp, vp, vp, vp]
+    L.hg_sketch_fasta_records.restype = i32
+    L.hg_sketch_fasta_records.argtypes = [vp, vp, vp, u32, pp, u32, vp, vp, vp, vp, vp, C.POINTER(u32)]
+    L.hg_fasta_records_stats.restype = i32
+    L.hg_fasta_records_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_float), C.POINTER(C.c_float)]
     L.hg_kmer_hash.restype = i32; L.hg_kmer_hash.argtypes = [vp, vp, vp, u32, pp, vp, u64, vp]
     L.hg_sketch_batch.restype = i32; L.hg_sketch_batch.argtypes = [vp, vp, vp, u32, pp, vp, vp, vp, vp, vp]
     L.hg_sketch_batch_dev.restype = i32; L.hg_sketch_batch_dev.argtypes = [vp, vp, vp, u32, pp, vp, vp, vp, vp, vp]
@@ -136,6 +144,8 @@ def load() -> C.CDLL:
     L.hg_group_size.restype = i32; L.hg_group_size.argtypes = [vp]
     L.hg_group_ctx.restype = vp; L.hg_group_ctx.argtypes = [vp, i32]
     L.hg_group_sketch_fasta_batch.restype = i32; L.hg_group_sketch_fasta_batch.argtypes = [vp, vp, vp, u32, pp, vp, vp, vp, vp, vp]
+    L.hg_group_sketch_fasta_records.restype = i32
+    L.hg_group_sketch_fasta_records.argtypes = [vp, vp, vp, u32, pp, u32, vp, vp, vp, vp, vp, C.POINTER(u32)]
     L.hg_group_dist_packed.restype = i32
     L.hg_group_dist_packed.argtypes = [vp, vp, u64, vp, vp, u32, vp, u64, vp, vp, u32, u32, u32, C.c_float, i32, i32, vp, vp, u64,
                                        C.POINTER(u64)]
@@ -260,6 +270,24 @@ def _cluster_stats(ctx_handle):
     counts, ms = (C.c_uint64 * 4)(), (C.c_float * 4)()
     _check(load().hg_cluster_stats(ctx_handle, counts, ms))
     return [int(x) for x in counts], [float(x) for x in ms]
+
+
+def _sketch_records(fn, h, files, params):
+    """hg_sketch_fasta_records / hg_group_sketch_fasta_records (fn) on the context / group h: raw FASTA file contents in,
+    dict(packed, quant_bits, norm2, n_hashes, records) out, one row per record.  rec_cap is the '>' bytes of all files
+    plus one per file, which no call can exceed."""
+    raw, off = Context._concat_files(files)
+    n = len(files)
+    cap = sum(bytes(f).count(b">") for f in files) + n
+    out = _sketch_out(cap, int(params.hv_d), False)
+    del out["hv"]
+    records = np.empty(cap, RECORD_DTYPE)
+    n_rec = C.c_uint32(0)
+    _check(fn(h, _ptr(raw) if raw.size else None, _ptr(off), n, C.byref(params), cap, _ptr(records), *map(_ptr, out.values()),
+              C.byref(n_rec)))
+    out = {k: v[: n_rec.value] for k, v in out.items()}
+    out["records"] = records[: n_rec.value]
+    return out
 
 
 def pinned_empty(shape, dtype) -> np.ndarray:
@@ -458,6 +486,18 @@ class Context:
         _check(load().hg_sketch_fasta_batch(self._h, _ptr(raw) if raw.size else None, _ptr(off), n, C.byref(params),
                                             *map(_ptr, out.values())))
         return out
+
+    def sketch_fasta_records(self, files, params: SketchParams):
+        """hg_sketch_fasta_records: raw FASTA file contents in, one sketch per record out ->
+        dict(packed, quant_bits, norm2, n_hashes, records) with records a RECORD_DTYPE array."""
+        return _sketch_records(load().hg_sketch_fasta_records, self._h, files, params)
+
+    def fasta_records_stats(self):
+        """hg_fasta_records_stats of the last records call -> ([chunks, records, table slots, 0],
+        [ms of merge, record index, k-mer hash, encode], host gap ms) (ms -1: profiling off)"""
+        counts, ms, gap = (C.c_uint64 * 4)(), (C.c_float * 4)(), C.c_float(0)
+        _check(load().hg_fasta_records_stats(self._h, counts, ms, C.byref(gap)))
+        return [int(x) for x in counts], [float(x) for x in ms], float(gap.value)
 
     def sketch_status(self):
         _check(load().hg_sketch_status(self._h))
@@ -768,6 +808,10 @@ class Group:
         _check(load().hg_group_sketch_fasta_batch(self._h, _ptr(raw) if raw.size else None, _ptr(off), n, C.byref(params),
                                                   *map(_ptr, out.values())))
         return out
+
+    def sketch_fasta_records(self, files, params: SketchParams):
+        """hg_group_sketch_fasta_records: Context.sketch_fasta_records over the GPUs of the group; same bytes."""
+        return _sketch_records(load().hg_group_sketch_fasta_records, self._h, files, params)
 
     def dist_packed(self, ref_packed, ref_bits, ref_norm2, qry_packed, qry_bits, qry_norm2, hv_d, ksize=21, ani_th=85.0,
                     symmetric=False, sorted_output=True, cap=None):

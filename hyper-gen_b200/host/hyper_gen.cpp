@@ -11,7 +11,10 @@
 //   utils::dump_ani_file            src/utils.rs:260-308     stable sort by ANI, reversed, >= threshold
 //
 // CLI (same flags as src/utils.rs:44-126):
-//   hyper-gen sketch -p <dir> -o <out> [-k 21] [-s 1500] [-S 123] [-d 4096] [-C true] [-t 16]
+//   hyper-gen sketch -p <dir> -o <out> [-k 21] [-s 1500] [-S 123] [-d 4096] [-C true] [-t 16] [-i false]
+//       -i true (--individual): one sketch per FASTA record instead of one per file (hg_group_sketch_fasta_records),
+//       named by the record ID (the header text up to the first space or tab), or `<file>#<record index in the file>`
+//       for sequence before a file's first header and for an empty ID.
 //   hyper-gen dist   -r <ref sketch> -q <query sketch> -o <out> [-a 85.0]
 //   hyper-gen search -r <ref sketch> -q <query sketch> -o <out> [-n 10] [-a 0.0]
 //       the -n best refs of every query with ANI >= -a (ties by ascending ref index), one line per result,
@@ -55,6 +58,7 @@ struct SketchParams {  // src/types.rs:83-113
   uint64_t seed = 123, scaled = 1500;
   size_t hv_d = 4096;
   int threads = 16;
+  bool individual = false;  // -i: one sketch per record
 };
 
 struct FileSketch {  // src/types.rs:224-235
@@ -237,10 +241,11 @@ void sketch_cuda(const types::SketchParams &params) {
   p.scaled = params.scaled; p.seed = params.seed; p.hv_d = (uint32_t)params.hv_d;
   p.ksize = params.ksize; p.canonical = params.canonical ? 1 : 0;
   const size_t D = params.hv_d;
-  std::vector<types::FileSketch> all(n_file);
+  std::vector<types::FileSketch> all(params.individual ? 0 : n_file);  // -i: appended record by record
   // By default the raw file bytes go to the GPU, which does read_merge_seq's job itself (hg_sketch_fasta_batch);
   // HG_HOST_PARSE=1 keeps the reference's host-side reader in the loop instead.
   const bool host_parse = getenv("HG_HOST_PARSE") != nullptr;
+  if (host_parse && params.individual) die("-i true needs the raw file bytes on the GPU: the host reader (HG_HOST_PARSE=1) has no record mode");
   const int nt_all = std::max(1, params.threads);
   auto parallel = [&](size_t count, const std::function<void(size_t)> &fn) {  // the reference's rayon par_iter over files
     const int nt = (int)std::min<size_t>((size_t)nt_all, std::max<size_t>(count, 1));
@@ -274,6 +279,12 @@ void sketch_cuda(const types::SketchParams &params) {
   for (int i = 0; i < (batches.size() > 1 ? 2 : 1); i++) check(hg_host_alloc(max_batch + 4096, (void **)&stage[i]), "hg_host_alloc");
   lap(t_alloc);
   std::vector<std::vector<uint64_t>> seg_offs(batches.size());
+  std::vector<uint64_t> n_gt(params.individual ? n_file : 0);  // '>' bytes per file: a file holds at most that + 1 records
+  auto count_gt = [](const uint8_t *p, uint64_t n) {
+    uint64_t c = 0;
+    for (const uint8_t *e = p + n; (p = (const uint8_t *)memchr(p, '>', (size_t)(e - p))) != nullptr; ++p) ++c;
+    return c;
+  };
   auto fill = [&](size_t bi) {  // batch bi into staging buffer bi % 2
     const size_t b0 = batches[bi].first, m = batches[bi].second - b0;
     std::vector<uint64_t> &seg_off = seg_offs[bi];
@@ -283,7 +294,10 @@ void sketch_cuda(const types::SketchParams &params) {
     if (host_parse)
       parallel(m, [&](size_t i) { if (fsize[b0 + i]) memcpy(dst + seg_off[i], parsed[b0 + i].data(), fsize[b0 + i]); });
     else
-      parallel(m, [&](size_t i) { fastx_reader::read_raw_into(files[b0 + i], dst + seg_off[i], fsize[b0 + i]); });
+      parallel(m, [&](size_t i) {
+        fastx_reader::read_raw_into(files[b0 + i], dst + seg_off[i], fsize[b0 + i]);
+        if (params.individual) n_gt[b0 + i] = count_gt(dst + seg_off[i], fsize[b0 + i]);
+      });
   };
   if (!batches.empty()) fill(0);
   lap(t_read);
@@ -292,6 +306,34 @@ void sketch_cuda(const types::SketchParams &params) {
     std::thread next;
     if (bi + 1 < batches.size()) next = std::thread(fill, bi + 1);  // overlaps the GPU call below
     const std::vector<uint64_t> &seg_off = seg_offs[bi];
+    if (params.individual) {
+      uint64_t cap = m;
+      for (size_t i = 0; i < m; i++) cap += n_gt[b0 + i];
+      if (cap > 0xFFFFFFFFull) cap = 0xFFFFFFFFull;  // the library refuses more records than that anyway
+      std::vector<hg_fasta_record> rec(cap);
+      std::vector<uint8_t> packed(cap * 2 * D), bits(cap);
+      std::vector<int32_t> norm2(cap);
+      uint32_t n_rec = 0;
+      check(hg_group_sketch_fasta_records(group, stage[bi & 1], seg_off.data(), (uint32_t)m, &p, (uint32_t)cap, rec.data(), packed.data(),
+                                          bits.data(), norm2.data(), nullptr, &n_rec),
+            "hg_group_sketch_fasta_records");
+      for (uint32_t r = 0, index = 0; r < n_rec; r++) {
+        index = r && rec[r].file == rec[r - 1].file ? index + 1 : 0;
+        types::FileSketch s;
+        s.ksize = params.ksize; s.scaled = params.scaled; s.seed = params.seed; s.canonical = params.canonical;
+        s.hv_d = D; s.hv_quant_bits = bits[r]; s.hv_norm_2 = norm2[r];
+        const char *h = (const char *)stage[bi & 1] + rec[r].name_off;
+        s.file_str = rec[r].has_header ? std::string(h, std::find_if(h, h + rec[r].name_len, [](char ch) { return ch == ' ' || ch == '\t'; }))
+                                       : std::string();
+        if (s.file_str.empty()) s.file_str = files[b0 + rec[r].file] + "#" + std::to_string(index);
+        const size_t nbytes = (size_t)bits[r] * D / 8;
+        s.hv.resize(nbytes / 2);
+        memcpy(s.hv.data(), packed.data() + (size_t)r * 2 * D, nbytes);
+        all.push_back(std::move(s));
+      }
+      if (next.joinable()) next.join();
+      continue;
+    }
     std::vector<uint8_t> packed(m * 2 * D), bits(m);
     std::vector<int32_t> norm2(m);
     std::vector<uint32_t> nh(m);
@@ -573,6 +615,7 @@ int main(int argc, char **argv) {
     }
     else if (k == "-t" || k == "--thread") sp.threads = atoi(v.c_str());
     else if (k == "-C" || k == "--canonical") sp.canonical = (v == "true" || v == "1");
+    else if (k == "-i" || k == "--individual") sp.individual = (v == "true" || v == "1");
     else if (k == "-k" || k == "--ksize") sp.ksize = (uint8_t)atoi(v.c_str());
     else if (k == "-S" || k == "--seed") sp.seed = strtoull(v.c_str(), nullptr, 10);
     else if (k == "-s" || k == "--scaled") sp.scaled = strtoull(v.c_str(), nullptr, 10);

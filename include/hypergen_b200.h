@@ -171,6 +171,36 @@ HG_API int hg_sketch_fasta_batch(hg_ctx *ctx, const uint8_t *raw, const uint64_t
                                  const hg_sketch_params *p, int16_t *hv, uint8_t *packed,
                                  uint8_t *quant_bits, int32_t *norm2, uint32_t *n_hashes);
 
+/* One record of a FASTA file, as hg_sketch_fasta_records reports it.  A file's records, in file
+ * order: every line that starts with '>' opens one; its sequence is the merged bytes (as
+ * hg_fasta_merge merges them) of its sequence lines up to the next header or the end of the file,
+ * without the header's own 'N'.  Merged bytes before a file's first header (or of a file without
+ * one) form one leading record first, with has_header = 0; a file with no such byte has none. */
+typedef struct hg_fasta_record {
+  uint64_t name_off;   /* index into raw (the indexing of file_off) of the first byte after '>'          */
+  uint64_t name_len;   /* header text bytes, without the line's '\n' and one '\r' before it              */
+  uint64_t seq_len;    /* bases of the record's merged sequence: what was hashed                          */
+  uint32_t file;       /* index of the record's file in this call                                         */
+  uint32_t has_header; /* 0 only for the leading record of a file (sequence before its first header)     */
+} hg_fasta_record;     /* 32 bytes */
+
+/* hg_sketch_fasta_batch with one sketch per record instead of one per file.  Record r's row of
+ * packed, quant_bits, norm2 and n_hashes is what hg_sketch_fasta_batch returns for a file holding
+ * that record alone (its header line, if any, and its sequence lines).  Records go out in file
+ * order, then record order; *n_records always receives their count.  A file that contains c '>'
+ * bytes holds at most c + 1 records, so rec_cap = (the '>' bytes of all files) + n_files always
+ * suffices.  More records than rec_cap: HG_E_CAPACITY and nothing else is written; more than
+ * 2^32 - 1: HG_E_UNSUPPORTED.  Any output pointer but n_records may be NULL (not copied). */
+HG_API int hg_sketch_fasta_records(hg_ctx *ctx, const uint8_t *raw, const uint64_t *file_off, uint32_t n_files,
+                                   const hg_sketch_params *p, uint32_t rec_cap, hg_fasta_record *records,
+                                   uint8_t *packed /* rec_cap rows of 2 * hv_d bytes */, uint8_t *quant_bits,
+                                   int32_t *norm2, uint32_t *n_hashes, uint32_t *n_records);
+/* The last hg_sketch_fasta_records call on this context: counts = [chunks, records, record table slots (one
+ * leading slot per file included), 0]; with hg_set_profiling on, ms = device ms of [merge, record index, k-mer
+ * hash, encode] summed over the chunks and host_gap_ms = the device time between the index pass and the hash
+ * stage spent waiting for the host (the two record table round trips and the planning); -1 otherwise. */
+HG_API int hg_fasta_records_stats(hg_ctx *ctx, uint64_t counts[4], float ms[4], float *host_gap_ms);
+
 /* ---- sketch format ---------------------------------------------------------------- */
 
 /* decompress_hd_sketch (src/hd.rs:184-212) for n sketches on the GPU: packed rows of
@@ -270,6 +300,12 @@ HG_API hg_ctx *hg_group_ctx(hg_group *g, int i);
 HG_API int hg_group_sketch_fasta_batch(hg_group *g, const uint8_t *raw, const uint64_t *file_off, uint32_t n_files,
                                        const hg_sketch_params *p, int16_t *hv, uint8_t *packed, uint8_t *quant_bits,
                                        int32_t *norm2, uint32_t *n_hashes);
+/* hg_sketch_fasta_records with the files split as hg_group_sketch_fasta_batch splits them; every GPU keeps its
+ * rows until the group has checked the total against rec_cap.  Same arguments, outputs and bytes as one GPU. */
+HG_API int hg_group_sketch_fasta_records(hg_group *g, const uint8_t *raw, const uint64_t *file_off, uint32_t n_files,
+                                         const hg_sketch_params *p, uint32_t rec_cap, hg_fasta_record *records,
+                                         uint8_t *packed, uint8_t *quant_bits, int32_t *norm2, uint32_t *n_hashes,
+                                         uint32_t *n_records);
 /* hg_dist_packed with the rows of both sketch files split into one block per GPU: each block crosses its
  * own GPU's PCIe link, is unpacked and brought into operand form there, the query operands are pushed to
  * every GPU, the output tiles are shared out, the hits land on GPU 0 (sorted there if asked).  Results are

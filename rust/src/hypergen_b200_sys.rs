@@ -14,6 +14,11 @@ pub struct hg_sketch_params { pub scaled: u64, pub seed: u64, pub hv_d: u32, pub
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct hg_hit { pub i: u32, pub j: u32, pub dot: i32, pub ani: f32 }
 
+/// one FASTA record of hg_sketch_fasta_records: header text span in raw, merged sequence length, file, 0 for the
+/// sequence before a file's first header
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct hg_fasta_record { pub name_off: u64, pub name_len: u64, pub seq_len: u64, pub file: u32, pub has_header: u32 }
+
 pub const HG_OK: c_int = 0;
 pub const HG_E_CAPACITY: c_int = -3;
 
@@ -28,6 +33,13 @@ extern "C" {
     pub fn hg_group_sketch_fasta_batch(g: *mut hg_group, raw: *const u8, file_off: *const u64, n_files: u32,
         p: *const hg_sketch_params, hv: *mut i16, packed: *mut u8, quant_bits: *mut u8, norm2: *mut i32,
         n_hashes: *mut u32) -> c_int;
+    // one sketch per FASTA record (`sketch -i`); rec_cap = the '>' bytes of all files + n_files always suffices
+    pub fn hg_sketch_fasta_records(ctx: *mut hg_ctx, raw: *const u8, file_off: *const u64, n_files: u32,
+        p: *const hg_sketch_params, rec_cap: u32, records: *mut hg_fasta_record, packed: *mut u8, quant_bits: *mut u8,
+        norm2: *mut i32, n_hashes: *mut u32, n_records: *mut u32) -> c_int;
+    pub fn hg_group_sketch_fasta_records(g: *mut hg_group, raw: *const u8, file_off: *const u64, n_files: u32,
+        p: *const hg_sketch_params, rec_cap: u32, records: *mut hg_fasta_record, packed: *mut u8, quant_bits: *mut u8,
+        norm2: *mut i32, n_hashes: *mut u32, n_records: *mut u32) -> c_int;
     pub fn hg_group_dist_packed(g: *mut hg_group, ref_packed: *const u8, ref_stride: u64, ref_quant_bits: *const u8,
         ref_norm2: *const i32, n_ref: u32, qry_packed: *const u8, qry_stride: u64, qry_quant_bits: *const u8,
         qry_norm2: *const i32, n_qry: u32, hv_d: u32, ksize: u32, ani_th: f32, symmetric: c_int, sorted: c_int,
